@@ -142,7 +142,10 @@ def run_reference(args):
     binding.build()
     threads = os.cpu_count() or 1
     log_n = pick_cpu_sample(binding, threads, args.steps + args.warmup, 150.0)
-    rate, mean = cpu_commit_rate(binding, log_n, threads, args.steps, args.warmup)
+    kept = {}
+    rate, mean = cpu_commit_rate(binding, log_n, threads, args.steps, args.warmup, keep=kept)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(kept["roots"], kept["last"], kept["transcript"])])
     sample = "reed_solomon + FriProverData::fold of one 2^%d-coefficient polynomial per step (workload is 2^%d)" % (log_n, args.log_n)
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -369,6 +372,22 @@ def pin_to_gpu_numa_node(local_rank):
         return {"pinned": False, "error": str(e)[:120]}
 
 
+def dump_outputs(out_dir, results):
+    """writes what the last timed step returned for each of the P polynomials (FriProverData's layer roots, last element, final
+    transcript state) as <out_dir>/<name>.npy.  All three are byte strings: every byte is stored as one float32 value, so any
+    changed bit stays a difference of at least 1 under a tolerance comparison."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"fri_layer_roots": [b"".join(roots) for roots, _, _ in results],  # (P, log_n, 32)
+              "last_element": [last.to_bytes(16, "little") for _, last, _ in results],  # (P, 16), little-endian field element
+              "transcript_state": [tr for _, _, tr in results]}  # (P, 32)
+    for name, rows in arrays.items():
+        a = np.array([np.frombuffer(r, dtype=np.uint8) for r in rows], dtype=np.float32)
+        if name == "fri_layer_roots":
+            a = a.reshape(len(rows), -1, 32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     from multilinear_b200 import api as ml
@@ -445,6 +464,8 @@ def run_ours(args):
     ms = e0.elapsed_time(e1) / args.steps
     launches = ml.kernel_launches() - launches0
     roots, last, tr0 = results[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, results)  # before the serial pass below overwrites results[0]
 
     # ---- serial pass of the same workload (one commit at a time) with per-kernel CUDA-event timing: per-kernel
     # durations are only well defined when commits do not share the GPU
@@ -765,7 +786,11 @@ def main():
     ap.add_argument("--e2e-polys", type=int, default=0, dest="e2e_polys",
                     help="concurrent commits in the end-to-end leg (more in flight hides the PCIe copies); default 12 on one GPU "
                          "(measured 1708 / 1727 / 1775 Melem/s at 6 / 8 / 12), 8 per rank under torchrun")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's polynomials) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

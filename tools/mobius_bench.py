@@ -1,5 +1,5 @@
 import ctypes as C, sys, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
 import torch
 from multilinear_b200 import api as ml
 from multilinear_b200 import load

@@ -1,5 +1,5 @@
-import ctypes as C, sys
-sys.path.insert(0, "/root/repo")
+import ctypes as C, os, sys
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
 L = load(); ml.set_device(0)
