@@ -322,6 +322,31 @@ int ml_shard_batched_pcs_prove_dev(ml_shard *sh, const uint8_t *inputs, size_t n
 int ml_shard_batched_pcs_prove(ml_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
                                const uint8_t *const *evals, ml_transcript *t, ml_bpcs_proof **out);
 
+/* ---- PCSProof::prove of ONE polynomial sharded over the GPUs of one box (multilinear_pcs.rs:90-136) ----
+ * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; rank b holds the contiguous block evals[b*n/G, (b+1)*n/G).  The blocks
+ * are encoded locally and combined into the global code by a column exchange (rank r owns code columns [r*N/G^2, (r+1)*N/G^2),
+ * N = 2n); the first log2(G) fold rounds run sharded (Merkle subtrees, sumcheck tables and FRI folds stay on their owners; the
+ * round polynomial and challenge are computed identically on every rank), then rank 0 runs the rest of the fold chain from N/G
+ * elements and the openings, reading the sharded layers from the owners' arenas (csrc/pcs_shard.cu).  Rank r therefore holds
+ * about 1/G of the encoded layers, trees and tables; rank 0 additionally the tail from N/G elements.
+ * The proof is byte-identical to ml_pcs_prove's and an ordinary ml_pcs_proof (ml_pcs_verify, the serializer work unchanged).
+ * Handles, records, calls and errors as for ml_shard_* above (the same 72-byte IPC records, MLB_SHARD_TIMEOUT_S bounds every
+ * wait).  Minimum size: n_vars >= max(1, 2*log2 G): G = 1: 1, 2: 2, 4: 4, 8: 6, 16: 8 (ML_ERR_SIZE below). */
+typedef struct ml_pcs_shard ml_pcs_shard;
+int ml_pcs_shard_create(int world, int n_local, const int *local_ranks, const int *local_devices, size_t n_vars, ml_pcs_shard **out);
+void ml_pcs_shard_free(ml_pcs_shard *sh);   /* multi-process: all ranks must have returned from their last call (caller's barrier) */
+int ml_pcs_shard_export(ml_pcs_shard *sh, uint8_t *records_out /* num_local * ml_shard_record_bytes() */);
+int ml_pcs_shard_connect(ml_pcs_shard *sh, const uint8_t *records, size_t n_records /* world */);
+void *ml_pcs_shard_stream(const ml_pcs_shard *sh, int local_index);  /* the local rank's main stream (for CUDA-event timing) */
+size_t ml_pcs_shard_arena_bytes(const ml_pcs_shard *sh);
+/* local_evals_dev[i]: local rank i's block evals[rank*n/G, (rank+1)*n/G) (device pointer, complete before the call).  Every process
+ * passes the same claim and its own transcript copy; all copies end in rank 0's final state. */
+int ml_pcs_shard_prove_dev(ml_pcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t output[16],
+                           const void *const *local_evals_dev, ml_transcript *t, ml_pcs_proof **out /* NULL unless rank 0 is local */);
+/* host evals (all n) and a handle that hosts every rank: the drop-in for multilinear_pcs.rs:90 */
+int ml_pcs_shard_prove(ml_pcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t output[16],
+                       const uint8_t *evals, size_t n, ml_transcript *t, ml_pcs_proof **out);
+
 /* ---- batched commit building blocks (round-1 API, kept): one rank's share of `Merkle::batch_commit`
  * (merkle_tree/mod.rs:110-131) over leaf range [leaf_begin, leaf_begin+leaf_count) of all codes.
  * codes_dev[j] points at code j's rows for this range laid out as pairs: leaf_count x 32 bytes.

@@ -315,8 +315,29 @@ class PCSProof {
     }
 
   private:
+    friend class ShardedPCSProver;
     PCSProof() = default;
     ml_pcs_proof* h_ = nullptr;
+};
+// PCSProof::prove of one polynomial over several GPUs from one process (ml_pcs_shard_*, csrc/pcs_shard.cu); `devices` may repeat
+// (virtual ranks).  The proof bytes equal PCSProof::prove's.
+class ShardedPCSProver {
+  public:
+    ShardedPCSProver(const std::vector<int>& devices, size_t n_vars) {
+        std::vector<int> ranks(devices.size());
+        for (size_t i = 0; i < ranks.size(); i++) ranks[i] = (int)i;
+        check(ml_pcs_shard_create((int)devices.size(), (int)devices.size(), ranks.data(), devices.data(), n_vars, &h_));
+    }
+    ShardedPCSProver(const ShardedPCSProver&) = delete;
+    ~ShardedPCSProver() { if (h_) ml_pcs_shard_free(h_); }
+    PCSProof prove(const std::vector<F>& inputs, F output, const MultilinearPolynomialEvals& poly, Transcript& t) {
+        PCSProof p;
+        check(ml_pcs_shard_prove(h_, raw(inputs), inputs.size(), output.bytes(), raw(poly.evals), poly.evals.size(), t.handle(), &p.h_));
+        return p;
+    }
+
+  private:
+    ml_pcs_shard* h_ = nullptr;
 };
 
 // src/fri/batched_pcs.rs:22-254

@@ -33,6 +33,10 @@ int ml_microbench(const char *what, size_t n, int iters, double *ms_out, double 
  * S4 wait for the matrix, chain incl. S5 first fold, openings + proof (the last three on rank 0 only).  Returns how many. */
 struct ml_shard;
 int ml_shard_phase_ms(const struct ml_shard *sh, double *out, int cap);
+/* sharded single PCS prover (ml_pcs_shard_*): the same for [S0 encode + exchange + tables, S1 combine, sharded rounds, tail fold
+ * chain (rank 0), openings + proof (rank 0)] */
+struct ml_pcs_shard;
+int ml_pcs_shard_phase_ms(const struct ml_pcs_shard *sh, double *out, int cap);
 
 #ifdef __cplusplus
 }

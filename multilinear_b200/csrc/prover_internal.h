@@ -35,6 +35,8 @@ void free_sumcheck(ml_sumcheck* s);
 int encode_into(Ctx* ctx, const fe* evals_dev, size_t n, fe* code, cudaStream_t s);
 void derive_indices(ml_transcript* t, size_t domain_size, std::vector<size_t>& idx);
 void fill_dirs(PathH& p, size_t index, int depth);
+// appends layer `code` (n elements) to f with its Merkle tree (build_tree) but without reading the root back
+int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree);
 int fri_open_queries(const ml_fri* f, const std::vector<size_t>& indices, std::vector<QueryH>& out, cudaStream_t s);
 hfe fingerprint_host(hfe r, const hfe* c, size_t n);
 

@@ -4,7 +4,7 @@
 // (the batched Merkle leaf i hashes the ReedSolomonPairs of ALL codes at i, merkle_tree/mod.rs:110-116).  Every rank owns
 //   * the polynomials j with j mod G == rank               (encode)
 //   * leaf rows [rank*rows, (rank+1)*rows), rows = n/G     (hash, fingerprint, first fold, openings)
-// and one peer-visible ARENA in HBM (cudaMalloc, mapped into the other ranks through CUDA IPC or plain peer access):
+// and one peer-visible ARENA in HBM (peer.h: cudaMalloc, mapped into the other ranks through CUDA IPC or plain peer access):
 //   mailbox (flags, subtree roots, challenge, final transcript) | pairs[B][rows][32] | digests of the row subtree |
 //   stage[G][n/G] (fingerprint partial sums) | matrix[n] | next[n]   (the last two are used on rank 0)
 // All data-path exchange is a kernel STORING into a peer's arena over NVLink, followed by a flag store (release, system scope);
@@ -33,6 +33,7 @@
 #include <cstdlib>
 #include <map>
 
+#include "peer.h"
 #include "prover_internal.h"
 #include "sha256.cuh"
 
@@ -48,13 +49,13 @@ using namespace mlbp;
 namespace {
 
 enum Phase { P1 = 0, P2, P3, P4, P5, P6, P7, N_PHASES };
-static const int MAXR = ML_MAX_PEERS;
+static const int MAXR = PEER_MAXR;
 
 // ---- arena layout (byte offsets; every section 256-byte aligned)
 struct Layout {
     size_t flags, roots, r0, final_tr, status, top, fr, prev, tr, tr_in, root_out, outputs, pairs, digests, stage, matrix, next, total;
 };
-static size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
+static size_t align_up(size_t x) { return peer_align(x); }
 static Layout make_layout(size_t B, size_t n, size_t G) {
     Layout L;
     size_t o = 0;
@@ -79,59 +80,6 @@ static Layout make_layout(size_t B, size_t n, size_t G) {
     L.next = take(n * 16);
     L.total = o;
     return L;
-}
-
-struct PeerPtrs {
-    uint8_t* base[MAXR];
-};
-
-// ------------------------------------------------------------------ flags
-__device__ __forceinline__ void flag_store_release(unsigned long long* p, unsigned long long v) {
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long flag_load_acquire(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-// thread g sets flag[phase][rank] = epoch in rank g's arena (only: a single target, or -1 for all ranks)
-__global__ void shard_signal_kernel(PeerPtrs peers, size_t off_flags, int world, int phase, int rank, unsigned long long epoch, int only) {
-    const int g = threadIdx.x;
-    if (g >= world || (only >= 0 && g != only)) return;
-    __threadfence_system();  // everything this rank's earlier kernels stored (stream order) is visible before the flag
-    flag_store_release(reinterpret_cast<unsigned long long*>(peers.base[g] + off_flags) + phase * MAXR + rank, epoch);
-}
-// thread g waits until flag[phase][g] >= epoch in the LOCAL arena (only_from: a single source, or -1 for all)
-__device__ __forceinline__ void wait_flags(const unsigned long long* flags, int world, int only_from, unsigned long long epoch,
-                                           unsigned long long timeout_ns, int* status) {
-    const int g = threadIdx.x;
-    if (g < world && (only_from < 0 || g == only_from)) {
-        const unsigned long long t0 = global_ns();
-        while (flag_load_acquire(flags + g) < epoch) {
-            if (global_ns() - t0 > timeout_ns) { atomicExch(status, ML_ERR_PEER); break; }
-            __nanosleep(200);
-        }
-    }
-}
-__global__ void shard_wait_kernel(const unsigned long long* flags, int world, int only_from, unsigned long long epoch,
-                                  unsigned long long timeout_ns, int* status) {
-    wait_flags(flags, world, only_from, epoch, timeout_ns, status);
-}
-// copy nbytes (multiple of 16, <= 128) from src to dst_off in the arenas of all ranks (or one), then raise the flag there
-__global__ void shard_push_kernel(const uint8_t* __restrict__ src, int nbytes, PeerPtrs peers, size_t dst_off, size_t off_flags, int world,
-                                  int phase, int rank, unsigned long long epoch, int only) {
-    const int g = threadIdx.x;
-    if (g >= world || (only >= 0 && g != only)) return;
-    const uint4* s4 = reinterpret_cast<const uint4*>(src);
-    uint4* d4 = reinterpret_cast<uint4*>(peers.base[g] + dst_off);
-    for (int i = 0; i < nbytes / 16; i++) d4[i] = s4[i];
-    __threadfence_system();
-    flag_store_release(reinterpret_cast<unsigned long long*>(peers.base[g] + off_flags) + phase * MAXR + rank, epoch);
 }
 
 // ------------------------------------------------------------------ S0: pack pass with the exchange fused in
@@ -309,14 +257,7 @@ __global__ void __launch_bounds__(64) shard_gather_kernel(const unsigned long lo
 }
 
 // ------------------------------------------------------------------ host side
-struct DevStreams {
-    cudaStream_t main = nullptr, enc2 = nullptr, side = nullptr;
-};
-struct ShardRank {
-    int rank = 0, device = 0;
-    Ctx* ctx = nullptr;
-    DevStreams st;
-    uint8_t* arena = nullptr;
+struct ShardRank : PeerRank {
     fe* code[2] = {nullptr, nullptr};
     cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr}, ev_fork = nullptr, ev_enc2 = nullptr, ev_side = nullptr;
     const fe** evals_ptrs_dev = nullptr;  // n_local_polys device pointers
@@ -330,60 +271,25 @@ struct ml_shard {
     size_t B = 0, n_vars = 0, n = 0, rows = 0, slice = 0, polys_per_rank = 0;
     Layout lay;
     std::vector<ShardRank> local;
-    std::map<int, DevStreams> streams;  // per device
-    uint8_t* peer_base[MAXR];
-    bool peer_mapped[MAXR];             // opened through IPC (must be closed)
-    bool connected = false;
-    unsigned long long epoch = 0;
+    PeerGroup grp;  // arenas of all ranks, flags, epoch, timeout (peer.h)
     // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
     static const int N_MARKS = 10;
     cudaEvent_t mark[N_MARKS] = {nullptr};
     int n_marks = 0;
-    unsigned long long timeout_ns = 20ull * 1000 * 1000 * 1000;
     unsigned pack_ctas = 32;
-    ml_shard() {
-        for (int g = 0; g < MAXR; g++) { peer_base[g] = nullptr; peer_mapped[g] = false; }
-    }
 };
 
 namespace {
 
-struct DeviceGuard {
-    int prev = 0;
-    DeviceGuard() { cudaGetDevice(&prev); }
-    ~DeviceGuard() { cudaSetDevice(prev); }
-};
-PeerPtrs peers_of(const ml_shard* sh) {
-    PeerPtrs p;
-    for (int g = 0; g < MAXR; g++) p.base[g] = sh->peer_base[g];
-    return p;
-}
-unsigned long long* flags_at(const ml_shard* sh, const ShardRank& r, int phase) {
-    return reinterpret_cast<unsigned long long*>(r.arena + sh->lay.flags) + phase * MAXR;
-}
-int* status_at(const ml_shard* sh, const ShardRank& r) { return reinterpret_cast<int*>(r.arena + sh->lay.status); }
-
-int signal(const ml_shard* sh, const ShardRank& r, int phase, int only, cudaStream_t s) {
-    shard_signal_kernel<<<1, 32, 0, s>>>(peers_of(sh), sh->lay.flags, sh->world, phase, r.rank, sh->epoch, only);
-    MLB_KERNEL_CHECK();
-    return ML_OK;
-}
-int wait(const ml_shard* sh, const ShardRank& r, int phase, int only_from, cudaStream_t s) {
-    shard_wait_kernel<<<1, 32, 0, s>>>(flags_at(sh, r, phase), sh->world, only_from, sh->epoch, sh->timeout_ns, status_at(sh, r));
-    MLB_KERNEL_CHECK();
-    return ML_OK;
-}
+PeerPtrs peers_of(const ml_shard* sh) { return sh->grp.peers(); }
+unsigned long long* flags_at(const ml_shard* sh, const ShardRank& r, int phase) { return sh->grp.flags(r, phase); }
+int* status_at(const ml_shard* sh, const ShardRank& r) { return sh->grp.status(r); }
+int signal(const ml_shard* sh, const ShardRank& r, int phase, int only, cudaStream_t s) { return peer_signal(sh->grp, r, phase, only, s); }
+int wait(const ml_shard* sh, const ShardRank& r, int phase, int only_from, cudaStream_t s) { return peer_wait(sh->grp, r, phase, only_from, s); }
 int push(const ml_shard* sh, const ShardRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s) {
-    shard_push_kernel<<<1, 32, 0, s>>>((const uint8_t*)src_dev, nbytes, peers_of(sh), dst_off, sh->lay.flags, sh->world, phase, r.rank, sh->epoch, only);
-    MLB_KERNEL_CHECK();
-    return ML_OK;
+    return peer_push(sh->grp, r, src_dev, nbytes, dst_off, phase, only, s);
 }
-unsigned grid_for(size_t n, size_t cap = 148 * 8) {
-    size_t b = (n + 255) / 256;
-    if (b > cap) b = cap;
-    if (b == 0) b = 1;
-    return (unsigned)b;
-}
+unsigned grid_for(size_t n) { return peer_grid(n); }
 
 void free_rank(ShardRank& r) {
     cudaSetDevice(r.device);
@@ -398,7 +304,7 @@ void free_rank(ShardRank& r) {
     if (r.ev_side) cudaEventDestroy(r.ev_side);
     if (r.evals_ptrs_dev) cudaFree((void*)r.evals_ptrs_dev);
     if (r.pinned) cudaFreeHost(r.pinned);
-    if (r.arena) cudaFree(r.arena);
+    peer_rank_free(r);
 }
 
 // ---- S0: encode + pack of one local rank (enqueue only)
@@ -443,7 +349,7 @@ int stage_subtree(ml_shard* sh, ShardRank& r) {
 int stage_root(ml_shard* sh, ShardRank& r, bool with_transcript) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
-    shard_root_kernel<<<1, 32, 0, s>>>(flags_at(sh, r, P2), sh->world, sh->epoch, sh->timeout_ns, status_at(sh, r), r.arena + sh->lay.roots,
+    shard_root_kernel<<<1, 32, 0, s>>>(flags_at(sh, r, P2), sh->world, sh->grp.epoch, sh->grp.timeout_ns, status_at(sh, r), r.arena + sh->lay.roots,
                                        r.arena + sh->lay.top, (const DevTranscript*)(r.arena + sh->lay.tr_in), (DevTranscript*)(r.arena + sh->lay.tr),
                                        (const fe*)(r.arena + sh->lay.outputs), (int)sh->B, (fe*)(r.arena + sh->lay.fr), (fe*)(r.arena + sh->lay.prev),
                                        r.arena + sh->lay.root_out, with_transcript ? 1 : 0);
@@ -464,7 +370,7 @@ int stage_fp_reduce(ml_shard* sh, ShardRank& r) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     MLB_TRY(wait(sh, r, P3, -1, s));
-    fe* out = reinterpret_cast<fe*>(sh->peer_base[0] + sh->lay.matrix) + (size_t)r.rank * sh->slice;
+    fe* out = reinterpret_cast<fe*>(sh->grp.base[0] + sh->lay.matrix) + (size_t)r.rank * sh->slice;
     shard_fp_reduce_kernel<<<grid_for(sh->slice), 256, 0, s>>>((const fe*)(r.arena + sh->lay.stage), sh->world, sh->slice, out);
     MLB_KERNEL_CHECK();
     return signal(sh, r, P4, 0, s);
@@ -477,7 +383,7 @@ int stage_first_fold(ml_shard* sh, ShardRank& r) {
     const RootTables* rt;
     MLB_TRY(get_root_tables(r.ctx, log_n0, s, &rt));  // exists since the encode; never a lazy build behind a spinning wait
     MLB_TRY(wait(sh, r, P5, 0, s));
-    fe* out = reinterpret_cast<fe*>(sh->peer_base[0] + sh->lay.next) + (size_t)r.rank * sh->rows;
+    fe* out = reinterpret_cast<fe*>(sh->grp.base[0] + sh->lay.next) + (size_t)r.rank * sh->rows;
     shard_first_fold_kernel<<<grid_for(sh->rows), 256, 0, s>>>(r.arena + sh->lay.pairs, (int)sh->B, sh->rows, (size_t)r.rank * sh->rows,
                                                               (const fe*)(r.arena + sh->lay.fr), (const fe*)(r.arena + sh->lay.r0), log_n0, rt->lo,
                                                               rt->hi, out);
@@ -500,10 +406,7 @@ ShardRank* rank0_of(ml_shard* sh) {
     return nullptr;
 }
 
-int check_ready(ml_shard* sh) {
-    if (!sh->connected) { set_error("ml_shard: arenas of the other ranks are not connected (ml_shard_connect)"); return ML_ERR_ARG; }
-    return ML_OK;
-}
+int check_ready(ml_shard* sh) { return peer_check_ready(sh->grp, "ml_shard"); }
 // upload the per-call small inputs of a rank through its pinned staging block (asynchronous, stream ordered)
 int upload_inputs(ml_shard* sh, ShardRank& r, const HostSha256* tr, const uint8_t* outputs, const void* const* evals) {
     MLB_CUDA(cudaSetDevice(r.device));
@@ -524,13 +427,7 @@ int upload_inputs(ml_shard* sh, ShardRank& r, const HostSha256* tr, const uint8_
     MLB_CUDA(cudaMemsetAsync(status_at(sh, r), 0, 16, s));
     return ML_OK;
 }
-int read_status(ml_shard* sh, ShardRank& r) {
-    int st = 0;
-    MLB_CUDA(cudaSetDevice(r.device));
-    MLB_TRY(d2h_sync(&st, status_at(sh, r), sizeof st, r.st.main));
-    if (st != 0) { set_error("ml_shard: rank %d timed out waiting for a peer rank (%.0f s)", r.rank, sh->timeout_ns * 1e-9); return ML_ERR_PEER; }
-    return ML_OK;
-}
+int read_status(ml_shard* sh, ShardRank& r) { return peer_read_status(sh->grp, r, "ml_shard"); }
 
 // batch layer openings + the rest of the proof on rank 0 (batched_fri.rs:207-225, 296-308)
 int shard_assemble(ml_shard* sh, ShardRank& r0, ml_fri* fri, ml_transcript* t, ml_bfri_proof* p, const uint8_t batch_root[32]) {
@@ -578,8 +475,7 @@ int shard_assemble(ml_shard* sh, ShardRank& r0, ml_fri* fri, ml_transcript* t, m
 extern "C" {
 
 int ml_shard_create(int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_polys, size_t n_vars, ml_shard** out) {
-    if (world < 1 || world > MAXR || (world & (world - 1)) || n_local < 1 || n_local > world) { set_error("ml_shard_create: world must be a power of two <= %d", MAXR); return ML_ERR_ARG; }
-    if (n_local != 1 && n_local != world) { set_error("ml_shard_create: a process hosts either one rank or all of them"); return ML_ERR_ARG; }
+    MLB_TRY(peer_check_world("ml_shard_create", world, n_local));
     if (n_vars < 1 || n_vars >= 40) { set_error("ml_shard_create: n_vars out of range"); return ML_ERR_SIZE; }
     const size_t n = (size_t)1 << n_vars;
     if (n_polys == 0 || n_polys % (size_t)world || n % (size_t)world || n / (size_t)world < 2) {
@@ -591,26 +487,20 @@ int ml_shard_create(int world, int n_local, const int* local_ranks, const int* l
     sh->world = world; sh->B = n_polys; sh->n_vars = n_vars; sh->n = n;
     sh->rows = n / world; sh->slice = n / world; sh->polys_per_rank = n_polys / world;
     sh->lay = make_layout(n_polys, n, world);
-    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->timeout_ns = (unsigned long long)(atof(e) * 1e9);
+    sh->grp.world = world;
+    sh->grp.arena_bytes = sh->lay.total;
+    sh->grp.off_flags = sh->lay.flags;
+    sh->grp.off_status = sh->lay.status;
+    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
     if (const char* e = getenv("MLB_SHARD_PACK_CTAS")) sh->pack_ctas = (unsigned)atoi(e);
     int st = ML_OK;
     for (int i = 0; i < n_local && st == ML_OK; i++) {
         ShardRank r;
         r.rank = local_ranks[i];
         r.device = local_devices[i];
-        if (r.rank < 0 || r.rank >= world) { set_error("ml_shard_create: rank out of range"); st = ML_ERR_ARG; break; }
-        if (cudaSetDevice(r.device) != cudaSuccess) { cudaGetLastError(); set_error("ml_shard_create: no CUDA device %d", r.device); st = ML_ERR_CUDA; break; }
-        st = get_ctx(&r.ctx);
-        if (st != ML_OK) break;
-        auto it = sh->streams.find(r.device);
-        if (it == sh->streams.end()) {
-            DevStreams ds;
-            if (lib_stream_create(&ds.main, true) != ML_OK || lib_stream_create(&ds.enc2, true) != ML_OK || lib_stream_create(&ds.side, true) != ML_OK) { st = ML_ERR_CUDA; break; }
-            it = sh->streams.emplace(r.device, ds).first;
-        }
-        r.st = it->second;
-        bool ok = cudaMalloc((void**)&r.arena, sh->lay.total) == cudaSuccess && cudaMemset(r.arena, 0, sh->lay.pairs) == cudaSuccess &&
-                  cudaMalloc((void**)&r.code[0], 2 * n * 16) == cudaSuccess && cudaMalloc((void**)&r.code[1], 2 * n * 16) == cudaSuccess &&
+        st = peer_rank_init(sh->grp, r, "ml_shard_create", sh->lay.pairs);
+        if (st != ML_OK && st != ML_ERR_ALLOC) break;
+        bool ok = st == ML_OK && cudaMalloc((void**)&r.code[0], 2 * n * 16) == cudaSuccess && cudaMalloc((void**)&r.code[1], 2 * n * 16) == cudaSuccess &&
                   cudaMalloc((void**)&r.evals_ptrs_dev, sh->polys_per_rank * sizeof(void*)) == cudaSuccess &&
                   cudaMallocHost((void**)&r.pinned, 128 + align_up(n_polys * 16) + sh->polys_per_rank * sizeof(void*)) == cudaSuccess;
         for (int b = 0; b < 2 && ok; b++)
@@ -621,19 +511,9 @@ int ml_shard_create(int world, int n_local, const int* local_ranks, const int* l
         if (!ok) { cudaGetLastError(); set_error("ml_shard_create: allocation of %zu bytes on device %d failed", sh->lay.total, r.device); st = ML_ERR_ALLOC; }
     }
     if (st == ML_OK && n_local == world) {
-        // all ranks in this process: plain pointers; distinct devices need peer access in both directions
-        for (auto& r : sh->local) sh->peer_base[r.rank] = r.arena;
-        for (auto& a : sh->local)
-            for (auto& b : sh->local) {
-                if (a.device == b.device) continue;
-                cudaSetDevice(a.device);
-                cudaError_t e = cudaDeviceEnablePeerAccess(b.device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) { set_error("no peer access from device %d to %d: %s", a.device, b.device, cudaGetErrorString(e)); st = ML_ERR_PEER; }
-                cudaGetLastError();
-            }
-        for (int g = 0; g < world; g++)
-            if (!sh->peer_base[g]) { set_error("ml_shard_create: rank %d is missing from local_ranks", g); st = ML_ERR_ARG; }
-        sh->connected = st == ML_OK;
+        std::vector<PeerRank*> ranks;
+        for (auto& r : sh->local) ranks.push_back(&r);
+        st = peer_link_local(sh->grp, ranks, "ml_shard_create");
     }
     if (st != ML_OK) { ml_shard_free(sh); return st; }
     *out = sh;
@@ -659,58 +539,21 @@ void ml_shard_free(ml_shard* sh) {
     for (int i = 0; i < ml_shard::N_MARKS; i++)
         if (sh->mark[i]) cudaEventDestroy(sh->mark[i]);
     for (auto& r : sh->local) free_rank(r);
-    if (!sh->local.empty()) cudaSetDevice(sh->local[0].device);
-    for (int g = 0; g < MAXR; g++)
-        if (sh->peer_mapped[g]) cudaIpcCloseMemHandle(sh->peer_base[g]);
-    for (auto& kv : sh->streams) {
-        cudaSetDevice(kv.first);
-        lib_stream_destroy(kv.second.main);
-        lib_stream_destroy(kv.second.enc2);
-        lib_stream_destroy(kv.second.side);
-    }
+    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
     delete sh;
 }
 
 /* one record per local rank: int32 rank | int32 reserved | 64-byte CUDA IPC handle of the arena */
-size_t ml_shard_record_bytes(void) { return 72; }
+size_t ml_shard_record_bytes(void) { return PEER_RECORD_BYTES; }
 int ml_shard_num_local(const ml_shard* sh) { return (int)sh->local.size(); }
 int ml_shard_export(ml_shard* sh, uint8_t* records_out) {
-    DeviceGuard guard;
-    for (size_t i = 0; i < sh->local.size(); i++) {
-        ShardRank& r = sh->local[i];
-        MLB_CUDA(cudaSetDevice(r.device));
-        int32_t hdr[2] = {r.rank, 0};
-        cudaIpcMemHandle_t h;
-        MLB_CUDA(cudaIpcGetMemHandle(&h, r.arena));
-        memcpy(records_out + 72 * i, hdr, 8);
-        memcpy(records_out + 72 * i + 8, &h, 64);
-    }
-    return ML_OK;
+    std::vector<PeerRank*> ranks;
+    for (auto& r : sh->local) ranks.push_back(&r);
+    return peer_export(ranks, records_out);
 }
 int ml_shard_connect(ml_shard* sh, const uint8_t* records, size_t n_records) {
-    DeviceGuard guard;
     if (sh->local.size() != 1) { set_error("ml_shard_connect: only for handles that host one rank"); return ML_ERR_ARG; }
-    ShardRank& me = sh->local[0];
-    MLB_CUDA(cudaSetDevice(me.device));
-    for (size_t i = 0; i < n_records; i++) {
-        int32_t hdr[2];
-        memcpy(hdr, records + 72 * i, 8);
-        const int g = hdr[0];
-        if (g < 0 || g >= sh->world) { set_error("ml_shard_connect: record with rank %d", g); return ML_ERR_ARG; }
-        if (g == me.rank) { sh->peer_base[g] = me.arena; continue; }
-        if (sh->peer_base[g]) continue;
-        cudaIpcMemHandle_t h;
-        memcpy(&h, records + 72 * i + 8, 64);
-        void* p = nullptr;
-        cudaError_t e = cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess);
-        if (e != cudaSuccess) { cudaGetLastError(); set_error("ml_shard_connect: cannot map the arena of rank %d: %s", g, cudaGetErrorString(e)); return ML_ERR_PEER; }
-        sh->peer_base[g] = (uint8_t*)p;
-        sh->peer_mapped[g] = true;
-    }
-    for (int g = 0; g < sh->world; g++)
-        if (!sh->peer_base[g]) { set_error("ml_shard_connect: no record for rank %d", g); return ML_ERR_ARG; }
-    sh->connected = true;
-    return ML_OK;
+    return peer_connect(sh->grp, sh->local[0], records, n_records, "ml_shard_connect");
 }
 void* ml_shard_stream(const ml_shard* sh, int local_index) {
     if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
@@ -723,7 +566,7 @@ size_t ml_shard_arena_bytes(const ml_shard* sh) { return sh->lay.total; }
 int ml_shard_batch_commit_dev(ml_shard* sh, const void* const* local_evals_dev, uint8_t root_out[32]) {
     MLB_TRY(check_ready(sh));
     DeviceGuard guard;
-    sh->epoch++;
+    sh->grp.epoch++;
     const size_t ppr = sh->polys_per_rank;
     for (size_t i = 0; i < sh->local.size(); i++) MLB_TRY(upload_inputs(sh, sh->local[i], nullptr, nullptr, local_evals_dev + i * ppr));
     sh->n_marks = 0;
@@ -749,7 +592,7 @@ int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n
     if (n_vars != sh->n_vars || n_polys != sh->B) { set_error("ml_shard_batched_pcs_prove: claim does not match the handle's shape"); return ML_ERR_SIZE; }
     DeviceGuard guard;
     *out = nullptr;
-    sh->epoch++;
+    sh->grp.epoch++;
     const size_t ppr = sh->polys_per_rank, n = sh->n, domain = n << ML_LOG_BLOWUP;
     // BatchedPCSProverData::init (:37-77): the claim enters the transcript first
     t->sha.update(inputs, n_vars * 16);    // :44-46

@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -139,6 +139,14 @@ extern "C" {
     pub fn ml_pcs_proof_sumcheck_coeffs(p: *const MlPcsProof, out: *mut u8) -> c_int;
     pub fn ml_pcs_prove(inputs: *const u8, n_vars: usize, output: *const u8, evals: *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlPcsProof) -> c_int;
     pub fn ml_pcs_prove_dev(inputs: *const u8, n_vars: usize, output: *const u8, evals_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlPcsProof) -> c_int;
+    pub fn ml_pcs_shard_arena_bytes(sh: *const MlPcsShard) -> usize;
+    pub fn ml_pcs_shard_connect(sh: *mut MlPcsShard, records: *const u8, n_records: usize) -> c_int;
+    pub fn ml_pcs_shard_create(world: c_int, n_local: c_int, local_ranks: *const c_int, local_devices: *const c_int, n_vars: usize, out: *mut *mut MlPcsShard) -> c_int;
+    pub fn ml_pcs_shard_export(sh: *mut MlPcsShard, records_out: *mut u8) -> c_int;
+    pub fn ml_pcs_shard_free(sh: *mut MlPcsShard);
+    pub fn ml_pcs_shard_prove(sh: *mut MlPcsShard, inputs: *const u8, n_vars: usize, output: *const u8, evals: *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlPcsProof) -> c_int;
+    pub fn ml_pcs_shard_prove_dev(sh: *mut MlPcsShard, inputs: *const u8, n_vars: usize, output: *const u8, local_evals_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlPcsProof) -> c_int;
+    pub fn ml_pcs_shard_stream(sh: *const MlPcsShard, local_index: c_int) -> *mut c_void;
     pub fn ml_pcs_verify(p: *const MlPcsProof, t: *mut MlTranscript) -> c_int;
     pub fn ml_poly_evaluate(coeffs: *const u8, n: usize, x: *const u8, out: *mut u8) -> c_int;
     pub fn ml_poly_evaluate_over_domain(coeffs: *const u8, n: usize, evals_out: *mut u8) -> c_int;
@@ -533,11 +541,48 @@ fn sumcheck_polys(flat: &[F]) -> Vec<SumcheckPolynomial<F>> {
 pub fn pcs_prove(inputs: Vec<F>, output: F, poly: MultilinearPolynomialEvals<F>, transcript: &mut Transcript) -> PCSProof<F> {
     let mut h = std::ptr::null_mut();
     check(unsafe { ml_pcs_prove(p(&inputs), inputs.len(), output.as_ref().as_ptr(), p(&poly.evals), poly.evals.len(), transcript.h, &mut h) });
-    let fri_proof = unsafe { fri_proof_from(ml_pcs_proof_fri(h)) };
-    let mut flat = zeros(2 * unsafe { ml_pcs_proof_num_rounds(h) });
-    check(unsafe { ml_pcs_proof_sumcheck_coeffs(h, pm(&mut flat)) });
-    unsafe { ml_pcs_proof_free(h) };
+    unsafe { pcs_proof_from(h, inputs, output) }
+}
+unsafe fn pcs_proof_from(h: *mut MlPcsProof, inputs: Vec<F>, output: F) -> PCSProof<F> {
+    let fri_proof = fri_proof_from(ml_pcs_proof_fri(h));
+    let mut flat = zeros(2 * ml_pcs_proof_num_rounds(h));
+    check(ml_pcs_proof_sumcheck_coeffs(h, pm(&mut flat)));
+    ml_pcs_proof_free(h);
     PCSProof { fri_proof, sumcheck_polynomials: sumcheck_polys(&flat), inputs, output }
+}
+/// `PCSProof::prove` of ONE polynomial over all GPUs of the box from one process (ml_pcs_shard_*, csrc/pcs_shard.cu): rank g holds
+/// the block evals[g*n/G, (g+1)*n/G); the first log2(G) fold rounds run sharded, rank 0 runs the rest.  Lower latency than
+/// `pcs_prove` from n_vars ~ 20 up, and polynomials too large for one GPU.  The handle is built once per n_vars and reused; the
+/// proof bytes equal `pcs_prove`'s.
+pub struct ShardedPcsProver {
+    h: *mut MlPcsShard,
+}
+impl ShardedPcsProver {
+    pub fn new(n_vars: usize) -> Self {
+        let mut count = 0;
+        check(unsafe { ml_device_count(&mut count) });
+        let mut world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
+        while world > 1 && n_vars < 2 * world.trailing_zeros() as usize {
+            world >>= 1; // n_vars >= 2 log2(world)
+        }
+        let world = world.min(16) as c_int;
+        let ids: Vec<c_int> = (0..world).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_pcs_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), n_vars, &mut h) });
+        Self { h }
+    }
+    pub fn prove(&mut self, inputs: Vec<F>, output: F, poly: MultilinearPolynomialEvals<F>, transcript: &mut Transcript) -> PCSProof<F> {
+        let mut h = std::ptr::null_mut();
+        check(unsafe {
+            ml_pcs_shard_prove(self.h, p(&inputs), inputs.len(), output.as_ref().as_ptr(), p(&poly.evals), poly.evals.len(), transcript.h, &mut h)
+        });
+        unsafe { pcs_proof_from(h, inputs, output) }
+    }
+}
+impl Drop for ShardedPcsProver {
+    fn drop(&mut self) {
+        unsafe { ml_pcs_shard_free(self.h) }
+    }
 }
 /// `BatchedFriProof` does not derive `Deserialize`; its blob is the bincode encoding of its parts in field order, and the parts
 /// that do derive it (`Vec<HashDigest>`, `MerkleInclusionPath<Vec<ReedSolomonPair<F>>>`, `QueryProof<F>`, `F`) are decoded one by one
