@@ -45,7 +45,8 @@ def claim(oracle, world, nv):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("world,nv", [(1, 1), (1, 6), (2, 2), (2, 9), (4, 4), (4, 12), (8, 6), (8, 14), (16, 8), (16, 13)])
+@pytest.mark.parametrize("world,nv", [(1, 1), (1, 6), (2, 2), (2, 9), (2, 20), (4, 4), (4, 12), (4, 20), (8, 6), (8, 14), (16, 8), (16, 13),
+                                      (16, 20)])
 def test_virtual_ranks_vs_oracle(ml, oracle, world, nv):
     ev, inp, out = claim(oracle, world, nv)
     sh = ml.ShardedPCSProver.single_process([0] * world, nv)
@@ -82,22 +83,32 @@ def test_reference_inputs_n20_world8(ml, oracle):
     sh.free()
 
 
-@pytest.mark.gpu
-def test_at_size_n24_world8_equals_unsharded(ml):
-    """n_vars 24 with 8 virtual ranks: the same bytes as the unsharded CUDA prover (itself pinned to the oracle at this size by
-    test_atsize_pcs_prove_n_vars_24)"""
+def at_size_n24_equals_unsharded(ml, world):
     nv, n = 24, 1 << 24
     evals = ml.synthetic_elements_dev(0xB200, n)
     inp = ml.synthetic_elements_dev(0xB2000001, nv).elems()
     out = ml.MultilinearPolynomialEvals(evals.elems()).evaluate(ml.to_ints(inp))
     t1 = ml.Transcript()
     single = ml.PCSProof.prove_dev(inp, out, evals, n, t1)
-    sh = ml.ShardedPCSProver.single_process([0] * 8, nv)
+    sh = ml.ShardedPCSProver.single_process([0] * world, nv)
     t = ml.Transcript()
-    proof = sh.prove_dev(inp, out, [evals.ptr.value + g * (n // 8) * 16 for g in range(8)], t)
+    proof = sh.prove_dev(inp, out, [evals.ptr.value + g * (n // world) * 16 for g in range(world)], t)
     assert proof.fri_proof.serialize() == single.fri_proof.serialize()
     assert proof.sumcheck_polynomials == single.sumcheck_polynomials and t.random() == t1.random()
     sh.free()
+
+
+@pytest.mark.gpu
+def test_at_size_n24_world8_equals_unsharded(ml):
+    """n_vars 24 with 8 virtual ranks: the same bytes as the unsharded CUDA prover (itself pinned to the oracle at this size by
+    test_atsize_pcs_prove_n_vars_24)"""
+    at_size_n24_equals_unsharded(ml, 8)
+
+
+@pytest.mark.gpu
+def test_at_size_n24_world16_equals_unsharded(ml):
+    """the same with 16 virtual ranks: the combine kernel for G = 16 and the tail chain from layer 4 at a realistic size"""
+    at_size_n24_equals_unsharded(ml, 16)
 
 
 @pytest.mark.gpu
