@@ -347,6 +347,32 @@ int ml_pcs_shard_prove_dev(ml_pcs_shard *sh, const uint8_t *inputs, size_t n_var
 int ml_pcs_shard_prove(ml_pcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t output[16],
                        const uint8_t *evals, size_t n, ml_transcript *t, ml_pcs_proof **out);
 
+/* ---- BatchedPCSProof::prove with every polynomial split by block over the GPUs of one box (batched_pcs.rs:130-180) ----
+ * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; rank b holds the block evals_j[b*n/G, (b+1)*n/G) of EVERY polynomial j,
+ * so any batch size B >= 1 runs on any G (ml_shard_* splits by polynomial and needs G | B).  Each code is encoded, exchanged and
+ * combined as in ml_pcs_shard_*; layer 0 is one batched Merkle tree over the B codes whose segment subtrees stay with their owners;
+ * rho, the fingerprinted sumcheck tables and the first log2(G) fold rounds are sharded, then rank 0 runs the rest of the fold
+ * chain from N/G elements and the openings (csrc/bpcs_shard.cu).  Rank r holds about 1/G of every code, of the batch tree and of
+ * the tables; the arena holds each code twice (layer 0 and its receive slice, ml_bpcs_shard_arena_bytes).
+ * The proof is byte-identical to ml_batched_pcs_prove's and an ordinary ml_bpcs_proof (ml_batched_pcs_verify, the serializer
+ * work unchanged).  Handles, records, calls and errors as for ml_shard_* above.  Minimum size: n_vars >= max(1, 2*log2 G):
+ * G = 1: 1, 2: 2, 4: 4, 8: 6, 16: 8 (ML_ERR_SIZE below, and for n_polys = 0). */
+typedef struct ml_bpcs_shard ml_bpcs_shard;
+int ml_bpcs_shard_create(int world, int n_local, const int *local_ranks, const int *local_devices, size_t n_polys, size_t n_vars,
+                         ml_bpcs_shard **out);
+void ml_bpcs_shard_free(ml_bpcs_shard *sh);   /* multi-process: all ranks must have returned from their last call (caller's barrier) */
+int ml_bpcs_shard_export(ml_bpcs_shard *sh, uint8_t *records_out /* num_local * ml_shard_record_bytes() */);
+int ml_bpcs_shard_connect(ml_bpcs_shard *sh, const uint8_t *records, size_t n_records /* world */);
+void *ml_bpcs_shard_stream(const ml_bpcs_shard *sh, int local_index);  /* the local rank's main stream (for CUDA-event timing) */
+size_t ml_bpcs_shard_arena_bytes(const ml_bpcs_shard *sh);
+/* local_evals_dev[i * n_polys + j]: local rank i's block of polynomial j (device pointers, complete before the call; rank-major).
+ * Every process passes the same claim and its own transcript copy; all copies end in rank 0's final state. */
+int ml_bpcs_shard_prove_dev(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
+                            const void *const *local_evals_dev, ml_transcript *t, ml_bpcs_proof **out /* NULL unless rank 0 is local */);
+/* host evals[j] (all n of each polynomial) and a handle that hosts every rank: the drop-in for batched_pcs.rs:130 */
+int ml_bpcs_shard_prove(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
+                        const uint8_t *const *evals, size_t n, ml_transcript *t, ml_bpcs_proof **out);
+
 /* ---- batched commit building blocks (round-1 API, kept): one rank's share of `Merkle::batch_commit`
  * (merkle_tree/mod.rs:110-131) over leaf range [leaf_begin, leaf_begin+leaf_count) of all codes.
  * codes_dev[j] points at code j's rows for this range laid out as pairs: leaf_count x 32 bytes.

@@ -366,6 +366,7 @@ class BatchedPCSProof {
 
   private:
     friend class ShardedBatchedProver;
+    friend class ShardedBatchedBlockProver;
     BatchedPCSProof() = default;
     ml_bpcs_proof* h_ = nullptr;
 };
@@ -389,6 +390,29 @@ class ShardedBatchedProver {
 
   private:
     ml_shard* h_ = nullptr;
+};
+// BatchedPCSProof::prove over several GPUs from one process with every polynomial split by block (ml_bpcs_shard_*,
+// csrc/bpcs_shard.cu): any n_polys >= 1 on any power-of-two number of ranks; `devices` may repeat (virtual ranks)
+class ShardedBatchedBlockProver {
+  public:
+    ShardedBatchedBlockProver(const std::vector<int>& devices, size_t n_polys, size_t n_vars) {
+        std::vector<int> ranks(devices.size());
+        for (size_t i = 0; i < ranks.size(); i++) ranks[i] = (int)i;
+        check(ml_bpcs_shard_create((int)devices.size(), (int)devices.size(), ranks.data(), devices.data(), n_polys, n_vars, &h_));
+    }
+    ShardedBatchedBlockProver(const ShardedBatchedBlockProver&) = delete;
+    ~ShardedBatchedBlockProver() { if (h_) ml_bpcs_shard_free(h_); }
+    BatchedPCSProof prove(const BatchedPCSClaim& claim, const std::vector<MultilinearPolynomialEvals>& polys, Transcript& t) {
+        std::vector<const uint8_t*> ptrs;
+        for (auto& p : polys) ptrs.push_back(raw(p.evals));
+        BatchedPCSProof p;
+        check(ml_bpcs_shard_prove(h_, raw(claim.inputs), claim.inputs.size(), raw(claim.outputs), polys.size(), ptrs.data(),
+                                  polys.empty() ? 0 : polys[0].evals.size(), t.handle(), &p.h_));
+        return p;
+    }
+
+  private:
+    ml_bpcs_shard* h_ = nullptr;
 };
 
 // src/polynomials.rs:3-98 — univariate helpers over the domain 0..n-1 (named Univariate* here: `Polynomial` above is src/ntt's)

@@ -37,6 +37,10 @@ int ml_shard_phase_ms(const struct ml_shard *sh, double *out, int cap);
  * chain (rank 0), openings + proof (rank 0)] */
 struct ml_pcs_shard;
 int ml_pcs_shard_phase_ms(const struct ml_pcs_shard *sh, double *out, int cap);
+/* block-sharded batched PCS prover (ml_bpcs_shard_*): [S0 encodes + exchange, S1 combine + batch tree, S2/S3 batch root + rho +
+ * fingerprinted tables, sharded rounds, tail fold chain (rank 0), openings + proof (rank 0)] */
+struct ml_bpcs_shard;
+int ml_bpcs_shard_phase_ms(const struct ml_bpcs_shard *sh, double *out, int cap);
 
 #ifdef __cplusplus
 }

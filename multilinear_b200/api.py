@@ -887,6 +887,90 @@ class ShardedBatchedProver:
             pass
 
 
+class BlockShardedBatchedProver:
+    """BatchedPCSProof::prove with every polynomial split by block over the GPUs of one box (ml_bpcs_shard_*,
+    csrc/bpcs_shard.cu).  Rank g holds the block evals_j[g*n/G, (g+1)*n/G) of every polynomial j, so any batch size works on any
+    power-of-two G.  Handles as for ShardedPCSProver: single_process (devices may repeat = virtual ranks on one GPU) or one_rank
+    with connect / connect_over.  The proof is an ordinary batched PCSProof, byte-identical to BatchedPCSProof.prove's."""
+
+    def __init__(self, h, world, local_ranks, n_polys, n_vars):
+        self.h, self.world, self.local_ranks, self.n_polys, self.n_vars = h, world, list(local_ranks), n_polys, n_vars
+
+    @staticmethod
+    def _create(world, ranks, devices, n_polys, n_vars):
+        h = C.c_void_p()
+        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
+        check(load().ml_bpcs_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_polys), _sz(n_vars), C.byref(h)))
+        return BlockShardedBatchedProver(h, world, ranks, n_polys, n_vars)
+
+    @staticmethod
+    def single_process(devices, n_polys, n_vars):
+        return BlockShardedBatchedProver._create(len(devices), list(range(len(devices))), list(devices), n_polys, n_vars)
+
+    @staticmethod
+    def one_rank(rank, world, device, n_polys, n_vars):
+        return BlockShardedBatchedProver._create(world, [rank], [device], n_polys, n_vars)
+
+    def export(self):
+        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
+        check(load().ml_bpcs_shard_export(self.h, _p(out)))
+        return out.tobytes()
+
+    def connect(self, records):
+        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
+        check(load().ml_bpcs_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
+
+    def connect_over(self, dist, device):
+        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
+        import torch
+        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
+        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
+        dist.all_gather(allr, mine)
+        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
+
+    def stream(self, local_index=0):
+        return load().ml_bpcs_shard_stream(self.h, C.c_int(local_index))
+
+    def arena_bytes(self):
+        return load().ml_bpcs_shard_arena_bytes(self.h)
+
+    def phase_ms(self):
+        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
+        out = (C.c_double * 16)()
+        n = load().ml_bpcs_shard_phase_ms(self.h, out, C.c_int(16))
+        return [out[i] for i in range(n)]
+
+    def prove_dev(self, inputs, outputs, local_evals_ptrs, transcript):
+        """local_evals_ptrs[i * n_polys + j]: device pointer to local rank i's block (n/G evaluations) of polynomial j;
+        None unless rank 0 is local"""
+        i, o = as_elems(inputs), as_elems(outputs)
+        ptrs = (C.c_void_p * len(local_evals_ptrs))(*local_evals_ptrs)
+        h = C.c_void_p()
+        check(load().ml_bpcs_shard_prove_dev(self.h, _p(i), _sz(i.shape[0]), _p(o), _sz(o.shape[0]), ptrs, transcript.h, C.byref(h)))
+        return PCSProof(h, batched=True) if h.value else None
+
+    def prove(self, inputs, outputs, polys, transcript):
+        """host evaluations (needs a single-process handle) — the drop-in for batched_pcs.rs:130"""
+        i, o = as_elems(inputs), as_elems(outputs)
+        ps = [p.evals if isinstance(p, MultilinearPolynomialEvals) else as_elems(p) for p in polys]
+        ptrs = (C.c_void_p * len(ps))(*[p.ctypes.data for p in ps])
+        h = C.c_void_p()
+        check(load().ml_bpcs_shard_prove(self.h, _p(i), _sz(i.shape[0]), _p(o), _sz(len(ps)), ptrs, _sz(ps[0].shape[0] if ps else 0),
+                                         transcript.h, C.byref(h)))
+        return PCSProof(h, batched=True)
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_bpcs_shard_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class ShardedPCSProver:
     """PCSProof::prove of one polynomial sharded over the GPUs of one box (ml_pcs_shard_*, csrc/pcs_shard.cu).  Rank g holds the
     block evals[g*n/G, (g+1)*n/G).  A handle hosts the ranks of one process: all of them (single_process; devices may repeat =

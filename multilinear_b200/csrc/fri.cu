@@ -135,7 +135,8 @@ int fri_batched_fold_launch(Ctx* ctx, const fe* const* codes, size_t n_codes, si
 
 // fingerprinted evaluation table (batched_pcs.rs:55-63): out[i] = Horner_rho(polys[0][i], ..., polys[B-1][i])
 __global__ void __launch_bounds__(256) fingerprint_rows_kernel(const fe* const* __restrict__ polys, int n_polys, size_t n, fe rho,
-                                                               fe* __restrict__ out) {
+                                                               const fe* __restrict__ rho_dev, fe* __restrict__ out) {
+    if (rho_dev) rho = fe_load(rho_dev);
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     for (; i < n; i += stride) {
@@ -144,8 +145,8 @@ __global__ void __launch_bounds__(256) fingerprint_rows_kernel(const fe* const* 
         fe_store(out + i, a);
     }
 }
-int fingerprint_rows_launch(const fe* const* polys, size_t n_polys, size_t n, hfe r, fe* out, cudaStream_t s) {
-    fingerprint_rows_kernel<<<grid_for(n), 256, 0, s>>>(polys, (int)n_polys, n, to_dev_fe(r), out);
+int fingerprint_rows_launch(const fe* const* polys, size_t n_polys, size_t n, hfe r, fe* out, cudaStream_t s, const fe* r_dev) {
+    fingerprint_rows_kernel<<<grid_for(n), 256, 0, s>>>(polys, (int)n_polys, n, to_dev_fe(r), r_dev, out);
     MLB_KERNEL_CHECK();
     return ML_OK;
 }

@@ -175,7 +175,8 @@ int merkle_upper_launch(uint8_t* digests, size_t n_leaves, cudaStream_t s);  // 
 int fri_fold_launch(Ctx* ctx, const fe* cur, size_t n_cur, fe* next, hfe r, const fe* r_dev, size_t k, int log_n0, cudaStream_t s);
 int fri_batched_fold_launch(Ctx* ctx, const fe* const* codes_dev_ptrs, size_t n_codes, size_t n, fe* next, hfe fingerprint_r, hfe r,
                             const fe* r_dev, int log_n0, cudaStream_t s);
-int fingerprint_rows_launch(const fe* const* polys_dev_ptrs, size_t n_polys, size_t n, hfe r, fe* out, cudaStream_t s);
+// r_dev: rho read from HBM instead of r
+int fingerprint_rows_launch(const fe* const* polys_dev_ptrs, size_t n_polys, size_t n, hfe r, fe* out, cudaStream_t s, const fe* r_dev = nullptr);
 // sumcheck.cu
 int sumcheck_sums_launch(Ctx* ctx, const fe* m, const fe* d, size_t height, hfe* s1, hfe* s2, cudaStream_t s);
 int sumcheck_partial_sum_launch(Ctx* ctx, const fe* m, const fe* d, size_t height, hfe r, hfe* out, cudaStream_t s);

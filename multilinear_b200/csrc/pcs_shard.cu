@@ -24,75 +24,17 @@
 //       fri_open_queries; the final transcript -> all + flag PF.  Every process's transcript ends in rank 0's state.
 //   G = 1 runs the same code without the exchange: the encode and the tables go straight into the tail buffers.
 #include <cstdlib>
+#include <memory>
 
-#include "peer.h"
-#include "prover_internal.h"
+#include "pcs_shard.h"
 #include "reduce.cuh"
 #include "sha256.cuh"
 
 using namespace mlb;
 using namespace mlbp;
+using namespace mlbs;
 
 namespace {
-
-enum Phase { PX = 0, PR0 = 1, PG = PR0 + 4, PF, N_PHASES };  // PR0 + k: round k (L <= 4)
-static const int MAXR = PEER_MAXR;
-static const int MAX_L = 4;
-static const size_t MAIL_ROOTS = (size_t)MAXR * MAXR / 2;  // run roots of layer 0 at G = ML_MAX_PEERS
-
-struct Layout {
-    size_t flags, status, tr, prev, r, sc, roots_out, final_tr, mail[MAX_L], top[MAX_L], part;  // mailbox (cleared at create)
-    size_t ycode, recv, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;
-};
-Layout make_layout(size_t n, int G) {
-    const int L = (int)ilog2((size_t)G);
-    const size_t NL = 2 * n / G, R = NL / G, nloc = n / G;
-    Layout a;
-    size_t o = 0;
-    auto take = [&](size_t bytes) { size_t r = o; o = peer_align(o + bytes); return r; };
-    a.flags = take((size_t)N_PHASES * MAXR * 8);
-    a.status = take(16);
-    a.tr = take(sizeof(DevTranscript));
-    a.prev = take(16);
-    a.r = take(32);
-    a.sc = take((size_t)MAX_L * 32);
-    a.roots_out = take((size_t)MAX_L * 32);
-    a.final_tr = take(sizeof(DevTranscript));
-    for (int k = 0; k < MAX_L; k++) a.mail[k] = take(MAIL_ROOTS * 32 + (size_t)MAXR * 32);  // run roots | partial pairs
-    for (int k = 0; k < MAX_L; k++) a.top[k] = take(2 * MAIL_ROOTS * 32);
-    a.part = take((size_t)(2 * sumcheck_max_blocks() + 2) * 16);
-    const bool sharded = G > 1;
-    a.ycode = take(sharded ? NL * 16 : 0);
-    a.recv = take(sharded ? NL * 16 : 0);
-    for (int k = 0; k < MAX_L; k++) {
-        a.layer[k] = take(k < L ? ((size_t)G >> k) * R * 16 : 0);
-        a.dig[k] = take(k < L ? ((size_t)G >> k) * R * 32 : 0);
-    }
-    a.m = take(sharded ? nloc * 16 : 0);
-    a.d = take(sharded ? nloc * 16 : 0);
-    a.tail_code = take(NL * 16);
-    a.tail_m = take(nloc * 16);
-    a.tail_d = take(nloc * 16);
-    a.total = o;
-    return a;
-}
-// mailbox of round k: run root of run q at roots + 32 q, partial pair of rank g at partials + 32 g
-size_t mail_partials(const Layout& a, int k) { return a.mail[k] + MAIL_ROOTS * 32; }
-
-__device__ __forceinline__ int ilog2_dev(size_t x) { return 63 - __clzll((unsigned long long)x); }
-// merkle_layer_offset on the device: layer l of a tree with n leaves starts at digest 2n - (2n >> l)
-__device__ __forceinline__ size_t layer_off(size_t n_leaves, int layer) { return 2 * n_leaves - ((2 * n_leaves) >> layer); }
-__device__ __forceinline__ fe root_pow(const fe* __restrict__ lo, const fe* __restrict__ hi, size_t e) {
-    fe w = fe_load_nc(lo + (e & (((size_t)1 << LO_BITS) - 1)));
-    if (e >> LO_BITS) w = fe_mul(w, fe_load_nc(hi + (e >> LO_BITS)));
-    return w;
-}
-// position of element j of run p in a layer with `runs` runs per rank (segment layout; one run: plain)
-__device__ __forceinline__ size_t run_pos(size_t runs, size_t p, size_t j, size_t R) {
-    if (runs == 1) return j;
-    const size_t half = runs >> 1;
-    return (p & (half - 1)) * 2 * R + (p >= half ? R : 0) + j;
-}
 
 // ------------------------------------------------------------------ S0: exchange of the local code, cyclic tables
 // code slice [dest*R, (dest+1)*R) -> rank dest's recv[rank*R ..]
@@ -163,7 +105,7 @@ __global__ void __launch_bounds__(256) pcs_shard_combine_kernel(const fe* __rest
 }
 
 // ------------------------------------------------------------------ rounds
-// A: this rank's partial sums (CTA partials -> one pair) and run roots -> every rank's round-k mailbox, then flag PR_k there
+// A: this rank's partial sums (CTA partials -> one pair; none if nb < 0) and run roots -> every rank's mailbox, then the flag there
 __global__ void __launch_bounds__(256) pcs_shard_post_kernel(const fe* __restrict__ part, int nb, const uint8_t* __restrict__ dig, size_t R, int segs,
                                                              int rank, int world, PeerPtrs peers, size_t off_roots, size_t off_partials, size_t off_flag,
                                                              unsigned long long epoch) {
@@ -185,8 +127,10 @@ __global__ void __launch_bounds__(256) pcs_shard_post_kernel(const fe* __restric
         d4[0] = src[0];
         d4[1] = src[1];
     }
-    fe_store(reinterpret_cast<fe*>(dst + off_partials) + 2 * rank, sums[0]);
-    fe_store(reinterpret_cast<fe*>(dst + off_partials) + 2 * rank + 1, sums[1]);
+    if (nb >= 0) {
+        fe_store(reinterpret_cast<fe*>(dst + off_partials) + 2 * rank, sums[0]);
+        fe_store(reinterpret_cast<fe*>(dst + off_partials) + 2 * rank + 1, sums[1]);
+    }
     __threadfence_system();
     flag_store_release(reinterpret_cast<unsigned long long*>(dst + off_flag) + rank, epoch);
 }
@@ -247,11 +191,11 @@ struct OpenArgs {
     size_t off_layer[MAX_L], off_dig[MAX_L];
     const uint8_t* top[MAX_L];  // rank 0's copies of the top trees
     size_t n, NL, R;
-    int L, world, log_R, stride;  // stride: bytes per (query, layer) record = 32 value + 32 * 64 path
+    int L, j0, world, log_R, stride;  // layers j0 .. L-1; stride: bytes per (query, layer) record = 32 value + 32 * 64 path
 };
 // block (q, j): pair and path of leaf idx[q] mod (n >> j) in layer j, from the owner's arena
 __global__ void __launch_bounds__(64) pcs_shard_open_kernel(const unsigned long long* __restrict__ idx, PeerPtrs peers, OpenArgs a, uint8_t* __restrict__ out) {
-    const int q = blockIdx.x, j = blockIdx.y, t = threadIdx.x;
+    const int q = blockIdx.x, j = blockIdx.y + a.j0, t = threadIdx.x;
     const size_t i = idx[q] % (a.n >> j);
     const size_t p = i / a.NL, k2 = i - p * a.NL, owner = k2 / a.R, jj = k2 - owner * a.R;
     const int cnt = (a.world * a.world) >> (j + 1), log_cnt = ilog2_dev((size_t)cnt);
@@ -277,67 +221,151 @@ __global__ void __launch_bounds__(64) pcs_shard_open_kernel(const unsigned long 
     }
 }
 
-struct PcsRank : PeerRank {};
-
 }  // namespace
 
-struct ml_pcs_shard {
-    int world = 1, L = 0;
-    size_t n_vars = 0, n = 0, NL = 0, R = 0, nloc = 0;
-    Layout lay;
-    std::vector<PcsRank> local;
-    PeerGroup grp;
-    // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
-    static const int N_MARKS = 8;
-    cudaEvent_t mark[N_MARKS] = {nullptr};
-    int n_marks = 0;
-};
+struct ml_pcs_shard : ShardCore {};
 
-namespace {
+namespace mlbs {
 
-const char* WHO = "ml_pcs_shard";
+Layout make_layout(size_t n, int G, size_t B) {
+    const int L = (int)ilog2((size_t)G);
+    const size_t NL = 2 * n / G, R = NL / G, nloc = n / G;
+    const bool sharded = G > 1, batched = B > 0;
+    Layout a;
+    size_t o = 0;
+    auto take = [&](size_t bytes) { size_t r = o; o = peer_align(o + bytes); return r; };
+    a.flags = take((size_t)N_PHASES * MAXR * 8);
+    a.status = take(16);
+    a.tr = take(sizeof(DevTranscript));
+    a.prev = take(16);
+    a.r = take(32);
+    a.sc = take((size_t)MAX_L * 32);
+    a.roots_out = take((size_t)MAX_L * 32);
+    a.final_tr = take(sizeof(DevTranscript));
+    for (int k = 0; k < MAX_L; k++) a.mail[k] = take(MAIL_ROOTS * 32 + (size_t)MAXR * 32);  // run roots | partial pairs
+    for (int k = 0; k < MAX_L; k++) a.top[k] = take(2 * MAIL_ROOTS * 32);
+    a.part = take((size_t)(2 * sumcheck_max_blocks() + 2) * 16);
+    a.rho = take(batched ? 16 : 0);
+    a.outs = take(B * 16);
+    a.eptrs = take(B * 8);
+    a.segptrs = take((sharded ? (size_t)G / 2 : 1) * B * 8);
+    // batched: two encode buffers (the encode of polynomial j+1 overlaps the exchange of j) and one recv slice per polynomial
+    a.ycode = take(sharded ? (batched ? 2 : 1) * NL * 16 : 0);
+    a.recv = take(sharded ? (batched ? B : 1) * NL * 16 : 0);
+    for (int k = 0; k < MAX_L; k++) {
+        const bool held = k < L || (k == 0 && batched);
+        a.layer[k] = take(held ? (k == 0 && batched ? B : 1) * ((size_t)G >> k) * R * 16 : 0);
+        a.dig[k] = take(held ? ((size_t)G >> k) * R * 32 : 0);
+    }
+    a.m = take(sharded ? nloc * 16 : 0);
+    a.d = take(sharded ? nloc * 16 : 0);
+    a.tail_code = take(NL * 16);
+    a.tail_m = take(nloc * 16);
+    a.tail_d = take(nloc * 16);
+    a.total = o;
+    return a;
+}
 
-void mark_phase(ml_pcs_shard* sh, int idx) {
-    if (idx >= ml_pcs_shard::N_MARKS || sh->local.empty()) return;
-    PcsRank& r = sh->local[0];
+void mark_phase(ShardCore* sh, int idx) {
+    if (idx >= ShardCore::N_MARKS || sh->local.empty()) return;
+    PeerRank& r = sh->local[0];
     cudaSetDevice(r.device);
     if (!sh->mark[idx] && cudaEventCreate(&sh->mark[idx]) != cudaSuccess) { cudaGetLastError(); return; }
     cudaEventRecord(sh->mark[idx], r.st.main);
     if (idx + 1 > sh->n_marks) sh->n_marks = idx + 1;
 }
-fe* at(const PcsRank& r, size_t off) { return reinterpret_cast<fe*>(r.arena + off); }
+PeerRank* rank0_of(ShardCore* sh) {
+    for (auto& r : sh->local)
+        if (r.rank == 0) return &r;
+    return nullptr;
+}
 
-// S0 of one rank: claim state, encode, exchange, tables
-int stage_encode(ml_pcs_shard* sh, PcsRank& r, const fe* evals, const uint8_t* claim_state, const std::vector<hfe>& pts) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    cudaStream_t s = r.st.main;
-    const Layout& a = sh->lay;
-    MLB_TRY(h2d(r.arena + a.tr, claim_state, sizeof(DevTranscript), s));
-    MLB_TRY(h2d(r.arena + a.prev, claim_state + sizeof(DevTranscript), 16, s));
-    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, s));
-    const int G = sh->world, L = sh->L, v = (int)sh->n_vars;
-    if (G == 1) {
-        MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.tail_code), s));
-        MLB_CUDA(cudaMemcpyAsync(at(r, a.tail_m), evals, sh->nloc * 16, cudaMemcpyDeviceToDevice, s));
-        return eq_table_launch(r.ctx, pts.data(), sh->n_vars, at(r, a.tail_d), s);
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who) {
+    const int L = (int)ilog2((size_t)world);
+    sh->world = world; sh->L = L; sh->n_vars = n_vars; sh->n = (size_t)1 << n_vars; sh->B = B;
+    sh->NL = 2 * sh->n / world; sh->R = sh->NL / world; sh->nloc = sh->n / world;
+    sh->lay = make_layout(sh->n, world, B);
+    sh->grp.world = world;
+    sh->grp.arena_bytes = sh->lay.total;
+    sh->grp.off_flags = sh->lay.flags;
+    sh->grp.off_status = sh->lay.status;
+    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
+    int st = ML_OK;
+    for (int i = 0; i < n_local && st == ML_OK; i++) {
+        PeerRank r;
+        r.rank = local_ranks[i];
+        r.device = local_devices[i];
+        st = peer_rank_init(sh->grp, r, who, sh->lay.ycode);
+        if (st == ML_OK || st == ML_ERR_ALLOC) sh->local.push_back(r);
     }
-    MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.ycode), s));
-    pcs_shard_exchange_kernel<<<peer_grid(sh->NL), 256, 0, s>>>(at(r, a.ycode), sh->NL, sh->R, r.rank, sh->grp.peers(), a.recv);
+    if (st == ML_OK && n_local == world) {
+        std::vector<PeerRank*> ranks;
+        for (auto& r : sh->local) ranks.push_back(&r);
+        st = peer_link_local(sh->grp, ranks, who);
+    }
+    return st;
+}
+
+void shard_free(ShardCore* sh) {
+    DeviceGuard guard;
+    for (int i = 0; i < ShardCore::N_MARKS; i++)
+        if (sh->mark[i]) cudaEventDestroy(sh->mark[i]);
+    for (auto& r : sh->local) {
+        cudaSetDevice(r.device);
+        cudaDeviceSynchronize();
+        peer_rank_free(r);
+    }
+    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
+}
+
+int shard_export(ShardCore* sh, uint8_t* records_out) {
+    std::vector<PeerRank*> ranks;
+    for (auto& r : sh->local) ranks.push_back(&r);
+    return peer_export(ranks, records_out);
+}
+int shard_connect(ShardCore* sh, const uint8_t* records, size_t n_records, const char* who) {
+    if (sh->local.size() != 1) { set_error("%s: only for handles that host one rank", who); return ML_ERR_ARG; }
+    return peer_connect(sh->grp, sh->local[0], records, n_records, who);
+}
+void* shard_stream(const ShardCore* sh, int local_index) {
+    if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
+    return (void*)sh->local[local_index].st.main;
+}
+int shard_phase_ms(const ShardCore* sh, double* out, int cap) {
+    int n = 0;
+    for (int i = 0; i + 1 < sh->n_marks && n < cap; i++) {
+        float ms = 0;
+        if (!sh->mark[i] || !sh->mark[i + 1] || cudaEventElapsedTime(&ms, sh->mark[i], sh->mark[i + 1]) != cudaSuccess) { cudaGetLastError(); ms = -1.f; }
+        out[n++] = ms;
+    }
+    return n;
+}
+
+int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s) {
+    pcs_shard_exchange_kernel<<<peer_grid(sh->NL), 256, 0, s>>>(ycode, sh->NL, sh->R, r.rank, sh->grp.peers(), off_recv);
     MLB_KERNEL_CHECK();
-    pcs_shard_tables_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(evals, sh->nloc, L, r.rank, sh->grp.peers(), a.m);
+    return ML_OK;
+}
+int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s) {
+    pcs_shard_tables_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(src, sh->nloc, sh->L, r.rank, sh->grp.peers(), off_m);
     MLB_KERNEL_CHECK();
-    MLB_TRY(eq_table_launch(r.ctx, pts.data(), (size_t)(v - L), at(r, a.d), s));
+    return ML_OK;
+}
+int local_eq_table(ShardCore* sh, PeerRank& r, const std::vector<hfe>& pts, fe* d, cudaStream_t s) {
+    const int L = sh->L, v = (int)sh->n_vars;
+    MLB_TRY(eq_table_launch(r.ctx, pts.data(), (size_t)(v - L), d, s));
+    if (L == 0) return ML_OK;
     hfe scale = 1;
     for (int b = 0; b < L; b++) {
         const hfe p = pts[(size_t)(v - 1 - b)];
         scale = hfe_mul(scale, ((r.rank >> b) & 1) ? p : hfe_sub(1, p));
     }
-    pcs_shard_scale_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(at(r, a.d), sh->nloc, to_dev_fe_h(scale));
+    pcs_shard_scale_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(d, sh->nloc, to_dev_fe_h(scale));
     MLB_KERNEL_CHECK();
-    return peer_signal(sh->grp, r, PX, -1, s);
+    return ML_OK;
 }
 
-int launch_combine(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s) {
+int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s) {
     const unsigned grid = peer_grid(R);
     switch (L) {
         case 1: pcs_shard_combine_kernel<1><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
@@ -350,8 +378,46 @@ int launch_combine(int L, const fe* recv, size_t R, int rank, int log_N, const R
     return ML_OK;
 }
 
+int post_launch(ShardCore* sh, PeerRank& r, const uint8_t* dig, size_t R, int segs, int nb, size_t off_roots, size_t off_partials, int phase) {
+    pcs_shard_post_kernel<<<1, 256, 0, r.st.main>>>(at(r, sh->lay.part), nb, dig, R, segs, r.rank, sh->world, sh->grp.peers(), off_roots, off_partials,
+                                                    sh->lay.flags + (size_t)phase * MAXR * 8, sh->grp.epoch);
+    MLB_KERNEL_CHECK();
+    return ML_OK;
+}
+int top_launch(ShardCore* sh, PeerRank& r, int phase, int k, int cnt) {
+    pcs_shard_top_kernel<<<1, 32, 0, r.st.main>>>(sh->grp.flags(r, phase), sh->world, sh->grp.epoch, sh->grp.timeout_ns, sh->grp.status(r),
+                                                  r.arena + sh->lay.mail[k], cnt, r.arena + sh->lay.top[k]);
+    MLB_KERNEL_CHECK();
+    return ML_OK;
+}
+int finish_launch(ShardCore* sh, PeerRank& r, int k, const uint8_t* root) {
+    const Layout& a = sh->lay;
+    return chain_sumcheck_finish_launch(at(r, mail_partials(a, k)), sh->world, at(r, a.prev), (DevTranscript*)(r.arena + a.tr), root, root ? 32 : 0,
+                                        root ? r.arena + a.roots_out + 32 * k : nullptr, at(r, a.sc) + 2 * k, at(r, a.r), r.st.main);
+}
+
+// S0 of one rank: claim state, encode, exchange, tables
+int stage_encode(ShardCore* sh, PeerRank& r, const fe* evals, const uint8_t* claim_state, const std::vector<hfe>& pts) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    cudaStream_t s = r.st.main;
+    const Layout& a = sh->lay;
+    MLB_TRY(h2d(r.arena + a.tr, claim_state, sizeof(DevTranscript), s));
+    MLB_TRY(h2d(r.arena + a.prev, claim_state + sizeof(DevTranscript), 16, s));
+    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, s));
+    if (sh->world == 1) {
+        MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.tail_code), s));
+        MLB_CUDA(cudaMemcpyAsync(at(r, a.tail_m), evals, sh->nloc * 16, cudaMemcpyDeviceToDevice, s));
+        return local_eq_table(sh, r, pts, at(r, a.tail_d), s);
+    }
+    MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.ycode), s));
+    MLB_TRY(exchange_launch(sh, r, at(r, a.ycode), a.recv, s));
+    MLB_TRY(tables_launch(sh, r, evals, a.m, s));
+    MLB_TRY(local_eq_table(sh, r, pts, at(r, a.d), s));
+    return peer_signal(sh->grp, r, PX, -1, s);
+}
+
 // S1 of one rank: wait for the slices, combine into layer 0, round-0 partial sums
-int stage_combine(ml_pcs_shard* sh, PcsRank& r, int* nb) {
+int stage_combine(ShardCore* sh, PeerRank& r, int* nb) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     const Layout& a = sh->lay;
@@ -359,80 +425,150 @@ int stage_combine(ml_pcs_shard* sh, PcsRank& r, int* nb) {
     const RootTables* rt;
     MLB_TRY(get_root_tables(r.ctx, log_N, s, &rt));  // never a lazy build behind a spinning wait
     MLB_TRY(peer_wait(sh->grp, r, PX, -1, s));
-    MLB_TRY(launch_combine(sh->L, at(r, a.recv), sh->R, r.rank, log_N, rt, at(r, a.layer[0]), s));
+    MLB_TRY(combine_launch(sh->L, at(r, a.recv), sh->R, r.rank, log_N, rt, at(r, a.layer[0]), s));
     return sumcheck_sums_partials_launch(at(r, a.m), at(r, a.d), sh->nloc, at(r, a.part), nb, s);
 }
 
 // round k, phase A: segment subtrees, post roots + partial sums
-int stage_post(ml_pcs_shard* sh, PcsRank& r, int k, int nb) {
+int stage_post(ShardCore* sh, PeerRank& r, int k, int nb) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     const Layout& a = sh->lay;
     const size_t segs = (size_t)sh->world >> (k + 1), R = sh->R;
     for (size_t p = 0; p < segs; p++) MLB_TRY(merkle_rs_launch(at(r, a.layer[k]) + p * 2 * R, 2 * R, r.arena + a.dig[k] + 32 * p * 2 * R, s));
-    pcs_shard_post_kernel<<<1, 256, 0, s>>>(at(r, a.part), nb, r.arena + a.dig[k], R, (int)segs, r.rank, sh->world, sh->grp.peers(), a.mail[k],
-                                            mail_partials(a, k), a.flags + (size_t)(PR0 + k) * MAXR * 8, sh->grp.epoch);
-    MLB_KERNEL_CHECK();
-    return ML_OK;
+    return post_launch(sh, r, r.arena + a.dig[k], R, (int)segs, nb, a.mail[k], mail_partials(a, k), PR0 + k);
 }
 // round k, phase B: top of the layer tree, round polynomial, challenge (same on every rank)
-int stage_round(ml_pcs_shard* sh, PcsRank& r, int k) {
+int stage_round(ShardCore* sh, PeerRank& r, int k) {
     MLB_CUDA(cudaSetDevice(r.device));
-    cudaStream_t s = r.st.main;
-    const Layout& a = sh->lay;
     const int cnt = (sh->world * sh->world) >> (k + 1);
-    pcs_shard_top_kernel<<<1, 32, 0, s>>>(sh->grp.flags(r, PR0 + k), sh->world, sh->grp.epoch, sh->grp.timeout_ns, sh->grp.status(r), r.arena + a.mail[k], cnt,
-                                          r.arena + a.top[k]);
-    MLB_KERNEL_CHECK();
-    const uint8_t* root = r.arena + a.top[k] + 32 * merkle_layer_offset((size_t)cnt, ilog2((size_t)cnt));
-    return chain_sumcheck_finish_launch(at(r, mail_partials(a, k)), sh->world, at(r, a.prev), (DevTranscript*)(r.arena + a.tr), root, 32,
-                                        r.arena + a.roots_out + 32 * k, at(r, a.sc) + 2 * k, at(r, a.r), s);
+    MLB_TRY(top_launch(sh, r, PR0 + k, k, cnt));
+    return finish_launch(sh, r, k, r.arena + sh->lay.top[k] + 32 * merkle_layer_offset((size_t)cnt, ilog2((size_t)cnt)));
 }
-// round k, phase C: fold tables and code; after the last sharded round, hand layer L and the tables to rank 0
-int stage_fold(ml_pcs_shard* sh, PcsRank& r, int k, int* nb) {
-    MLB_CUDA(cudaSetDevice(r.device));
+fe* fold_target(ShardCore* sh, PeerRank& r, int k) {
+    if (k + 1 == sh->L) return reinterpret_cast<fe*>(sh->grp.base[0] + sh->lay.tail_code) + (size_t)r.rank * sh->R;
+    return at(r, sh->lay.layer[k + 1]);
+}
+int fold_tables(ShardCore* sh, PeerRank& r, int k, int* nb) {
     cudaStream_t s = r.st.main;
     const Layout& a = sh->lay;
-    const int log_N = (int)sh->n_vars + ML_LOG_BLOWUP;
-    const RootTables* rt;
-    MLB_TRY(get_root_tables(r.ctx, log_N, s, &rt));
-    const size_t h = sh->nloc >> k, segs = (size_t)sh->world >> (k + 1);
-    const bool last = k + 1 == sh->L;
-    fe* out = last ? reinterpret_cast<fe*>(sh->grp.base[0] + a.tail_code) + (size_t)r.rank * sh->R : at(r, a.layer[k + 1]);
-    pcs_shard_fold_kernel<<<peer_grid(segs * sh->R), 256, 0, s>>>(at(r, a.layer[k]), segs, sh->R, sh->NL, r.rank, k, log_N, at(r, a.r), rt->lo, rt->hi, out);
-    MLB_KERNEL_CHECK();
-    if (!last) return sumcheck_fold_sums_launch(at(r, a.m), at(r, a.d), h, at(r, a.r), at(r, a.part), nb, s);  // h >= 4 here
+    const size_t h = sh->nloc >> k;
+    if (k + 1 < sh->L) return sumcheck_fold_sums_launch(at(r, a.m), at(r, a.d), h, at(r, a.r), at(r, a.part), nb, s);  // h >= 4 here
     MLB_TRY(sumcheck_fold_launch(at(r, a.m), at(r, a.d), h, 0, at(r, a.r), s));
     pcs_shard_gather_tables_kernel<<<peer_grid(h / 2), 256, 0, s>>>(at(r, a.m), at(r, a.d), h / 2, r.rank, sh->world,
                                                                    reinterpret_cast<fe*>(sh->grp.base[0] + a.tail_m), reinterpret_cast<fe*>(sh->grp.base[0] + a.tail_d));
     MLB_KERNEL_CHECK();
     return peer_signal(sh->grp, r, PG, 0, s);
 }
+// round k, phase C: fold tables and code; after the last sharded round, hand layer L and the tables to rank 0
+int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    cudaStream_t s = r.st.main;
+    const Layout& a = sh->lay;
+    const int log_N = (int)sh->n_vars + ML_LOG_BLOWUP;
+    const RootTables* rt;
+    MLB_TRY(get_root_tables(r.ctx, log_N, s, &rt));
+    const size_t segs = (size_t)sh->world >> (k + 1);
+    pcs_shard_fold_kernel<<<peer_grid(segs * sh->R), 256, 0, s>>>(at(r, a.layer[k]), segs, sh->R, sh->NL, r.rank, k, log_N, at(r, a.r), rt->lo, rt->hi,
+                                                                  fold_target(sh, r, k));
+    MLB_KERNEL_CHECK();
+    return fold_tables(sh, r, k, nb);
+}
+
+int open_sharded(ShardCore* sh, PeerRank& r0, const std::vector<size_t>& idx, int j0, std::vector<uint8_t>& host, int* stride) {
+    cudaStream_t s = r0.st.main;
+    const int L = sh->L;
+    const size_t nq = idx.size();
+    OpenArgs oa;
+    memset(&oa, 0, sizeof oa);
+    oa.stride = *stride = 32 + 32 * 64;
+    if (j0 >= L) return ML_OK;
+    for (int j = 0; j < L; j++) { oa.off_layer[j] = sh->lay.layer[j]; oa.off_dig[j] = sh->lay.dig[j]; oa.top[j] = r0.arena + sh->lay.top[j]; }
+    oa.n = sh->n; oa.NL = sh->NL; oa.R = sh->R; oa.L = L; oa.j0 = j0; oa.world = sh->world; oa.log_R = (int)ilog2(sh->R);
+    std::vector<unsigned long long> idx64(idx.begin(), idx.end());
+    Scratch didx(s), dout(s);
+    MLB_TRY(didx.alloc(nq * 8));
+    MLB_TRY(dout.alloc(nq * L * (size_t)oa.stride));
+    MLB_TRY(h2d(didx.p, idx64.data(), nq * 8, s));
+    pcs_shard_open_kernel<<<dim3((unsigned)nq, (unsigned)(L - j0)), 64, 0, s>>>(didx.as<unsigned long long>(), sh->grp.peers(), oa, dout.as<uint8_t>());
+    MLB_KERNEL_CHECK();
+    host.resize(nq * L * (size_t)oa.stride);
+    return d2h_sync(host.data(), dout.p, host.size(), s);
+}
+
+int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, hfe* sumcheck, uint8_t* roots_lo, ml_transcript* t, int mark_base) {
+    MLB_CUDA(cudaSetDevice(r0.device));
+    cudaStream_t s = r0.st.main;
+    const Layout& a = sh->lay;
+    const int L = sh->L;
+    if (L > 0) MLB_TRY(peer_wait(sh->grp, r0, PG, -1, s));
+    if (&r0 == &sh->local[0]) mark_phase(sh, mark_base);
+    f->log_n0 = (int)sh->n_vars + ML_LOG_BLOWUP;
+    f->stream = s;
+    if (!hooks.first_fold) MLB_TRY(fri_push_layer(f, at(r0, a.tail_code), sh->NL, false, s, true));  // layer L, committed, root not absorbed yet
+    ml_sumcheck sc;  // tables in the arena: not freed by the chain
+    sc.matrix = at(r0, a.tail_m);
+    sc.delta = at(r0, a.tail_d);
+    sc.owns_matrix = false;
+    sc.height = sh->nloc;
+    sc.stream = s;
+    ChainHooks h = hooks;
+    h.tr_dev = (const DevTranscript*)(r0.arena + a.tr);
+    h.prev_dev = at(r0, a.prev);
+    MLB_TRY(fold_chain_dev(r0.ctx, f, &h, &sc, 0, sumcheck + 2 * L, (size_t)L, !hooks.first_fold, t, s));
+    if (&r0 == &sh->local[0]) mark_phase(sh, mark_base + 1);
+    if (L > 0) {  // sumcheck (c1, c2) and layer roots of the sharded rounds
+        uint8_t lo[MAX_L * 32];
+        MLB_CUDA(cudaMemcpyAsync(lo, r0.arena + a.sc, (size_t)L * 32, cudaMemcpyDeviceToHost, s));
+        MLB_TRY(d2h_sync(roots_lo, r0.arena + a.roots_out, (size_t)L * 32, s));
+        for (int i = 0; i < 2 * L; i++) sumcheck[i] = hfe_load(lo + 16 * i);
+    }
+    return peer_read_status(sh->grp, r0, sh->who);
+}
+
+int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t) {
+    if (sh->world == 1) return ML_OK;
+    cudaStream_t s = r0.st.main;
+    Scratch trd(s);
+    MLB_TRY(trd.alloc(128));
+    MLB_TRY(h2d(trd.p, &t->sha, sizeof(DevTranscript), s));
+    MLB_TRY(peer_push(sh->grp, r0, trd.p, (int)(sizeof(DevTranscript) + 15) / 16 * 16, sh->lay.final_tr, PF, -1, s));
+    return stream_wait_blocking(s);
+}
+
+// ranks other than 0: wait for the end of the proof (their buffers are read by rank 0's openings until then)
+int finish_ranks(ShardCore* sh, ml_transcript* t, int st) {
+    for (auto& r : sh->local) {
+        if (r.rank == 0) continue;
+        MLB_CUDA(cudaSetDevice(r.device));
+        MLB_TRY(peer_wait(sh->grp, r, PF, 0, r.st.main));
+        int s1 = peer_read_status(sh->grp, r, sh->who);
+        if (s1 != ML_OK) { st = s1; continue; }
+        if (!rank0_of(sh)) {  // another process holds rank 0: adopt its final transcript
+            HostSha256 fin;
+            MLB_TRY(d2h_sync(&fin, r.arena + sh->lay.final_tr, sizeof(DevTranscript), r.st.main));
+            t->sha = fin;
+        }
+    }
+    return st;
+}
+
+}  // namespace mlbs
+
+namespace {
+
+const char* WHO = "ml_pcs_shard";
 
 // openings and the proof on rank 0 (:113-129): layers < L from the owners' arenas, layers >= L from the tail's FriProverData
-int assemble(ml_pcs_shard* sh, PcsRank& r0, const ml_fri* f, ml_transcript* t, ml_fri_proof* p, const uint8_t* roots_lo) {
+int assemble(ml_pcs_shard* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_fri_proof* p, const uint8_t* roots_lo) {
     cudaStream_t s = r0.st.main;
     const int L = sh->L;
     std::vector<size_t> idx;
     derive_indices(t, 2 * sh->n, idx);
     const size_t nq = idx.size();
     std::vector<uint8_t> host;
-    OpenArgs oa;
-    memset(&oa, 0, sizeof oa);
-    oa.stride = 32 + 32 * 64;
-    if (L > 0) {
-        for (int j = 0; j < L; j++) { oa.off_layer[j] = sh->lay.layer[j]; oa.off_dig[j] = sh->lay.dig[j]; oa.top[j] = r0.arena + sh->lay.top[j]; }
-        oa.n = sh->n; oa.NL = sh->NL; oa.R = sh->R; oa.L = L; oa.world = sh->world; oa.log_R = (int)ilog2(sh->R);
-        std::vector<unsigned long long> idx64(idx.begin(), idx.end());
-        Scratch didx(s), dout(s);
-        MLB_TRY(didx.alloc(nq * 8));
-        MLB_TRY(dout.alloc(nq * L * (size_t)oa.stride));
-        MLB_TRY(h2d(didx.p, idx64.data(), nq * 8, s));
-        pcs_shard_open_kernel<<<dim3((unsigned)nq, (unsigned)L), 64, 0, s>>>(didx.as<unsigned long long>(), sh->grp.peers(), oa, dout.as<uint8_t>());
-        MLB_KERNEL_CHECK();
-        host.resize(nq * L * (size_t)oa.stride);
-        MLB_TRY(d2h_sync(host.data(), dout.p, host.size(), s));
-    }
+    int stride = 0;
+    MLB_TRY(open_sharded(sh, r0, idx, 0, host, &stride));
     std::vector<size_t> sub(nq);
     for (size_t q = 0; q < nq; q++) sub[q] = idx[q] % (sh->n >> L);
     std::vector<QueryH> qs;
@@ -442,7 +578,7 @@ int assemble(ml_pcs_shard* sh, PcsRank& r0, const ml_fri* f, ml_transcript* t, m
         std::vector<PathH>& paths = p->queries[q].paths;
         paths.resize(L);
         for (int j = 0; j < L; j++) {
-            const uint8_t* rec = host.data() + (q * L + j) * (size_t)oa.stride;
+            const uint8_t* rec = host.data() + (q * L + j) * (size_t)stride;
             const int depth = (int)ilog2(sh->n >> j);
             paths[j].value.assign(rec, rec + 32);
             paths[j].digests.assign(rec + 32, rec + 32 + 32 * (size_t)depth);
@@ -458,59 +594,22 @@ int assemble(ml_pcs_shard* sh, PcsRank& r0, const ml_fri* f, ml_transcript* t, m
 }
 
 // rank 0: the rest of the fold chain from layer L, the openings, the final transcript to everybody
-int prove_tail(ml_pcs_shard* sh, PcsRank& r0, const uint8_t* inputs, const uint8_t* output, ml_transcript* t, ml_pcs_proof** out) {
-    MLB_CUDA(cudaSetDevice(r0.device));
-    cudaStream_t s = r0.st.main;
-    const Layout& a = sh->lay;
-    const int L = sh->L;
-    if (L > 0) MLB_TRY(peer_wait(sh->grp, r0, PG, -1, s));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 3);
+int prove_tail(ml_pcs_shard* sh, PeerRank& r0, const uint8_t* inputs, const uint8_t* output, ml_transcript* t, ml_pcs_proof** out) {
     ml_fri* f = new ml_fri();
-    f->log_n0 = (int)sh->n_vars + ML_LOG_BLOWUP;
-    f->stream = s;
     struct FriGuard { ml_fri* p; ~FriGuard() { free_fri(p); } } fri_guard{f};
-    MLB_TRY(fri_push_layer(f, at(r0, a.tail_code), sh->NL, false, s, true));  // layer L, committed, root not absorbed yet
-    ml_sumcheck sc;  // tables in the arena: not freed by the chain
-    sc.matrix = at(r0, a.tail_m);
-    sc.delta = at(r0, a.tail_d);
-    sc.owns_matrix = false;
-    sc.height = sh->nloc;
-    sc.stream = s;
-    ChainHooks hooks;
-    hooks.tr_dev = (const DevTranscript*)(r0.arena + a.tr);
-    hooks.prev_dev = at(r0, a.prev);
     ml_pcs_proof* p = new ml_pcs_proof();
     std::unique_ptr<ml_pcs_proof> guard(p);
     p->sumcheck.resize(2 * sh->n_vars);
-    MLB_TRY(fold_chain_dev(r0.ctx, f, &hooks, &sc, 0, p->sumcheck.data() + 2 * L, (size_t)L, true, t, s));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 4);
-    uint8_t lo[MAX_L * 32 * 2];  // sumcheck (c1, c2) and layer roots of the sharded rounds
-    if (L > 0) {
-        MLB_CUDA(cudaMemcpyAsync(lo, r0.arena + a.sc, (size_t)L * 32, cudaMemcpyDeviceToHost, s));
-        MLB_TRY(d2h_sync(lo + MAX_L * 32, r0.arena + a.roots_out, (size_t)L * 32, s));
-        for (int i = 0; i < 2 * L; i++) p->sumcheck[i] = hfe_load(lo + 16 * i);
-    }
-    MLB_TRY(peer_read_status(sh->grp, r0, WHO));
-    MLB_TRY(assemble(sh, r0, f, t, &p->fri, lo + MAX_L * 32));
+    uint8_t roots_lo[MAX_L * 32];
+    MLB_TRY(tail_chain(sh, r0, f, ChainHooks(), p->sumcheck.data(), roots_lo, t, 3));
+    MLB_TRY(assemble(sh, r0, f, t, &p->fri, roots_lo));
     if (&r0 == &sh->local[0]) mark_phase(sh, 5);
     p->inputs.resize(sh->n_vars);
     for (size_t i = 0; i < sh->n_vars; i++) p->inputs[i] = hfe_load(inputs + 16 * i);
     p->output = hfe_load(output);
-    if (sh->world > 1) {  // final transcript to everybody; also releases the other ranks' buffers for the next call
-        Scratch trd(s);
-        MLB_TRY(trd.alloc(128));
-        MLB_TRY(h2d(trd.p, &t->sha, sizeof(DevTranscript), s));
-        MLB_TRY(peer_push(sh->grp, r0, trd.p, (int)(sizeof(DevTranscript) + 15) / 16 * 16, a.final_tr, PF, -1, s));
-        MLB_TRY(stream_wait_blocking(s));
-    }
+    MLB_TRY(tail_release(sh, r0, t));  // also releases the other ranks' buffers for the next call
     *out = guard.release();
     return ML_OK;
-}
-
-PcsRank* rank0_of(ml_pcs_shard* sh) {
-    for (auto& r : sh->local)
-        if (r.rank == 0) return &r;
-    return nullptr;
 }
 
 }  // namespace
@@ -526,27 +625,7 @@ int ml_pcs_shard_create(int world, int n_local, const int* local_ranks, const in
     }
     DeviceGuard guard;
     ml_pcs_shard* sh = new ml_pcs_shard();
-    sh->world = world; sh->L = L; sh->n_vars = n_vars; sh->n = (size_t)1 << n_vars;
-    sh->NL = 2 * sh->n / world; sh->R = sh->NL / world; sh->nloc = sh->n / world;
-    sh->lay = make_layout(sh->n, world);
-    sh->grp.world = world;
-    sh->grp.arena_bytes = sh->lay.total;
-    sh->grp.off_flags = sh->lay.flags;
-    sh->grp.off_status = sh->lay.status;
-    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
-    int st = ML_OK;
-    for (int i = 0; i < n_local && st == ML_OK; i++) {
-        PcsRank r;
-        r.rank = local_ranks[i];
-        r.device = local_devices[i];
-        st = peer_rank_init(sh->grp, r, "ml_pcs_shard_create", sh->lay.ycode);
-        if (st == ML_OK || st == ML_ERR_ALLOC) sh->local.push_back(r);
-    }
-    if (st == ML_OK && n_local == world) {
-        std::vector<PeerRank*> ranks;
-        for (auto& r : sh->local) ranks.push_back(&r);
-        st = peer_link_local(sh->grp, ranks, "ml_pcs_shard_create");
-    }
+    int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, 0, "ml_pcs_shard_create");
     if (st != ML_OK) { ml_pcs_shard_free(sh); return st; }
     *out = sh;
     return ML_OK;
@@ -554,45 +633,19 @@ int ml_pcs_shard_create(int world, int n_local, const int* local_ranks, const in
 
 void ml_pcs_shard_free(ml_pcs_shard* sh) {
     if (!sh) return;
-    DeviceGuard guard;
-    for (int i = 0; i < ml_pcs_shard::N_MARKS; i++)
-        if (sh->mark[i]) cudaEventDestroy(sh->mark[i]);
-    for (auto& r : sh->local) {
-        cudaSetDevice(r.device);
-        cudaDeviceSynchronize();
-        peer_rank_free(r);
-    }
-    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
+    shard_free(sh);
     delete sh;
 }
 
-int ml_pcs_shard_export(ml_pcs_shard* sh, uint8_t* records_out) {
-    std::vector<PeerRank*> ranks;
-    for (auto& r : sh->local) ranks.push_back(&r);
-    return peer_export(ranks, records_out);
-}
-int ml_pcs_shard_connect(ml_pcs_shard* sh, const uint8_t* records, size_t n_records) {
-    if (sh->local.size() != 1) { set_error("ml_pcs_shard_connect: only for handles that host one rank"); return ML_ERR_ARG; }
-    return peer_connect(sh->grp, sh->local[0], records, n_records, "ml_pcs_shard_connect");
-}
-void* ml_pcs_shard_stream(const ml_pcs_shard* sh, int local_index) {
-    if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
-    return (void*)sh->local[local_index].st.main;
-}
+int ml_pcs_shard_export(ml_pcs_shard* sh, uint8_t* records_out) { return shard_export(sh, records_out); }
+int ml_pcs_shard_connect(ml_pcs_shard* sh, const uint8_t* records, size_t n_records) { return shard_connect(sh, records, n_records, "ml_pcs_shard_connect"); }
+void* ml_pcs_shard_stream(const ml_pcs_shard* sh, int local_index) { return shard_stream(sh, local_index); }
 size_t ml_pcs_shard_arena_bytes(const ml_pcs_shard* sh) { return sh->lay.total; }
 
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: [S0 encode + exchange + tables, S1 combine, sharded rounds, tail chain, openings] (the last two
 // on rank 0 only).  Returns the count.
-int ml_pcs_shard_phase_ms(const ml_pcs_shard* sh, double* out, int cap) {
-    int n = 0;
-    for (int i = 0; i + 1 < sh->n_marks && n < cap; i++) {
-        float ms = 0;
-        if (!sh->mark[i] || !sh->mark[i + 1] || cudaEventElapsedTime(&ms, sh->mark[i], sh->mark[i + 1]) != cudaSuccess) { cudaGetLastError(); ms = -1.f; }
-        out[n++] = ms;
-    }
-    return n;
-}
+int ml_pcs_shard_phase_ms(const ml_pcs_shard* sh, double* out, int cap) { return shard_phase_ms(sh, out, cap); }
 
 // PCSProof::prove (multilinear_pcs.rs:90-136).  Every process calls it with the same claim and its own transcript copy; the proof
 // comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the same state.
@@ -626,20 +679,8 @@ int ml_pcs_shard_prove_dev(ml_pcs_shard* sh, const uint8_t* inputs, size_t n_var
         mark_phase(sh, 2);
     }
     int st = ML_OK;
-    if (PcsRank* r0 = rank0_of(sh)) st = prove_tail(sh, *r0, inputs, output, t, out);
-    // ranks other than 0: wait for the end of the proof (their buffers are read by rank 0's openings until then)
-    for (auto& r : sh->local) {
-        if (r.rank == 0) continue;
-        MLB_CUDA(cudaSetDevice(r.device));
-        MLB_TRY(peer_wait(sh->grp, r, PF, 0, r.st.main));
-        int s1 = peer_read_status(sh->grp, r, WHO);
-        if (s1 != ML_OK) { st = s1; continue; }
-        if (!rank0_of(sh)) {  // another process holds rank 0: adopt its final transcript
-            HostSha256 fin;
-            MLB_TRY(d2h_sync(&fin, r.arena + sh->lay.final_tr, sizeof(DevTranscript), r.st.main));
-            t->sha = fin;
-        }
-    }
+    if (PeerRank* r0 = rank0_of(sh)) st = prove_tail(sh, *r0, inputs, output, t, out);
+    st = finish_ranks(sh, t, st);
     if (st != ML_OK && *out) { ml_pcs_proof_free(*out); *out = nullptr; }
     return st;
 }
@@ -653,7 +694,7 @@ int ml_pcs_shard_prove(ml_pcs_shard* sh, const uint8_t* inputs, size_t n_vars, c
     std::vector<void*> dev(sh->local.size(), nullptr);
     int st = ML_OK;
     for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        PcsRank& r = sh->local[i];
+        PeerRank& r = sh->local[i];
         if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
         st = pmalloc(&dev[i], sh->nloc * 16, r.st.main);
         if (st == ML_OK) st = h2d(dev[i], evals + (size_t)r.rank * sh->nloc * 16, sh->nloc * 16, r.st.main);

@@ -1,0 +1,102 @@
+// Stages of the block-sharded PCS provers, shared by pcs_shard.cu (one PCSProof::prove, ml_pcs_shard_*) and bpcs_shard.cu
+// (one BatchedPCSProof::prove, ml_bpcs_shard_*).  Both split every polynomial by block over G ranks and keep the sharded layers
+// in the segment layout described at the top of pcs_shard.cu; the batched prover only adds a batched layer 0 and round 0.
+#pragma once
+#include "peer.h"
+#include "prover_internal.h"
+
+namespace mlbs {
+using namespace mlb;
+using namespace mlbp;
+
+enum Phase { PX = 0, PR0 = 1, PG = PR0 + 4, PF, PB, PT, N_PHASES };  // PR0 + k: round k (L <= 4); PB, PT: batched prover only
+static const int MAXR = PEER_MAXR;
+static const int MAX_L = 4;
+static const size_t MAIL_ROOTS = (size_t)MAXR * MAXR / 2;  // run roots of layer 0 at G = ML_MAX_PEERS
+
+struct Layout {
+    size_t flags, status, tr, prev, r, sc, roots_out, final_tr, mail[MAX_L], top[MAX_L], part;  // mailbox (cleared at create)
+    size_t rho, outs, eptrs, segptrs;                                                          // batched prover only
+    size_t ycode, recv, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;
+};
+// B = 0: one polynomial; B >= 1: a batch of B polynomials (layer 0 holds B codes)
+Layout make_layout(size_t n, int G, size_t B);
+// mailbox of round k: run root of run q at roots + 32 q, partial pair of rank g at partials + 32 g
+inline size_t mail_partials(const Layout& a, int k) { return a.mail[k] + MAIL_ROOTS * 32; }
+
+struct ShardCore {
+    int world = 1, L = 0;
+    size_t n_vars = 0, n = 0, NL = 0, R = 0, nloc = 0, B = 0;
+    const char* who = "ml_pcs_shard";  // prefix of error messages
+    Layout lay;
+    std::vector<PeerRank> local;
+    PeerGroup grp;
+    // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
+    static const int N_MARKS = 8;
+    cudaEvent_t mark[N_MARKS] = {nullptr};
+    int n_marks = 0;
+};
+
+inline fe* at(const PeerRank& r, size_t off) { return reinterpret_cast<fe*>(r.arena + off); }
+void mark_phase(ShardCore* sh, int idx);
+PeerRank* rank0_of(ShardCore* sh);
+
+// handle plumbing (arguments already checked by the caller)
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who);
+void shard_free(ShardCore* sh);
+int shard_export(ShardCore* sh, uint8_t* records_out);
+int shard_connect(ShardCore* sh, const uint8_t* records, size_t n_records, const char* who);
+void* shard_stream(const ShardCore* sh, int local_index);
+int shard_phase_ms(const ShardCore* sh, double* out, int cap);
+
+// S0 exchange: slice r of the local code `ycode` -> rank r's recv at off_recv (G > 1)
+int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s);
+// cyclic transpose of a local table of nloc entries into the owners' tables at off_m
+int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s);
+// the rank's eq table: eq over all variables (G = 1) or the local part times the rank's factor for the top L variables
+int local_eq_table(ShardCore* sh, PeerRank& r, const std::vector<hfe>& pts, fe* d, cudaStream_t s);
+int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s);
+// run roots of `segs` segment subtrees (digests at dig, segment p at 32 * p * 2 R) -> every rank's mailbox at off_roots, and
+// (nb >= 0) the rank's partial sums from its CTA partials -> off_partials; then flag `phase` there
+int post_launch(ShardCore* sh, PeerRank& r, const uint8_t* dig, size_t R, int segs, int nb, size_t off_roots, size_t off_partials, int phase);
+// wait for `phase` from every rank, then hash the top of a tree over cnt run roots of mailbox k into top[k]
+int top_launch(ShardCore* sh, PeerRank& r, int phase, int k, int cnt);
+// round polynomial of round k from the posted partial sums (absorbing `root` first if given), challenge r_k, claim update
+int finish_launch(ShardCore* sh, PeerRank& r, int k, const uint8_t* root);
+
+// sharded round k >= 0 of a single code layer: A (subtrees + post), B (top + transcript), C (folds)
+int stage_post(ShardCore* sh, PeerRank& r, int k, int nb);
+int stage_round(ShardCore* sh, PeerRank& r, int k);
+int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb);
+// where round k writes its fold: layer k+1 in the segment layout, or rank 0's tail code after the last sharded round
+fe* fold_target(ShardCore* sh, PeerRank& r, int k);
+// fold of the tables of round k; after the last sharded round, hand the tables to rank 0 and flag PG
+int fold_tables(ShardCore* sh, PeerRank& r, int k, int* nb);
+
+// rank 0: the fold chain from layer L (first_fold: a batched round 0 at G = 1), sumcheck coefficients and roots of the sharded
+// rounds (sumcheck: 2 * n_vars, roots_lo: 32 * L); marks mark_base and mark_base + 1
+int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, hfe* sumcheck, uint8_t* roots_lo, ml_transcript* t, int mark_base);
+// rank 0: records (value pair | path) of layers j0 .. L-1 for every query index, from the owners' arenas; record (q, j) at
+// (q * L + j) * *stride
+int open_sharded(ShardCore* sh, PeerRank& r0, const std::vector<size_t>& idx, int j0, std::vector<uint8_t>& host, int* stride);
+// rank 0: final transcript to every rank (releases their buffers); the other local ranks wait for it and adopt it
+int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t);
+int finish_ranks(ShardCore* sh, ml_transcript* t, int st);
+
+// segment-layout helpers on the device
+__device__ __forceinline__ int ilog2_dev(size_t x) { return 63 - __clzll((unsigned long long)x); }
+// merkle_layer_offset on the device: layer l of a tree with n leaves starts at digest 2n - (2n >> l)
+__device__ __forceinline__ size_t layer_off(size_t n_leaves, int layer) { return 2 * n_leaves - ((2 * n_leaves) >> layer); }
+__device__ __forceinline__ fe root_pow(const fe* __restrict__ lo, const fe* __restrict__ hi, size_t e) {
+    fe w = fe_load_nc(lo + (e & (((size_t)1 << LO_BITS) - 1)));
+    if (e >> LO_BITS) w = fe_mul(w, fe_load_nc(hi + (e >> LO_BITS)));
+    return w;
+}
+// position of element j of run p in a layer with `runs` runs per rank (segment layout; one run: plain)
+__device__ __forceinline__ size_t run_pos(size_t runs, size_t p, size_t j, size_t R) {
+    if (runs == 1) return j;
+    const size_t half = runs >> 1;
+    return (p & (half - 1)) * 2 * R + (p >= half ? R : 0) + j;
+}
+
+}  // namespace mlbs

@@ -149,11 +149,8 @@ __global__ void __launch_bounds__(32) shard_root_kernel(const unsigned long long
     for (int i = 0; i < 32; i++) root_out[i] = root[i];
     if (!with_transcript) return;
     DevTranscript tr = *tr_in;
-    dt_absorb(&tr, root, 32);
-    fe rho = dt_challenge(&tr);
-    dt_absorb_fe(&tr, rho);
-    fe acc = fe_zero();
-    for (int j = 0; j < n_outputs; j++) acc = fe_add(fe_mul(acc, rho), fe_load(outputs + j));
+    fe rho;
+    const fe acc = dt_batch_root(&tr, root, outputs, n_outputs, &rho);
     fe_store(fr_out, rho);
     fe_store(prev_out, acc);
     *tr_out = tr;

@@ -76,4 +76,16 @@ __device__ inline fe dt_challenge(const DevTranscript* t) {
     return fe_new(fe{{sha_bswap(st[0]), sha_bswap(st[1]), sha_bswap(st[2]), sha_bswap(st[3])}});
 }
 
+// BatchedFriProverData::init after the batch tree (batched_fri.rs:80-86) and the claim of BatchedPCSProof::prove
+// (batched_pcs.rs:92-94): absorb the batch root, draw rho = fingerprint_r and absorb it; returns fingerprint(rho, outputs)
+__device__ inline fe dt_batch_root(DevTranscript* t, const uint8_t* root, const fe* outputs, int n_outputs, fe* rho_out) {
+    dt_absorb(t, root, 32);
+    const fe rho = dt_challenge(t);
+    dt_absorb_fe(t, rho);
+    fe acc = fe_zero();
+    for (int j = 0; j < n_outputs; j++) acc = fe_add(fe_mul(acc, rho), fe_load(outputs + j));
+    *rho_out = rho;
+    return acc;
+}
+
 }  // namespace mlb

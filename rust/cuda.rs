@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -61,6 +61,14 @@ extern "C" {
     pub fn ml_bpcs_proof_fri(p: *const MlBpcsProof) -> *const MlBfriProof;
     pub fn ml_bpcs_proof_num_rounds(p: *const MlBpcsProof) -> usize;
     pub fn ml_bpcs_proof_sumcheck_coeffs(p: *const MlBpcsProof, out: *mut u8) -> c_int;
+    pub fn ml_bpcs_shard_arena_bytes(sh: *const MlBpcsShard) -> usize;
+    pub fn ml_bpcs_shard_connect(sh: *mut MlBpcsShard, records: *const u8, n_records: usize) -> c_int;
+    pub fn ml_bpcs_shard_create(world: c_int, n_local: c_int, local_ranks: *const c_int, local_devices: *const c_int, n_polys: usize, n_vars: usize, out: *mut *mut MlBpcsShard) -> c_int;
+    pub fn ml_bpcs_shard_export(sh: *mut MlBpcsShard, records_out: *mut u8) -> c_int;
+    pub fn ml_bpcs_shard_free(sh: *mut MlBpcsShard);
+    pub fn ml_bpcs_shard_prove(sh: *mut MlBpcsShard, inputs: *const u8, n_vars: usize, outputs: *const u8, n_polys: usize, evals: *const *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlBpcsProof) -> c_int;
+    pub fn ml_bpcs_shard_prove_dev(sh: *mut MlBpcsShard, inputs: *const u8, n_vars: usize, outputs: *const u8, n_polys: usize, local_evals_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlBpcsProof) -> c_int;
+    pub fn ml_bpcs_shard_stream(sh: *const MlBpcsShard, local_index: c_int) -> *mut c_void;
     pub fn ml_delta_evaluate(data: *const u8, points: *const u8, n: usize, out: *mut u8) -> c_int;
     pub fn ml_dev_alloc(bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn ml_dev_download(dst_host: *mut c_void, src_dev: *const c_void, bytes: usize) -> c_int;
@@ -701,22 +709,31 @@ pub fn batched_pcs_prove(claim: BatchedPCSClaim<F>, poly: &[MultilinearPolynomia
 
 /// `BatchedPCSProof::prove` over all GPUs of the box from ONE process (ml_shard_*, csrc/shard.cu): the polynomials are encoded where
 /// they land (j mod G), leaves are hashed by leaf range, the exchange is NVLink stores between the GPUs' arenas.  The handle is
-/// built once per shape (n_polys, n_vars) and reused; the proof bytes equal `batched_pcs_prove`'s.
+/// built once per shape (n_polys, n_vars) and reused; the proof bytes equal `batched_pcs_prove`'s.  Shapes that ml_shard_* cannot
+/// split by polynomial (the chosen world is not a power of two or does not divide n_polys) go to `BlockShardedBatchedProver`.
 pub struct ShardedBatchedProver {
     h: *mut MlShard,
+    block: Option<BlockShardedBatchedProver>,
 }
 impl ShardedBatchedProver {
     pub fn new(n_polys: usize, n_vars: usize) -> Self {
         let mut count = 0;
         check(unsafe { ml_device_count(&mut count) });
         let world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
-        let world = world.min(n_polys).min(16) as c_int;
+        let world = world.min(n_polys).min(16);
+        if !world.is_power_of_two() || n_polys % world != 0 {
+            return Self { h: std::ptr::null_mut(), block: Some(BlockShardedBatchedProver::new(n_polys, n_vars)) };
+        }
+        let world = world as c_int;
         let ids: Vec<c_int> = (0..world).collect();
         let mut h = std::ptr::null_mut();
         check(unsafe { ml_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), n_polys, n_vars, &mut h) });
-        Self { h }
+        Self { h, block: None }
     }
     pub fn prove(&mut self, claim: BatchedPCSClaim<F>, poly: &[MultilinearPolynomialEvals<F>], transcript: &mut Transcript) -> BatchedPCSProof<F> {
+        if let Some(b) = self.block.as_mut() {
+            return b.prove(claim, poly, transcript);
+        }
         let ptrs: Vec<*const u8> = poly.iter().map(|m| p(&m.evals)).collect();
         let mut h = std::ptr::null_mut();
         check(unsafe {
@@ -727,7 +744,45 @@ impl ShardedBatchedProver {
 }
 impl Drop for ShardedBatchedProver {
     fn drop(&mut self) {
-        unsafe { ml_shard_free(self.h) }
+        if !self.h.is_null() {
+            unsafe { ml_shard_free(self.h) }
+        }
+    }
+}
+
+/// `BatchedPCSProof::prove` over all GPUs of the box from ONE process with every polynomial split by block (ml_bpcs_shard_*,
+/// csrc/bpcs_shard.cu): rank g holds evals_j[g*n/G, (g+1)*n/G) of every polynomial, so any n_polys >= 1 runs on every GPU.  The
+/// handle is built once per shape (n_polys, n_vars) and reused; the proof bytes equal `batched_pcs_prove`'s.
+pub struct BlockShardedBatchedProver {
+    h: *mut MlBpcsShard,
+}
+impl BlockShardedBatchedProver {
+    pub fn new(n_polys: usize, n_vars: usize) -> Self {
+        let mut count = 0;
+        check(unsafe { ml_device_count(&mut count) });
+        let mut world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
+        while world > 1 && n_vars < 2 * world.trailing_zeros() as usize {
+            world >>= 1; // n_vars >= 2 log2(world)
+        }
+        let world = world.min(16) as c_int;
+        let ids: Vec<c_int> = (0..world).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_bpcs_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), n_polys, n_vars, &mut h) });
+        Self { h }
+    }
+    pub fn prove(&mut self, claim: BatchedPCSClaim<F>, poly: &[MultilinearPolynomialEvals<F>], transcript: &mut Transcript) -> BatchedPCSProof<F> {
+        let ptrs: Vec<*const u8> = poly.iter().map(|m| p(&m.evals)).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe {
+            ml_bpcs_shard_prove(self.h, p(&claim.inputs), claim.inputs.len(), p(&claim.outputs), poly.len(), ptrs.as_ptr(), poly[0].evals.len(),
+                                transcript.h, &mut h)
+        });
+        unsafe { bpcs_proof_from(h, claim) }
+    }
+}
+impl Drop for BlockShardedBatchedProver {
+    fn drop(&mut self) {
+        unsafe { ml_bpcs_shard_free(self.h) }
     }
 }
 
