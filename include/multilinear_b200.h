@@ -373,6 +373,38 @@ int ml_bpcs_shard_prove_dev(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_v
 int ml_bpcs_shard_prove(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
                         const uint8_t *const *evals, size_t n, ml_transcript *t, ml_bpcs_proof **out);
 
+/* ---- the width-w System sumcheck sharded over the GPUs of one box (SumcheckTables::compute_sumcheck_polynomials,
+ * src/constraint_system/sumcheck.rs:147-202) ----
+ * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; rank b holds the contiguous row block matrix[b*h/G, (b+1)*h/G) of the
+ * row-major [h][width] trace (at width 1 the block ml_pcs_shard_prove_dev takes).  The rows go to CYCLIC tables (rank g owns rows
+ * i = g mod G), so every fold pair is local and the single-GPU round kernels run on each rank; each round's td point sums are
+ * exchanged through the arenas, the round polynomial and challenge are computed identically on every rank, and once the tables
+ * have 2^12 rows they are all-gathered and every rank runs the last rounds itself (csrc/wsumcheck_shard.cu).  Rank r holds about
+ * (width + 1) * 16 * h / G bytes of tables; the caller's blocks are only read (they stay valid for a following PCS call).
+ * One call computes exactly what ml_wsumcheck_build + ml_wsumcheck_set_composition + ml_wsumcheck_compute_polynomials compute:
+ * every coefficient, every challenge and the final transcript, and EVERY process gets the whole result.
+ * Handles, records, calls and errors as for ml_pcs_shard_* above.  width 1..16; n_vars >= max(1, log2 G) (ML_ERR_SIZE below);
+ * composition_degree 0..3 (ML_ERR_ARG above); composition limits and errors as for ml_wsumcheck_set_composition. */
+typedef struct ml_wsumcheck_shard ml_wsumcheck_shard;
+int ml_wsumcheck_shard_create(int world, int n_local, const int *local_ranks, const int *local_devices, size_t width, size_t n_vars,
+                              ml_wsumcheck_shard **out);
+void ml_wsumcheck_shard_free(ml_wsumcheck_shard *sh);   /* multi-process: all ranks must have returned from their last call (caller's barrier) */
+int ml_wsumcheck_shard_export(ml_wsumcheck_shard *sh, uint8_t *records_out /* num_local * ml_shard_record_bytes() */);
+int ml_wsumcheck_shard_connect(ml_wsumcheck_shard *sh, const uint8_t *records, size_t n_records /* world */);
+void *ml_wsumcheck_shard_stream(const ml_wsumcheck_shard *sh, int local_index);  /* the local rank's main stream (for CUDA-event timing) */
+size_t ml_wsumcheck_shard_arena_bytes(const ml_wsumcheck_shard *sh);
+/* the composition, as for ml_wsumcheck_set_composition; uploaded to every local rank */
+int ml_wsumcheck_shard_set_composition(ml_wsumcheck_shard *sh, size_t n_terms, const uint8_t *coefs, const uint32_t *term_lens, const uint32_t *term_cols);
+/* local_blocks_dev[i]: local rank i's row block (device pointer, complete before the call).  Every process passes the same row
+ * point, sum and transcript copy; coeffs_out: n_vars * (composition_degree + 1) elements, randoms_out: n_vars */
+int ml_wsumcheck_shard_compute_polynomials_dev(ml_wsumcheck_shard *sh, const uint8_t *row_point, size_t n_vars, const void *const *local_blocks_dev,
+                                               size_t composition_degree, ml_transcript *t, const uint8_t sum[16], uint8_t *coeffs_out,
+                                               uint8_t *randoms_out);
+/* host rows (all height) and a handle that hosts every rank */
+int ml_wsumcheck_shard_compute_polynomials(ml_wsumcheck_shard *sh, const uint8_t *row_point, size_t n_vars, const uint8_t *matrix, size_t width,
+                                           size_t height, size_t composition_degree, ml_transcript *t, const uint8_t sum[16], uint8_t *coeffs_out,
+                                           uint8_t *randoms_out);
+
 /* ---- batched commit building blocks (round-1 API, kept): one rank's share of `Merkle::batch_commit`
  * (merkle_tree/mod.rs:110-131) over leaf range [leaf_begin, leaf_begin+leaf_count) of all codes.
  * codes_dev[j] points at code j's rows for this range laid out as pairs: leaf_count x 32 bytes.

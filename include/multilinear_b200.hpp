@@ -296,6 +296,45 @@ class SumcheckTables {
     SumcheckTables() = default;
     ml_wsumcheck* h_ = nullptr;
 };
+// the width-w sumcheck over several GPUs from one process (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu); `devices` may repeat
+// (virtual ranks).  The result equals SumcheckTables::build + set_composition + compute_sumcheck_polynomials exactly.
+class ShardedWideSumcheckTables {
+  public:
+    ShardedWideSumcheckTables(const std::vector<int>& devices, size_t width, size_t n_vars) : width_(width) {
+        std::vector<int> ranks(devices.size());
+        for (size_t i = 0; i < ranks.size(); i++) ranks[i] = (int)i;
+        check(ml_wsumcheck_shard_create((int)devices.size(), (int)devices.size(), ranks.data(), devices.data(), width, n_vars, &h_));
+    }
+    ShardedWideSumcheckTables(const ShardedWideSumcheckTables&) = delete;
+    ~ShardedWideSumcheckTables() { if (h_) ml_wsumcheck_shard_free(h_); }
+    void set_composition(const std::vector<CompositionTerm>& terms) {
+        std::vector<F> coefs;
+        std::vector<uint32_t> lens, cols;
+        for (auto& t : terms) {
+            coefs.push_back(t.coef);
+            lens.push_back((uint32_t)t.cols.size());
+            cols.insert(cols.end(), t.cols.begin(), t.cols.end());
+        }
+        if (cols.empty()) cols.push_back(0);
+        check(ml_wsumcheck_shard_set_composition(h_, terms.size(), raw(coefs), lens.data(), cols.data()));
+    }
+    // :147-172 of the trace `matrix` (row-major [2^n_vars][width]) at `row_point` — returns (polynomials, randoms)
+    std::pair<std::vector<SumcheckPolynomial>, std::vector<F>> compute_sumcheck_polynomials(const std::vector<F>& row_point, const std::vector<F>& matrix,
+                                                                                          size_t composition_degree, Transcript& t, F sum) {
+        const size_t rounds = row_point.size(), td = composition_degree + 1;
+        std::vector<F> coeffs(rounds * td + 1), randoms(rounds + 1);
+        check(ml_wsumcheck_shard_compute_polynomials(h_, raw(row_point), rounds, raw(matrix), width_, matrix.size() / width_, composition_degree, t.handle(),
+                                                     sum.bytes(), raw(coeffs), raw(randoms)));
+        std::vector<SumcheckPolynomial> pols(rounds);
+        for (size_t k = 0; k < rounds; k++) pols[k].nonzero_coeffs.assign(coeffs.begin() + k * td, coeffs.begin() + (k + 1) * td);
+        randoms.resize(rounds);
+        return {std::move(pols), std::move(randoms)};
+    }
+
+  private:
+    ml_wsumcheck_shard* h_ = nullptr;
+    size_t width_;
+};
 
 // src/fri/multilinear_pcs.rs:79-191
 class PCSProof {

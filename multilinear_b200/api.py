@@ -1052,6 +1052,92 @@ class ShardedPCSProver:
             pass
 
 
+class ShardedWideSumcheck:
+    """The width-w System sumcheck over the GPUs of one box (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu).  Rank g holds the row
+    block matrix[g*h/G, (g+1)*h/G) of the row-major trace.  Handles as for ShardedPCSProver.  One call equals
+    WideSumcheckTables.build + set_composition + compute_sumcheck_polynomials exactly, and every process gets the whole result."""
+
+    def __init__(self, h, world, local_ranks, width, n_vars):
+        self.h, self.world, self.local_ranks, self.width, self.n_vars = h, world, list(local_ranks), width, n_vars
+
+    @staticmethod
+    def _create(world, ranks, devices, width, n_vars):
+        h = C.c_void_p()
+        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
+        check(load().ml_wsumcheck_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(width), _sz(n_vars), C.byref(h)))
+        return ShardedWideSumcheck(h, world, ranks, width, n_vars)
+
+    @staticmethod
+    def single_process(devices, width, n_vars):
+        return ShardedWideSumcheck._create(len(devices), list(range(len(devices))), list(devices), width, n_vars)
+
+    @staticmethod
+    def one_rank(rank, world, device, width, n_vars):
+        return ShardedWideSumcheck._create(world, [rank], [device], width, n_vars)
+
+    def export(self):
+        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
+        check(load().ml_wsumcheck_shard_export(self.h, _p(out)))
+        return out.tobytes()
+
+    def connect(self, records):
+        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
+        check(load().ml_wsumcheck_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
+
+    def connect_over(self, dist, device):
+        """all-gather the IPC records over a torch.distributed process group"""
+        import torch
+        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
+        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
+        dist.all_gather(allr, mine)
+        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
+
+    def stream(self, local_index=0):
+        return load().ml_wsumcheck_shard_stream(self.h, C.c_int(local_index))
+
+    def arena_bytes(self):
+        return load().ml_wsumcheck_shard_arena_bytes(self.h)
+
+    def set_composition(self, terms):
+        """terms: [(coefficient, [column, ...]), ...] as for WideSumcheckTables.set_composition"""
+        coefs = as_elems([c for c, _ in terms]) if terms else elems_empty(1)[:0]
+        lens = np.ascontiguousarray([len(cs) for _, cs in terms], dtype=np.uint32)
+        cols = np.ascontiguousarray([c for _, cs in terms for c in cs] or [0], dtype=np.uint32)
+        check(load().ml_wsumcheck_shard_set_composition(self.h, _sz(len(terms)), _p(coefs), _p(lens), _p(cols)))
+
+    def _outputs(self, composition_degree):
+        n, td = self.n_vars, composition_degree + 1
+        return n, td, np.empty((max(n, 1) * td, 16), dtype=np.uint8), np.empty((max(n, 1), 16), dtype=np.uint8)
+
+    def compute_sumcheck_polynomials_dev(self, row_point, local_blocks_ptrs, composition_degree, transcript, s):
+        """local_blocks_ptrs[i]: device pointer to local rank i's row block -> (flat nonzero coeffs, randoms)"""
+        rp, sb = as_elems(row_point), _fe1(s)
+        n, td, co, rs = self._outputs(composition_degree)
+        ptrs = (C.c_void_p * len(local_blocks_ptrs))(*local_blocks_ptrs)
+        check(load().ml_wsumcheck_shard_compute_polynomials_dev(self.h, _p(rp), _sz(rp.shape[0]), ptrs, _sz(composition_degree), transcript.h,
+                                                                _p(sb), _p(co), _p(rs)))
+        return to_ints(co[:n * td]), to_ints(rs[:n])
+
+    def compute_sumcheck_polynomials(self, row_point, matrix, composition_degree, transcript, s):
+        """host rows (needs a single-process handle) -> (flat nonzero coeffs, randoms)"""
+        rp, m, sb = as_elems(row_point), as_elems(matrix), _fe1(s)
+        n, td, co, rs = self._outputs(composition_degree)
+        check(load().ml_wsumcheck_shard_compute_polynomials(self.h, _p(rp), _sz(rp.shape[0]), _p(m), _sz(self.width), _sz(m.shape[0] // self.width),
+                                                            _sz(composition_degree), transcript.h, _p(sb), _p(co), _p(rs)))
+        return to_ints(co[:n * td]), to_ints(rs[:n])
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_wsumcheck_shard_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 _INSTR = None
 
 

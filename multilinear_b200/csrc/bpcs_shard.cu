@@ -170,9 +170,9 @@ int bstage_tables(ml_bpcs_shard* sh, PeerRank& r, const std::vector<hfe>& pts) {
     MLB_KERNEL_CHECK();
     fe* fp = sh->world == 1 ? at(r, a.tail_m) : at(r, a.ycode);  // the encode buffers are free once S0 is done
     MLB_TRY(fingerprint_rows_launch((const fe* const*)(r.arena + a.eptrs), sh->B, sh->nloc, 0, fp, s, at(r, a.rho)));
-    if (sh->world == 1) return local_eq_table(sh, r, pts, at(r, a.tail_d), s);
+    if (sh->world == 1) return local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.tail_d), s);
     MLB_TRY(tables_launch(sh, r, fp, a.m, s));
-    MLB_TRY(local_eq_table(sh, r, pts, at(r, a.d), s));
+    MLB_TRY(local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.d), s));
     return peer_signal(sh->grp, r, PT, -1, s);
 }
 

@@ -351,16 +351,16 @@ int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaS
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
-int local_eq_table(ShardCore* sh, PeerRank& r, const std::vector<hfe>& pts, fe* d, cudaStream_t s) {
-    const int L = sh->L, v = (int)sh->n_vars;
-    MLB_TRY(eq_table_launch(r.ctx, pts.data(), (size_t)(v - L), d, s));
+int local_eq_table(Ctx* ctx, const std::vector<hfe>& pts, int v, int L, int rank, fe* d, cudaStream_t s) {
+    MLB_TRY(eq_table_launch(ctx, pts.data(), (size_t)(v - L), d, s));
     if (L == 0) return ML_OK;
     hfe scale = 1;
     for (int b = 0; b < L; b++) {
         const hfe p = pts[(size_t)(v - 1 - b)];
-        scale = hfe_mul(scale, ((r.rank >> b) & 1) ? p : hfe_sub(1, p));
+        scale = hfe_mul(scale, ((rank >> b) & 1) ? p : hfe_sub(1, p));
     }
-    pcs_shard_scale_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(d, sh->nloc, to_dev_fe_h(scale));
+    const size_t nloc = (size_t)1 << (v - L);
+    pcs_shard_scale_kernel<<<peer_grid(nloc), 256, 0, s>>>(d, nloc, to_dev_fe_h(scale));
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
@@ -407,12 +407,12 @@ int stage_encode(ShardCore* sh, PeerRank& r, const fe* evals, const uint8_t* cla
     if (sh->world == 1) {
         MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.tail_code), s));
         MLB_CUDA(cudaMemcpyAsync(at(r, a.tail_m), evals, sh->nloc * 16, cudaMemcpyDeviceToDevice, s));
-        return local_eq_table(sh, r, pts, at(r, a.tail_d), s);
+        return local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.tail_d), s);
     }
     MLB_TRY(encode_into(r.ctx, evals, sh->nloc, at(r, a.ycode), s));
     MLB_TRY(exchange_launch(sh, r, at(r, a.ycode), a.recv, s));
     MLB_TRY(tables_launch(sh, r, evals, a.m, s));
-    MLB_TRY(local_eq_table(sh, r, pts, at(r, a.d), s));
+    MLB_TRY(local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.d), s));
     return peer_signal(sh->grp, r, PX, -1, s);
 }
 

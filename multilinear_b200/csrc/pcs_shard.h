@@ -53,8 +53,9 @@ int shard_phase_ms(const ShardCore* sh, double* out, int cap);
 int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s);
 // cyclic transpose of a local table of nloc entries into the owners' tables at off_m
 int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s);
-// the rank's eq table: eq over all variables (G = 1) or the local part times the rank's factor for the top L variables
-int local_eq_table(ShardCore* sh, PeerRank& r, const std::vector<hfe>& pts, fe* d, cudaStream_t s);
+// the eq table of rank `rank`'s cyclic share of the 2^v rows (rows i = m*2^L + rank): eq over the low v-L variables times the
+// rank's factor for the top L variables (L = 0: eq over all variables); also used by wsumcheck_shard.cu
+int local_eq_table(Ctx* ctx, const std::vector<hfe>& pts, int v, int L, int rank, fe* d, cudaStream_t s);
 int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s);
 // run roots of `segs` segment subtrees (digests at dig, segment p at 32 * p * 2 R) -> every rank's mailbox at off_roots, and
 // (nb >= 0) the rank's partial sums from its CTA partials -> off_partials; then flag `phase` there

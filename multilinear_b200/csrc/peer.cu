@@ -143,8 +143,9 @@ int peer_signal(const PeerGroup& g, const PeerRank& r, int phase, int only, cuda
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
-int peer_wait(const PeerGroup& g, const PeerRank& r, int phase, int only_from, cudaStream_t s) {
-    peer_wait_kernel<<<1, 32, 0, s>>>(g.flags(r, phase), g.world, only_from, g.epoch, g.timeout_ns, g.status(r));
+int peer_wait(const PeerGroup& g, const PeerRank& r, int phase, int only_from, cudaStream_t s) { return peer_wait_for(g, r, phase, only_from, g.epoch, s); }
+int peer_wait_for(const PeerGroup& g, const PeerRank& r, int phase, int only_from, unsigned long long epoch, cudaStream_t s) {
+    peer_wait_kernel<<<1, 32, 0, s>>>(g.flags(r, phase), g.world, only_from, epoch, g.timeout_ns, g.status(r));
     MLB_KERNEL_CHECK();
     return ML_OK;
 }

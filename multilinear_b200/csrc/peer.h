@@ -110,6 +110,8 @@ int peer_check_ready(const PeerGroup& g, const char* who);
 int peer_signal(const PeerGroup& g, const PeerRank& r, int phase, int only, cudaStream_t s);
 // wait for flag[phase][*] >= epoch in r's arena (only_from: a single source, or -1 for all)
 int peer_wait(const PeerGroup& g, const PeerRank& r, int phase, int only_from, cudaStream_t s);
+// the same for flags raised by an earlier call: flag[phase][*] >= epoch
+int peer_wait_for(const PeerGroup& g, const PeerRank& r, int phase, int only_from, unsigned long long epoch, cudaStream_t s);
 // copy nbytes (multiple of 16, <= 128) from src_dev to dst_off in the arenas of all ranks (or one), then raise the flag there
 int peer_push(const PeerGroup& g, const PeerRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s);
 // ML_ERR_PEER if a wait of r's timed out (synchronises r's main stream)

@@ -1012,6 +1012,32 @@ int bfri_verify_queries(const ml_bfri_proof* p, ml_transcript* t, const hfe* rs,
     return memcmp(lr, p->last_random, 32) == 0 ? ML_V_OK : ML_V_LAST_RANDOM;
 }
 
+int wsumcheck_check_terms(size_t width, size_t n_terms, const uint32_t* term_lens, const uint32_t* term_cols, std::vector<uint32_t>& off, size_t* total) {
+    if (n_terms > (size_t)wsumcheck_limits(1)) { set_error("at most %d composition terms", wsumcheck_limits(1)); return ML_ERR_ARG; }
+    off.assign(n_terms ? n_terms : 1, 0);
+    *total = 0;
+    for (size_t t = 0; t < n_terms; t++) {
+        off[t] = (uint32_t)*total;
+        for (uint32_t k = 0; k < term_lens[t]; k++)
+            if (term_cols[*total + k] >= width) { set_error("composition term %zu references column %u of a width-%zu trace", t, term_cols[*total + k], width); return ML_ERR_OUT_OF_RANGE; }
+        *total += term_lens[t];
+    }
+    if (*total > (size_t)wsumcheck_limits(2)) { set_error("at most %d column references", wsumcheck_limits(2)); return ML_ERR_ARG; }
+    return ML_OK;
+}
+int wsumcheck_lagrange(size_t td, std::vector<uint8_t>& lag) {
+    const size_t n = td + 1;
+    std::vector<uint8_t> unit(n * 16), col(n * 16);
+    lag.assign(n * n * 16, 0);
+    for (size_t j = 0; j < n; j++) {
+        std::fill(unit.begin(), unit.end(), 0);
+        unit[16 * j] = 1;
+        MLB_TRY(ml_poly_interpolate(unit.data(), n, col.data()));
+        for (size_t i = 0; i < n; i++) memcpy(&lag[(i * n + j) * 16], &col[16 * i], 16);
+    }
+    return ML_OK;
+}
+
 }  // namespace mlbp
 using namespace mlbp;
 
@@ -1491,16 +1517,9 @@ size_t ml_wsumcheck_width(const ml_wsumcheck* w) { return w->width; }
 int ml_wsumcheck_set_composition(ml_wsumcheck* w, size_t n_terms, const uint8_t* coefs, const uint32_t* term_lens, const uint32_t* term_cols) {
     API_BEGIN
     (void)ctx;
-    if (n_terms > (size_t)wsumcheck_limits(1)) { set_error("at most %d composition terms", wsumcheck_limits(1)); return ML_ERR_ARG; }
-    std::vector<uint32_t> off(n_terms ? n_terms : 1, 0);
+    std::vector<uint32_t> off;
     size_t total = 0;
-    for (size_t t = 0; t < n_terms; t++) {
-        off[t] = (uint32_t)total;
-        for (uint32_t k = 0; k < term_lens[t]; k++)
-            if (term_cols[total + k] >= w->width) { set_error("composition term %zu references column %u of a width-%zu trace", t, term_cols[total + k], w->width); return ML_ERR_OUT_OF_RANGE; }
-        total += term_lens[t];
-    }
-    if (total > (size_t)wsumcheck_limits(2)) { set_error("at most %d column references", wsumcheck_limits(2)); return ML_ERR_ARG; }
+    MLB_TRY(wsumcheck_check_terms(w->width, n_terms, term_lens, term_cols, off, &total));
     cudaStream_t s = w->stream;
     pfree(w->coef, s); pfree(w->len, s); pfree(w->off, s); pfree(w->cols, s);
     w->coef = nullptr; w->len = w->off = w->cols = nullptr;
@@ -1553,15 +1572,8 @@ int ml_wsumcheck_compute_polynomials(ml_wsumcheck* w, size_t composition_degree,
         // every round on the device: points kernel -> one-CTA bookkeeping (Lagrange matrix, transcript in HBM, challenge) -> fold
         // reading the challenge from HBM; the last WTAIL_LOG rounds in one CTA; one synchronisation at the end
         cudaStream_t s = w->stream;
-        const size_t n = td + 1;
-        // Lagrange coefficient matrix over x = 0..td: lag[i][j] = coefficient of x^i in L_j (polynomials.rs:51-86 for unit vectors)
-        std::vector<uint8_t> lag_h(n * n * 16), unit(n * 16), col(n * 16);
-        for (size_t j = 0; j < n; j++) {
-            std::fill(unit.begin(), unit.end(), 0);
-            unit[16 * j] = 1;
-            MLB_TRY(ml_poly_interpolate(unit.data(), n, col.data()));
-            for (size_t i = 0; i < n; i++) memcpy(&lag_h[(i * n + j) * 16], &col[16 * i], 16);
-        }
+        std::vector<uint8_t> lag_h;
+        MLB_TRY(wsumcheck_lagrange(td, lag_h));
         const int max_nb = sumcheck_max_blocks();
         Scratch blk(s);
         const size_t off_tr = 0, off_r = 128, off_prev = 144, off_lag = 160, off_co = off_lag + 32 * 16, off_rs = off_co + 64 * W_MAX_TD * 16,

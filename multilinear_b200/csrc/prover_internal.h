@@ -39,6 +39,10 @@ void fill_dirs(PathH& p, size_t index, int depth);
 int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree);
 int fri_open_queries(const ml_fri* f, const std::vector<size_t>& indices, std::vector<QueryH>& out, cudaStream_t s);
 hfe fingerprint_host(hfe r, const hfe* c, size_t n);
+// width-w composition terms (ml_wsumcheck_set_composition's checks): per-term offsets into term_cols and the total count
+int wsumcheck_check_terms(size_t width, size_t n_terms, const uint32_t* term_lens, const uint32_t* term_cols, std::vector<uint32_t>& off, size_t* total);
+// Lagrange coefficient matrix over x = 0..td: lag[i][j] = coefficient of x^i in L_j (polynomials.rs:51-86 for unit vectors)
+int wsumcheck_lagrange(size_t td, std::vector<uint8_t>& lag);
 
 // Optional pieces of the sync-free fold chain supplied by the caller.
 struct ChainHooks {

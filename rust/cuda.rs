@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -213,6 +213,15 @@ extern "C" {
     pub fn ml_wsumcheck_height(w: *const MlWSumcheck) -> usize;
     pub fn ml_wsumcheck_partial_sum(w: *mut MlWSumcheck, r: *const u8, out: *mut u8) -> c_int;
     pub fn ml_wsumcheck_set_composition(w: *mut MlWSumcheck, n_terms: usize, coefs: *const u8, term_lens: *const u32, term_cols: *const u32) -> c_int;
+    pub fn ml_wsumcheck_shard_arena_bytes(sh: *const MlWSumcheckShard) -> usize;
+    pub fn ml_wsumcheck_shard_compute_polynomials(sh: *mut MlWSumcheckShard, row_point: *const u8, n_vars: usize, matrix: *const u8, width: usize, height: usize, composition_degree: usize, t: *mut MlTranscript, sum: *const u8, coeffs_out: *mut u8, randoms_out: *mut u8) -> c_int;
+    pub fn ml_wsumcheck_shard_compute_polynomials_dev(sh: *mut MlWSumcheckShard, row_point: *const u8, n_vars: usize, local_blocks_dev: *const *const c_void, composition_degree: usize, t: *mut MlTranscript, sum: *const u8, coeffs_out: *mut u8, randoms_out: *mut u8) -> c_int;
+    pub fn ml_wsumcheck_shard_connect(sh: *mut MlWSumcheckShard, records: *const u8, n_records: usize) -> c_int;
+    pub fn ml_wsumcheck_shard_create(world: c_int, n_local: c_int, local_ranks: *const c_int, local_devices: *const c_int, width: usize, n_vars: usize, out: *mut *mut MlWSumcheckShard) -> c_int;
+    pub fn ml_wsumcheck_shard_export(sh: *mut MlWSumcheckShard, records_out: *mut u8) -> c_int;
+    pub fn ml_wsumcheck_shard_free(sh: *mut MlWSumcheckShard);
+    pub fn ml_wsumcheck_shard_set_composition(sh: *mut MlWSumcheckShard, n_terms: usize, coefs: *const u8, term_lens: *const u32, term_cols: *const u32) -> c_int;
+    pub fn ml_wsumcheck_shard_stream(sh: *const MlWSumcheckShard, local_index: c_int) -> *mut c_void;
     pub fn ml_wsumcheck_tables(w: *const MlWSumcheck, matrix_out: *mut u8, delta_out: *mut u8) -> c_int;
     pub fn ml_wsumcheck_width(w: *const MlWSumcheck) -> usize;
     // ---- END GENERATED
@@ -826,5 +835,50 @@ impl CudaWideSumcheckTables {
 impl Drop for CudaWideSumcheckTables {
     fn drop(&mut self) {
         unsafe { ml_wsumcheck_free(self.h) }
+    }
+}
+/// The width-w sumcheck over all GPUs of the box from one process (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu): rank g holds the
+/// row block matrix[g*h/G, (g+1)*h/G); the result equals `CudaWideSumcheckTables::build` + `set_composition` +
+/// `compute_sumcheck_polynomials` exactly.  For traces too large for one GPU.  The handle is built once per (width, n_vars).
+pub struct ShardedWideSumcheckTables {
+    h: *mut MlWSumcheckShard,
+    width: usize,
+}
+impl ShardedWideSumcheckTables {
+    pub fn new(width: usize, n_vars: usize) -> Self {
+        let mut count = 0;
+        check(unsafe { ml_device_count(&mut count) });
+        let mut world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
+        while world > 1 && n_vars < world.trailing_zeros() as usize {
+            world >>= 1; // n_vars >= log2(world)
+        }
+        let world = world.min(16) as c_int;
+        let ids: Vec<c_int> = (0..world).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_wsumcheck_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), width, n_vars, &mut h) });
+        Self { h, width }
+    }
+    pub fn set_composition(&mut self, terms: &[(F, &[u32])]) {
+        let coefs: Vec<F> = terms.iter().map(|t| t.0).collect();
+        let lens: Vec<u32> = terms.iter().map(|t| t.1.len() as u32).collect();
+        let cols: Vec<u32> = terms.iter().flat_map(|t| t.1.iter().copied()).collect();
+        check(unsafe { ml_wsumcheck_shard_set_composition(self.h, terms.len(), p(&coefs), lens.as_ptr(), cols.as_ptr()) });
+    }
+    /// `compute_sumcheck_polynomials` (:147-172) of the trace `matrix` (row-major [2^n_vars][width]) at `row_point`
+    pub fn compute_sumcheck_polynomials(&mut self, row_point: &[F], matrix: &[F], composition_degree: usize, transcript: &mut Transcript, sum: F)
+        -> (Vec<SumcheckPolynomial<F>>, Vec<F>) {
+        let rounds = row_point.len();
+        let td = composition_degree + 1;
+        let (mut coeffs, mut randoms) = (zeros(rounds * td), zeros(rounds));
+        check(unsafe {
+            ml_wsumcheck_shard_compute_polynomials(self.h, p(row_point), rounds, p(matrix), self.width, matrix.len() / self.width, composition_degree,
+                                                   transcript.h, sum.as_ref().as_ptr(), pm(&mut coeffs), pm(&mut randoms))
+        });
+        (coeffs.chunks_exact(td).map(|c| SumcheckPolynomial { nonzero_coeffs: c.into() }).collect(), randoms)
+    }
+}
+impl Drop for ShardedWideSumcheckTables {
+    fn drop(&mut self) {
+        unsafe { ml_wsumcheck_shard_free(self.h) }
     }
 }
