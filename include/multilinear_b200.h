@@ -213,12 +213,14 @@ size_t ml_sumcheck_height(const ml_sumcheck *s);
 int ml_sumcheck_tables(const ml_sumcheck *s, uint8_t *matrix_out, uint8_t *delta_out);  /* current `height` entries each */
 int ml_sumcheck_partial_sum(const ml_sumcheck *s, const uint8_t r[16], uint8_t out[16]);   /* partial_sum :204-232 */
 int ml_sumcheck_fold(ml_sumcheck *s, const uint8_t r[16]);                                 /* fold :234-247 */
-/* compute_sumcheck_polynomial :174-202 — total_degree must be 2 on this path (multilinear_pcs.rs:57) */
+/* compute_sumcheck_polynomial :174-202 — total_degree 1..16, else ML_ERR_ARG (the PCS uses 2, multilinear_pcs.rs:57; at 0 the
+ * reference panics) */
 int ml_sumcheck_compute_polynomial(ml_sumcheck *s, size_t total_degree, uint8_t previous_sum[16], ml_transcript *t,
                                    uint8_t *nonzero_coeffs_out /* total_degree*16 */, uint8_t r_out[16]);
-/* compute_sumcheck_polynomials :147-172 — composition_degree must be 1 */
+/* compute_sumcheck_polynomials :147-172 — composition_degree 0..15, else ML_ERR_ARG.  The PCS degree 1 runs every round on the
+ * device; any other degree runs one host round per variable */
 int ml_sumcheck_compute_polynomials(ml_sumcheck *s, size_t composition_degree, ml_transcript *t, const uint8_t sum[16],
-                                    uint8_t *coeffs_out /* rounds*2*16 */, uint8_t *randoms_out /* rounds*16 */);
+                                    uint8_t *coeffs_out /* rounds*(composition_degree+1)*16 */, uint8_t *randoms_out /* rounds*16 */);
 int ml_delta_evaluate(const uint8_t *data, const uint8_t *points, size_t n, uint8_t out[16]); /* Delta::evaluate, evaluation.rs:80-90 (host) */
 
 /* ---- multilinear PCS (src/fri/multilinear_pcs.rs) ---- */
@@ -278,7 +280,12 @@ int ml_bpcs_proof_sumcheck_coeffs(const ml_bpcs_proof *p, uint8_t *out);
  * polynomial it computes over the row:  comp(x) = sum_t coefs[t] * prod_{k < term_lens[t]} x[term_cols[...]]
  * (term_cols is the concatenation of the terms' column lists; a term of length 0 is the constant coefs[t]).
  * System::evaluate_composition (evaluation.rs:5-12) = sum_k constraint_mask[k] * expr_k(row) has exactly this form once
- * the masks and trace challenges are folded into the coefficients.  matrix: the trace, row-major [height][width]. */
+ * the masks and trace challenges are folded into the coefficients.  matrix: the trace, row-major [height][width].
+ * Limits: width 1..16 (ML_ERR_ARG); at most 64 terms and 256 column references in all (ML_ERR_ARG); a column >= width is
+ * ML_ERR_OUT_OF_RANGE.  A rejected ml_wsumcheck_set_composition leaves the previous composition in place.
+ * ml_wsumcheck_compute_polynomials: composition_degree 0..15 (ML_ERR_ARG above); coeffs_out holds
+ * n_vars * (composition_degree + 1) elements.  Degrees 0..3 run every round on the device; 4..15 run one host round per
+ * variable.  A term may be longer than composition_degree: the result is then what the reference computes with that degree. */
 typedef struct ml_wsumcheck ml_wsumcheck;
 int ml_wsumcheck_build(const uint8_t *row_point, size_t n_vars, const uint8_t *matrix, size_t width, size_t height, ml_wsumcheck **out);
 int ml_wsumcheck_build_dev(const uint8_t *row_point, size_t n_vars, const void *matrix_dev, size_t width, size_t height, void *stream, ml_wsumcheck **out);

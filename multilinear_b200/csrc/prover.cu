@@ -439,8 +439,7 @@ int sumcheck_round(Ctx* ctx, ml_sumcheck* sc, size_t total_degree, hfe* previous
         for (size_t i = 1; i <= total_degree; i++)
             MLB_TRY(sumcheck_partial_sum_launch(ctx, sc->matrix, sc->delta, sc->height, hfe_new((hfe)i), &evals[i], s));
     }
-    if (total_degree >= 1) evals[0] = hfe_sub(*previous_sum, evals[1]);  // :188
-    else evals[0] = *previous_sum;
+    evals[0] = hfe_sub(*previous_sum, evals[1]);                          // :188 (total_degree >= 1)
     interpolate(evals, coeffs);                                           // :189-192
     for (size_t i = 1; i <= total_degree; i++) { nonzero_out[i - 1] = coeffs[i]; absorb_fe(t, coeffs[i]); }  // :193-197
     hfe r = challenge(t);                                                 // :198
@@ -1408,9 +1407,10 @@ int ml_sumcheck_fold(ml_sumcheck* sc, const uint8_t r[16]) {
 int ml_sumcheck_compute_polynomial(ml_sumcheck* sc, size_t total_degree, uint8_t previous_sum[16], ml_transcript* t,
                                    uint8_t* nonzero_coeffs_out, uint8_t r_out[16]) {
     API_BEGIN
-    if (total_degree > 16) { set_error("total_degree too large"); return ML_ERR_ARG; }
+    // total_degree 0: the reference reads evals[1] of a one-point round (:188) and panics
+    if (total_degree < 1 || total_degree > 16) { set_error("total_degree must be 1..16"); return ML_ERR_ARG; }
     hfe prev = hfe_load(previous_sum), r;
-    std::vector<hfe> nz(total_degree ? total_degree : 1);
+    std::vector<hfe> nz(total_degree);
     MLB_TRY(sumcheck_round(ctx, sc, total_degree, &prev, t, nz.data(), &r, lib_stream(ctx)));
     for (size_t i = 0; i < total_degree; i++) hfe_store(nonzero_coeffs_out + 16 * i, nz[i]);
     hfe_store(previous_sum, prev);

@@ -421,9 +421,11 @@ class OrSumcheck:
         self.L.or_sumcheck_fold(self.h, buf(rb))
 
     def compute_sumcheck_polynomial(self, total_degree, previous_sum, t):
-        prev, co, r = fe1(previous_sum), np.empty((total_degree, 16), dtype=np.uint8), np.empty(16, dtype=np.uint8)
-        self.L.or_sumcheck_compute_polynomial(self.h, sz(total_degree), buf(prev), t.h, buf(co), buf(r))
-        return fe_ints(co), fe_int(r), fe_int(prev)
+        prev, co, r = fe1(previous_sum), np.empty((max(total_degree, 1), 16), dtype=np.uint8), np.empty(16, dtype=np.uint8)
+        st = self.L.or_sumcheck_compute_polynomial(self.h, sz(total_degree), buf(prev), t.h, buf(co), buf(r))
+        if st:
+            raise ValueError("or_sumcheck_compute_polynomial: status %d (total_degree %d)" % (st, total_degree))
+        return fe_ints(co[:total_degree]), fe_int(r), fe_int(prev)
 
     def compute_sumcheck_polynomials(self, composition_degree, t, s):
         n = (self.height()).bit_length() - 1

@@ -763,12 +763,14 @@ static fe sumcheck_round(or_sumcheck *s, size_t total_degree, fe *previous_sum, 
     free(evals); free(coeffs);
     return r;
 }
-void or_sumcheck_compute_polynomial(or_sumcheck *s, size_t total_degree, uint8_t previous_sum[16], or_transcript *t,
-                                    uint8_t *nonzero_coeffs_out, uint8_t r_out[16]) {
+int or_sumcheck_compute_polynomial(or_sumcheck *s, size_t total_degree, uint8_t previous_sum[16], or_transcript *t,
+                                   uint8_t *nonzero_coeffs_out, uint8_t r_out[16]) {
+    if (total_degree == 0) return OR_ERR_SIZE; /* :188 indexes evals[1] */
     fe prev = fe_load(previous_sum);
     fe r = sumcheck_round(s, total_degree, &prev, t, (fe *)nonzero_coeffs_out);
     fe_store(previous_sum, prev);
     fe_store(r_out, r);
+    return OR_OK;
 }
 void or_sumcheck_compute_polynomials(or_sumcheck *s, size_t composition_degree, or_transcript *t, const uint8_t sum[16],
                                      uint8_t *coeffs_out, uint8_t *randoms_out) { /* :147-172 */

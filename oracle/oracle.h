@@ -117,8 +117,9 @@ size_t or_sumcheck_height(const or_sumcheck *s);
 void or_sumcheck_tables(const or_sumcheck *s, uint8_t *matrix_out, uint8_t *delta_out); /* current height entries each */
 void or_sumcheck_partial_sum(const or_sumcheck *s, const uint8_t r[16], uint8_t out[16]); /* :204-232, composition x[0] */
 void or_sumcheck_fold(or_sumcheck *s, const uint8_t r[16]);                               /* :234-247 */
-void or_sumcheck_compute_polynomial(or_sumcheck *s, size_t total_degree, uint8_t previous_sum[16], or_transcript *t,
-                                    uint8_t *nonzero_coeffs_out, uint8_t r_out[16]);      /* :174-202 */
+/* :174-202; total_degree 0 (the reference reads evals[1] of one point and panics): OR_ERR_SIZE, nothing touched */
+int or_sumcheck_compute_polynomial(or_sumcheck *s, size_t total_degree, uint8_t previous_sum[16], or_transcript *t,
+                                   uint8_t *nonzero_coeffs_out, uint8_t r_out[16]);
 void or_sumcheck_compute_polynomials(or_sumcheck *s, size_t composition_degree, or_transcript *t, const uint8_t sum[16],
                                      uint8_t *coeffs_out, uint8_t *randoms_out);          /* :147-172 */
 void or_delta_evaluate(const uint8_t *data, const uint8_t *points, size_t n, uint8_t out[16]); /* evaluation.rs:80-90 */
