@@ -380,6 +380,39 @@ int ml_bpcs_shard_prove_dev(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_v
 int ml_bpcs_shard_prove(ml_bpcs_shard *sh, const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
                         const uint8_t *const *evals, size_t n, ml_transcript *t, ml_bpcs_proof **out);
 
+/* ---- FriProof::prove of ONE polynomial sharded over the GPUs of one box (fri/mod.rs:261-285), from its coefficients
+ * (reed_solomon + prove, fri/mod.rs:19-28) or from its code ----
+ * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; n = 2^log_n coefficients, code length N = 2n.  From coefficients, rank
+ * b holds the block coeffs[b*n/G, (b+1)*n/G): a cyclic transpose over the peers gives each rank one residue class of the
+ * coefficients mod G, which it RS-encodes at length N/G; the column exchange and the combine of ml_pcs_shard_* (without its
+ * Moebius step) give the global code.  From a code, rank b holds the block code[b*N/G, (b+1)*N/G), stored straight into the
+ * owners' layer 0.  The first log2(G) fold rounds run sharded (Merkle subtrees and folds stay on their owners; every rank absorbs
+ * the layer root and draws the same challenge), then rank 0 runs the rest of the fold chain from N/G elements and the openings
+ * (csrc/fri_shard.cu).  Rank r holds about 1/G of the encoded layers and trees; rank 0 additionally the tail from N/G elements;
+ * there are no sumcheck tables (ml_fri_shard_arena_bytes).
+ * The proof is byte-identical to ml_rs_fri_prove's / ml_fri_prove's and an ordinary ml_fri_proof (ml_fri_verify and the
+ * serializer work unchanged).  A code that is not an RS code gives ML_ERR_NOT_RS_CODE on every rank, in every process, within
+ * the call; the handle proves normally afterwards.  Handles, records, calls and errors as for ml_pcs_shard_* above.  Minimum
+ * size: log_n >= max(1, 2*log2 G): G = 1: 1, 2: 2, 4: 4, 8: 6, 16: 8 (ML_ERR_SIZE below). */
+typedef struct ml_fri_shard ml_fri_shard;
+int ml_fri_shard_create(int world, int n_local, const int *local_ranks, const int *local_devices, size_t log_n, ml_fri_shard **out);
+void ml_fri_shard_free(ml_fri_shard *sh);   /* multi-process: all ranks must have returned from their last call (caller's barrier) */
+int ml_fri_shard_export(ml_fri_shard *sh, uint8_t *records_out /* num_local * ml_shard_record_bytes() */);
+int ml_fri_shard_connect(ml_fri_shard *sh, const uint8_t *records, size_t n_records /* world */);
+void *ml_fri_shard_stream(const ml_fri_shard *sh, int local_index);  /* the local rank's main stream (for CUDA-event timing) */
+size_t ml_fri_shard_arena_bytes(const ml_fri_shard *sh);
+/* local_coeffs_dev[i]: local rank i's block coeffs[rank*n/G, (rank+1)*n/G) (device pointer, complete before the call; only read).
+ * Every process passes its own transcript copy; all copies end in rank 0's final state. */
+int ml_fri_shard_rs_prove_dev(ml_fri_shard *sh, const void *const *local_coeffs_dev, ml_transcript *t, ml_fri_proof **out /* NULL unless rank 0 is local */);
+/* local_code_dev[i]: local rank i's block code[rank*N/G, (rank+1)*N/G) (device pointer, complete before the call; only read) */
+int ml_fri_shard_prove_dev(ml_fri_shard *sh, const void *const *local_code_dev, ml_transcript *t, ml_fri_proof **out /* NULL unless rank 0 is local */);
+/* host coefficients (all n) and a handle that hosts every rank: reed_solomon + prove (= ml_rs_fri_prove) */
+int ml_fri_shard_rs_prove(ml_fri_shard *sh, const uint8_t *coeffs, size_t n, ml_transcript *t, ml_fri_proof **out);
+/* host code (n = its length, N) and a handle that hosts every rank: the drop-in for fri/mod.rs:261.  gen_pows follows the
+ * RESTRICTION of ml_fri_prove (NULL, or the domain generator's powers: ML_ERR_SIZE / ML_ERR_GENERATOR otherwise). */
+int ml_fri_shard_prove(ml_fri_shard *sh, const uint8_t *code, size_t n, const uint8_t *gen_pows, size_t gen_pows_len,
+                       ml_transcript *t, ml_fri_proof **out);
+
 /* ---- the width-w System sumcheck sharded over the GPUs of one box (SumcheckTables::compute_sumcheck_polynomials,
  * src/constraint_system/sumcheck.rs:147-202) ----
  * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; rank b holds the contiguous row block matrix[b*h/G, (b+1)*h/G) of the

@@ -239,6 +239,7 @@ class FriProof {
     }
 
   private:
+    friend class ShardedFriProver;
     FriProof() = default;
     ml_fri_proof* h_ = nullptr;
 };
@@ -377,6 +378,31 @@ class ShardedPCSProver {
 
   private:
     ml_pcs_shard* h_ = nullptr;
+};
+// FriProof::prove of one polynomial over several GPUs from one process (ml_fri_shard_*, csrc/fri_shard.cu), from its code or from
+// its 2^log_n coefficients (reed_solomon + prove); `devices` may repeat (virtual ranks).  The proof bytes equal FriProof::prove's.
+class ShardedFriProver {
+  public:
+    ShardedFriProver(const std::vector<int>& devices, size_t log_n) {
+        std::vector<int> ranks(devices.size());
+        for (size_t i = 0; i < ranks.size(); i++) ranks[i] = (int)i;
+        check(ml_fri_shard_create((int)devices.size(), (int)devices.size(), ranks.data(), devices.data(), log_n, &h_));
+    }
+    ShardedFriProver(const ShardedFriProver&) = delete;
+    ~ShardedFriProver() { if (h_) ml_fri_shard_free(h_); }
+    FriProof prove(const std::vector<F>& code, const std::vector<F>& gen_pows, Transcript& t) {  // fri/mod.rs:261-285
+        FriProof p;
+        check(ml_fri_shard_prove(h_, raw(code), code.size(), raw(gen_pows), gen_pows.size(), t.handle(), &p.h_));
+        return p;
+    }
+    FriProof rs_prove(const std::vector<F>& coeffs, Transcript& t) {  // reed_solomon (fri/mod.rs:19-28) + prove
+        FriProof p;
+        check(ml_fri_shard_rs_prove(h_, raw(coeffs), coeffs.size(), t.handle(), &p.h_));
+        return p;
+    }
+
+  private:
+    ml_fri_shard* h_ = nullptr;
 };
 
 // src/fri/batched_pcs.rs:22-254

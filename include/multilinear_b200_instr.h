@@ -41,6 +41,10 @@ int ml_pcs_shard_phase_ms(const struct ml_pcs_shard *sh, double *out, int cap);
  * fingerprinted tables, sharded rounds, tail fold chain (rank 0), openings + proof (rank 0)] */
 struct ml_bpcs_shard;
 int ml_bpcs_shard_phase_ms(const struct ml_bpcs_shard *sh, double *out, int cap);
+/* sharded FRI prover (ml_fri_shard_*): [S0 transpose + encode + exchange (from a code: the placement into layer 0), S1 combine
+ * (from a code: the wait), sharded rounds, tail fold chain (rank 0), openings + proof (rank 0)] */
+struct ml_fri_shard;
+int ml_fri_shard_phase_ms(const struct ml_fri_shard *sh, double *out, int cap);
 
 #ifdef __cplusplus
 }

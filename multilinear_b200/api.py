@@ -1052,6 +1052,101 @@ class ShardedPCSProver:
             pass
 
 
+class ShardedFriProver:
+    """FriProof::prove of one polynomial sharded over the GPUs of one box (ml_fri_shard_*, csrc/fri_shard.cu), from its 2^log_n
+    coefficients (reed_solomon + prove) or from its code of 2^(log_n+1) elements.  Rank g holds the block coeffs[g*n/G, (g+1)*n/G)
+    or code[g*N/G, (g+1)*N/G).  Handles as for ShardedPCSProver.  The proof is an ordinary FriProof, byte-identical to
+    FriProof.prove_from_coeffs's / FriProof.prove's."""
+
+    def __init__(self, h, world, local_ranks, log_n):
+        self.h, self.world, self.local_ranks, self.log_n = h, world, list(local_ranks), log_n
+
+    @staticmethod
+    def _create(world, ranks, devices, log_n):
+        h = C.c_void_p()
+        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
+        check(load().ml_fri_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(log_n), C.byref(h)))
+        return ShardedFriProver(h, world, ranks, log_n)
+
+    @staticmethod
+    def single_process(devices, log_n):
+        return ShardedFriProver._create(len(devices), list(range(len(devices))), list(devices), log_n)
+
+    @staticmethod
+    def one_rank(rank, world, device, log_n):
+        return ShardedFriProver._create(world, [rank], [device], log_n)
+
+    def export(self):
+        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
+        check(load().ml_fri_shard_export(self.h, _p(out)))
+        return out.tobytes()
+
+    def connect(self, records):
+        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
+        check(load().ml_fri_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
+
+    def connect_over(self, dist, device):
+        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
+        import torch
+        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
+        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
+        dist.all_gather(allr, mine)
+        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
+
+    def stream(self, local_index=0):
+        return load().ml_fri_shard_stream(self.h, C.c_int(local_index))
+
+    def arena_bytes(self):
+        return load().ml_fri_shard_arena_bytes(self.h)
+
+    def phase_ms(self):
+        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
+        out = (C.c_double * 16)()
+        n = load().ml_fri_shard_phase_ms(self.h, out, C.c_int(16))
+        return [out[i] for i in range(n)]
+
+    def rs_prove_dev(self, local_coeffs_ptrs, transcript):
+        """local_coeffs_ptrs[i]: device pointer to local rank i's block of n/G coefficients; None unless rank 0 is local"""
+        ptrs = (C.c_void_p * len(local_coeffs_ptrs))(*local_coeffs_ptrs)
+        h = C.c_void_p()
+        check(load().ml_fri_shard_rs_prove_dev(self.h, ptrs, transcript.h, C.byref(h)))
+        return FriProof(h) if h.value else None
+
+    def prove_dev(self, local_code_ptrs, transcript):
+        """local_code_ptrs[i]: device pointer to local rank i's block of N/G code elements; None unless rank 0 is local"""
+        ptrs = (C.c_void_p * len(local_code_ptrs))(*local_code_ptrs)
+        h = C.c_void_p()
+        check(load().ml_fri_shard_prove_dev(self.h, ptrs, transcript.h, C.byref(h)))
+        return FriProof(h) if h.value else None
+
+    def rs_prove(self, coeffs, transcript):
+        """host coefficients (needs a single-process handle): reed_solomon + FriProof::prove"""
+        c = as_elems(coeffs)
+        h = C.c_void_p()
+        check(load().ml_fri_shard_rs_prove(self.h, _p(c), _sz(c.shape[0]), transcript.h, C.byref(h)))
+        return FriProof(h)
+
+    def prove(self, code, gen_pows, transcript):
+        """host code (needs a single-process handle) — the drop-in for fri/mod.rs:261"""
+        c = as_elems(code)
+        gp = as_elems(gen_pows) if gen_pows is not None else None
+        h = C.c_void_p()
+        check(load().ml_fri_shard_prove(self.h, _p(c), _sz(c.shape[0]), _p(gp) if gp is not None else None,
+                                        _sz(gp.shape[0] if gp is not None else 0), transcript.h, C.byref(h)))
+        return FriProof(h)
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_fri_shard_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class ShardedWideSumcheck:
     """The width-w System sumcheck over the GPUs of one box (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu).  Rank g holds the row
     block matrix[g*h/G, (g+1)*h/G) of the row-major trace.  Handles as for ShardedPCSProver.  One call equals

@@ -45,12 +45,15 @@ __global__ void __launch_bounds__(256) pcs_shard_exchange_kernel(const fe* __res
         reinterpret_cast<uint4*>(peers.base[dest] + off_recv)[(size_t)rank * R + j] = __ldg(reinterpret_cast<const uint4*>(code + k));
     }
 }
-// block entry o (global b*nloc + o) -> table of rank o mod G at (b*nloc + o) / G; stores are contiguous per destination
+// block entry o (global b*nloc + o) -> table of rank o mod G (REV: rank rev_L(o mod G)) at (b*nloc + o) / G; stores are
+// contiguous per destination
+template <bool REV>
 __global__ void __launch_bounds__(256) pcs_shard_tables_kernel(const fe* __restrict__ evals, size_t nloc, int L, int rank, PeerPtrs peers, size_t off_m) {
     const size_t per = nloc >> L, stride = (size_t)gridDim.x * blockDim.x;
     for (size_t x = (size_t)blockIdx.x * blockDim.x + threadIdx.x; x < nloc; x += stride) {
-        const size_t dest = x / per, ml = x - dest * per;
-        reinterpret_cast<uint4*>(peers.base[dest] + off_m)[(size_t)rank * per + ml] = __ldg(reinterpret_cast<const uint4*>(evals + (ml << L) + dest));
+        const size_t cls = x / per, ml = x - cls * per;
+        const size_t dest = REV ? (__brev((unsigned)cls) >> (32 - L)) : cls;
+        reinterpret_cast<uint4*>(peers.base[dest] + off_m)[(size_t)rank * per + ml] = __ldg(reinterpret_cast<const uint4*>(evals + (ml << L) + cls));
     }
 }
 __global__ void __launch_bounds__(256) pcs_shard_scale_kernel(fe* __restrict__ d, size_t n, fe s) {
@@ -59,7 +62,8 @@ __global__ void __launch_bounds__(256) pcs_shard_scale_kernel(fe* __restrict__ d
 }
 
 // ------------------------------------------------------------------ S1: Moebius over the rank bits + twiddle + G-point DFT
-template <int LG>
+// (MOBIUS = false: the local codes encode coefficients, the FRI prover's S1 is twiddle + DFT only)
+template <int LG, bool MOBIUS>
 __global__ void __launch_bounds__(256) pcs_shard_combine_kernel(const fe* __restrict__ recv, size_t R, int rank, int log_N, const fe* __restrict__ lo,
                                                                 const fe* __restrict__ hi, fe* __restrict__ layer0) {
     constexpr int G = 1 << LG;
@@ -71,11 +75,13 @@ __global__ void __launch_bounds__(256) pcs_shard_combine_kernel(const fe* __rest
         fe a[G];
 #pragma unroll
         for (int b = 0; b < G; b++) a[b] = fe_load_nc(recv + (size_t)b * R + j);
+        if (MOBIUS) {
 #pragma unroll
-        for (int m = 1; m < G; m <<= 1)  // to_coefficient over the rank bits (polynomials.rs:150-163)
+            for (int m = 1; m < G; m <<= 1)  // to_coefficient over the rank bits (polynomials.rs:150-163)
 #pragma unroll
-            for (int b = 0; b < G; b++)
-                if (b & m) a[b] = fe_sub(a[b], a[b ^ m]);
+                for (int b = 0; b < G; b++)
+                    if (b & m) a[b] = fe_sub(a[b], a[b ^ m]);
+        }
         // a[b] *= w^(rev(b) * k2): input j1 = rev(b) of the DFT, already in the bit-reversed order the butterflies below take
         const size_t k2 = (size_t)rank * R + j;
         const fe wk = root_pow(lo, hi, k2);
@@ -227,7 +233,7 @@ struct ml_pcs_shard : ShardCore {};
 
 namespace mlbs {
 
-Layout make_layout(size_t n, int G, size_t B) {
+Layout make_layout(size_t n, int G, size_t B, bool fri) {
     const int L = (int)ilog2((size_t)G);
     const size_t NL = 2 * n / G, R = NL / G, nloc = n / G;
     const bool sharded = G > 1, batched = B > 0;
@@ -244,7 +250,7 @@ Layout make_layout(size_t n, int G, size_t B) {
     a.final_tr = take(sizeof(DevTranscript));
     for (int k = 0; k < MAX_L; k++) a.mail[k] = take(MAIL_ROOTS * 32 + (size_t)MAXR * 32);  // run roots | partial pairs
     for (int k = 0; k < MAX_L; k++) a.top[k] = take(2 * MAIL_ROOTS * 32);
-    a.part = take((size_t)(2 * sumcheck_max_blocks() + 2) * 16);
+    a.part = take(fri ? 0 : (size_t)(2 * sumcheck_max_blocks() + 2) * 16);
     a.rho = take(batched ? 16 : 0);
     a.outs = take(B * 16);
     a.eptrs = take(B * 8);
@@ -252,16 +258,17 @@ Layout make_layout(size_t n, int G, size_t B) {
     // batched: two encode buffers (the encode of polynomial j+1 overlaps the exchange of j) and one recv slice per polynomial
     a.ycode = take(sharded ? (batched ? 2 : 1) * NL * 16 : 0);
     a.recv = take(sharded ? (batched ? B : 1) * NL * 16 : 0);
+    a.coef = take(sharded && fri ? nloc * 16 : 0);
     for (int k = 0; k < MAX_L; k++) {
         const bool held = k < L || (k == 0 && batched);
         a.layer[k] = take(held ? (k == 0 && batched ? B : 1) * ((size_t)G >> k) * R * 16 : 0);
         a.dig[k] = take(held ? ((size_t)G >> k) * R * 32 : 0);
     }
-    a.m = take(sharded ? nloc * 16 : 0);
-    a.d = take(sharded ? nloc * 16 : 0);
+    a.m = take(sharded && !fri ? nloc * 16 : 0);
+    a.d = take(sharded && !fri ? nloc * 16 : 0);
     a.tail_code = take(NL * 16);
-    a.tail_m = take(nloc * 16);
-    a.tail_d = take(nloc * 16);
+    a.tail_m = take(fri ? 0 : nloc * 16);
+    a.tail_d = take(fri ? 0 : nloc * 16);
     a.total = o;
     return a;
 }
@@ -280,11 +287,12 @@ PeerRank* rank0_of(ShardCore* sh) {
     return nullptr;
 }
 
-int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who) {
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who,
+               bool fri) {
     const int L = (int)ilog2((size_t)world);
     sh->world = world; sh->L = L; sh->n_vars = n_vars; sh->n = (size_t)1 << n_vars; sh->B = B;
     sh->NL = 2 * sh->n / world; sh->R = sh->NL / world; sh->nloc = sh->n / world;
-    sh->lay = make_layout(sh->n, world, B);
+    sh->lay = make_layout(sh->n, world, B, fri);
     sh->grp.world = world;
     sh->grp.arena_bytes = sh->lay.total;
     sh->grp.off_flags = sh->lay.flags;
@@ -346,8 +354,9 @@ int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
-int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s) {
-    pcs_shard_tables_kernel<<<peer_grid(sh->nloc), 256, 0, s>>>(src, sh->nloc, sh->L, r.rank, sh->grp.peers(), off_m);
+int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s, bool rev_dest) {
+    if (rev_dest) pcs_shard_tables_kernel<true><<<peer_grid(sh->nloc), 256, 0, s>>>(src, sh->nloc, sh->L, r.rank, sh->grp.peers(), off_m);
+    else pcs_shard_tables_kernel<false><<<peer_grid(sh->nloc), 256, 0, s>>>(src, sh->nloc, sh->L, r.rank, sh->grp.peers(), off_m);
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
@@ -365,17 +374,21 @@ int local_eq_table(Ctx* ctx, const std::vector<hfe>& pts, int v, int L, int rank
     return ML_OK;
 }
 
-int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s) {
+template <bool MOBIUS>
+int combine_launch_t(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s) {
     const unsigned grid = peer_grid(R);
     switch (L) {
-        case 1: pcs_shard_combine_kernel<1><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
-        case 2: pcs_shard_combine_kernel<2><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
-        case 3: pcs_shard_combine_kernel<3><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
-        case 4: pcs_shard_combine_kernel<4><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
+        case 1: pcs_shard_combine_kernel<1, MOBIUS><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
+        case 2: pcs_shard_combine_kernel<2, MOBIUS><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
+        case 3: pcs_shard_combine_kernel<3, MOBIUS><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
+        case 4: pcs_shard_combine_kernel<4, MOBIUS><<<grid, 256, 0, s>>>(recv, R, rank, log_N, rt->lo, rt->hi, layer0); break;
         default: set_error("ml_pcs_shard: log2(world) = %d out of range", L); return ML_ERR_ARG;
     }
     MLB_KERNEL_CHECK();
     return ML_OK;
+}
+int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s, bool mobius) {
+    return mobius ? combine_launch_t<true>(L, recv, R, rank, log_N, rt, layer0, s) : combine_launch_t<false>(L, recv, R, rank, log_N, rt, layer0, s);
 }
 
 int post_launch(ShardCore* sh, PeerRank& r, const uint8_t* dig, size_t R, int segs, int nb, size_t off_roots, size_t off_partials, int phase) {
@@ -462,6 +475,10 @@ int fold_tables(ShardCore* sh, PeerRank& r, int k, int* nb) {
 }
 // round k, phase C: fold tables and code; after the last sharded round, hand layer L and the tables to rank 0
 int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb) {
+    MLB_TRY(fold_code(sh, r, k));
+    return fold_tables(sh, r, k, nb);
+}
+int fold_code(ShardCore* sh, PeerRank& r, int k) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     const Layout& a = sh->lay;
@@ -472,7 +489,7 @@ int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb) {
     pcs_shard_fold_kernel<<<peer_grid(segs * sh->R), 256, 0, s>>>(at(r, a.layer[k]), segs, sh->R, sh->NL, r.rank, k, log_N, at(r, a.r), rt->lo, rt->hi,
                                                                   fold_target(sh, r, k));
     MLB_KERNEL_CHECK();
-    return fold_tables(sh, r, k, nb);
+    return ML_OK;
 }
 
 int open_sharded(ShardCore* sh, PeerRank& r0, const std::vector<size_t>& idx, int j0, std::vector<uint8_t>& host, int* stride) {
@@ -515,13 +532,14 @@ int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, 
     ChainHooks h = hooks;
     h.tr_dev = (const DevTranscript*)(r0.arena + a.tr);
     h.prev_dev = at(r0, a.prev);
-    MLB_TRY(fold_chain_dev(r0.ctx, f, &h, &sc, 0, sumcheck + 2 * L, (size_t)L, !hooks.first_fold, t, s));
+    MLB_TRY(fold_chain_dev(r0.ctx, f, &h, sumcheck ? &sc : nullptr, 0, sumcheck ? sumcheck + 2 * L : nullptr, (size_t)L, !hooks.first_fold, t, s));
     if (&r0 == &sh->local[0]) mark_phase(sh, mark_base + 1);
     if (L > 0) {  // sumcheck (c1, c2) and layer roots of the sharded rounds
         uint8_t lo[MAX_L * 32];
-        MLB_CUDA(cudaMemcpyAsync(lo, r0.arena + a.sc, (size_t)L * 32, cudaMemcpyDeviceToHost, s));
+        if (sumcheck) MLB_CUDA(cudaMemcpyAsync(lo, r0.arena + a.sc, (size_t)L * 32, cudaMemcpyDeviceToHost, s));
         MLB_TRY(d2h_sync(roots_lo, r0.arena + a.roots_out, (size_t)L * 32, s));
-        for (int i = 0; i < 2 * L; i++) sumcheck[i] = hfe_load(lo + 16 * i);
+        if (sumcheck)
+            for (int i = 0; i < 2 * L; i++) sumcheck[i] = hfe_load(lo + 16 * i);
     }
     return peer_read_status(sh->grp, r0, sh->who);
 }
@@ -533,6 +551,16 @@ int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t) {
     MLB_TRY(trd.alloc(128));
     MLB_TRY(h2d(trd.p, &t->sha, sizeof(DevTranscript), s));
     MLB_TRY(peer_push(sh->grp, r0, trd.p, (int)(sizeof(DevTranscript) + 15) / 16 * 16, sh->lay.final_tr, PF, -1, s));
+    return stream_wait_blocking(s);
+}
+int tail_fail(ShardCore* sh, PeerRank& r0, int st) {
+    if (sh->world == 1) return ML_OK;
+    cudaStream_t s = r0.st.main;
+    const int word[4] = {st, 0, 0, 0};
+    Scratch d(s);
+    MLB_TRY(d.alloc(16));
+    MLB_TRY(h2d(d.p, word, 16, s));
+    MLB_TRY(peer_push(sh->grp, r0, d.p, 16, sh->lay.status, PF, -1, s));
     return stream_wait_blocking(s);
 }
 
@@ -553,14 +581,7 @@ int finish_ranks(ShardCore* sh, ml_transcript* t, int st) {
     return st;
 }
 
-}  // namespace mlbs
-
-namespace {
-
-const char* WHO = "ml_pcs_shard";
-
-// openings and the proof on rank 0 (:113-129): layers < L from the owners' arenas, layers >= L from the tail's FriProverData
-int assemble(ml_pcs_shard* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_fri_proof* p, const uint8_t* roots_lo) {
+int assemble_fri(ShardCore* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_fri_proof* p, const uint8_t* roots_lo) {
     cudaStream_t s = r0.st.main;
     const int L = sh->L;
     std::vector<size_t> idx;
@@ -593,7 +614,13 @@ int assemble(ml_pcs_shard* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, 
     return ML_OK;
 }
 
-// rank 0: the rest of the fold chain from layer L, the openings, the final transcript to everybody
+}  // namespace mlbs
+
+namespace {
+
+const char* WHO = "ml_pcs_shard";
+
+// rank 0: the rest of the fold chain from layer L, the openings (:113-129), the final transcript to everybody
 int prove_tail(ml_pcs_shard* sh, PeerRank& r0, const uint8_t* inputs, const uint8_t* output, ml_transcript* t, ml_pcs_proof** out) {
     ml_fri* f = new ml_fri();
     struct FriGuard { ml_fri* p; ~FriGuard() { free_fri(p); } } fri_guard{f};
@@ -602,7 +629,7 @@ int prove_tail(ml_pcs_shard* sh, PeerRank& r0, const uint8_t* inputs, const uint
     p->sumcheck.resize(2 * sh->n_vars);
     uint8_t roots_lo[MAX_L * 32];
     MLB_TRY(tail_chain(sh, r0, f, ChainHooks(), p->sumcheck.data(), roots_lo, t, 3));
-    MLB_TRY(assemble(sh, r0, f, t, &p->fri, roots_lo));
+    MLB_TRY(assemble_fri(sh, r0, f, t, &p->fri, roots_lo));
     if (&r0 == &sh->local[0]) mark_phase(sh, 5);
     p->inputs.resize(sh->n_vars);
     for (size_t i = 0; i < sh->n_vars; i++) p->inputs[i] = hfe_load(inputs + 16 * i);

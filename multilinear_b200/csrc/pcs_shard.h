@@ -1,6 +1,7 @@
-// Stages of the block-sharded PCS provers, shared by pcs_shard.cu (one PCSProof::prove, ml_pcs_shard_*) and bpcs_shard.cu
-// (one BatchedPCSProof::prove, ml_bpcs_shard_*).  Both split every polynomial by block over G ranks and keep the sharded layers
-// in the segment layout described at the top of pcs_shard.cu; the batched prover only adds a batched layer 0 and round 0.
+// Stages of the block-sharded provers, shared by pcs_shard.cu (one PCSProof::prove, ml_pcs_shard_*), bpcs_shard.cu (one
+// BatchedPCSProof::prove, ml_bpcs_shard_*) and fri_shard.cu (one FriProof::prove, ml_fri_shard_*).  All split every polynomial by
+// block over G ranks and keep the sharded layers in the segment layout described at the top of pcs_shard.cu; the batched prover
+// only adds a batched layer 0 and round 0, the FRI prover drops the sumcheck tables.
 #pragma once
 #include "peer.h"
 #include "prover_internal.h"
@@ -9,7 +10,8 @@ namespace mlbs {
 using namespace mlb;
 using namespace mlbp;
 
-enum Phase { PX = 0, PR0 = 1, PG = PR0 + 4, PF, PB, PT, N_PHASES };  // PR0 + k: round k (L <= 4); PB, PT: batched prover only
+// PR0 + k: round k (L <= 4); PB, PT: batched prover only; PC: FRI prover only (coefficient transpose)
+enum Phase { PX = 0, PR0 = 1, PG = PR0 + 4, PF, PB, PT, PC, N_PHASES };
 static const int MAXR = PEER_MAXR;
 static const int MAX_L = 4;
 static const size_t MAIL_ROOTS = (size_t)MAXR * MAXR / 2;  // run roots of layer 0 at G = ML_MAX_PEERS
@@ -17,10 +19,11 @@ static const size_t MAIL_ROOTS = (size_t)MAXR * MAXR / 2;  // run roots of layer
 struct Layout {
     size_t flags, status, tr, prev, r, sc, roots_out, final_tr, mail[MAX_L], top[MAX_L], part;  // mailbox (cleared at create)
     size_t rho, outs, eptrs, segptrs;                                                          // batched prover only
-    size_t ycode, recv, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;
+    size_t ycode, recv, coef, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;  // coef: FRI prover only
 };
-// B = 0: one polynomial; B >= 1: a batch of B polynomials (layer 0 holds B codes)
-Layout make_layout(size_t n, int G, size_t B);
+// B = 0: one polynomial; B >= 1: a batch of B polynomials (layer 0 holds B codes); fri: one polynomial without sumcheck tables,
+// with a receive buffer for the transposed coefficients instead
+Layout make_layout(size_t n, int G, size_t B, bool fri = false);
 // mailbox of round k: run root of run q at roots + 32 q, partial pair of rank g at partials + 32 g
 inline size_t mail_partials(const Layout& a, int k) { return a.mail[k] + MAIL_ROOTS * 32; }
 
@@ -42,7 +45,8 @@ void mark_phase(ShardCore* sh, int idx);
 PeerRank* rank0_of(ShardCore* sh);
 
 // handle plumbing (arguments already checked by the caller)
-int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who);
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who,
+               bool fri = false);
 void shard_free(ShardCore* sh);
 int shard_export(ShardCore* sh, uint8_t* records_out);
 int shard_connect(ShardCore* sh, const uint8_t* records, size_t n_records, const char* who);
@@ -51,12 +55,14 @@ int shard_phase_ms(const ShardCore* sh, double* out, int cap);
 
 // S0 exchange: slice r of the local code `ycode` -> rank r's recv at off_recv (G > 1)
 int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s);
-// cyclic transpose of a local table of nloc entries into the owners' tables at off_m
-int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s);
+// cyclic transpose of a local table of nloc entries into the owners' tables at off_m: entry o of the block goes to rank
+// (o mod G), or rank rev_L(o mod G) with rev_dest (the FRI prover's coefficients), at (b*nloc + o) / G
+int tables_launch(ShardCore* sh, PeerRank& r, const fe* src, size_t off_m, cudaStream_t s, bool rev_dest = false);
 // the eq table of rank `rank`'s cyclic share of the 2^v rows (rows i = m*2^L + rank): eq over the low v-L variables times the
 // rank's factor for the top L variables (L = 0: eq over all variables); also used by wsumcheck_shard.cu
 int local_eq_table(Ctx* ctx, const std::vector<hfe>& pts, int v, int L, int rank, fe* d, cudaStream_t s);
-int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s);
+// S1: layer 0 from the received columns; mobius: the local codes encode evaluations (PCS), else coefficients (FRI)
+int combine_launch(int L, const fe* recv, size_t R, int rank, int log_N, const RootTables* rt, fe* layer0, cudaStream_t s, bool mobius = true);
 // run roots of `segs` segment subtrees (digests at dig, segment p at 32 * p * 2 R) -> every rank's mailbox at off_roots, and
 // (nb >= 0) the rank's partial sums from its CTA partials -> off_partials; then flag `phase` there
 int post_launch(ShardCore* sh, PeerRank& r, const uint8_t* dig, size_t R, int segs, int nb, size_t off_roots, size_t off_partials, int phase);
@@ -68,20 +74,28 @@ int finish_launch(ShardCore* sh, PeerRank& r, int k, const uint8_t* root);
 // sharded round k >= 0 of a single code layer: A (subtrees + post), B (top + transcript), C (folds)
 int stage_post(ShardCore* sh, PeerRank& r, int k, int nb);
 int stage_round(ShardCore* sh, PeerRank& r, int k);
-int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb);
+int stage_fold(ShardCore* sh, PeerRank& r, int k, int* nb);  // fold_code + fold_tables
+// FRI fold of the code of layer k into fold_target
+int fold_code(ShardCore* sh, PeerRank& r, int k);
 // where round k writes its fold: layer k+1 in the segment layout, or rank 0's tail code after the last sharded round
 fe* fold_target(ShardCore* sh, PeerRank& r, int k);
 // fold of the tables of round k; after the last sharded round, hand the tables to rank 0 and flag PG
 int fold_tables(ShardCore* sh, PeerRank& r, int k, int* nb);
 
 // rank 0: the fold chain from layer L (first_fold: a batched round 0 at G = 1), sumcheck coefficients and roots of the sharded
-// rounds (sumcheck: 2 * n_vars, roots_lo: 32 * L); marks mark_base and mark_base + 1
+// rounds (sumcheck: 2 * n_vars, or nullptr for a plain FRI proof without tables; roots_lo: 32 * L); marks mark_base and
+// mark_base + 1
 int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, hfe* sumcheck, uint8_t* roots_lo, ml_transcript* t, int mark_base);
 // rank 0: records (value pair | path) of layers j0 .. L-1 for every query index, from the owners' arenas; record (q, j) at
 // (q * L + j) * *stride
 int open_sharded(ShardCore* sh, PeerRank& r0, const std::vector<size_t>& idx, int j0, std::vector<uint8_t>& host, int* stride);
+// rank 0: openings and the FriProof of one code (fri/mod.rs:261-285): layers < L from the owners' arenas, layers >= L from the
+// tail's FriProverData; roots_lo: the roots of the sharded layers
+int assemble_fri(ShardCore* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_fri_proof* p, const uint8_t* roots_lo);
 // rank 0: final transcript to every rank (releases their buffers); the other local ranks wait for it and adopt it
 int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t);
+// rank 0 after a failed call: its status into every rank's status word, then the same release (finish_ranks returns it)
+int tail_fail(ShardCore* sh, PeerRank& r0, int st);
 int finish_ranks(ShardCore* sh, ml_transcript* t, int st);
 
 // segment-layout helpers on the device

@@ -158,8 +158,10 @@ int peer_read_status(const PeerGroup& g, const PeerRank& r, const char* who) {
     int st = 0;
     MLB_CUDA(cudaSetDevice(r.device));
     MLB_TRY(mlbp::d2h_sync(&st, g.status(r), sizeof st, r.st.main));
-    if (st != 0) { set_error("%s: rank %d timed out waiting for a peer rank (%.0f s)", who, r.rank, g.timeout_ns * 1e-9); return ML_ERR_PEER; }
-    return ML_OK;
+    if (st == 0) return ML_OK;
+    if (st != ML_ERR_PEER) { set_error("%s: rank %d: rank 0 ended the call with status %d", who, r.rank, st); return st; }  // relayed (tail_fail)
+    set_error("%s: rank %d timed out waiting for a peer rank (%.0f s)", who, r.rank, g.timeout_ns * 1e-9);
+    return ML_ERR_PEER;
 }
 
 }  // namespace mlb

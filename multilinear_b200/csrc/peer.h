@@ -114,7 +114,7 @@ int peer_wait(const PeerGroup& g, const PeerRank& r, int phase, int only_from, c
 int peer_wait_for(const PeerGroup& g, const PeerRank& r, int phase, int only_from, unsigned long long epoch, cudaStream_t s);
 // copy nbytes (multiple of 16, <= 128) from src_dev to dst_off in the arenas of all ranks (or one), then raise the flag there
 int peer_push(const PeerGroup& g, const PeerRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s);
-// ML_ERR_PEER if a wait of r's timed out (synchronises r's main stream)
+// ML_ERR_PEER if a wait of r's timed out, or the status rank 0 stored into r's status word (synchronises r's main stream)
 int peer_read_status(const PeerGroup& g, const PeerRank& r, const char* who);
 
 }  // namespace mlb

@@ -1037,6 +1037,26 @@ int wsumcheck_lagrange(size_t td, std::vector<uint8_t>& lag) {
     return ML_OK;
 }
 
+int check_gen_pows(int log_n0, const uint8_t* gen_pows, size_t gen_pows_len) {
+    if (!gen_pows) return ML_OK;
+    if (gen_pows_len != ((size_t)1 << log_n0)) { set_error("gen_pows.len() must equal the domain size"); return ML_ERR_SIZE; }
+    // The kernels read their own root tables (powers of pow_2_generator(log2 domain)), not this array, so a caller-supplied table is
+    // only accepted if it IS that table.  Checked at [0], [1], [2], [len/2], [len-1] and 16 spread positions (host scalar pow): a table
+    // of the right length that disagrees anywhere else would be a table the reference's own callers never build (they all pass
+    // pow_2_generator_powers, src/fri/mod.rs:352, multilinear_pcs.rs:98); the restriction is stated in the header.
+    hfe w;
+    hfe_pow2_generator((uint64_t)log_n0, &w);
+    size_t probe[21] = {0, 1, 2, gen_pows_len / 2, gen_pows_len - 1};
+    for (int i = 0; i < 16; i++) probe[5 + i] = (size_t)(((unsigned __int128)gen_pows_len * (2 * i + 1)) / 33) ^ (size_t)(i * 2654435761u % 97);
+    for (size_t idx : probe) {
+        if (idx >= gen_pows_len) continue;
+        if (hfe_load(gen_pows + 16 * idx) != hfe_pow(w, (hfe)idx)) {
+            set_error("gen_pows[%zu] is not pow_2_generator(%d)^%zu: only the domain's own power table is supported", idx, log_n0, idx);
+            return ML_ERR_GENERATOR;
+        }
+    }
+    return ML_OK;
+}
 }  // namespace mlbp
 using namespace mlbp;
 
@@ -1165,29 +1185,9 @@ int ml_fri_init(const uint8_t* code_host, size_t n, ml_transcript* t, ml_fri** o
     if (st != ML_OK) { pfree(code, s); return st; }
     return fri_init_owned(out, code, n, true, t, s);
 }
-static int check_gen_pows(const ml_fri* f, const uint8_t* gen_pows, size_t gen_pows_len) {
-    if (!gen_pows) return ML_OK;
-    if (gen_pows_len != ((size_t)1 << f->log_n0)) { set_error("gen_pows.len() must equal the domain size"); return ML_ERR_SIZE; }
-    // The kernels read their own root tables (powers of pow_2_generator(log2 domain)), not this array, so a caller-supplied table is
-    // only accepted if it IS that table.  Checked at [0], [1], [2], [len/2], [len-1] and 16 spread positions (host scalar pow): a table
-    // of the right length that disagrees anywhere else would be a table the reference's own callers never build (they all pass
-    // pow_2_generator_powers, src/fri/mod.rs:352, multilinear_pcs.rs:98); the restriction is stated in the header.
-    hfe w;
-    hfe_pow2_generator((uint64_t)f->log_n0, &w);
-    size_t probe[21] = {0, 1, 2, gen_pows_len / 2, gen_pows_len - 1};
-    for (int i = 0; i < 16; i++) probe[5 + i] = (size_t)(((unsigned __int128)gen_pows_len * (2 * i + 1)) / 33) ^ (size_t)(i * 2654435761u % 97);
-    for (size_t idx : probe) {
-        if (idx >= gen_pows_len) continue;
-        if (hfe_load(gen_pows + 16 * idx) != hfe_pow(w, (hfe)idx)) {
-            set_error("gen_pows[%zu] is not pow_2_generator(%d)^%zu: only the domain's own power table is supported", idx, f->log_n0, idx);
-            return ML_ERR_GENERATOR;
-        }
-    }
-    return ML_OK;
-}
 int ml_fri_fold_step(ml_fri* f, const uint8_t* gen_pows, size_t gen_pows_len, size_t k, const uint8_t r[16], ml_transcript* t) {
     API_BEGIN
-    MLB_TRY(check_gen_pows(f, gen_pows, gen_pows_len));
+    MLB_TRY(check_gen_pows(f->log_n0, gen_pows, gen_pows_len));
     return fri_fold_step_impl(ctx, f, k, hfe_load(r), t, lib_stream(ctx));
 }
 static int fri_from_copy(const void* src, size_t n, bool src_on_device, cudaStream_t s, ml_fri** out) {
@@ -1211,7 +1211,7 @@ int ml_fri_fold(const uint8_t* gen_pows, size_t gen_pows_len, const uint8_t* cod
     API_BEGIN
     ml_fri* f;
     MLB_TRY(fri_from_copy(code, n, false, lib_stream(ctx), &f));
-    int st = check_gen_pows(f, gen_pows, gen_pows_len);
+    int st = check_gen_pows(f->log_n0, gen_pows, gen_pows_len);
     if (st == ML_OK) st = fold_chain_dev(ctx, f, nullptr, nullptr, 0, nullptr, 0, true, t, lib_stream(ctx));
     if (st != ML_OK) { free_fri(f); return st; }
     *out = f;
@@ -1297,7 +1297,7 @@ int ml_fri_prove(const uint8_t* code, size_t n, const uint8_t* gen_pows, size_t 
     API_BEGIN
     ml_fri* f;
     MLB_TRY(fri_from_copy(code, n, false, lib_stream(ctx), &f));
-    int st = check_gen_pows(f, gen_pows, gen_pows_len);
+    int st = check_gen_pows(f->log_n0, gen_pows, gen_pows_len);
     if (st != ML_OK) { free_fri(f); return st; }
     return fri_prove_from(ctx, f, n, t, lib_stream(ctx), out);
 }
@@ -1815,7 +1815,7 @@ int ml_bfri_init(const uint8_t* const* codes, size_t n_codes, size_t n, ml_trans
 }
 int ml_bfri_batched_fold_step(ml_bfri* h, const uint8_t* gen_pows, size_t gen_pows_len, const uint8_t r[16], ml_transcript* t) {  // :101-181
     API_BEGIN
-    if (gen_pows) MLB_TRY(check_gen_pows(h->b.fri, gen_pows, gen_pows_len));
+    if (gen_pows) MLB_TRY(check_gen_pows(h->b.fri->log_n0, gen_pows, gen_pows_len));
     return bfri_batched_fold_step(ctx, &h->b, hfe_load(r), t, lib_stream(ctx));
 }
 int ml_bfri_fold(const uint8_t* gen_pows, size_t gen_pows_len, const uint8_t* const* codes, size_t n_codes, size_t n, ml_transcript* t,
@@ -1826,7 +1826,7 @@ int ml_bfri_fold(const uint8_t* gen_pows, size_t gen_pows_len, const uint8_t* co
     ml_bfri* h = new ml_bfri();
     int st = bfri_upload_codes(h, codes, n_codes, n, s);
     if (st == ML_OK) st = bfri_init(&h->b, t, s);
-    if (st == ML_OK && gen_pows) st = check_gen_pows(h->b.fri, gen_pows, gen_pows_len);
+    if (st == ML_OK && gen_pows) st = check_gen_pows(h->b.fri->log_n0, gen_pows, gen_pows_len);
     if (st == ML_OK) {
         ChainHooks hooks;
         mlbp::BatchedFri* b = &h->b;

@@ -38,6 +38,8 @@ void fill_dirs(PathH& p, size_t index, int depth);
 // appends layer `code` (n elements) to f with its Merkle tree (build_tree) but without reading the root back
 int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree);
 int fri_open_queries(const ml_fri* f, const std::vector<size_t>& indices, std::vector<QueryH>& out, cudaStream_t s);
+// the RESTRICTION on a caller's gen_pows (include/multilinear_b200.h): NULL, or the powers of pow_2_generator(log_n0)
+int check_gen_pows(int log_n0, const uint8_t* gen_pows, size_t gen_pows_len);
 hfe fingerprint_host(hfe r, const hfe* c, size_t n);
 // width-w composition terms (ml_wsumcheck_set_composition's checks): per-term offsets into term_cols and the total count
 int wsumcheck_check_terms(size_t width, size_t n_terms, const uint32_t* term_lens, const uint32_t* term_cols, std::vector<uint32_t>& off, size_t* total);

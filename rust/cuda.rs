@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -103,6 +103,16 @@ extern "C" {
     pub fn ml_fri_proof_serialized_len(p: *const MlFriProof) -> usize;
     pub fn ml_fri_prove(code: *const u8, n: usize, gen_pows: *const u8, gen_pows_len: usize, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
     pub fn ml_fri_prove_dev(code_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_shard_arena_bytes(sh: *const MlFriShard) -> usize;
+    pub fn ml_fri_shard_connect(sh: *mut MlFriShard, records: *const u8, n_records: usize) -> c_int;
+    pub fn ml_fri_shard_create(world: c_int, n_local: c_int, local_ranks: *const c_int, local_devices: *const c_int, log_n: usize, out: *mut *mut MlFriShard) -> c_int;
+    pub fn ml_fri_shard_export(sh: *mut MlFriShard, records_out: *mut u8) -> c_int;
+    pub fn ml_fri_shard_free(sh: *mut MlFriShard);
+    pub fn ml_fri_shard_prove(sh: *mut MlFriShard, code: *const u8, n: usize, gen_pows: *const u8, gen_pows_len: usize, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_shard_prove_dev(sh: *mut MlFriShard, local_code_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_shard_rs_prove(sh: *mut MlFriShard, coeffs: *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_shard_rs_prove_dev(sh: *mut MlFriShard, local_coeffs_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_shard_stream(sh: *const MlFriShard, local_index: c_int) -> *mut c_void;
     pub fn ml_fri_tree(f: *const MlFri, i: usize, tree: *mut *const MlMerkle) -> c_int;
     pub fn ml_fri_tree_data(f: *const MlFri, i: usize, pairs_out: *mut u8) -> c_int;
     pub fn ml_fri_verify(p: *const MlFriProof) -> c_int;
@@ -599,6 +609,49 @@ impl ShardedPcsProver {
 impl Drop for ShardedPcsProver {
     fn drop(&mut self) {
         unsafe { ml_pcs_shard_free(self.h) }
+    }
+}
+/// `FriProof::prove` of ONE polynomial over all GPUs of the box from one process (ml_fri_shard_*, csrc/fri_shard.cu), from its
+/// 2^log_n coefficients (`reed_solomon` + prove) or from its code of 2^(log_n+1) elements: rank g holds the block g of G; the first
+/// log2(G) fold rounds run sharded, rank 0 runs the rest.  The handle is built once per log_n and reused; the proof bytes equal
+/// `rs_fri_prove`'s / `fri_prove`'s.
+pub struct ShardedFriProver {
+    h: *mut MlFriShard,
+}
+impl ShardedFriProver {
+    pub fn new(log_n: usize) -> Self {
+        let mut count = 0;
+        check(unsafe { ml_device_count(&mut count) });
+        let mut world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
+        while world > 1 && log_n < 2 * world.trailing_zeros() as usize {
+            world >>= 1; // log_n >= 2 log2(world)
+        }
+        let world = world.min(16) as c_int;
+        let ids: Vec<c_int> = (0..world).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_fri_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), log_n, &mut h) });
+        Self { h }
+    }
+    /// body of `FriProof::prove` (src/fri/mod.rs:261-285) for a code of the handle's length
+    pub fn prove(&mut self, code: &[F], gen_pows: &[F], transcript: &mut Transcript) -> FriProof<F> {
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_fri_shard_prove(self.h, p(code), code.len(), p(gen_pows), gen_pows.len(), transcript.h, &mut h) });
+        let proof = unsafe { fri_proof_from(h) };
+        unsafe { ml_fri_proof_free(h) };
+        proof
+    }
+    /// `reed_solomon` (src/fri/mod.rs:19-28) + `FriProof::prove` of the handle's number of coefficients
+    pub fn rs_prove(&mut self, coeffs: &[F], transcript: &mut Transcript) -> FriProof<F> {
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_fri_shard_rs_prove(self.h, p(coeffs), coeffs.len(), transcript.h, &mut h) });
+        let proof = unsafe { fri_proof_from(h) };
+        unsafe { ml_fri_proof_free(h) };
+        proof
+    }
+}
+impl Drop for ShardedFriProver {
+    fn drop(&mut self) {
+        unsafe { ml_fri_shard_free(self.h) }
     }
 }
 /// `BatchedFriProof` does not derive `Deserialize`; its blob is the bincode encoding of its parts in field order, and the parts
