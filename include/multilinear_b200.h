@@ -413,6 +413,41 @@ int ml_fri_shard_rs_prove(ml_fri_shard *sh, const uint8_t *coeffs, size_t n, ml_
 int ml_fri_shard_prove(ml_fri_shard *sh, const uint8_t *code, size_t n, const uint8_t *gen_pows, size_t gen_pows_len,
                        ml_transcript *t, ml_fri_proof **out);
 
+/* ---- BatchedFriProof::prove of B codes sharded by block over the GPUs of one box (batched_fri.rs:286-318), from the
+ * polynomials' coefficients (reed_solomon of each + prove) or from their codes ----
+ * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; B = n_codes (1 <= B <= 2^20) polynomials of n = 2^log_n coefficients
+ * each, code length N = 2n.  Rank b holds block b of every polynomial: coefficients [b*n/G, (b+1)*n/G) or code elements
+ * [b*N/G, (b+1)*N/G).  Each code is built and placed as by ml_fri_shard_*; layer 0 is one batched Merkle tree over the B codes
+ * whose subtrees stay with their owners (as ml_bpcs_shard_*); every rank absorbs the batch root, draws rho and the first
+ * challenge; round 0 folds the fingerprinted pairs on their owners, rounds 1 .. log2(G)-1 run sharded, then rank 0 runs the rest
+ * of the fold chain from N/G elements and the openings (csrc/bfri_shard.cu).  Rank r holds B received slices and the B layer-0
+ * blocks (2B * 16 N/G bytes; the transposed coefficients share the layer-0 space) plus about 1/G of the other layers and trees;
+ * rank 0 additionally the tail from N/G elements; there are no sumcheck tables (ml_bfri_shard_arena_bytes).
+ * The proof is byte-identical to ml_batched_fri_prove's on the same codes (on reed_solomon of each polynomial for the coefficient
+ * entries) and an ordinary ml_bfri_proof (ml_batched_fri_verify and the serializer work unchanged).  A code that is not an RS
+ * code gives ML_ERR_NOT_RS_CODE on every rank, in every process, within the call; the handle proves normally afterwards.
+ * Handles, records, calls and errors as for ml_pcs_shard_* above.  Minimum size: log_n >= max(1, 2*log2 G) (ML_ERR_SIZE below);
+ * log_n = 1 at G = 1 has no folded layer and gives ML_ERR_OUT_OF_RANGE, as ml_batched_fri_prove does. */
+typedef struct ml_bfri_shard ml_bfri_shard;
+int ml_bfri_shard_create(int world, int n_local, const int *local_ranks, const int *local_devices, size_t n_codes, size_t log_n,
+                         ml_bfri_shard **out);
+void ml_bfri_shard_free(ml_bfri_shard *sh);   /* multi-process: all ranks must have returned from their last call (caller's barrier) */
+int ml_bfri_shard_export(ml_bfri_shard *sh, uint8_t *records_out /* num_local * ml_shard_record_bytes() */);
+int ml_bfri_shard_connect(ml_bfri_shard *sh, const uint8_t *records, size_t n_records /* world */);
+void *ml_bfri_shard_stream(const ml_bfri_shard *sh, int local_index);  /* the local rank's main stream (for CUDA-event timing) */
+size_t ml_bfri_shard_arena_bytes(const ml_bfri_shard *sh);
+/* local_coeffs_dev[i * n_codes + j]: local rank i's block of the coefficients of polynomial j, n/G elements (device pointers,
+ * complete before the call; only read).  Every process passes its own transcript copy; all copies end in rank 0's final state. */
+int ml_bfri_shard_rs_prove_dev(ml_bfri_shard *sh, const void *const *local_coeffs_dev, ml_transcript *t, ml_bfri_proof **out /* NULL unless rank 0 is local */);
+/* local_codes_dev[i * n_codes + j]: local rank i's block of code j, N/G elements (device pointers, complete before the call; only read) */
+int ml_bfri_shard_prove_dev(ml_bfri_shard *sh, const void *const *local_codes_dev, ml_transcript *t, ml_bfri_proof **out /* NULL unless rank 0 is local */);
+/* host coefficients (n_codes arrays of n) and a handle that hosts every rank: reed_solomon of each + prove */
+int ml_bfri_shard_rs_prove(ml_bfri_shard *sh, const uint8_t *const *coeffs, size_t n_codes, size_t n, ml_transcript *t, ml_bfri_proof **out);
+/* host codes (n_codes arrays of n = N elements) and a handle that hosts every rank: the drop-in for batched_fri.rs:286.  gen_pows
+ * follows the RESTRICTION of ml_fri_prove (NULL, or the domain generator's powers: ML_ERR_SIZE / ML_ERR_GENERATOR otherwise). */
+int ml_bfri_shard_prove(ml_bfri_shard *sh, const uint8_t *const *codes, size_t n_codes, size_t n, const uint8_t *gen_pows,
+                        size_t gen_pows_len, ml_transcript *t, ml_bfri_proof **out);
+
 /* ---- the width-w System sumcheck sharded over the GPUs of one box (SumcheckTables::compute_sumcheck_polynomials,
  * src/constraint_system/sumcheck.rs:147-202) ----
  * G ranks (a power of two <= ML_MAX_PEERS), one GPU each; rank b holds the contiguous row block matrix[b*h/G, (b+1)*h/G) of the

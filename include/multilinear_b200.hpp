@@ -404,6 +404,60 @@ class ShardedFriProver {
   private:
     ml_fri_shard* h_ = nullptr;
 };
+// src/fri/batched_fri.rs:284-398
+class BatchedFriProof {
+  public:
+    static BatchedFriProof prove(const std::vector<std::vector<F>>& codes, const std::vector<F>& gen_pows, Transcript& t) {  // :286-318
+        std::vector<const uint8_t*> ptrs;
+        for (auto& c : codes) ptrs.push_back(raw(c));
+        BatchedFriProof p;
+        check(ml_batched_fri_prove(ptrs.data(), codes.size(), codes.empty() ? 0 : codes[0].size(), raw(gen_pows), gen_pows.size(), t.handle(), &p.h_));
+        return p;
+    }
+    BatchedFriProof(BatchedFriProof&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+    ~BatchedFriProof() { if (h_) ml_bfri_proof_free(h_); }
+    int verify() const { return ml_batched_fri_verify(h_); }  // :320-354; 0 = Ok(())
+    std::vector<uint8_t> serialize() const {  // bincode
+        std::vector<uint8_t> out(ml_bfri_proof_serialized_len(h_));
+        check(ml_bfri_proof_serialize(h_, out.data()));
+        return out;
+    }
+
+  private:
+    friend class ShardedBatchedFriProver;
+    BatchedFriProof() = default;
+    ml_bfri_proof* h_ = nullptr;
+};
+// BatchedFriProof::prove of B codes over several GPUs from one process, every code split by block (ml_bfri_shard_*,
+// csrc/bfri_shard.cu), from the codes or from the polynomials' 2^log_n coefficients (reed_solomon of each + prove); `devices` may
+// repeat (virtual ranks).  The proof bytes equal BatchedFriProof::prove's.
+class ShardedBatchedFriProver {
+  public:
+    ShardedBatchedFriProver(const std::vector<int>& devices, size_t n_codes, size_t log_n) {
+        std::vector<int> ranks(devices.size());
+        for (size_t i = 0; i < ranks.size(); i++) ranks[i] = (int)i;
+        check(ml_bfri_shard_create((int)devices.size(), (int)devices.size(), ranks.data(), devices.data(), n_codes, log_n, &h_));
+    }
+    ShardedBatchedFriProver(const ShardedBatchedFriProver&) = delete;
+    ~ShardedBatchedFriProver() { if (h_) ml_bfri_shard_free(h_); }
+    BatchedFriProof prove(const std::vector<std::vector<F>>& codes, const std::vector<F>& gen_pows, Transcript& t) {  // batched_fri.rs:286-318
+        std::vector<const uint8_t*> ptrs;
+        for (auto& c : codes) ptrs.push_back(raw(c));
+        BatchedFriProof p;
+        check(ml_bfri_shard_prove(h_, ptrs.data(), codes.size(), codes.empty() ? 0 : codes[0].size(), raw(gen_pows), gen_pows.size(), t.handle(), &p.h_));
+        return p;
+    }
+    BatchedFriProof rs_prove(const std::vector<std::vector<F>>& coeffs, Transcript& t) {  // reed_solomon of each + prove
+        std::vector<const uint8_t*> ptrs;
+        for (auto& c : coeffs) ptrs.push_back(raw(c));
+        BatchedFriProof p;
+        check(ml_bfri_shard_rs_prove(h_, ptrs.data(), coeffs.size(), coeffs.empty() ? 0 : coeffs[0].size(), t.handle(), &p.h_));
+        return p;
+    }
+
+  private:
+    ml_bfri_shard* h_ = nullptr;
+};
 
 // src/fri/batched_pcs.rs:22-254
 struct BatchedPCSClaim {

@@ -45,6 +45,10 @@ int ml_bpcs_shard_phase_ms(const struct ml_bpcs_shard *sh, double *out, int cap)
  * (from a code: the wait), sharded rounds, tail fold chain (rank 0), openings + proof (rank 0)] */
 struct ml_fri_shard;
 int ml_fri_shard_phase_ms(const struct ml_fri_shard *sh, double *out, int cap);
+/* sharded batched FRI prover (ml_bfri_shard_*): [S0 transposes + encodes + exchange (from codes: the placement into layer 0), S1
+ * combine + batch tree, S2 batch root, sharded rounds, tail fold chain (rank 0), openings + proof (rank 0)] */
+struct ml_bfri_shard;
+int ml_bfri_shard_phase_ms(const struct ml_bfri_shard *sh, double *out, int cap);
 
 #ifdef __cplusplus
 }

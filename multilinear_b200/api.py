@@ -1147,6 +1147,110 @@ class ShardedFriProver:
             pass
 
 
+class ShardedBatchedFriProver:
+    """BatchedFriProof::prove of B codes sharded by block over the GPUs of one box (ml_bfri_shard_*, csrc/bfri_shard.cu), from the
+    2^log_n coefficients of each polynomial (reed_solomon of each + prove) or from their codes of 2^(log_n+1) elements.  Rank g
+    holds block g of every polynomial: coeffs_j[g*n/G, (g+1)*n/G) or code_j[g*N/G, (g+1)*N/G).  Handles as for ShardedPCSProver.
+    The proof is an ordinary batched FriProof, byte-identical to BatchedFriProof.prove's."""
+
+    def __init__(self, h, world, local_ranks, n_codes, log_n):
+        self.h, self.world, self.local_ranks, self.n_codes, self.log_n = h, world, list(local_ranks), n_codes, log_n
+
+    @staticmethod
+    def _create(world, ranks, devices, n_codes, log_n):
+        h = C.c_void_p()
+        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
+        check(load().ml_bfri_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_codes), _sz(log_n), C.byref(h)))
+        return ShardedBatchedFriProver(h, world, ranks, n_codes, log_n)
+
+    @staticmethod
+    def single_process(devices, n_codes, log_n):
+        return ShardedBatchedFriProver._create(len(devices), list(range(len(devices))), list(devices), n_codes, log_n)
+
+    @staticmethod
+    def one_rank(rank, world, device, n_codes, log_n):
+        return ShardedBatchedFriProver._create(world, [rank], [device], n_codes, log_n)
+
+    def export(self):
+        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
+        check(load().ml_bfri_shard_export(self.h, _p(out)))
+        return out.tobytes()
+
+    def connect(self, records):
+        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
+        check(load().ml_bfri_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
+
+    def connect_over(self, dist, device):
+        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
+        import torch
+        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
+        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
+        dist.all_gather(allr, mine)
+        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
+
+    def stream(self, local_index=0):
+        return load().ml_bfri_shard_stream(self.h, C.c_int(local_index))
+
+    def arena_bytes(self):
+        return load().ml_bfri_shard_arena_bytes(self.h)
+
+    def phase_ms(self):
+        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
+        out = (C.c_double * 16)()
+        n = load().ml_bfri_shard_phase_ms(self.h, out, C.c_int(16))
+        return [out[i] for i in range(n)]
+
+    def rs_prove_dev(self, local_coeffs_ptrs, transcript):
+        """local_coeffs_ptrs[i * n_codes + j]: device pointer to local rank i's block (n/G coefficients) of polynomial j;
+        None unless rank 0 is local"""
+        ptrs = (C.c_void_p * len(local_coeffs_ptrs))(*local_coeffs_ptrs)
+        h = C.c_void_p()
+        check(load().ml_bfri_shard_rs_prove_dev(self.h, ptrs, transcript.h, C.byref(h)))
+        return FriProof(h, batched=True) if h.value else None
+
+    def prove_dev(self, local_codes_ptrs, transcript):
+        """local_codes_ptrs[i * n_codes + j]: device pointer to local rank i's block (N/G elements) of code j; None unless rank 0
+        is local"""
+        ptrs = (C.c_void_p * len(local_codes_ptrs))(*local_codes_ptrs)
+        h = C.c_void_p()
+        check(load().ml_bfri_shard_prove_dev(self.h, ptrs, transcript.h, C.byref(h)))
+        return FriProof(h, batched=True) if h.value else None
+
+    @staticmethod
+    def _arrays(xs):
+        cs = [as_elems(x) for x in xs]
+        if any(c.shape != cs[0].shape for c in cs):
+            raise SizeMismatch(2, "All codes must have the same size")
+        return cs, (C.c_void_p * len(cs))(*[c.ctypes.data for c in cs]), (cs[0].shape[0] if cs else 0)
+
+    def rs_prove(self, coeffs_list, transcript):
+        """host coefficients, one array per polynomial (needs a single-process handle): reed_solomon of each + BatchedFriProof::prove"""
+        cs, ptrs, n = self._arrays(coeffs_list)
+        h = C.c_void_p()
+        check(load().ml_bfri_shard_rs_prove(self.h, ptrs, _sz(len(cs)), _sz(n), transcript.h, C.byref(h)))
+        return FriProof(h, batched=True)
+
+    def prove(self, codes, gen_pows, transcript):
+        """host codes (needs a single-process handle) — the drop-in for batched_fri.rs:286"""
+        cs, ptrs, n = self._arrays(codes)
+        gp = as_elems(gen_pows) if gen_pows is not None else None
+        h = C.c_void_p()
+        check(load().ml_bfri_shard_prove(self.h, ptrs, _sz(len(cs)), _sz(n), _p(gp) if gp is not None else None,
+                                         _sz(gp.shape[0] if gp is not None else 0), transcript.h, C.byref(h)))
+        return FriProof(h, batched=True)
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_bfri_shard_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class ShardedWideSumcheck:
     """The width-w System sumcheck over the GPUs of one box (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu).  Rank g holds the row
     block matrix[g*h/G, (g+1)*h/G) of the row-major trace.  Handles as for ShardedPCSProver.  One call equals

@@ -1,7 +1,8 @@
 // One BatchedPCSProof::prove (batched_pcs.rs:130-180) with every polynomial split by block over G ranks, one GPU each; the proof is
 // byte-identical to ml_batched_pcs_prove's.  Notation and the segment layout are pcs_shard.cu's; rank b holds the block
 // evals_j[b*n/G, (b+1)*n/G) of each of the B polynomials.  Only what a batched proof does differently lives here; the encode
-// exchange, the combine, rounds 1 .. L-1, the tail and the openings of layers >= 1 are the stages of pcs_shard.h.
+// exchange, the combine, rounds 1 .. L-1, the tail and the openings of layers >= 1 are the stages of pcs_shard.h.  The batched
+// layer 0 (pipeline, commit, round-0 fold, openings and the BatchedFriProof) is shared with bfri_shard.cu through pcs_shard.h.
 //
 //   S0  per polynomial j: encode the local block (encode_into) into one of two buffers on the main stream while the side stream
 //       stores slice r of code j-1 into rank r's recv slice j-1 (one recv slice per polynomial); flag PX -> all.
@@ -97,37 +98,53 @@ __global__ void __launch_bounds__(64) bpcs_shard_open0_kernel(const unsigned lon
 
 }  // namespace
 
-struct ml_bpcs_shard : ShardCore {
-    struct Events { cudaEvent_t done[2] = {nullptr, nullptr}, free[2] = {nullptr, nullptr}, join = nullptr; };
-    std::vector<Events> ev;  // per local rank: the S0 encode / exchange pipeline
-    size_t R0 = 0;           // leaves of a layer-0 segment (R, or N/2 at G = 1)
-    int segs0 = 1, cnt0 = 1; // layer-0 segments per rank, run roots of the batch tree
-};
+namespace mlbs {
 
-namespace {
+int batch_init(BatchCore* sh) {
+    const size_t B = sh->B;
+    sh->R0 = sh->world == 1 ? sh->n : sh->R;
+    sh->segs0 = sh->world == 1 ? 1 : sh->world / 2;
+    sh->cnt0 = sh->world == 1 ? 1 : sh->world * sh->world / 2;
+    sh->ev.resize(sh->local.size());
+    int st = ML_OK;
+    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
+        PeerRank& r = sh->local[i];
+        cudaSetDevice(r.device);
+        BatchCore::Events& e = sh->ev[i];
+        for (cudaEvent_t* x : {&e.done[0], &e.done[1], &e.free[0], &e.free[1], &e.join})
+            if (cudaEventCreateWithFlags(x, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); st = ML_ERR_CUDA; }
+        // code pointers of every layer-0 segment: segment p of code c at layer0 + c * NL + p * 2 R0
+        std::vector<const fe*> ptrs((size_t)sh->segs0 * B);
+        for (int p = 0; p < sh->segs0; p++)
+            for (size_t c = 0; c < B; c++) ptrs[(size_t)p * B + c] = at(r, sh->lay.layer[0]) + c * sh->NL + (size_t)p * 2 * sh->R0;
+        if (st == ML_OK && cudaMemcpy(r.arena + sh->lay.segptrs, ptrs.data(), ptrs.size() * sizeof(void*), cudaMemcpyHostToDevice) != cudaSuccess) {
+            cudaGetLastError();
+            st = ML_ERR_CUDA;
+        }
+    }
+    return st;
+}
 
-const char* WHO = "ml_bpcs_shard";
+void batch_free(BatchCore* sh) {
+    DeviceGuard guard;
+    for (size_t i = 0; i < sh->ev.size(); i++) {
+        cudaSetDevice(sh->local[i].device);
+        BatchCore::Events& e = sh->ev[i];
+        for (cudaEvent_t x : {e.done[0], e.done[1], e.free[0], e.free[1], e.join})
+            if (x) cudaEventDestroy(x);
+    }
+}
 
-// S0 of one rank: transcript and claim, B encodes, each exchanged while the next one runs
-int bstage_encode(ml_bpcs_shard* sh, size_t li, const void* const* evals, const uint8_t* tr_state, const uint8_t* outputs) {
+int batch_encode_exchange(BatchCore* sh, size_t li, const std::function<int(size_t j, fe* y, cudaStream_t s)>& encode) {
     PeerRank& r = sh->local[li];
-    MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main, side = r.st.side;
     const Layout& a = sh->lay;
-    const size_t B = sh->B, NL = sh->NL;
-    MLB_TRY(h2d(r.arena + a.tr, tr_state, sizeof(DevTranscript), s));
-    MLB_TRY(h2d(r.arena + a.outs, outputs, B * 16, s));
-    MLB_TRY(h2d(r.arena + a.eptrs, evals, B * sizeof(void*), s));
-    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, s));
-    if (sh->world == 1) {
-        for (size_t j = 0; j < B; j++) MLB_TRY(encode_into(r.ctx, (const fe*)evals[j], sh->nloc, at(r, a.layer[0]) + j * NL, s));
-        return ML_OK;
-    }
-    ml_bpcs_shard::Events& e = sh->ev[li];
-    for (size_t j = 0; j < B; j++) {
+    const size_t NL = sh->NL;
+    BatchCore::Events& e = sh->ev[li];
+    for (size_t j = 0; j < sh->B; j++) {
         fe* y = at(r, a.ycode) + (j & 1) * NL;
         MLB_CUDA(cudaStreamWaitEvent(s, e.free[j & 1], 0));  // the exchange of polynomial j-2 has read this buffer
-        MLB_TRY(encode_into(r.ctx, (const fe*)evals[j], sh->nloc, y, s));
+        MLB_TRY(encode(j, y, s));
         MLB_CUDA(cudaEventRecord(e.done[j & 1], s));
         MLB_CUDA(cudaStreamWaitEvent(side, e.done[j & 1], 0));
         MLB_TRY(exchange_launch(sh, r, y, a.recv + j * NL * 16, side));
@@ -138,8 +155,7 @@ int bstage_encode(ml_bpcs_shard* sh, size_t li, const void* const* evals, const 
     return peer_signal(sh->grp, r, PX, -1, s);
 }
 
-// S1 of one rank: combine every code into layer 0, batched segment subtrees, run roots -> all (flag PB)
-int bstage_commit(ml_bpcs_shard* sh, PeerRank& r) {
+int batch_commit(BatchCore* sh, PeerRank& r, bool combine, bool mobius) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     const Layout& a = sh->lay;
@@ -149,48 +165,20 @@ int bstage_commit(ml_bpcs_shard* sh, PeerRank& r) {
         const RootTables* rt;
         MLB_TRY(get_root_tables(r.ctx, log_N, s, &rt));  // never a lazy build behind a spinning wait
         MLB_TRY(peer_wait(sh->grp, r, PX, -1, s));
-        for (size_t j = 0; j < B; j++) MLB_TRY(combine_launch(sh->L, at(r, a.recv) + j * NL, sh->R, r.rank, log_N, rt, at(r, a.layer[0]) + j * NL, s));
+        if (combine)
+            for (size_t j = 0; j < B; j++)
+                MLB_TRY(combine_launch(sh->L, at(r, a.recv) + j * NL, sh->R, r.rank, log_N, rt, at(r, a.layer[0]) + j * NL, s, mobius));
     }
     const fe* const* ptrs = reinterpret_cast<const fe* const*>(r.arena + a.segptrs);
     for (int p = 0; p < sh->segs0; p++) MLB_TRY(merkle_batched_rs_launch(ptrs + (size_t)p * B, B, 2 * R0, r.arena + a.dig[0] + 32 * (size_t)p * 2 * R0, s));
     return post_launch(sh, r, r.arena + a.dig[0], R0, sh->segs0, -1, a.mail[0], mail_partials(a, 0), PB);
 }
 
-const uint8_t* batch_root(const ml_bpcs_shard* sh, const PeerRank& r) {
+const uint8_t* batch_root(const BatchCore* sh, const PeerRank& r) {
     return r.arena + sh->lay.top[0] + 32 * merkle_layer_offset((size_t)sh->cnt0, ilog2((size_t)sh->cnt0));
 }
 
-// S2 + S3 of one rank: batch root, rho and claim; fingerprinted tables -> owners (flag PT); eq table
-int bstage_tables(ml_bpcs_shard* sh, PeerRank& r, const std::vector<hfe>& pts) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    cudaStream_t s = r.st.main;
-    const Layout& a = sh->lay;
-    MLB_TRY(top_launch(sh, r, PB, 0, sh->cnt0));
-    bpcs_shard_root_kernel<<<1, 32, 0, s>>>(batch_root(sh, r), (DevTranscript*)(r.arena + a.tr), at(r, a.outs), (int)sh->B, at(r, a.rho), at(r, a.prev));
-    MLB_KERNEL_CHECK();
-    fe* fp = sh->world == 1 ? at(r, a.tail_m) : at(r, a.ycode);  // the encode buffers are free once S0 is done
-    MLB_TRY(fingerprint_rows_launch((const fe* const*)(r.arena + a.eptrs), sh->B, sh->nloc, 0, fp, s, at(r, a.rho)));
-    if (sh->world == 1) return local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.tail_d), s);
-    MLB_TRY(tables_launch(sh, r, fp, a.m, s));
-    MLB_TRY(local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.d), s));
-    return peer_signal(sh->grp, r, PT, -1, s);
-}
-
-// round 0, phase A: wait for the tables, partial sums -> all (flag PR_0)
-int bstage_post0(ml_bpcs_shard* sh, PeerRank& r, int* nb) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    const Layout& a = sh->lay;
-    MLB_TRY(peer_wait(sh->grp, r, PT, -1, r.st.main));
-    MLB_TRY(sumcheck_sums_partials_launch(at(r, a.m), at(r, a.d), sh->nloc, at(r, a.part), nb, r.st.main));
-    return post_launch(sh, r, nullptr, sh->R, 0, *nb, a.mail[0], mail_partials(a, 0), PR0);
-}
-// round 0, phase B: round polynomial and r_0 (no root: the batch root was absorbed in S2)
-int bstage_round0(ml_bpcs_shard* sh, PeerRank& r) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    MLB_TRY(peer_wait(sh->grp, r, PR0, -1, r.st.main));
-    return finish_launch(sh, r, 0, nullptr);
-}
-int launch_fold0(ml_bpcs_shard* sh, PeerRank& r, const fe* r_dev, fe* out, cudaStream_t s) {
+int batch_fold0_launch(BatchCore* sh, PeerRank& r, const fe* r_dev, fe* out, cudaStream_t s) {
     const int log_N = (int)sh->n_vars + ML_LOG_BLOWUP;
     const RootTables* rt;
     MLB_TRY(get_root_tables(r.ctx, log_N, s, &rt));
@@ -200,16 +188,8 @@ int launch_fold0(ml_bpcs_shard* sh, PeerRank& r, const fe* r_dev, fe* out, cudaS
     MLB_KERNEL_CHECK();
     return ML_OK;
 }
-// round 0, phase C: fingerprint + first fold of the codes, fold of the tables
-int bstage_fold0(ml_bpcs_shard* sh, PeerRank& r, int* nb) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    MLB_TRY(launch_fold0(sh, r, at(r, sh->lay.r), fold_target(sh, r, 0), r.st.main));
-    return fold_tables(sh, r, 0, nb);
-}
 
-// openings and the proof on rank 0 (batched_fri.rs:296-308): layer 0 and layers 1 .. L-1 from the owners' arenas, the rest from
-// the tail's FriProverData
-int bassemble(ml_bpcs_shard* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_bfri_proof* p, const uint8_t* roots_lo) {
+int assemble_bfri(BatchCore* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_bfri_proof* p, const uint8_t* roots_lo) {
     cudaStream_t s = r0.st.main;
     if (f->layers.empty()) { set_error("open_query_at: no folded layer (domain too small)"); return ML_ERR_OUT_OF_RANGE; }  // n_vars = 1
     const int L = sh->L, Ls = L > 1 ? L : 1;  // layers held outside the tail's FriProverData
@@ -265,6 +245,69 @@ int bassemble(ml_bpcs_shard* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t
     return ML_OK;
 }
 
+}  // namespace mlbs
+
+struct ml_bpcs_shard : BatchCore {};
+
+namespace {
+
+const char* WHO = "ml_bpcs_shard";
+
+// S0 of one rank: transcript and claim, B encodes, each exchanged while the next one runs
+int bstage_encode(ml_bpcs_shard* sh, size_t li, const void* const* evals, const uint8_t* tr_state, const uint8_t* outputs) {
+    PeerRank& r = sh->local[li];
+    MLB_CUDA(cudaSetDevice(r.device));
+    cudaStream_t s = r.st.main;
+    const Layout& a = sh->lay;
+    const size_t B = sh->B, NL = sh->NL;
+    MLB_TRY(h2d(r.arena + a.tr, tr_state, sizeof(DevTranscript), s));
+    MLB_TRY(h2d(r.arena + a.outs, outputs, B * 16, s));
+    MLB_TRY(h2d(r.arena + a.eptrs, evals, B * sizeof(void*), s));
+    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, s));
+    if (sh->world == 1) {
+        for (size_t j = 0; j < B; j++) MLB_TRY(encode_into(r.ctx, (const fe*)evals[j], sh->nloc, at(r, a.layer[0]) + j * NL, s));
+        return ML_OK;
+    }
+    return batch_encode_exchange(sh, li, [&](size_t j, fe* y, cudaStream_t st) { return encode_into(r.ctx, (const fe*)evals[j], sh->nloc, y, st); });
+}
+
+// S2 + S3 of one rank: batch root, rho and claim; fingerprinted tables -> owners (flag PT); eq table
+int bstage_tables(ml_bpcs_shard* sh, PeerRank& r, const std::vector<hfe>& pts) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    cudaStream_t s = r.st.main;
+    const Layout& a = sh->lay;
+    MLB_TRY(top_launch(sh, r, PB, 0, sh->cnt0));
+    bpcs_shard_root_kernel<<<1, 32, 0, s>>>(batch_root(sh, r), (DevTranscript*)(r.arena + a.tr), at(r, a.outs), (int)sh->B, at(r, a.rho), at(r, a.prev));
+    MLB_KERNEL_CHECK();
+    fe* fp = sh->world == 1 ? at(r, a.tail_m) : at(r, a.ycode);  // the encode buffers are free once S0 is done
+    MLB_TRY(fingerprint_rows_launch((const fe* const*)(r.arena + a.eptrs), sh->B, sh->nloc, 0, fp, s, at(r, a.rho)));
+    if (sh->world == 1) return local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.tail_d), s);
+    MLB_TRY(tables_launch(sh, r, fp, a.m, s));
+    MLB_TRY(local_eq_table(r.ctx, pts, (int)sh->n_vars, sh->L, r.rank, at(r, a.d), s));
+    return peer_signal(sh->grp, r, PT, -1, s);
+}
+
+// round 0, phase A: wait for the tables, partial sums -> all (flag PR_0)
+int bstage_post0(ml_bpcs_shard* sh, PeerRank& r, int* nb) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    const Layout& a = sh->lay;
+    MLB_TRY(peer_wait(sh->grp, r, PT, -1, r.st.main));
+    MLB_TRY(sumcheck_sums_partials_launch(at(r, a.m), at(r, a.d), sh->nloc, at(r, a.part), nb, r.st.main));
+    return post_launch(sh, r, nullptr, sh->R, 0, *nb, a.mail[0], mail_partials(a, 0), PR0);
+}
+// round 0, phase B: round polynomial and r_0 (no root: the batch root was absorbed in S2)
+int bstage_round0(ml_bpcs_shard* sh, PeerRank& r) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    MLB_TRY(peer_wait(sh->grp, r, PR0, -1, r.st.main));
+    return finish_launch(sh, r, 0, nullptr);
+}
+// round 0, phase C: fingerprint + first fold of the codes, fold of the tables
+int bstage_fold0(ml_bpcs_shard* sh, PeerRank& r, int* nb) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    MLB_TRY(batch_fold0_launch(sh, r, at(r, sh->lay.r), fold_target(sh, r, 0), r.st.main));
+    return fold_tables(sh, r, 0, nb);
+}
+
 // rank 0: the rest of the fold chain (at G = 1 from the batched first fold), the openings, the final transcript to everybody
 int bprove_tail(ml_bpcs_shard* sh, PeerRank& r0, const std::vector<hfe>& pts, const uint8_t* outputs, ml_transcript* t, ml_bpcs_proof** out) {
     ml_fri* f = new ml_fri();
@@ -277,11 +320,11 @@ int bprove_tail(ml_bpcs_shard* sh, PeerRank& r0, const std::vector<hfe>& pts, co
         hooks.first_fold = [&](const fe* r_dev, fe** next, bool* owns) {
             *owns = false;  // the tail code buffer of the arena
             *next = at(r0, sh->lay.tail_code);
-            return launch_fold0(sh, r0, r_dev, *next, r0.st.main);
+            return batch_fold0_launch(sh, r0, r_dev, *next, r0.st.main);
         };
     uint8_t roots_lo[MAX_L * 32] = {0};
     MLB_TRY(tail_chain(sh, r0, f, hooks, p->sumcheck.data(), roots_lo, t, 4));
-    MLB_TRY(bassemble(sh, r0, f, t, &p->fri, roots_lo));
+    MLB_TRY(assemble_bfri(sh, r0, f, t, &p->fri, roots_lo));
     if (&r0 == &sh->local[0]) mark_phase(sh, 6);
     p->inputs = pts;
     p->outputs.resize(sh->B);
@@ -297,13 +340,7 @@ extern "C" {
 
 void ml_bpcs_shard_free(ml_bpcs_shard* sh) {
     if (!sh) return;
-    DeviceGuard guard;
-    for (size_t i = 0; i < sh->ev.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        ml_bpcs_shard::Events& e = sh->ev[i];
-        for (cudaEvent_t x : {e.done[0], e.done[1], e.free[0], e.free[1], e.join})
-            if (x) cudaEventDestroy(x);
-    }
+    batch_free(sh);
     shard_free(sh);
     delete sh;
 }
@@ -320,25 +357,7 @@ int ml_bpcs_shard_create(int world, int n_local, const int* local_ranks, const i
     ml_bpcs_shard* sh = new ml_bpcs_shard();
     sh->who = WHO;
     int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, n_polys, "ml_bpcs_shard_create");
-    sh->R0 = world == 1 ? sh->n : sh->R;
-    sh->segs0 = world == 1 ? 1 : world / 2;
-    sh->cnt0 = world == 1 ? 1 : world * world / 2;
-    sh->ev.resize(sh->local.size());
-    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        cudaSetDevice(r.device);
-        ml_bpcs_shard::Events& e = sh->ev[i];
-        for (cudaEvent_t* x : {&e.done[0], &e.done[1], &e.free[0], &e.free[1], &e.join})
-            if (cudaEventCreateWithFlags(x, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); st = ML_ERR_CUDA; }
-        // code pointers of every layer-0 segment: segment p of code c at layer0 + c * NL + p * 2 R0
-        std::vector<const fe*> ptrs((size_t)sh->segs0 * n_polys);
-        for (int p = 0; p < sh->segs0; p++)
-            for (size_t c = 0; c < n_polys; c++) ptrs[(size_t)p * n_polys + c] = at(r, sh->lay.layer[0]) + c * sh->NL + (size_t)p * 2 * sh->R0;
-        if (st == ML_OK && cudaMemcpy(r.arena + sh->lay.segptrs, ptrs.data(), ptrs.size() * sizeof(void*), cudaMemcpyHostToDevice) != cudaSuccess) {
-            cudaGetLastError();
-            st = ML_ERR_CUDA;
-        }
-    }
+    if (st == ML_OK) st = batch_init(sh);
     if (st != ML_OK) { ml_bpcs_shard_free(sh); return st; }
     *out = sh;
     return ML_OK;
@@ -378,7 +397,7 @@ int ml_bpcs_shard_prove_dev(ml_bpcs_shard* sh, const uint8_t* inputs, size_t n_v
     mark_phase(sh, 0);
     for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_encode(sh, i, local_evals_dev + i * n_polys, tr_state, outputs));
     mark_phase(sh, 1);
-    for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_commit(sh, sh->local[i]));
+    for (size_t i = 0; i < nl; i++) MLB_TRY(batch_commit(sh, sh->local[i], true, true));
     mark_phase(sh, 2);
     for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_tables(sh, sh->local[i], pts));
     mark_phase(sh, 3);

@@ -2,7 +2,8 @@
 // (reed_solomon + prove, fri/mod.rs:19-28) or by its code; the proof is byte-identical to ml_rs_fri_prove's / ml_fri_prove's.
 // Notation and the segment layout are pcs_shard.cu's: L = log2 G, n coefficients, N = 2n, NL = N/G, R = N/G^2, w = w_N.
 // Only what a FRI proof does differently lives here; the column exchange, the combine, the segment subtrees, the top hash, the
-// fold, the tail and the openings of the sharded layers are the stages of pcs_shard.h.
+// fold, the tail and the openings of the sharded layers are the stages of pcs_shard.h.  The placement of a given code and the
+// table-free round (fri_round, fri_fold) are shared with bfri_shard.cu through pcs_shard.h.
 //
 //   Coefficients.  With j = j1 + G*j2 and Y_j1 = reed_solomon(c[j1 + G*j2 : j2 < n/G], w^G) (the RS-encode NTT at length NL),
 //       code[k2 + NL*k1] = sum_j1 w_G^(j1*k1) * w^(j1*k2) * Y_j1[k2]:
@@ -30,7 +31,7 @@ using namespace mlbs;
 
 namespace {
 
-// S0 of the code entry: slice [dest*R, (dest+1)*R) of this rank's block = run `rank` of rank dest's layer 0
+// S0 of the code entry: slice [dest*R, (dest+1)*R) of this rank's block = run `rank` of rank dest's code at off_layer0
 __global__ void __launch_bounds__(256) fri_shard_place_kernel(const fe* __restrict__ code, size_t NL, size_t R, int rank, int world, PeerPtrs peers,
                                                               size_t off_layer0) {
     const size_t stride = (size_t)gridDim.x * blockDim.x;
@@ -42,6 +43,35 @@ __global__ void __launch_bounds__(256) fri_shard_place_kernel(const fe* __restri
 
 }  // namespace
 
+namespace mlbs {
+
+int fri_begin(ShardCore* sh, PeerRank& r, const uint8_t* tr_state) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    MLB_TRY(h2d(r.arena + sh->lay.tr, tr_state, sizeof(DevTranscript), r.st.main));
+    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, r.st.main));
+    return ML_OK;
+}
+int place_launch(ShardCore* sh, PeerRank& r, const fe* code, size_t off_code, cudaStream_t s) {
+    fri_shard_place_kernel<<<peer_grid(sh->NL), 256, 0, s>>>(code, sh->NL, sh->R, r.rank, sh->world, sh->grp.peers(), off_code);
+    MLB_KERNEL_CHECK();
+    return ML_OK;
+}
+int fri_round(ShardCore* sh, PeerRank& r, int k) {
+    MLB_CUDA(cudaSetDevice(r.device));
+    const Layout& a = sh->lay;
+    const int cnt = (sh->world * sh->world) >> (k + 1);
+    MLB_TRY(top_launch(sh, r, PR0 + k, k, cnt));
+    const uint8_t* root = r.arena + a.top[k] + 32 * merkle_layer_offset((size_t)cnt, ilog2((size_t)cnt));
+    return chain_challenge_launch((DevTranscript*)(r.arena + a.tr), root, 32, r.arena + a.roots_out + 32 * k, at(r, a.r), true, r.st.main);
+}
+int fri_fold(ShardCore* sh, PeerRank& r, int k) {
+    MLB_TRY(fold_code(sh, r, k));
+    if (k + 1 < sh->L) return ML_OK;
+    return peer_signal(sh->grp, r, PG, 0, r.st.main);
+}
+
+}  // namespace mlbs
+
 struct ml_fri_shard : ShardCore {};
 
 namespace {
@@ -50,17 +80,9 @@ const char* WHO = "ml_fri_shard";
 
 int log_N_of(const ml_fri_shard* sh) { return (int)sh->n_vars + ML_LOG_BLOWUP; }
 
-// transcript state and status word of one rank at the start of a call
-int fstage_begin(ml_fri_shard* sh, PeerRank& r, const uint8_t* tr_state) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    MLB_TRY(h2d(r.arena + sh->lay.tr, tr_state, sizeof(DevTranscript), r.st.main));
-    MLB_CUDA(cudaMemsetAsync(sh->grp.status(r), 0, 16, r.st.main));
-    return ML_OK;
-}
-
 // G = 1: layer 0 straight into the tail buffer
 int fstage_local(ml_fri_shard* sh, PeerRank& r, const fe* src, bool rs, const uint8_t* tr_state) {
-    MLB_TRY(fstage_begin(sh, r, tr_state));
+    MLB_TRY(fri_begin(sh, r, tr_state));
     fe* code = at(r, sh->lay.tail_code);
     if (rs) return ntt_launch(r.ctx, src, code, log_N_of(sh), false, true, r.st.main);
     MLB_CUDA(cudaMemcpyAsync(code, src, sh->NL * 16, cudaMemcpyDeviceToDevice, r.st.main));
@@ -69,7 +91,7 @@ int fstage_local(ml_fri_shard* sh, PeerRank& r, const fe* src, bool rs, const ui
 
 // S0, coefficients: the caller's block -> the owners' coefficient buffers (flag PC)
 int fstage_transpose(ml_fri_shard* sh, PeerRank& r, const fe* coeffs, const uint8_t* tr_state) {
-    MLB_TRY(fstage_begin(sh, r, tr_state));
+    MLB_TRY(fri_begin(sh, r, tr_state));
     const RootTables* rt;
     MLB_TRY(get_root_tables(r.ctx, log_N_of(sh), r.st.main, &rt));  // never a lazy build behind a spinning wait
     MLB_TRY(tables_launch(sh, r, coeffs, sh->lay.coef, r.st.main, true));
@@ -87,11 +109,10 @@ int fstage_encode(ml_fri_shard* sh, PeerRank& r) {
 }
 // S0, code: the caller's block -> run `rank` of every rank's layer 0 (flag PX)
 int fstage_place(ml_fri_shard* sh, PeerRank& r, const fe* code, const uint8_t* tr_state) {
-    MLB_TRY(fstage_begin(sh, r, tr_state));
+    MLB_TRY(fri_begin(sh, r, tr_state));
     const RootTables* rt;
     MLB_TRY(get_root_tables(r.ctx, log_N_of(sh), r.st.main, &rt));
-    fri_shard_place_kernel<<<peer_grid(sh->NL), 256, 0, r.st.main>>>(code, sh->NL, sh->R, r.rank, sh->world, sh->grp.peers(), sh->lay.layer[0]);
-    MLB_KERNEL_CHECK();
+    MLB_TRY(place_launch(sh, r, code, sh->lay.layer[0], r.st.main));
     return peer_signal(sh->grp, r, PX, -1, r.st.main);
 }
 // S1: wait PX; coefficients: combine the received columns into layer 0
@@ -103,22 +124,6 @@ int fstage_combine(ml_fri_shard* sh, PeerRank& r, bool rs) {
     if (!rs) return ML_OK;
     return combine_launch(sh->L, at(r, sh->lay.recv), sh->R, r.rank, log_N_of(sh), rt, at(r, sh->lay.layer[0]), r.st.main, false);
 }
-// round k, phase B: top of the layer tree; absorb its root, draw r_k (identical on every rank)
-int fstage_round(ml_fri_shard* sh, PeerRank& r, int k) {
-    MLB_CUDA(cudaSetDevice(r.device));
-    const Layout& a = sh->lay;
-    const int cnt = (sh->world * sh->world) >> (k + 1);
-    MLB_TRY(top_launch(sh, r, PR0 + k, k, cnt));
-    const uint8_t* root = r.arena + a.top[k] + 32 * merkle_layer_offset((size_t)cnt, ilog2((size_t)cnt));
-    return chain_challenge_launch((DevTranscript*)(r.arena + a.tr), root, 32, r.arena + a.roots_out + 32 * k, at(r, a.r), true, r.st.main);
-}
-// round k, phase C: fold; after the last sharded round layer L is in rank 0's tail code (flag PG)
-int fstage_fold(ml_fri_shard* sh, PeerRank& r, int k) {
-    MLB_TRY(fold_code(sh, r, k));
-    if (k + 1 < sh->L) return ML_OK;
-    return peer_signal(sh->grp, r, PG, 0, r.st.main);
-}
-
 // rank 0: the rest of the fold chain from layer L, the openings, the final transcript to everybody
 int fprove_tail(ml_fri_shard* sh, PeerRank& r0, ml_transcript* t, ml_fri_proof** out) {
     ml_fri* f = new ml_fri();
@@ -160,8 +165,8 @@ int fri_shard_run(ml_fri_shard* sh, const void* const* blocks, bool rs, ml_trans
         mark_phase(sh, 2);
         for (int k = 0; k < sh->L; k++) {
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_post(sh, sh->local[i], k, -1));
-            for (size_t i = 0; i < nl; i++) MLB_TRY(fstage_round(sh, sh->local[i], k));
-            for (size_t i = 0; i < nl; i++) MLB_TRY(fstage_fold(sh, sh->local[i], k));
+            for (size_t i = 0; i < nl; i++) MLB_TRY(fri_round(sh, sh->local[i], k));
+            for (size_t i = 0; i < nl; i++) MLB_TRY(fri_fold(sh, sh->local[i], k));
         }
     }
     int st0 = ML_OK;

@@ -252,18 +252,19 @@ Layout make_layout(size_t n, int G, size_t B, bool fri) {
     for (int k = 0; k < MAX_L; k++) a.top[k] = take(2 * MAIL_ROOTS * 32);
     a.part = take(fri ? 0 : (size_t)(2 * sumcheck_max_blocks() + 2) * 16);
     a.rho = take(batched ? 16 : 0);
-    a.outs = take(B * 16);
-    a.eptrs = take(B * 8);
+    a.outs = take(fri ? 0 : B * 16);
+    a.eptrs = take(fri ? 0 : B * 8);
     a.segptrs = take((sharded ? (size_t)G / 2 : 1) * B * 8);
     // batched: two encode buffers (the encode of polynomial j+1 overlaps the exchange of j) and one recv slice per polynomial
     a.ycode = take(sharded ? (batched ? 2 : 1) * NL * 16 : 0);
     a.recv = take(sharded ? (batched ? B : 1) * NL * 16 : 0);
-    a.coef = take(sharded && fri ? nloc * 16 : 0);
+    a.coef = take(sharded && fri && !batched ? nloc * 16 : 0);
     for (int k = 0; k < MAX_L; k++) {
         const bool held = k < L || (k == 0 && batched);
         a.layer[k] = take(held ? (k == 0 && batched ? B : 1) * ((size_t)G >> k) * R * 16 : 0);
         a.dig[k] = take(held ? ((size_t)G >> k) * R * 32 : 0);
     }
+    if (sharded && fri && batched) a.coef = a.layer[0];  // B slices of nloc: read by the encodes, before any combine writes layer 0
     a.m = take(sharded && !fri ? nloc * 16 : 0);
     a.d = take(sharded && !fri ? nloc * 16 : 0);
     a.tail_code = take(NL * 16);

@@ -1,7 +1,8 @@
 // Stages of the block-sharded provers, shared by pcs_shard.cu (one PCSProof::prove, ml_pcs_shard_*), bpcs_shard.cu (one
-// BatchedPCSProof::prove, ml_bpcs_shard_*) and fri_shard.cu (one FriProof::prove, ml_fri_shard_*).  All split every polynomial by
-// block over G ranks and keep the sharded layers in the segment layout described at the top of pcs_shard.cu; the batched prover
-// only adds a batched layer 0 and round 0, the FRI prover drops the sumcheck tables.
+// BatchedPCSProof::prove, ml_bpcs_shard_*), fri_shard.cu (one FriProof::prove, ml_fri_shard_*) and bfri_shard.cu (one
+// BatchedFriProof::prove, ml_bfri_shard_*).  All split every polynomial by block over G ranks and keep the sharded layers in the
+// segment layout described at the top of pcs_shard.cu; the batched provers add a batched layer 0 and round 0 (implemented in
+// bpcs_shard.cu), the FRI provers drop the sumcheck tables (their table-free stages are implemented in fri_shard.cu).
 #pragma once
 #include "peer.h"
 #include "prover_internal.h"
@@ -10,7 +11,7 @@ namespace mlbs {
 using namespace mlb;
 using namespace mlbp;
 
-// PR0 + k: round k (L <= 4); PB, PT: batched prover only; PC: FRI prover only (coefficient transpose)
+// PR0 + k: round k (L <= 4); PB: batched provers only; PT: batched PCS prover only; PC: FRI provers only (coefficient transpose)
 enum Phase { PX = 0, PR0 = 1, PG = PR0 + 4, PF, PB, PT, PC, N_PHASES };
 static const int MAXR = PEER_MAXR;
 static const int MAX_L = 4;
@@ -19,10 +20,10 @@ static const size_t MAIL_ROOTS = (size_t)MAXR * MAXR / 2;  // run roots of layer
 struct Layout {
     size_t flags, status, tr, prev, r, sc, roots_out, final_tr, mail[MAX_L], top[MAX_L], part;  // mailbox (cleared at create)
     size_t rho, outs, eptrs, segptrs;                                                          // batched prover only
-    size_t ycode, recv, coef, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;  // coef: FRI prover only
+    size_t ycode, recv, coef, layer[MAX_L], dig[MAX_L], m, d, tail_code, tail_m, tail_d, total;  // coef: FRI provers only
 };
-// B = 0: one polynomial; B >= 1: a batch of B polynomials (layer 0 holds B codes); fri: one polynomial without sumcheck tables,
-// with a receive buffer for the transposed coefficients instead
+// B = 0: one polynomial; B >= 1: a batch of B polynomials (layer 0 holds B codes); fri: no sumcheck tables, with a receive buffer
+// for the transposed coefficients instead (batched: B slices of n/G inside layer 0, which is written only after they are encoded)
 Layout make_layout(size_t n, int G, size_t B, bool fri = false);
 // mailbox of round k: run root of run q at roots + 32 q, partial pair of rank g at partials + 32 g
 inline size_t mail_partials(const Layout& a, int k) { return a.mail[k] + MAIL_ROOTS * 32; }
@@ -97,6 +98,39 @@ int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t);
 // rank 0 after a failed call: its status into every rank's status word, then the same release (finish_ranks returns it)
 int tail_fail(ShardCore* sh, PeerRank& r0, int st);
 int finish_ranks(ShardCore* sh, ml_transcript* t, int st);
+
+// ---- the FRI provers (fri_shard.cu): no sumcheck tables, every layer root absorbed before its challenge
+// transcript state and status word of one rank at the start of a call
+int fri_begin(ShardCore* sh, PeerRank& r, const uint8_t* tr_state);
+// S0 of a given code: slice [r*R, (r+1)*R) of this rank's block `code` (N/G elements) = run `rank` of rank r's code at off_code
+int place_launch(ShardCore* sh, PeerRank& r, const fe* code, size_t off_code, cudaStream_t s);
+// round k, phase B: top of the layer tree; absorb its root, draw r_k (identical on every rank)
+int fri_round(ShardCore* sh, PeerRank& r, int k);
+// round k, phase C: fold; after the last sharded round layer L is in rank 0's tail code (flag PG)
+int fri_fold(ShardCore* sh, PeerRank& r, int k);
+
+// ---- the batched provers (bpcs_shard.cu): B codes in layer 0 under one batched tree
+struct BatchCore : ShardCore {
+    struct Events { cudaEvent_t done[2] = {nullptr, nullptr}, free[2] = {nullptr, nullptr}, join = nullptr; };
+    std::vector<Events> ev;  // per local rank: the S0 encode / exchange pipeline
+    size_t R0 = 0;           // leaves of a layer-0 segment (R, or N/2 at G = 1)
+    int segs0 = 1, cnt0 = 1; // layer-0 segments per rank, run roots of the batch tree
+};
+// after shard_init: the pipeline events and the code pointers of every layer-0 segment
+int batch_init(BatchCore* sh);
+void batch_free(BatchCore* sh);  // the events; then shard_free
+// S0 of local rank li (G > 1): per code j, encode(j, y, main) into one of two buffers on the main stream while the side stream
+// stores slice r of code j-1 into rank r's recv slice j-1; flag PX -> all
+int batch_encode_exchange(BatchCore* sh, size_t li, const std::function<int(size_t j, fe* y, cudaStream_t s)>& encode);
+// S1: G > 1: wait PX, then (combine) recv slice j -> layer-0 code j for every j; batched subtree of every segment, run roots -> all
+// (flag PB)
+int batch_commit(BatchCore* sh, PeerRank& r, bool combine, bool mobius);
+const uint8_t* batch_root(const BatchCore* sh, const PeerRank& r);
+// round 0: fingerprint (rho from the arena) + fold of the B layer-0 codes with the global leaf index into out
+int batch_fold0_launch(BatchCore* sh, PeerRank& r, const fe* r_dev, fe* out, cudaStream_t s);
+// rank 0: openings and the BatchedFriProof (batched_fri.rs:296-308): layer 0 and layers 1 .. L-1 from the owners' arenas, the
+// rest from the tail's FriProverData; roots_lo: the roots of the sharded layers (round 0 absorbed none)
+int assemble_bfri(BatchCore* sh, PeerRank& r0, const ml_fri* f, ml_transcript* t, ml_bfri_proof* p, const uint8_t* roots_lo);
 
 // segment-layout helpers on the device
 __device__ __forceinline__ int ilog2_dev(size_t x) { return 63 - __clzll((unsigned long long)x); }

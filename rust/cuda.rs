@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard, MlBfriShard);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -56,6 +56,16 @@ extern "C" {
     pub fn ml_bfri_proof_num_commitments(p: *const MlBfriProof) -> usize;
     pub fn ml_bfri_proof_serialize(p: *const MlBfriProof, out: *mut u8) -> c_int;
     pub fn ml_bfri_proof_serialized_len(p: *const MlBfriProof) -> usize;
+    pub fn ml_bfri_shard_arena_bytes(sh: *const MlBfriShard) -> usize;
+    pub fn ml_bfri_shard_connect(sh: *mut MlBfriShard, records: *const u8, n_records: usize) -> c_int;
+    pub fn ml_bfri_shard_create(world: c_int, n_local: c_int, local_ranks: *const c_int, local_devices: *const c_int, n_codes: usize, log_n: usize, out: *mut *mut MlBfriShard) -> c_int;
+    pub fn ml_bfri_shard_export(sh: *mut MlBfriShard, records_out: *mut u8) -> c_int;
+    pub fn ml_bfri_shard_free(sh: *mut MlBfriShard);
+    pub fn ml_bfri_shard_prove(sh: *mut MlBfriShard, codes: *const *const u8, n_codes: usize, n: usize, gen_pows: *const u8, gen_pows_len: usize, t: *mut MlTranscript, out: *mut *mut MlBfriProof) -> c_int;
+    pub fn ml_bfri_shard_prove_dev(sh: *mut MlBfriShard, local_codes_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlBfriProof) -> c_int;
+    pub fn ml_bfri_shard_rs_prove(sh: *mut MlBfriShard, coeffs: *const *const u8, n_codes: usize, n: usize, t: *mut MlTranscript, out: *mut *mut MlBfriProof) -> c_int;
+    pub fn ml_bfri_shard_rs_prove_dev(sh: *mut MlBfriShard, local_coeffs_dev: *const *const c_void, t: *mut MlTranscript, out: *mut *mut MlBfriProof) -> c_int;
+    pub fn ml_bfri_shard_stream(sh: *const MlBfriShard, local_index: c_int) -> *mut c_void;
     pub fn ml_bit_reverse_permutation(values: *mut u8, n: usize, elem_bytes: usize) -> c_int;
     pub fn ml_bpcs_proof_free(p: *mut MlBpcsProof);
     pub fn ml_bpcs_proof_fri(p: *const MlBpcsProof) -> *const MlBfriProof;
@@ -684,6 +694,51 @@ pub fn batched_fri_prove(codes: &[Vec<F>], gen_pows: &[F], transcript: &mut Tran
     let proof = unsafe { bfri_proof_from(h) };
     unsafe { ml_bfri_proof_free(h) };
     proof
+}
+/// `BatchedFriProof::prove` of B codes over all GPUs of the box from one process, every code split by block (ml_bfri_shard_*,
+/// csrc/bfri_shard.cu), from the codes of 2^(log_n+1) elements or from the polynomials' 2^log_n coefficients (`reed_solomon` of each
+/// + prove): rank g holds block g of G of every polynomial; round 0 and the next log2(G)-1 fold rounds run sharded, rank 0 runs the
+/// rest.  The handle is built once per shape (n_codes, log_n) and reused; the proof bytes equal `batched_fri_prove`'s.
+pub struct ShardedBatchedFriProver {
+    h: *mut MlBfriShard,
+}
+impl ShardedBatchedFriProver {
+    pub fn new(n_codes: usize, log_n: usize) -> Self {
+        let mut count = 0;
+        check(unsafe { ml_device_count(&mut count) });
+        let mut world = 1usize << (usize::BITS - 1 - (count.max(1) as usize).leading_zeros()); // largest power of two <= GPUs
+        while world > 1 && log_n < 2 * world.trailing_zeros() as usize {
+            world >>= 1; // log_n >= 2 log2(world)
+        }
+        let world = world.min(16) as c_int;
+        let ids: Vec<c_int> = (0..world).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_bfri_shard_create(world, world, ids.as_ptr(), ids.as_ptr(), n_codes, log_n, &mut h) });
+        Self { h }
+    }
+    /// body of `BatchedFriProof::prove` (src/fri/batched_fri.rs:286-318) for codes of the handle's shape
+    pub fn prove(&mut self, codes: &[Vec<F>], gen_pows: &[F], transcript: &mut Transcript) -> BatchedFriProof<F> {
+        let ptrs: Vec<*const u8> = codes.iter().map(|c| p(c)).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_bfri_shard_prove(self.h, ptrs.as_ptr(), codes.len(), codes[0].len(), p(gen_pows), gen_pows.len(), transcript.h, &mut h) });
+        let proof = unsafe { bfri_proof_from(h) };
+        unsafe { ml_bfri_proof_free(h) };
+        proof
+    }
+    /// `reed_solomon` (src/fri/mod.rs:19-28) of every polynomial + `BatchedFriProof::prove`
+    pub fn rs_prove(&mut self, coeffs: &[Vec<F>], transcript: &mut Transcript) -> BatchedFriProof<F> {
+        let ptrs: Vec<*const u8> = coeffs.iter().map(|c| p(c)).collect();
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_bfri_shard_rs_prove(self.h, ptrs.as_ptr(), coeffs.len(), coeffs[0].len(), transcript.h, &mut h) });
+        let proof = unsafe { bfri_proof_from(h) };
+        unsafe { ml_bfri_proof_free(h) };
+        proof
+    }
+}
+impl Drop for ShardedBatchedFriProver {
+    fn drop(&mut self) {
+        unsafe { ml_bfri_shard_free(self.h) }
+    }
 }
 /// `BatchedFriProverData<F>` (src/fri/batched_fri.rs:9-14) with the batch layer and every tree resident in HBM:
 /// init :41-99, batched_fold_step :101-181, fold :183-205, open_query_at :207-225; `fri_data()` borrows the inner FriProverData

@@ -11,7 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HANDLES = {"ml_transcript": "MlTranscript", "ml_merkle": "MlMerkle", "ml_fri": "MlFri", "ml_fri_proof": "MlFriProof", "ml_sumcheck": "MlSumcheck",
            "ml_wsumcheck": "MlWSumcheck", "ml_pcs_proof": "MlPcsProof", "ml_bfri_proof": "MlBfriProof", "ml_bpcs_proof": "MlBpcsProof",
            "ml_shard": "MlShard", "ml_bfri": "MlBfri", "ml_pcs_shard": "MlPcsShard", "ml_bpcs_shard": "MlBpcsShard",
-           "ml_wsumcheck_shard": "MlWSumcheckShard", "ml_fri_shard": "MlFriShard"}
+           "ml_wsumcheck_shard": "MlWSumcheckShard", "ml_fri_shard": "MlFriShard", "ml_bfri_shard": "MlBfriShard"}
 SCALARS = {"int": "c_int", "unsigned": "c_uint", "size_t": "usize", "uint64_t": "u64", "int64_t": "i64", "uint32_t": "u32", "uint8_t": "u8",
            "double": "f64", "char": "c_char", "void": "c_void"}
 BEGIN, END = "    // ---- GENERATED from include/multilinear_b200.h by tools/abi_tools.py (do not edit by hand)\n", "    // ---- END GENERATED\n"
