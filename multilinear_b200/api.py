@@ -800,37 +800,44 @@ class BatchedPCSProof:
         return PCSProof(h, batched=True)
 
 
-class ShardedBatchedProver:
-    """BatchedPCSProof::prove sharded over the GPUs of one box (ml_shard_*, csrc/shard.cu).  A handle hosts the ranks of one
-    process: all of them (single_process; devices may repeat = virtual ranks on one GPU) or one (one_rank; the records of all
-    processes are all-gathered by the caller's transport and passed to connect)."""
+class _ShardedHandle:
+    """What every sharded handle shares, over the C entries <_PREFIX>_create, _export, _connect, _stream, _arena_bytes,
+    _phase_ms and _free.  A handle hosts the ranks of one process: all of them (single_process; devices may repeat = virtual
+    ranks on one GPU) or one (one_rank; the records of all processes are all-gathered by the caller's transport and passed to
+    connect).  _SHAPE names the shape arguments, in the order the create entry takes them."""
+    _PREFIX, _SHAPE = None, ()
 
-    def __init__(self, h, world, local_ranks, n_polys, n_vars):
-        self.h, self.world, self.local_ranks, self.n_polys, self.n_vars = h, world, list(local_ranks), n_polys, n_vars
+    def __init__(self, h, world, local_ranks, *shape):
+        self.h, self.world, self.local_ranks = h, world, list(local_ranks)
+        for name, v in zip(self._SHAPE, shape):
+            setattr(self, name, v)
 
-    @staticmethod
-    def _create(world, ranks, devices, n_polys, n_vars):
+    def _fn(self, name):
+        return getattr(load(), "%s_%s" % (self._PREFIX, name))
+
+    @classmethod
+    def _create(cls, world, ranks, devices, *shape):
         h = C.c_void_p()
         ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_polys), _sz(n_vars), C.byref(h)))
-        return ShardedBatchedProver(h, world, ranks, n_polys, n_vars)
+        check(getattr(load(), cls._PREFIX + "_create")(C.c_int(world), C.c_int(len(ranks)), ra, da, *[_sz(v) for v in shape], C.byref(h)))
+        return cls(h, world, ranks, *shape)
 
-    @staticmethod
-    def single_process(devices, n_polys, n_vars):
-        return ShardedBatchedProver._create(len(devices), list(range(len(devices))), list(devices), n_polys, n_vars)
+    @classmethod
+    def single_process(cls, devices, *shape):
+        return cls._create(len(devices), list(range(len(devices))), list(devices), *shape)
 
-    @staticmethod
-    def one_rank(rank, world, device, n_polys, n_vars):
-        return ShardedBatchedProver._create(world, [rank], [device], n_polys, n_vars)
+    @classmethod
+    def one_rank(cls, rank, world, device, *shape):
+        return cls._create(world, [rank], [device], *shape)
 
     def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_shard_export(self.h, _p(out)))
+        out = np.empty(load().ml_shard_record_bytes() * len(self.local_ranks), dtype=np.uint8)
+        check(self._fn("export")(self.h, _p(out)))
         return out.tobytes()
 
     def connect(self, records):
         buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
+        check(self._fn("connect")(self.h, _p(buf), _sz(len(buf) // load().ml_shard_record_bytes())))
 
     def connect_over(self, dist, device):
         """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
@@ -841,13 +848,35 @@ class ShardedBatchedProver:
         self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
 
     def stream(self, local_index=0):
-        return load().ml_shard_stream(self.h, C.c_int(local_index))
+        return self._fn("stream")(self.h, C.c_int(local_index))
+
+    def arena_bytes(self):
+        return self._fn("arena_bytes")(self.h)
 
     def phase_ms(self):
         """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
         out = (C.c_double * 16)()
-        n = load().ml_shard_phase_ms(self.h, out, C.c_int(16))
+        n = self._fn("phase_ms")(self.h, out, C.c_int(16))
         return [out[i] for i in range(n)]
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            self._fn("free")(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+class ShardedBatchedProver(_ShardedHandle):
+    """BatchedPCSProof::prove sharded over the GPUs of one box (ml_shard_*, csrc/shard.cu).  A handle hosts the ranks of one
+    process: all of them (single_process; devices may repeat = virtual ranks on one GPU) or one (one_rank; the records of all
+    processes are all-gathered by the caller's transport and passed to connect)."""
+
+    _PREFIX, _SHAPE = "ml_shard", ("n_polys", "n_vars")
 
     def local_polys(self):
         """global polynomial indices in the order local_evals must be given: for each local rank, rank, rank + world, ..."""
@@ -875,70 +904,14 @@ class ShardedBatchedProver:
         check(load().ml_shard_batched_pcs_prove(self.h, _p(i), _sz(i.shape[0]), _p(o), _sz(len(ps)), ptrs, transcript.h, C.byref(h)))
         return PCSProof(h, batched=True)
 
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_shard_free(self.h)
-        self.h = None
 
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
-
-
-class BlockShardedBatchedProver:
+class BlockShardedBatchedProver(_ShardedHandle):
     """BatchedPCSProof::prove with every polynomial split by block over the GPUs of one box (ml_bpcs_shard_*,
     csrc/bpcs_shard.cu).  Rank g holds the block evals_j[g*n/G, (g+1)*n/G) of every polynomial j, so any batch size works on any
     power-of-two G.  Handles as for ShardedPCSProver: single_process (devices may repeat = virtual ranks on one GPU) or one_rank
     with connect / connect_over.  The proof is an ordinary batched PCSProof, byte-identical to BatchedPCSProof.prove's."""
 
-    def __init__(self, h, world, local_ranks, n_polys, n_vars):
-        self.h, self.world, self.local_ranks, self.n_polys, self.n_vars = h, world, list(local_ranks), n_polys, n_vars
-
-    @staticmethod
-    def _create(world, ranks, devices, n_polys, n_vars):
-        h = C.c_void_p()
-        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_bpcs_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_polys), _sz(n_vars), C.byref(h)))
-        return BlockShardedBatchedProver(h, world, ranks, n_polys, n_vars)
-
-    @staticmethod
-    def single_process(devices, n_polys, n_vars):
-        return BlockShardedBatchedProver._create(len(devices), list(range(len(devices))), list(devices), n_polys, n_vars)
-
-    @staticmethod
-    def one_rank(rank, world, device, n_polys, n_vars):
-        return BlockShardedBatchedProver._create(world, [rank], [device], n_polys, n_vars)
-
-    def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_bpcs_shard_export(self.h, _p(out)))
-        return out.tobytes()
-
-    def connect(self, records):
-        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_bpcs_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
-
-    def connect_over(self, dist, device):
-        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
-        import torch
-        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
-        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
-        dist.all_gather(allr, mine)
-        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
-
-    def stream(self, local_index=0):
-        return load().ml_bpcs_shard_stream(self.h, C.c_int(local_index))
-
-    def arena_bytes(self):
-        return load().ml_bpcs_shard_arena_bytes(self.h)
-
-    def phase_ms(self):
-        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
-        out = (C.c_double * 16)()
-        n = load().ml_bpcs_shard_phase_ms(self.h, out, C.c_int(16))
-        return [out[i] for i in range(n)]
+    _PREFIX, _SHAPE = "ml_bpcs_shard", ("n_polys", "n_vars")
 
     def prove_dev(self, inputs, outputs, local_evals_ptrs, transcript):
         """local_evals_ptrs[i * n_polys + j]: device pointer to local rank i's block (n/G evaluations) of polynomial j;
@@ -959,70 +932,14 @@ class BlockShardedBatchedProver:
                                          transcript.h, C.byref(h)))
         return PCSProof(h, batched=True)
 
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_bpcs_shard_free(self.h)
-        self.h = None
 
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
-
-
-class ShardedPCSProver:
+class ShardedPCSProver(_ShardedHandle):
     """PCSProof::prove of one polynomial sharded over the GPUs of one box (ml_pcs_shard_*, csrc/pcs_shard.cu).  Rank g holds the
     block evals[g*n/G, (g+1)*n/G).  A handle hosts the ranks of one process: all of them (single_process; devices may repeat =
     virtual ranks on one GPU) or one (one_rank; the records of all processes are all-gathered by the caller's transport and
     passed to connect).  The proof is an ordinary PCSProof, byte-identical to PCSProof.prove's."""
 
-    def __init__(self, h, world, local_ranks, n_vars):
-        self.h, self.world, self.local_ranks, self.n_vars = h, world, list(local_ranks), n_vars
-
-    @staticmethod
-    def _create(world, ranks, devices, n_vars):
-        h = C.c_void_p()
-        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_pcs_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_vars), C.byref(h)))
-        return ShardedPCSProver(h, world, ranks, n_vars)
-
-    @staticmethod
-    def single_process(devices, n_vars):
-        return ShardedPCSProver._create(len(devices), list(range(len(devices))), list(devices), n_vars)
-
-    @staticmethod
-    def one_rank(rank, world, device, n_vars):
-        return ShardedPCSProver._create(world, [rank], [device], n_vars)
-
-    def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_pcs_shard_export(self.h, _p(out)))
-        return out.tobytes()
-
-    def connect(self, records):
-        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_pcs_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
-
-    def connect_over(self, dist, device):
-        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
-        import torch
-        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
-        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
-        dist.all_gather(allr, mine)
-        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
-
-    def stream(self, local_index=0):
-        return load().ml_pcs_shard_stream(self.h, C.c_int(local_index))
-
-    def arena_bytes(self):
-        return load().ml_pcs_shard_arena_bytes(self.h)
-
-    def phase_ms(self):
-        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
-        out = (C.c_double * 16)()
-        n = load().ml_pcs_shard_phase_ms(self.h, out, C.c_int(16))
-        return [out[i] for i in range(n)]
+    _PREFIX, _SHAPE = "ml_pcs_shard", ("n_vars",)
 
     def prove_dev(self, inputs, output, local_evals_ptrs, transcript):
         """local_evals_ptrs[i]: device pointer to local rank i's block of n/G evaluations; None unless rank 0 is local"""
@@ -1040,70 +957,14 @@ class ShardedPCSProver:
         check(load().ml_pcs_shard_prove(self.h, _p(i), _sz(i.shape[0]), _p(o), _p(e), _sz(e.shape[0]), transcript.h, C.byref(h)))
         return PCSProof(h)
 
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_pcs_shard_free(self.h)
-        self.h = None
 
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
-
-
-class ShardedFriProver:
+class ShardedFriProver(_ShardedHandle):
     """FriProof::prove of one polynomial sharded over the GPUs of one box (ml_fri_shard_*, csrc/fri_shard.cu), from its 2^log_n
     coefficients (reed_solomon + prove) or from its code of 2^(log_n+1) elements.  Rank g holds the block coeffs[g*n/G, (g+1)*n/G)
     or code[g*N/G, (g+1)*N/G).  Handles as for ShardedPCSProver.  The proof is an ordinary FriProof, byte-identical to
     FriProof.prove_from_coeffs's / FriProof.prove's."""
 
-    def __init__(self, h, world, local_ranks, log_n):
-        self.h, self.world, self.local_ranks, self.log_n = h, world, list(local_ranks), log_n
-
-    @staticmethod
-    def _create(world, ranks, devices, log_n):
-        h = C.c_void_p()
-        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_fri_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(log_n), C.byref(h)))
-        return ShardedFriProver(h, world, ranks, log_n)
-
-    @staticmethod
-    def single_process(devices, log_n):
-        return ShardedFriProver._create(len(devices), list(range(len(devices))), list(devices), log_n)
-
-    @staticmethod
-    def one_rank(rank, world, device, log_n):
-        return ShardedFriProver._create(world, [rank], [device], log_n)
-
-    def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_fri_shard_export(self.h, _p(out)))
-        return out.tobytes()
-
-    def connect(self, records):
-        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_fri_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
-
-    def connect_over(self, dist, device):
-        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
-        import torch
-        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
-        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
-        dist.all_gather(allr, mine)
-        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
-
-    def stream(self, local_index=0):
-        return load().ml_fri_shard_stream(self.h, C.c_int(local_index))
-
-    def arena_bytes(self):
-        return load().ml_fri_shard_arena_bytes(self.h)
-
-    def phase_ms(self):
-        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
-        out = (C.c_double * 16)()
-        n = load().ml_fri_shard_phase_ms(self.h, out, C.c_int(16))
-        return [out[i] for i in range(n)]
+    _PREFIX, _SHAPE = "ml_fri_shard", ("log_n",)
 
     def rs_prove_dev(self, local_coeffs_ptrs, transcript):
         """local_coeffs_ptrs[i]: device pointer to local rank i's block of n/G coefficients; None unless rank 0 is local"""
@@ -1135,70 +996,14 @@ class ShardedFriProver:
                                         _sz(gp.shape[0] if gp is not None else 0), transcript.h, C.byref(h)))
         return FriProof(h)
 
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_fri_shard_free(self.h)
-        self.h = None
 
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
-
-
-class ShardedBatchedFriProver:
+class ShardedBatchedFriProver(_ShardedHandle):
     """BatchedFriProof::prove of B codes sharded by block over the GPUs of one box (ml_bfri_shard_*, csrc/bfri_shard.cu), from the
     2^log_n coefficients of each polynomial (reed_solomon of each + prove) or from their codes of 2^(log_n+1) elements.  Rank g
     holds block g of every polynomial: coeffs_j[g*n/G, (g+1)*n/G) or code_j[g*N/G, (g+1)*N/G).  Handles as for ShardedPCSProver.
     The proof is an ordinary batched FriProof, byte-identical to BatchedFriProof.prove's."""
 
-    def __init__(self, h, world, local_ranks, n_codes, log_n):
-        self.h, self.world, self.local_ranks, self.n_codes, self.log_n = h, world, list(local_ranks), n_codes, log_n
-
-    @staticmethod
-    def _create(world, ranks, devices, n_codes, log_n):
-        h = C.c_void_p()
-        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_bfri_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(n_codes), _sz(log_n), C.byref(h)))
-        return ShardedBatchedFriProver(h, world, ranks, n_codes, log_n)
-
-    @staticmethod
-    def single_process(devices, n_codes, log_n):
-        return ShardedBatchedFriProver._create(len(devices), list(range(len(devices))), list(devices), n_codes, log_n)
-
-    @staticmethod
-    def one_rank(rank, world, device, n_codes, log_n):
-        return ShardedBatchedFriProver._create(world, [rank], [device], n_codes, log_n)
-
-    def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_bfri_shard_export(self.h, _p(out)))
-        return out.tobytes()
-
-    def connect(self, records):
-        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_bfri_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
-
-    def connect_over(self, dist, device):
-        """all-gather the IPC records over a torch.distributed process group (the only use of the collective library)"""
-        import torch
-        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
-        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
-        dist.all_gather(allr, mine)
-        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
-
-    def stream(self, local_index=0):
-        return load().ml_bfri_shard_stream(self.h, C.c_int(local_index))
-
-    def arena_bytes(self):
-        return load().ml_bfri_shard_arena_bytes(self.h)
-
-    def phase_ms(self):
-        """device time between the phase marks of the last call (instrumentation, multilinear_b200_instr.h)"""
-        out = (C.c_double * 16)()
-        n = load().ml_bfri_shard_phase_ms(self.h, out, C.c_int(16))
-        return [out[i] for i in range(n)]
+    _PREFIX, _SHAPE = "ml_bfri_shard", ("n_codes", "log_n")
 
     def rs_prove_dev(self, local_coeffs_ptrs, transcript):
         """local_coeffs_ptrs[i * n_codes + j]: device pointer to local rank i's block (n/G coefficients) of polynomial j;
@@ -1239,63 +1044,13 @@ class ShardedBatchedFriProver:
                                          _sz(gp.shape[0] if gp is not None else 0), transcript.h, C.byref(h)))
         return FriProof(h, batched=True)
 
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_bfri_shard_free(self.h)
-        self.h = None
 
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
-
-
-class ShardedWideSumcheck:
+class ShardedWideSumcheck(_ShardedHandle):
     """The width-w System sumcheck over the GPUs of one box (ml_wsumcheck_shard_*, csrc/wsumcheck_shard.cu).  Rank g holds the row
     block matrix[g*h/G, (g+1)*h/G) of the row-major trace.  Handles as for ShardedPCSProver.  One call equals
     WideSumcheckTables.build + set_composition + compute_sumcheck_polynomials exactly, and every process gets the whole result."""
 
-    def __init__(self, h, world, local_ranks, width, n_vars):
-        self.h, self.world, self.local_ranks, self.width, self.n_vars = h, world, list(local_ranks), width, n_vars
-
-    @staticmethod
-    def _create(world, ranks, devices, width, n_vars):
-        h = C.c_void_p()
-        ra, da = (C.c_int * len(ranks))(*ranks), (C.c_int * len(devices))(*devices)
-        check(load().ml_wsumcheck_shard_create(C.c_int(world), C.c_int(len(ranks)), ra, da, _sz(width), _sz(n_vars), C.byref(h)))
-        return ShardedWideSumcheck(h, world, ranks, width, n_vars)
-
-    @staticmethod
-    def single_process(devices, width, n_vars):
-        return ShardedWideSumcheck._create(len(devices), list(range(len(devices))), list(devices), width, n_vars)
-
-    @staticmethod
-    def one_rank(rank, world, device, width, n_vars):
-        return ShardedWideSumcheck._create(world, [rank], [device], width, n_vars)
-
-    def export(self):
-        out = np.empty(72 * len(self.local_ranks), dtype=np.uint8)
-        check(load().ml_wsumcheck_shard_export(self.h, _p(out)))
-        return out.tobytes()
-
-    def connect(self, records):
-        buf = np.frombuffer(bytes(records), dtype=np.uint8).copy()
-        check(load().ml_wsumcheck_shard_connect(self.h, _p(buf), _sz(len(buf) // 72)))
-
-    def connect_over(self, dist, device):
-        """all-gather the IPC records over a torch.distributed process group"""
-        import torch
-        mine = torch.tensor(list(self.export()), dtype=torch.uint8, device=device)
-        allr = [torch.empty_like(mine) for _ in range(dist.get_world_size())]
-        dist.all_gather(allr, mine)
-        self.connect(b"".join(bytes(r.cpu().numpy().tobytes()) for r in allr))
-
-    def stream(self, local_index=0):
-        return load().ml_wsumcheck_shard_stream(self.h, C.c_int(local_index))
-
-    def arena_bytes(self):
-        return load().ml_wsumcheck_shard_arena_bytes(self.h)
+    _PREFIX, _SHAPE = "ml_wsumcheck_shard", ("width", "n_vars")
 
     def set_composition(self, terms):
         """terms: [(coefficient, [column, ...]), ...] as for WideSumcheckTables.set_composition"""
@@ -1324,17 +1079,6 @@ class ShardedWideSumcheck:
         check(load().ml_wsumcheck_shard_compute_polynomials(self.h, _p(rp), _sz(rp.shape[0]), _p(m), _sz(self.width), _sz(m.shape[0] // self.width),
                                                             _sz(composition_degree), transcript.h, _p(sb), _p(co), _p(rs)))
         return to_ints(co[:n * td]), to_ints(rs[:n])
-
-    def free(self):
-        if self.h is not None and self.h.value:
-            load().ml_wsumcheck_shard_free(self.h)
-        self.h = None
-
-    def __del__(self):
-        try:
-            self.free()
-        except Exception:
-            pass
 
 
 _INSTR = None

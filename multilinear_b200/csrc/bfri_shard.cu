@@ -22,7 +22,6 @@
 //   G = 1 runs the same code without any exchange: the encodes (or copies) go straight into layer 0 as one segment, S2 only
 //   absorbs the root and rho, and round 0 runs inside the tail's fold chain as its batched first fold (as ml_batched_fri_prove).
 #include <memory>
-#include <string>
 
 #include "pcs_shard.h"
 #include "transcript.cuh"
@@ -127,7 +126,7 @@ int bfprove_tail(ml_bfri_shard* sh, PeerRank& r0, ml_transcript* t, ml_bfri_proo
     uint8_t roots_lo[MAX_L * 32] = {0};
     MLB_TRY(tail_chain(sh, r0, f, hooks, nullptr, roots_lo, t, 4));
     MLB_TRY(assemble_bfri(sh, r0, f, t, p.get(), roots_lo));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 6);
+    if (&r0 == &sh->local[0]) sh->mark_phase(6);
     MLB_TRY(tail_release(sh, r0, t));  // also releases the other ranks' buffers for the next call
     *out = p.release();
     return ML_OK;
@@ -135,7 +134,7 @@ int bfprove_tail(ml_bfri_shard* sh, PeerRank& r0, ml_transcript* t, ml_bfri_proo
 
 // one call on every local rank; blocks[i * B + j]: local rank i's block of polynomial j, coefficients (rs) or code
 int bfri_shard_run(ml_bfri_shard* sh, const void* const* blocks, bool rs, ml_transcript* t, ml_bfri_proof** out) {
-    MLB_TRY(peer_check_ready(sh->grp, WHO));
+    MLB_TRY(sh->check_ready());
     DeviceGuard guard;
     *out = nullptr;
     sh->grp.epoch++;
@@ -143,7 +142,7 @@ int bfri_shard_run(ml_bfri_shard* sh, const void* const* blocks, bool rs, ml_tra
     memcpy(tr_state, &t->sha, sizeof tr_state);
     const size_t nl = sh->local.size(), B = sh->B;
     sh->n_marks = 0;
-    mark_phase(sh, 0);
+    sh->mark_phase(0);
     if (sh->L == 0) {
         MLB_TRY(bfstage_local(sh, sh->local[0], blocks, rs, tr_state));
     } else if (rs) {
@@ -152,11 +151,11 @@ int bfri_shard_run(ml_bfri_shard* sh, const void* const* blocks, bool rs, ml_tra
     } else {
         for (size_t i = 0; i < nl; i++) MLB_TRY(bfstage_place(sh, sh->local[i], blocks + i * B, tr_state));
     }
-    mark_phase(sh, 1);
+    sh->mark_phase(1);
     for (size_t i = 0; i < nl; i++) MLB_TRY(batch_commit(sh, sh->local[i], rs, false));
-    mark_phase(sh, 2);
+    sh->mark_phase(2);
     for (size_t i = 0; i < nl; i++) MLB_TRY(bfstage_root(sh, sh->local[i]));
-    mark_phase(sh, 3);
+    sh->mark_phase(3);
     if (sh->L > 0) {
         for (size_t i = 0; i < nl; i++) MLB_TRY(bfstage_fold0(sh, sh->local[i]));
         for (int k = 1; k < sh->L; k++) {
@@ -165,52 +164,20 @@ int bfri_shard_run(ml_bfri_shard* sh, const void* const* blocks, bool rs, ml_tra
             for (size_t i = 0; i < nl; i++) MLB_TRY(fri_fold(sh, sh->local[i], k));
         }
     }
-    int st0 = ML_OK;
-    std::string msg;
-    if (PeerRank* r0 = rank0_of(sh)) {
-        st0 = bfprove_tail(sh, *r0, t, out);
-        if (st0 != ML_OK) {
-            msg = ml_last_error();
-            tail_fail(sh, *r0, st0);  // the other ranks wait for PF: release them with this status instead of letting them time out
-        }
-    }
-    int st = finish_ranks(sh, t, st0);
-    if (st0 != ML_OK) { set_error("%s", msg.c_str()); st = st0; }
-    if (st != ML_OK && *out) { ml_bfri_proof_free(*out); *out = nullptr; }
-    return st;
+    return end_call(sh, t, out, ml_bfri_proof_free, [&](PeerRank& r0) { return bfprove_tail(sh, r0, t, out); });
 }
 
-// host arrays src[j] (the whole polynomial j) cut into blocks of `per` elements (a handle that hosts every rank)
-int bfri_shard_host(ml_bfri_shard* sh, const uint8_t* const* src, size_t per, bool rs, ml_transcript* t, ml_bfri_proof** out) {
-    DeviceGuard guard;
-    const size_t nl = sh->local.size(), B = sh->B;
-    std::vector<void*> dev(nl * B, nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < nl && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        for (size_t j = 0; j < B && st == ML_OK; j++) {
-            st = pmalloc(&dev[i * B + j], per * 16, r.st.main);
-            if (st == ML_OK) st = h2d(dev[i * B + j], src[j] + (size_t)r.rank * per * 16, per * 16, r.st.main);
-        }
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK) st = bfri_shard_run(sh, dev.data(), rs, t, out);
-    for (size_t i = 0; i < nl; i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        for (size_t j = 0; j < B; j++) pfree(dev[i * B + j], sh->local[i].st.main);
-    }
-    return st;
-}
-
-int check_host_call(const ml_bfri_shard* sh, const char* who, size_t n_codes, size_t n, size_t want_n) {
-    if ((int)sh->local.size() != sh->world) { set_error("%s: host-pointer entry needs a handle that hosts every rank", who); return ML_ERR_ARG; }
+// host arrays src[j] (the whole polynomial j: n coefficients (rs) or code elements), cut into the ranks' blocks
+int bfri_shard_host(ml_bfri_shard* sh, const char* entry, const uint8_t* const* src, size_t n_codes, size_t n, bool rs, const uint8_t* gen_pows,
+                    size_t gen_pows_len, ml_transcript* t, ml_bfri_proof** out) {
+    const size_t want_n = rs ? sh->n : 2 * sh->n, bytes = want_n / sh->world * 16;
     if (n_codes != sh->B || n != want_n) {
-        set_error("%s: %zu arrays of %zu elements, the handle takes %zu of %zu", who, n_codes, n, sh->B, want_n);
+        set_error("%s: %zu arrays of %zu elements, the handle takes %zu of %zu", entry, n_codes, n, sh->B, want_n);
         return ML_ERR_SIZE;
     }
-    return ML_OK;
+    if (!rs) MLB_TRY(check_gen_pows(log_N_of(sh), gen_pows, gen_pows_len));
+    return sh->host_call(entry, sh->B, bytes, [&](int rank, size_t j) { return src[j] + (size_t)rank * bytes; },
+                         [&](const void* const* dev) { return bfri_shard_run(sh, dev, rs, t, out); });
 }
 
 }  // namespace
@@ -228,29 +195,24 @@ int ml_bfri_shard_create(int world, int n_local, const int* local_ranks, const i
     DeviceGuard guard;
     ml_bfri_shard* sh = new ml_bfri_shard();
     sh->who = WHO;
-    int st = shard_init(sh, world, n_local, local_ranks, local_devices, log_n, n_codes, "ml_bfri_shard_create", true);
+    int st = shard_init(sh, world, n_local, local_ranks, local_devices, log_n, n_codes, true);
     if (st == ML_OK) st = batch_init(sh);
-    if (st != ML_OK) { ml_bfri_shard_free(sh); return st; }
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
 
-void ml_bfri_shard_free(ml_bfri_shard* sh) {
-    if (!sh) return;
-    batch_free(sh);
-    shard_free(sh);
-    delete sh;
-}
+void ml_bfri_shard_free(ml_bfri_shard* sh) { delete sh; }
 
-int ml_bfri_shard_export(ml_bfri_shard* sh, uint8_t* records_out) { return shard_export(sh, records_out); }
-int ml_bfri_shard_connect(ml_bfri_shard* sh, const uint8_t* records, size_t n_records) { return shard_connect(sh, records, n_records, "ml_bfri_shard_connect"); }
-void* ml_bfri_shard_stream(const ml_bfri_shard* sh, int local_index) { return shard_stream(sh, local_index); }
+int ml_bfri_shard_export(ml_bfri_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_bfri_shard_connect(ml_bfri_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_bfri_shard_stream(const ml_bfri_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_bfri_shard_arena_bytes(const ml_bfri_shard* sh) { return sh->lay.total; }
 
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: [S0 transpose + encodes + exchange (or placement), S1 combine + batch tree, S2 batch root, sharded
 // rounds, tail chain, openings] (the last two on rank 0 only).  Returns the count.
-int ml_bfri_shard_phase_ms(const ml_bfri_shard* sh, double* out, int cap) { return shard_phase_ms(sh, out, cap); }
+int ml_bfri_shard_phase_ms(const ml_bfri_shard* sh, double* out, int cap) { return sh->phase_ms(out, cap); }
 
 // reed_solomon of every polynomial + BatchedFriProof::prove (batched_fri.rs:286-318).  Every process calls it with its own
 // transcript copy; the proof comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the
@@ -265,16 +227,13 @@ int ml_bfri_shard_prove_dev(ml_bfri_shard* sh, const void* const* local_codes_de
 
 // host coefficients (n_codes arrays of n) and a handle that hosts every rank
 int ml_bfri_shard_rs_prove(ml_bfri_shard* sh, const uint8_t* const* coeffs, size_t n_codes, size_t n, ml_transcript* t, ml_bfri_proof** out) {
-    MLB_TRY(check_host_call(sh, "ml_bfri_shard_rs_prove", n_codes, n, sh->n));
-    return bfri_shard_host(sh, coeffs, sh->nloc, true, t, out);
+    return bfri_shard_host(sh, "ml_bfri_shard_rs_prove", coeffs, n_codes, n, true, nullptr, 0, t, out);
 }
 // host codes (n_codes arrays of n = 2^(log_n + 1)) and a handle that hosts every rank: the drop-in for batched_fri.rs:286;
 // gen_pows as for ml_fri_prove
 int ml_bfri_shard_prove(ml_bfri_shard* sh, const uint8_t* const* codes, size_t n_codes, size_t n, const uint8_t* gen_pows, size_t gen_pows_len,
                         ml_transcript* t, ml_bfri_proof** out) {
-    MLB_TRY(check_host_call(sh, "ml_bfri_shard_prove", n_codes, n, 2 * sh->n));
-    MLB_TRY(check_gen_pows(log_N_of(sh), gen_pows, gen_pows_len));
-    return bfri_shard_host(sh, codes, sh->NL, false, t, out);
+    return bfri_shard_host(sh, "ml_bfri_shard_prove", codes, n_codes, n, false, gen_pows, gen_pows_len, t, out);
 }
 
 }  // extern "C"

@@ -19,7 +19,6 @@
 //       and the path from the owner's arena (upper path from rank 0's copy of the top tree).
 //   G = 1 runs the same code without the exchange: the encodes go straight into layer 0 (one segment of N/2 leaves), the
 //       fingerprint straight into the tail tables, and round 0 runs inside the tail's fold chain as its batched first fold.
-#include <cstdlib>
 #include <memory>
 
 #include "pcs_shard.h"
@@ -125,11 +124,11 @@ int batch_init(BatchCore* sh) {
     return st;
 }
 
-void batch_free(BatchCore* sh) {
+BatchCore::~BatchCore() {
     DeviceGuard guard;
-    for (size_t i = 0; i < sh->ev.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        BatchCore::Events& e = sh->ev[i];
+    for (size_t i = 0; i < ev.size(); i++) {
+        cudaSetDevice(local[i].device);
+        Events& e = ev[i];
         for (cudaEvent_t x : {e.done[0], e.done[1], e.free[0], e.free[1], e.join})
             if (x) cudaEventDestroy(x);
     }
@@ -325,7 +324,7 @@ int bprove_tail(ml_bpcs_shard* sh, PeerRank& r0, const std::vector<hfe>& pts, co
     uint8_t roots_lo[MAX_L * 32] = {0};
     MLB_TRY(tail_chain(sh, r0, f, hooks, p->sumcheck.data(), roots_lo, t, 4));
     MLB_TRY(assemble_bfri(sh, r0, f, t, &p->fri, roots_lo));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 6);
+    if (&r0 == &sh->local[0]) sh->mark_phase(6);
     p->inputs = pts;
     p->outputs.resize(sh->B);
     for (size_t j = 0; j < sh->B; j++) p->outputs[j] = hfe_load(outputs + 16 * j);
@@ -338,12 +337,7 @@ int bprove_tail(ml_bpcs_shard* sh, PeerRank& r0, const std::vector<hfe>& pts, co
 
 extern "C" {
 
-void ml_bpcs_shard_free(ml_bpcs_shard* sh) {
-    if (!sh) return;
-    batch_free(sh);
-    shard_free(sh);
-    delete sh;
-}
+void ml_bpcs_shard_free(ml_bpcs_shard* sh) { delete sh; }
 
 int ml_bpcs_shard_create(int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_polys, size_t n_vars, ml_bpcs_shard** out) {
     MLB_TRY(peer_check_world("ml_bpcs_shard_create", world, n_local));
@@ -356,28 +350,28 @@ int ml_bpcs_shard_create(int world, int n_local, const int* local_ranks, const i
     DeviceGuard guard;
     ml_bpcs_shard* sh = new ml_bpcs_shard();
     sh->who = WHO;
-    int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, n_polys, "ml_bpcs_shard_create");
+    int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, n_polys);
     if (st == ML_OK) st = batch_init(sh);
-    if (st != ML_OK) { ml_bpcs_shard_free(sh); return st; }
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
 
-int ml_bpcs_shard_export(ml_bpcs_shard* sh, uint8_t* records_out) { return shard_export(sh, records_out); }
-int ml_bpcs_shard_connect(ml_bpcs_shard* sh, const uint8_t* records, size_t n_records) { return shard_connect(sh, records, n_records, "ml_bpcs_shard_connect"); }
-void* ml_bpcs_shard_stream(const ml_bpcs_shard* sh, int local_index) { return shard_stream(sh, local_index); }
+int ml_bpcs_shard_export(ml_bpcs_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_bpcs_shard_connect(ml_bpcs_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_bpcs_shard_stream(const ml_bpcs_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_bpcs_shard_arena_bytes(const ml_bpcs_shard* sh) { return sh->lay.total; }
 
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: [S0 encodes + exchange, S1 combine + batch tree, S2/S3 root + tables, sharded rounds, tail chain,
 // openings] (the last two on rank 0 only).  Returns the count.
-int ml_bpcs_shard_phase_ms(const ml_bpcs_shard* sh, double* out, int cap) { return shard_phase_ms(sh, out, cap); }
+int ml_bpcs_shard_phase_ms(const ml_bpcs_shard* sh, double* out, int cap) { return sh->phase_ms(out, cap); }
 
 // BatchedPCSProof::prove (batched_pcs.rs:130-180).  Every process calls it with the same claim and its own transcript copy; the
 // proof comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the same state.
 int ml_bpcs_shard_prove_dev(ml_bpcs_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t* outputs, size_t n_polys,
                             const void* const* local_evals_dev, ml_transcript* t, ml_bpcs_proof** out) {
-    MLB_TRY(peer_check_ready(sh->grp, WHO));
+    MLB_TRY(sh->check_ready());
     if (n_vars != sh->n_vars || n_polys != sh->B) {
         set_error("ml_bpcs_shard_prove: the claim has %zu polynomials of %zu variables, the handle %zu of %zu", n_polys, n_vars, sh->B, sh->n_vars);
         return ML_ERR_SIZE;
@@ -394,13 +388,13 @@ int ml_bpcs_shard_prove_dev(ml_bpcs_shard* sh, const uint8_t* inputs, size_t n_v
     const size_t nl = sh->local.size();
     std::vector<int> nb(nl, 0);
     sh->n_marks = 0;
-    mark_phase(sh, 0);
+    sh->mark_phase(0);
     for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_encode(sh, i, local_evals_dev + i * n_polys, tr_state, outputs));
-    mark_phase(sh, 1);
+    sh->mark_phase(1);
     for (size_t i = 0; i < nl; i++) MLB_TRY(batch_commit(sh, sh->local[i], true, true));
-    mark_phase(sh, 2);
+    sh->mark_phase(2);
     for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_tables(sh, sh->local[i], pts));
-    mark_phase(sh, 3);
+    sh->mark_phase(3);
     if (sh->L > 0) {
         for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_post0(sh, sh->local[i], &nb[i]));
         for (size_t i = 0; i < nl; i++) MLB_TRY(bstage_round0(sh, sh->local[i]));
@@ -411,41 +405,19 @@ int ml_bpcs_shard_prove_dev(ml_bpcs_shard* sh, const uint8_t* inputs, size_t n_v
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_fold(sh, sh->local[i], k, &nb[i]));
         }
     }
-    int st = ML_OK;
-    if (PeerRank* r0 = rank0_of(sh)) st = bprove_tail(sh, *r0, pts, outputs, t, out);
-    st = finish_ranks(sh, t, st);
-    if (st != ML_OK && *out) { ml_bpcs_proof_free(*out); *out = nullptr; }
-    return st;
+    return end_call(sh, t, out, ml_bpcs_proof_free, [&](PeerRank& r0) { return bprove_tail(sh, r0, pts, outputs, t, out); });
 }
 
 // host evaluations (n_polys arrays of n) and a handle that hosts every rank: the drop-in for batched_pcs.rs:130
 int ml_bpcs_shard_prove(ml_bpcs_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t* outputs, size_t n_polys, const uint8_t* const* evals,
                         size_t n, ml_transcript* t, ml_bpcs_proof** out) {
-    if ((int)sh->local.size() != sh->world) { set_error("ml_bpcs_shard_prove: host-pointer entry needs a handle that hosts every rank"); return ML_ERR_ARG; }
     if (n_vars != sh->n_vars || n != sh->n || n_polys != sh->B) {
         set_error("ml_bpcs_shard_prove: need 2^n_vars == evals[j].len() == the handle's size and n_polys == the handle's");
         return ML_ERR_SIZE;
     }
-    DeviceGuard guard;
-    const size_t nl = sh->local.size(), B = sh->B, bytes = sh->nloc * 16;
-    std::vector<void*> dev(nl * B, nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < nl && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        for (size_t j = 0; j < B && st == ML_OK; j++) {
-            st = pmalloc(&dev[i * B + j], bytes, r.st.main);
-            if (st == ML_OK) st = h2d(dev[i * B + j], evals[j] + (size_t)r.rank * bytes, bytes, r.st.main);
-        }
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK) st = ml_bpcs_shard_prove_dev(sh, inputs, n_vars, outputs, n_polys, dev.data(), t, out);
-    for (size_t i = 0; i < nl; i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        for (size_t j = 0; j < B; j++) pfree(dev[i * B + j], sh->local[i].st.main);
-    }
-    return st;
+    const size_t bytes = sh->nloc * 16;
+    return sh->host_call("ml_bpcs_shard_prove", sh->B, bytes, [&](int rank, size_t j) { return evals[j] + (size_t)rank * bytes; },
+                         [&](const void* const* dev) { return ml_bpcs_shard_prove_dev(sh, inputs, n_vars, outputs, n_polys, dev, t, out); });
 }
 
 }  // extern "C"

@@ -21,7 +21,6 @@
 //       ends in a non-constant last fold) hands its status to every rank instead, so every rank returns it at once.
 //   G = 1 runs the same code without any exchange: the encode (or a copy of the code) goes straight into the tail.
 #include <memory>
-#include <string>
 
 #include "pcs_shard.h"
 
@@ -132,7 +131,7 @@ int fprove_tail(ml_fri_shard* sh, PeerRank& r0, ml_transcript* t, ml_fri_proof**
     uint8_t roots_lo[MAX_L * 32];
     MLB_TRY(tail_chain(sh, r0, f, ChainHooks(), nullptr, roots_lo, t, 3));
     MLB_TRY(assemble_fri(sh, r0, f, t, p.get(), roots_lo));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 5);
+    if (&r0 == &sh->local[0]) sh->mark_phase(5);
     MLB_TRY(tail_release(sh, r0, t));  // also releases the other ranks' buffers for the next call
     *out = p.release();
     return ML_OK;
@@ -140,7 +139,7 @@ int fprove_tail(ml_fri_shard* sh, PeerRank& r0, ml_transcript* t, ml_fri_proof**
 
 // one call on every local rank; blocks[i]: local rank i's block of the coefficients (rs) or of the code
 int fri_shard_run(ml_fri_shard* sh, const void* const* blocks, bool rs, ml_transcript* t, ml_fri_proof** out) {
-    MLB_TRY(peer_check_ready(sh->grp, WHO));
+    MLB_TRY(sh->check_ready());
     DeviceGuard guard;
     *out = nullptr;
     sh->grp.epoch++;
@@ -148,11 +147,11 @@ int fri_shard_run(ml_fri_shard* sh, const void* const* blocks, bool rs, ml_trans
     memcpy(tr_state, &t->sha, sizeof tr_state);
     const size_t nl = sh->local.size();
     sh->n_marks = 0;
-    mark_phase(sh, 0);
+    sh->mark_phase(0);
     if (sh->L == 0) {
         MLB_TRY(fstage_local(sh, sh->local[0], (const fe*)blocks[0], rs, tr_state));
-        mark_phase(sh, 1);
-        mark_phase(sh, 2);
+        sh->mark_phase(1);
+        sh->mark_phase(2);
     } else {
         if (rs) {
             for (size_t i = 0; i < nl; i++) MLB_TRY(fstage_transpose(sh, sh->local[i], (const fe*)blocks[i], tr_state));
@@ -160,54 +159,16 @@ int fri_shard_run(ml_fri_shard* sh, const void* const* blocks, bool rs, ml_trans
         } else {
             for (size_t i = 0; i < nl; i++) MLB_TRY(fstage_place(sh, sh->local[i], (const fe*)blocks[i], tr_state));
         }
-        mark_phase(sh, 1);
+        sh->mark_phase(1);
         for (size_t i = 0; i < nl; i++) MLB_TRY(fstage_combine(sh, sh->local[i], rs));
-        mark_phase(sh, 2);
+        sh->mark_phase(2);
         for (int k = 0; k < sh->L; k++) {
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_post(sh, sh->local[i], k, -1));
             for (size_t i = 0; i < nl; i++) MLB_TRY(fri_round(sh, sh->local[i], k));
             for (size_t i = 0; i < nl; i++) MLB_TRY(fri_fold(sh, sh->local[i], k));
         }
     }
-    int st0 = ML_OK;
-    std::string msg;
-    if (PeerRank* r0 = rank0_of(sh)) {
-        st0 = fprove_tail(sh, *r0, t, out);
-        if (st0 != ML_OK) {
-            msg = ml_last_error();
-            tail_fail(sh, *r0, st0);  // the other ranks wait for PF: release them with this status instead of letting them time out
-        }
-    }
-    int st = finish_ranks(sh, t, st0);
-    if (st0 != ML_OK) { set_error("%s", msg.c_str()); st = st0; }
-    if (st != ML_OK && *out) { ml_fri_proof_free(*out); *out = nullptr; }
-    return st;
-}
-
-// host blocks of `per` elements each (a handle that hosts every rank)
-int fri_shard_host(ml_fri_shard* sh, const uint8_t* src, size_t per, bool rs, ml_transcript* t, ml_fri_proof** out) {
-    DeviceGuard guard;
-    std::vector<void*> dev(sh->local.size(), nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        st = pmalloc(&dev[i], per * 16, r.st.main);
-        if (st == ML_OK) st = h2d(dev[i], src + (size_t)r.rank * per * 16, per * 16, r.st.main);
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK) st = fri_shard_run(sh, dev.data(), rs, t, out);
-    for (size_t i = 0; i < sh->local.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        pfree(dev[i], sh->local[i].st.main);
-    }
-    return st;
-}
-
-int check_hosts_all(const ml_fri_shard* sh, const char* who) {
-    if ((int)sh->local.size() != sh->world) { set_error("%s: host-pointer entry needs a handle that hosts every rank", who); return ML_ERR_ARG; }
-    return ML_OK;
+    return end_call(sh, t, out, ml_fri_proof_free, [&](PeerRank& r0) { return fprove_tail(sh, r0, t, out); });
 }
 
 }  // namespace
@@ -224,27 +185,23 @@ int ml_fri_shard_create(int world, int n_local, const int* local_ranks, const in
     DeviceGuard guard;
     ml_fri_shard* sh = new ml_fri_shard();
     sh->who = WHO;
-    int st = shard_init(sh, world, n_local, local_ranks, local_devices, log_n, 0, "ml_fri_shard_create", true);
-    if (st != ML_OK) { ml_fri_shard_free(sh); return st; }
+    int st = shard_init(sh, world, n_local, local_ranks, local_devices, log_n, 0, true);
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
 
-void ml_fri_shard_free(ml_fri_shard* sh) {
-    if (!sh) return;
-    shard_free(sh);
-    delete sh;
-}
+void ml_fri_shard_free(ml_fri_shard* sh) { delete sh; }
 
-int ml_fri_shard_export(ml_fri_shard* sh, uint8_t* records_out) { return shard_export(sh, records_out); }
-int ml_fri_shard_connect(ml_fri_shard* sh, const uint8_t* records, size_t n_records) { return shard_connect(sh, records, n_records, "ml_fri_shard_connect"); }
-void* ml_fri_shard_stream(const ml_fri_shard* sh, int local_index) { return shard_stream(sh, local_index); }
+int ml_fri_shard_export(ml_fri_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_fri_shard_connect(ml_fri_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_fri_shard_stream(const ml_fri_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_fri_shard_arena_bytes(const ml_fri_shard* sh) { return sh->lay.total; }
 
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: [S0 transpose + encode + exchange (or placement), S1 combine (or the wait), sharded rounds, tail
 // chain, openings] (the last two on rank 0 only).  Returns the count.
-int ml_fri_shard_phase_ms(const ml_fri_shard* sh, double* out, int cap) { return shard_phase_ms(sh, out, cap); }
+int ml_fri_shard_phase_ms(const ml_fri_shard* sh, double* out, int cap) { return sh->phase_ms(out, cap); }
 
 // reed_solomon + FriProof::prove (fri/mod.rs:19-28, :261-285).  Every process calls it with its own transcript copy; the proof
 // comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the same state.
@@ -258,18 +215,20 @@ int ml_fri_shard_prove_dev(ml_fri_shard* sh, const void* const* local_code_dev, 
 
 // host coefficients (all n) and a handle that hosts every rank
 int ml_fri_shard_rs_prove(ml_fri_shard* sh, const uint8_t* coeffs, size_t n, ml_transcript* t, ml_fri_proof** out) {
-    MLB_TRY(check_hosts_all(sh, "ml_fri_shard_rs_prove"));
     if (n != sh->n) { set_error("ml_fri_shard_rs_prove: %zu coefficients, the handle takes %zu", n, sh->n); return ML_ERR_SIZE; }
-    return fri_shard_host(sh, coeffs, sh->nloc, true, t, out);
+    const size_t bytes = sh->nloc * 16;
+    return sh->host_call("ml_fri_shard_rs_prove", 1, bytes, [&](int rank, size_t) { return coeffs + (size_t)rank * bytes; },
+                         [&](const void* const* dev) { return fri_shard_run(sh, dev, true, t, out); });
 }
 // host code (all n = 2^(log_n + 1) elements) and a handle that hosts every rank: the drop-in for fri/mod.rs:261; gen_pows as
 // for ml_fri_prove
 int ml_fri_shard_prove(ml_fri_shard* sh, const uint8_t* code, size_t n, const uint8_t* gen_pows, size_t gen_pows_len, ml_transcript* t,
                        ml_fri_proof** out) {
-    MLB_TRY(check_hosts_all(sh, "ml_fri_shard_prove"));
     if (n != 2 * sh->n) { set_error("ml_fri_shard_prove: a code of %zu elements, the handle takes %zu", n, 2 * sh->n); return ML_ERR_SIZE; }
     MLB_TRY(check_gen_pows(log_N_of(sh), gen_pows, gen_pows_len));
-    return fri_shard_host(sh, code, sh->NL, false, t, out);
+    const size_t bytes = sh->NL * 16;
+    return sh->host_call("ml_fri_shard_prove", 1, bytes, [&](int rank, size_t) { return code + (size_t)rank * bytes; },
+                         [&](const void* const* dev) { return fri_shard_run(sh, dev, false, t, out); });
 }
 
 }  // extern "C"

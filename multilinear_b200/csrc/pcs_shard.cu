@@ -23,7 +23,6 @@
 //       the owners' arenas by peer loads (upper path from rank 0's copy of the layer's top tree), layers >= L by
 //       fri_open_queries; the final transcript -> all + flag PF.  Every process's transcript ends in rank 0's state.
 //   G = 1 runs the same code without the exchange: the encode and the tables go straight into the tail buffers.
-#include <cstdlib>
 #include <memory>
 
 #include "pcs_shard.h"
@@ -274,80 +273,11 @@ Layout make_layout(size_t n, int G, size_t B, bool fri) {
     return a;
 }
 
-void mark_phase(ShardCore* sh, int idx) {
-    if (idx >= ShardCore::N_MARKS || sh->local.empty()) return;
-    PeerRank& r = sh->local[0];
-    cudaSetDevice(r.device);
-    if (!sh->mark[idx] && cudaEventCreate(&sh->mark[idx]) != cudaSuccess) { cudaGetLastError(); return; }
-    cudaEventRecord(sh->mark[idx], r.st.main);
-    if (idx + 1 > sh->n_marks) sh->n_marks = idx + 1;
-}
-PeerRank* rank0_of(ShardCore* sh) {
-    for (auto& r : sh->local)
-        if (r.rank == 0) return &r;
-    return nullptr;
-}
-
-int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who,
-               bool fri) {
-    const int L = (int)ilog2((size_t)world);
-    sh->world = world; sh->L = L; sh->n_vars = n_vars; sh->n = (size_t)1 << n_vars; sh->B = B;
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, bool fri) {
+    sh->L = (int)ilog2((size_t)world); sh->n_vars = n_vars; sh->n = (size_t)1 << n_vars; sh->B = B;
     sh->NL = 2 * sh->n / world; sh->R = sh->NL / world; sh->nloc = sh->n / world;
     sh->lay = make_layout(sh->n, world, B, fri);
-    sh->grp.world = world;
-    sh->grp.arena_bytes = sh->lay.total;
-    sh->grp.off_flags = sh->lay.flags;
-    sh->grp.off_status = sh->lay.status;
-    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
-    int st = ML_OK;
-    for (int i = 0; i < n_local && st == ML_OK; i++) {
-        PeerRank r;
-        r.rank = local_ranks[i];
-        r.device = local_devices[i];
-        st = peer_rank_init(sh->grp, r, who, sh->lay.ycode);
-        if (st == ML_OK || st == ML_ERR_ALLOC) sh->local.push_back(r);
-    }
-    if (st == ML_OK && n_local == world) {
-        std::vector<PeerRank*> ranks;
-        for (auto& r : sh->local) ranks.push_back(&r);
-        st = peer_link_local(sh->grp, ranks, who);
-    }
-    return st;
-}
-
-void shard_free(ShardCore* sh) {
-    DeviceGuard guard;
-    for (int i = 0; i < ShardCore::N_MARKS; i++)
-        if (sh->mark[i]) cudaEventDestroy(sh->mark[i]);
-    for (auto& r : sh->local) {
-        cudaSetDevice(r.device);
-        cudaDeviceSynchronize();
-        peer_rank_free(r);
-    }
-    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
-}
-
-int shard_export(ShardCore* sh, uint8_t* records_out) {
-    std::vector<PeerRank*> ranks;
-    for (auto& r : sh->local) ranks.push_back(&r);
-    return peer_export(ranks, records_out);
-}
-int shard_connect(ShardCore* sh, const uint8_t* records, size_t n_records, const char* who) {
-    if (sh->local.size() != 1) { set_error("%s: only for handles that host one rank", who); return ML_ERR_ARG; }
-    return peer_connect(sh->grp, sh->local[0], records, n_records, who);
-}
-void* shard_stream(const ShardCore* sh, int local_index) {
-    if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
-    return (void*)sh->local[local_index].st.main;
-}
-int shard_phase_ms(const ShardCore* sh, double* out, int cap) {
-    int n = 0;
-    for (int i = 0; i + 1 < sh->n_marks && n < cap; i++) {
-        float ms = 0;
-        if (!sh->mark[i] || !sh->mark[i + 1] || cudaEventElapsedTime(&ms, sh->mark[i], sh->mark[i + 1]) != cudaSuccess) { cudaGetLastError(); ms = -1.f; }
-        out[n++] = ms;
-    }
-    return n;
+    return sh->init(world, n_local, local_ranks, local_devices, sh->lay.total, sh->lay.flags, sh->lay.status, sh->lay.ycode);
 }
 
 int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s) {
@@ -520,7 +450,7 @@ int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, 
     const Layout& a = sh->lay;
     const int L = sh->L;
     if (L > 0) MLB_TRY(peer_wait(sh->grp, r0, PG, -1, s));
-    if (&r0 == &sh->local[0]) mark_phase(sh, mark_base);
+    if (&r0 == &sh->local[0]) sh->mark_phase(mark_base);
     f->log_n0 = (int)sh->n_vars + ML_LOG_BLOWUP;
     f->stream = s;
     if (!hooks.first_fold) MLB_TRY(fri_push_layer(f, at(r0, a.tail_code), sh->NL, false, s, true));  // layer L, committed, root not absorbed yet
@@ -534,7 +464,7 @@ int tail_chain(ShardCore* sh, PeerRank& r0, ml_fri* f, const ChainHooks& hooks, 
     h.tr_dev = (const DevTranscript*)(r0.arena + a.tr);
     h.prev_dev = at(r0, a.prev);
     MLB_TRY(fold_chain_dev(r0.ctx, f, &h, sumcheck ? &sc : nullptr, 0, sumcheck ? sumcheck + 2 * L : nullptr, (size_t)L, !hooks.first_fold, t, s));
-    if (&r0 == &sh->local[0]) mark_phase(sh, mark_base + 1);
+    if (&r0 == &sh->local[0]) sh->mark_phase(mark_base + 1);
     if (L > 0) {  // sumcheck (c1, c2) and layer roots of the sharded rounds
         uint8_t lo[MAX_L * 32];
         if (sumcheck) MLB_CUDA(cudaMemcpyAsync(lo, r0.arena + a.sc, (size_t)L * 32, cudaMemcpyDeviceToHost, s));
@@ -573,7 +503,7 @@ int finish_ranks(ShardCore* sh, ml_transcript* t, int st) {
         MLB_TRY(peer_wait(sh->grp, r, PF, 0, r.st.main));
         int s1 = peer_read_status(sh->grp, r, sh->who);
         if (s1 != ML_OK) { st = s1; continue; }
-        if (!rank0_of(sh)) {  // another process holds rank 0: adopt its final transcript
+        if (!sh->rank0()) {  // another process holds rank 0: adopt its final transcript
             HostSha256 fin;
             MLB_TRY(d2h_sync(&fin, r.arena + sh->lay.final_tr, sizeof(DevTranscript), r.st.main));
             t->sha = fin;
@@ -631,7 +561,7 @@ int prove_tail(ml_pcs_shard* sh, PeerRank& r0, const uint8_t* inputs, const uint
     uint8_t roots_lo[MAX_L * 32];
     MLB_TRY(tail_chain(sh, r0, f, ChainHooks(), p->sumcheck.data(), roots_lo, t, 3));
     MLB_TRY(assemble_fri(sh, r0, f, t, &p->fri, roots_lo));
-    if (&r0 == &sh->local[0]) mark_phase(sh, 5);
+    if (&r0 == &sh->local[0]) sh->mark_phase(5);
     p->inputs.resize(sh->n_vars);
     for (size_t i = 0; i < sh->n_vars; i++) p->inputs[i] = hfe_load(inputs + 16 * i);
     p->output = hfe_load(output);
@@ -653,33 +583,29 @@ int ml_pcs_shard_create(int world, int n_local, const int* local_ranks, const in
     }
     DeviceGuard guard;
     ml_pcs_shard* sh = new ml_pcs_shard();
-    int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, 0, "ml_pcs_shard_create");
-    if (st != ML_OK) { ml_pcs_shard_free(sh); return st; }
+    sh->who = WHO;
+    int st = shard_init(sh, world, n_local, local_ranks, local_devices, n_vars, 0);
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
 
-void ml_pcs_shard_free(ml_pcs_shard* sh) {
-    if (!sh) return;
-    shard_free(sh);
-    delete sh;
-}
-
-int ml_pcs_shard_export(ml_pcs_shard* sh, uint8_t* records_out) { return shard_export(sh, records_out); }
-int ml_pcs_shard_connect(ml_pcs_shard* sh, const uint8_t* records, size_t n_records) { return shard_connect(sh, records, n_records, "ml_pcs_shard_connect"); }
-void* ml_pcs_shard_stream(const ml_pcs_shard* sh, int local_index) { return shard_stream(sh, local_index); }
+void ml_pcs_shard_free(ml_pcs_shard* sh) { delete sh; }
+int ml_pcs_shard_export(ml_pcs_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_pcs_shard_connect(ml_pcs_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_pcs_shard_stream(const ml_pcs_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_pcs_shard_arena_bytes(const ml_pcs_shard* sh) { return sh->lay.total; }
 
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: [S0 encode + exchange + tables, S1 combine, sharded rounds, tail chain, openings] (the last two
 // on rank 0 only).  Returns the count.
-int ml_pcs_shard_phase_ms(const ml_pcs_shard* sh, double* out, int cap) { return shard_phase_ms(sh, out, cap); }
+int ml_pcs_shard_phase_ms(const ml_pcs_shard* sh, double* out, int cap) { return sh->phase_ms(out, cap); }
 
 // PCSProof::prove (multilinear_pcs.rs:90-136).  Every process calls it with the same claim and its own transcript copy; the proof
 // comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the same state.
 int ml_pcs_shard_prove_dev(ml_pcs_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t output[16], const void* const* local_evals_dev,
                            ml_transcript* t, ml_pcs_proof** out) {
-    MLB_TRY(peer_check_ready(sh->grp, WHO));
+    MLB_TRY(sh->check_ready());
     if (n_vars != sh->n_vars) { set_error("ml_pcs_shard_prove: the claim has %zu variables, the handle %zu", n_vars, sh->n_vars); return ML_ERR_SIZE; }
     DeviceGuard guard;
     *out = nullptr;
@@ -692,49 +618,30 @@ int ml_pcs_shard_prove_dev(ml_pcs_shard* sh, const uint8_t* inputs, size_t n_var
     const size_t nl = sh->local.size();
     std::vector<int> nb(nl, 0);
     sh->n_marks = 0;
-    mark_phase(sh, 0);
+    sh->mark_phase(0);
     for (size_t i = 0; i < nl; i++) MLB_TRY(stage_encode(sh, sh->local[i], (const fe*)local_evals_dev[i], claim_state, pts));
-    mark_phase(sh, 1);
+    sh->mark_phase(1);
     if (sh->L > 0) {
         for (size_t i = 0; i < nl; i++) MLB_TRY(stage_combine(sh, sh->local[i], &nb[i]));
-        mark_phase(sh, 2);
+        sh->mark_phase(2);
         for (int k = 0; k < sh->L; k++) {
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_post(sh, sh->local[i], k, nb[i]));
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_round(sh, sh->local[i], k));
             for (size_t i = 0; i < nl; i++) MLB_TRY(stage_fold(sh, sh->local[i], k, &nb[i]));
         }
     } else {
-        mark_phase(sh, 2);
+        sh->mark_phase(2);
     }
-    int st = ML_OK;
-    if (PeerRank* r0 = rank0_of(sh)) st = prove_tail(sh, *r0, inputs, output, t, out);
-    st = finish_ranks(sh, t, st);
-    if (st != ML_OK && *out) { ml_pcs_proof_free(*out); *out = nullptr; }
-    return st;
+    return end_call(sh, t, out, ml_pcs_proof_free, [&](PeerRank& r0) { return prove_tail(sh, r0, inputs, output, t, out); });
 }
 
 // host evaluations (all n) and a handle that hosts every rank: the drop-in for multilinear_pcs.rs:90
 int ml_pcs_shard_prove(ml_pcs_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t output[16], const uint8_t* evals, size_t n,
                        ml_transcript* t, ml_pcs_proof** out) {
-    if ((int)sh->local.size() != sh->world) { set_error("ml_pcs_shard_prove: host-pointer entry needs a handle that hosts every rank"); return ML_ERR_ARG; }
     if (n_vars != sh->n_vars || n != sh->n) { set_error("ml_pcs_shard_prove: need 2^n_vars == evals.len() == the handle's size"); return ML_ERR_SIZE; }
-    DeviceGuard guard;
-    std::vector<void*> dev(sh->local.size(), nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        st = pmalloc(&dev[i], sh->nloc * 16, r.st.main);
-        if (st == ML_OK) st = h2d(dev[i], evals + (size_t)r.rank * sh->nloc * 16, sh->nloc * 16, r.st.main);
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK) st = ml_pcs_shard_prove_dev(sh, inputs, n_vars, output, dev.data(), t, out);
-    for (size_t i = 0; i < sh->local.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        pfree(dev[i], sh->local[i].st.main);
-    }
-    return st;
+    const size_t bytes = sh->nloc * 16;
+    return sh->host_call("ml_pcs_shard_prove", 1, bytes, [&](int rank, size_t) { return evals + (size_t)rank * bytes; },
+                         [&](const void* const* dev) { return ml_pcs_shard_prove_dev(sh, inputs, n_vars, output, dev, t, out); });
 }
 
 }  // extern "C"

@@ -1,9 +1,12 @@
 // Stages of the block-sharded provers, shared by pcs_shard.cu (one PCSProof::prove, ml_pcs_shard_*), bpcs_shard.cu (one
 // BatchedPCSProof::prove, ml_bpcs_shard_*), fri_shard.cu (one FriProof::prove, ml_fri_shard_*) and bfri_shard.cu (one
-// BatchedFriProof::prove, ml_bfri_shard_*).  All split every polynomial by block over G ranks and keep the sharded layers in the
-// segment layout described at the top of pcs_shard.cu; the batched provers add a batched layer 0 and round 0 (implemented in
-// bpcs_shard.cu), the FRI provers drop the sumcheck tables (their table-free stages are implemented in fri_shard.cu).
+// BatchedFriProof::prove, ml_bfri_shard_*); wsumcheck_shard.cu uses local_eq_table.  All split every polynomial by block over G
+// ranks and keep the sharded layers in the segment layout described at the top of pcs_shard.cu; the batched provers add a
+// batched layer 0 and round 0 (implemented in bpcs_shard.cu), the FRI provers drop the sumcheck tables (their table-free stages
+// are implemented in fri_shard.cu).  The handle plumbing (create, free, records, streams, marks) is PeerHandle's (peer.h).
 #pragma once
+#include <string>
+
 #include "peer.h"
 #include "prover_internal.h"
 
@@ -28,31 +31,16 @@ Layout make_layout(size_t n, int G, size_t B, bool fri = false);
 // mailbox of round k: run root of run q at roots + 32 q, partial pair of rank g at partials + 32 g
 inline size_t mail_partials(const Layout& a, int k) { return a.mail[k] + MAIL_ROOTS * 32; }
 
-struct ShardCore {
-    int world = 1, L = 0;
+struct ShardCore : PeerHandle {
+    int L = 0;
     size_t n_vars = 0, n = 0, NL = 0, R = 0, nloc = 0, B = 0;
-    const char* who = "ml_pcs_shard";  // prefix of error messages
     Layout lay;
-    std::vector<PeerRank> local;
-    PeerGroup grp;
-    // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
-    static const int N_MARKS = 8;
-    cudaEvent_t mark[N_MARKS] = {nullptr};
-    int n_marks = 0;
 };
 
 inline fe* at(const PeerRank& r, size_t off) { return reinterpret_cast<fe*>(r.arena + off); }
-void mark_phase(ShardCore* sh, int idx);
-PeerRank* rank0_of(ShardCore* sh);
 
-// handle plumbing (arguments already checked by the caller)
-int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, const char* who,
-               bool fri = false);
-void shard_free(ShardCore* sh);
-int shard_export(ShardCore* sh, uint8_t* records_out);
-int shard_connect(ShardCore* sh, const uint8_t* records, size_t n_records, const char* who);
-void* shard_stream(const ShardCore* sh, int local_index);
-int shard_phase_ms(const ShardCore* sh, double* out, int cap);
+// the shape and arena layout, then PeerHandle::init (arguments already checked by the caller, sh->who set)
+int shard_init(ShardCore* sh, int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_vars, size_t B, bool fri = false);
 
 // S0 exchange: slice r of the local code `ycode` -> rank r's recv at off_recv (G > 1)
 int exchange_launch(ShardCore* sh, PeerRank& r, const fe* ycode, size_t off_recv, cudaStream_t s);
@@ -98,6 +86,24 @@ int tail_release(ShardCore* sh, PeerRank& r0, ml_transcript* t);
 // rank 0 after a failed call: its status into every rank's status word, then the same release (finish_ranks returns it)
 int tail_fail(ShardCore* sh, PeerRank& r0, int st);
 int finish_ranks(ShardCore* sh, ml_transcript* t, int st);
+// the end of a call: rank 0's tail (if local; it sets *out); when it fails, its status and message are the call's and the other
+// ranks are released with that status (tail_fail) instead of timing out; then finish_ranks; on error *out is freed
+template <class Proof>
+int end_call(ShardCore* sh, ml_transcript* t, Proof** out, void (*free_proof)(Proof*), const std::function<int(PeerRank& r0)>& tail) {
+    int st0 = ML_OK;
+    std::string msg;
+    if (PeerRank* r0 = sh->rank0()) {
+        st0 = tail(*r0);
+        if (st0 != ML_OK) {
+            msg = ml_last_error();
+            tail_fail(sh, *r0, st0);
+        }
+    }
+    int st = finish_ranks(sh, t, st0);
+    if (st0 != ML_OK) { set_error("%s", msg.c_str()); st = st0; }
+    if (st != ML_OK && *out) { free_proof(*out); *out = nullptr; }
+    return st;
+}
 
 // ---- the FRI provers (fri_shard.cu): no sumcheck tables, every layer root absorbed before its challenge
 // transcript state and status word of one rank at the start of a call
@@ -111,6 +117,7 @@ int fri_fold(ShardCore* sh, PeerRank& r, int k);
 
 // ---- the batched provers (bpcs_shard.cu): B codes in layer 0 under one batched tree
 struct BatchCore : ShardCore {
+    ~BatchCore();  // the events, before the base frees the arenas
     struct Events { cudaEvent_t done[2] = {nullptr, nullptr}, free[2] = {nullptr, nullptr}, join = nullptr; };
     std::vector<Events> ev;  // per local rank: the S0 encode / exchange pipeline
     size_t R0 = 0;           // leaves of a layer-0 segment (R, or N/2 at G = 1)
@@ -118,7 +125,6 @@ struct BatchCore : ShardCore {
 };
 // after shard_init: the pipeline events and the code pointers of every layer-0 segment
 int batch_init(BatchCore* sh);
-void batch_free(BatchCore* sh);  // the events; then shard_free
 // S0 of local rank li (G > 1): per code j, encode(j, y, main) into one of two buffers on the main stream while the side stream
 // stores slice r of code j-1 into rank r's recv slice j-1; flag PX -> all
 int batch_encode_exchange(BatchCore* sh, size_t li, const std::function<int(size_t j, fe* y, cudaStream_t s)>& encode);

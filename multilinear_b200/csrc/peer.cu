@@ -1,5 +1,6 @@
-// Peer plumbing shared by the sharded provers: arenas, flags, push / wait kernels, IPC records (peer.h).
+// Peer plumbing shared by the sharded handles: arenas, flags, push / wait kernels, IPC records, the handle core (peer.h).
 #include <cstdlib>
+#include <string>
 
 #include "peer.h"
 #include "prover_internal.h"
@@ -162,6 +163,106 @@ int peer_read_status(const PeerGroup& g, const PeerRank& r, const char* who) {
     if (st != ML_ERR_PEER) { set_error("%s: rank %d: rank 0 ended the call with status %d", who, r.rank, st); return st; }  // relayed (tail_fail)
     set_error("%s: rank %d timed out waiting for a peer rank (%.0f s)", who, r.rank, g.timeout_ns * 1e-9);
     return ML_ERR_PEER;
+}
+
+
+PeerHandle::~PeerHandle() {
+    DeviceGuard guard;
+    for (int i = 0; i < N_MARKS; i++)
+        if (mark[i]) cudaEventDestroy(mark[i]);
+    for (auto& r : local) {
+        cudaSetDevice(r.device);
+        cudaDeviceSynchronize();
+        peer_rank_free(r);
+    }
+    peer_group_release(grp, local.empty() ? guard.prev : local[0].device);
+}
+
+int PeerHandle::init(int world_, int n_local, const int* local_ranks, const int* local_devices, size_t arena_bytes, size_t off_flags,
+                     size_t off_status, size_t zero_bytes) {
+    const std::string create = std::string(who) + "_create";
+    world = world_;
+    grp.world = world;
+    grp.arena_bytes = arena_bytes;
+    grp.off_flags = off_flags;
+    grp.off_status = off_status;
+    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
+    int st = ML_OK;
+    for (int i = 0; i < n_local && st == ML_OK; i++) {
+        PeerRank r;
+        r.rank = local_ranks[i];
+        r.device = local_devices[i];
+        st = peer_rank_init(grp, r, create.c_str(), zero_bytes);
+        if (st == ML_OK || st == ML_ERR_ALLOC) local.push_back(r);
+    }
+    if (st == ML_OK && n_local == world) {
+        std::vector<PeerRank*> ranks;
+        for (auto& r : local) ranks.push_back(&r);
+        st = peer_link_local(grp, ranks, create.c_str());
+    }
+    return st;
+}
+
+int PeerHandle::export_records(uint8_t* records_out) {
+    std::vector<PeerRank*> ranks;
+    for (auto& r : local) ranks.push_back(&r);
+    return peer_export(ranks, records_out);
+}
+int PeerHandle::connect(const uint8_t* records, size_t n_records) {
+    const std::string entry = std::string(who) + "_connect";
+    if (local.size() != 1) { set_error("%s: only for handles that host one rank", entry.c_str()); return ML_ERR_ARG; }
+    return peer_connect(grp, local[0], records, n_records, entry.c_str());
+}
+void* PeerHandle::stream(int local_index) const {
+    if (local_index < 0 || (size_t)local_index >= local.size()) return nullptr;
+    return (void*)local[local_index].st.main;
+}
+int PeerHandle::phase_ms(double* out, int cap) const {
+    int n = 0;
+    for (int i = 0; i + 1 < n_marks && n < cap; i++) {
+        float ms = 0;
+        if (!mark[i] || !mark[i + 1] || cudaEventElapsedTime(&ms, mark[i], mark[i + 1]) != cudaSuccess) { cudaGetLastError(); ms = -1.f; }
+        out[n++] = ms;
+    }
+    return n;
+}
+void PeerHandle::mark_phase(int idx) {
+    if (idx >= N_MARKS || local.empty()) return;
+    PeerRank& r = local[0];
+    cudaSetDevice(r.device);
+    if (!mark[idx] && cudaEventCreate(&mark[idx]) != cudaSuccess) { cudaGetLastError(); return; }
+    cudaEventRecord(mark[idx], r.st.main);
+    if (idx + 1 > n_marks) n_marks = idx + 1;
+}
+PeerRank* PeerHandle::rank0() {
+    for (auto& r : local)
+        if (r.rank == 0) return &r;
+    return nullptr;
+}
+
+int PeerHandle::host_call(const char* entry, size_t n_blocks, size_t bytes, const std::function<const uint8_t*(int rank, size_t j)>& src,
+                          const std::function<int(const void* const* dev)>& run) {
+    if ((int)local.size() != world) { set_error("%s: host-pointer entry needs a handle that hosts every rank", entry); return ML_ERR_ARG; }
+    DeviceGuard guard;
+    std::vector<void*> dev(local.size() * n_blocks, nullptr);
+    int st = ML_OK;
+    for (size_t i = 0; i < local.size() && st == ML_OK; i++) {
+        PeerRank& r = local[i];
+        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
+        for (size_t j = 0; j < n_blocks && st == ML_OK; j++) {
+            void*& d = dev[i * n_blocks + j];
+            st = mlbp::pmalloc(&d, bytes, r.st.main);
+            if (st == ML_OK) st = mlbp::h2d(d, src(r.rank, j), bytes, r.st.main);
+        }
+        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
+    }
+    if (st == ML_OK) st = run(dev.data());
+    for (size_t i = 0; i < local.size(); i++) {
+        cudaSetDevice(local[i].device);
+        cudaStreamSynchronize(local[i].st.main);
+        for (size_t j = 0; j < n_blocks; j++) mlbp::pfree(dev[i * n_blocks + j], local[i].st.main);
+    }
+    return st;
 }
 
 }  // namespace mlb

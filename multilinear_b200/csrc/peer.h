@@ -1,4 +1,5 @@
-// Peer plumbing shared by the sharded provers (shard.cu: batched proof, pcs_shard.cu: one PCS proof).
+// Peer plumbing shared by every sharded handle (ml_shard_*, ml_pcs_shard_*, ml_bpcs_shard_*, ml_fri_shard_*, ml_bfri_shard_*,
+// ml_wsumcheck_shard_*): arenas, flags, push / wait kernels, IPC records, and the handle core PeerHandle.
 //
 // Every rank owns one peer-visible ARENA in HBM (cudaMalloc; mapped into the other ranks through CUDA IPC, or plain peer access
 // when one process hosts all ranks).  The arena starts with a mailbox of flags: flag[phase][rank].  All data-path exchange is a
@@ -11,6 +12,7 @@
 // and the host enqueues phase by phase over the local ranks, so on a shared device every wait is already satisfied when it is
 // enqueued.
 #pragma once
+#include <functional>
 #include <map>
 #include <vector>
 
@@ -116,5 +118,35 @@ int peer_wait_for(const PeerGroup& g, const PeerRank& r, int phase, int only_fro
 int peer_push(const PeerGroup& g, const PeerRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s);
 // ML_ERR_PEER if a wait of r's timed out, or the status rank 0 stored into r's status word (synchronises r's main stream)
 int peer_read_status(const PeerGroup& g, const PeerRank& r, const char* who);
+
+// The host side of a sharded handle: the ranks this process hosts, their group and the phase marks of the last call.  A handle
+// type derives from it and adds its shape, arena layout and stages.
+struct PeerHandle {
+    int world = 1;
+    const char* who = "";  // ABI prefix of the handle (ml_pcs_shard, ...), the prefix of its error messages
+    std::vector<PeerRank> local;
+    PeerGroup grp;
+    // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
+    static const int N_MARKS = 10;
+    cudaEvent_t mark[N_MARKS] = {nullptr};
+    int n_marks = 0;
+
+    ~PeerHandle();  // marks, arenas (each device idle first), IPC mappings and streams
+    // the group over an arena layout (timeout from MLB_SHARD_TIMEOUT_S), every local rank (first zero_bytes of its arena
+    // cleared) and, when this process hosts every rank, the links between them (arguments checked by peer_check_world)
+    int init(int world, int n_local, const int* local_ranks, const int* local_devices, size_t arena_bytes, size_t off_flags, size_t off_status,
+             size_t zero_bytes);
+    int export_records(uint8_t* records_out);
+    int connect(const uint8_t* records, size_t n_records);  // a handle that hosts one rank
+    void* stream(int local_index) const;
+    int phase_ms(double* out, int cap) const;  // device time between consecutive marks
+    void mark_phase(int idx);
+    PeerRank* rank0();  // nullptr unless this process hosts rank 0
+    int check_ready() const { return peer_check_ready(grp, who); }
+    // host-pointer entry `entry` (a handle that hosts every rank): uploads n_blocks blocks of `bytes` to every local rank, block j of
+    // rank r from src(r, j), runs run(dev) with block j of local rank i at dev[i * n_blocks + j], then frees the blocks
+    int host_call(const char* entry, size_t n_blocks, size_t bytes, const std::function<const uint8_t*(int rank, size_t j)>& src,
+                  const std::function<int(const void* const* dev)>& run);
+};
 
 }  // namespace mlb

@@ -254,7 +254,8 @@ __global__ void __launch_bounds__(64) shard_gather_kernel(const unsigned long lo
 }
 
 // ------------------------------------------------------------------ host side
-struct ShardRank : PeerRank {
+// the buffers of one local rank beside its arena
+struct ShardBufs {
     fe* code[2] = {nullptr, nullptr};
     cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr}, ev_fork = nullptr, ev_enc2 = nullptr, ev_side = nullptr;
     const fe** evals_ptrs_dev = nullptr;  // n_local_polys device pointers
@@ -263,77 +264,58 @@ struct ShardRank : PeerRank {
 
 }  // namespace
 
-struct ml_shard {
-    int world = 1;
+struct ml_shard : PeerHandle {
     size_t B = 0, n_vars = 0, n = 0, rows = 0, slice = 0, polys_per_rank = 0;
     Layout lay;
-    std::vector<ShardRank> local;
-    PeerGroup grp;  // arenas of all ranks, flags, epoch, timeout (peer.h)
-    // device-time marks of the last call on the first local rank's main stream (include/multilinear_b200_instr.h)
-    static const int N_MARKS = 10;
-    cudaEvent_t mark[N_MARKS] = {nullptr};
-    int n_marks = 0;
+    std::vector<ShardBufs> bufs;  // per local rank
     unsigned pack_ctas = 32;
+    ~ml_shard();  // the buffers, before the base frees the arenas
 };
 
 namespace {
 
 PeerPtrs peers_of(const ml_shard* sh) { return sh->grp.peers(); }
-unsigned long long* flags_at(const ml_shard* sh, const ShardRank& r, int phase) { return sh->grp.flags(r, phase); }
-int* status_at(const ml_shard* sh, const ShardRank& r) { return sh->grp.status(r); }
-int signal(const ml_shard* sh, const ShardRank& r, int phase, int only, cudaStream_t s) { return peer_signal(sh->grp, r, phase, only, s); }
-int wait(const ml_shard* sh, const ShardRank& r, int phase, int only_from, cudaStream_t s) { return peer_wait(sh->grp, r, phase, only_from, s); }
-int push(const ml_shard* sh, const ShardRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s) {
+unsigned long long* flags_at(const ml_shard* sh, const PeerRank& r, int phase) { return sh->grp.flags(r, phase); }
+int* status_at(const ml_shard* sh, const PeerRank& r) { return sh->grp.status(r); }
+int signal(const ml_shard* sh, const PeerRank& r, int phase, int only, cudaStream_t s) { return peer_signal(sh->grp, r, phase, only, s); }
+int wait(const ml_shard* sh, const PeerRank& r, int phase, int only_from, cudaStream_t s) { return peer_wait(sh->grp, r, phase, only_from, s); }
+int push(const ml_shard* sh, const PeerRank& r, const void* src_dev, int nbytes, size_t dst_off, int phase, int only, cudaStream_t s) {
     return peer_push(sh->grp, r, src_dev, nbytes, dst_off, phase, only, s);
 }
 unsigned grid_for(size_t n) { return peer_grid(n); }
 
-void free_rank(ShardRank& r) {
-    cudaSetDevice(r.device);
-    cudaDeviceSynchronize();
-    for (int b = 0; b < 2; b++) {
-        if (r.code[b]) cudaFree(r.code[b]);
-        if (r.ev_done[b]) cudaEventDestroy(r.ev_done[b]);
-        if (r.ev_free[b]) cudaEventDestroy(r.ev_free[b]);
-    }
-    if (r.ev_fork) cudaEventDestroy(r.ev_fork);
-    if (r.ev_enc2) cudaEventDestroy(r.ev_enc2);
-    if (r.ev_side) cudaEventDestroy(r.ev_side);
-    if (r.evals_ptrs_dev) cudaFree((void*)r.evals_ptrs_dev);
-    if (r.pinned) cudaFreeHost(r.pinned);
-    peer_rank_free(r);
-}
-
-// ---- S0: encode + pack of one local rank (enqueue only)
-int stage_encode_pack(ml_shard* sh, ShardRank& r, const void* const* evals /* this rank's polynomials */) {
+// ---- S0: encode + pack of local rank li (enqueue only)
+int stage_encode_pack(ml_shard* sh, size_t li, const void* const* evals /* this rank's polynomials */) {
+    PeerRank& r = sh->local[li];
+    ShardBufs& x = sh->bufs[li];
     MLB_CUDA(cudaSetDevice(r.device));
     const size_t n = sh->n, N = 2 * n;
     cudaStream_t main = r.st.main, es[2] = {r.st.main, r.st.enc2}, side = r.st.side;
-    MLB_CUDA(cudaEventRecord(r.ev_fork, main));
-    MLB_CUDA(cudaStreamWaitEvent(r.st.enc2, r.ev_fork, 0));
-    MLB_CUDA(cudaStreamWaitEvent(side, r.ev_fork, 0));
+    MLB_CUDA(cudaEventRecord(x.ev_fork, main));
+    MLB_CUDA(cudaStreamWaitEvent(r.st.enc2, x.ev_fork, 0));
+    MLB_CUDA(cudaStreamWaitEvent(side, x.ev_fork, 0));
     const PeerPtrs peers = peers_of(sh);
     size_t blocks = (n + 255) / 256;
     if (blocks > sh->pack_ctas) blocks = sh->pack_ctas;
     for (size_t l = 0; l < sh->polys_per_rank; l++) {
         const int b = (int)(l & 1);
-        if (l >= 2) MLB_CUDA(cudaStreamWaitEvent(es[b], r.ev_free[b], 0));  // the store pass has finished reading code buffer b
-        MLB_TRY(encode_into(r.ctx, (const fe*)evals[l], n, r.code[b], es[b]));
-        MLB_CUDA(cudaEventRecord(r.ev_done[b], es[b]));
-        MLB_CUDA(cudaStreamWaitEvent(side, r.ev_done[b], 0));
+        if (l >= 2) MLB_CUDA(cudaStreamWaitEvent(es[b], x.ev_free[b], 0));  // the store pass has finished reading code buffer b
+        MLB_TRY(encode_into(r.ctx, (const fe*)evals[l], n, x.code[b], es[b]));
+        MLB_CUDA(cudaEventRecord(x.ev_done[b], es[b]));
+        MLB_CUDA(cudaStreamWaitEvent(side, x.ev_done[b], 0));
         // the store pass runs on a small grid: it is NVLink-latency bound and must leave the SMs to the next polynomial's NTT
-        shard_pack_kernel<<<(unsigned)blocks, 256, 0, side>>>(r.code[b], N / 2, sh->rows, (size_t)r.rank + l * sh->world, peers, sh->lay.pairs);
+        shard_pack_kernel<<<(unsigned)blocks, 256, 0, side>>>(x.code[b], N / 2, sh->rows, (size_t)r.rank + l * sh->world, peers, sh->lay.pairs);
         MLB_KERNEL_CHECK();
-        MLB_CUDA(cudaEventRecord(r.ev_free[b], side));
+        MLB_CUDA(cudaEventRecord(x.ev_free[b], side));
     }
-    MLB_CUDA(cudaEventRecord(r.ev_enc2, r.st.enc2));
-    MLB_CUDA(cudaStreamWaitEvent(main, r.ev_enc2, 0));
-    MLB_CUDA(cudaEventRecord(r.ev_side, side));
-    MLB_CUDA(cudaStreamWaitEvent(main, r.ev_side, 0));
+    MLB_CUDA(cudaEventRecord(x.ev_enc2, r.st.enc2));
+    MLB_CUDA(cudaStreamWaitEvent(main, x.ev_enc2, 0));
+    MLB_CUDA(cudaEventRecord(x.ev_side, side));
+    MLB_CUDA(cudaStreamWaitEvent(main, x.ev_side, 0));
     return signal(sh, r, P1, -1, main);
 }
 // ---- S1: leaf range subtree, root to everybody
-int stage_subtree(ml_shard* sh, ShardRank& r) {
+int stage_subtree(ml_shard* sh, PeerRank& r) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     MLB_TRY(wait(sh, r, P1, -1, s));
@@ -343,7 +325,7 @@ int stage_subtree(ml_shard* sh, ShardRank& r) {
     return push(sh, r, root, 32, sh->lay.roots + 32 * (size_t)r.rank, P2, -1, s);
 }
 // ---- S2a: batch root (+ transcript, rho, claimed sum)
-int stage_root(ml_shard* sh, ShardRank& r, bool with_transcript) {
+int stage_root(ml_shard* sh, PeerRank& r, bool with_transcript) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     shard_root_kernel<<<1, 32, 0, s>>>(flags_at(sh, r, P2), sh->world, sh->grp.epoch, sh->grp.timeout_ns, status_at(sh, r), r.arena + sh->lay.roots,
@@ -354,16 +336,17 @@ int stage_root(ml_shard* sh, ShardRank& r, bool with_transcript) {
     return ML_OK;
 }
 // ---- S2b: fingerprint partial sums into the slice owners' stage areas
-int stage_fp_partial(ml_shard* sh, ShardRank& r) {
+int stage_fp_partial(ml_shard* sh, size_t li) {
+    PeerRank& r = sh->local[li];
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
-    shard_fp_partial_kernel<<<grid_for(sh->n), 256, 0, s>>>(r.evals_ptrs_dev, (int)sh->polys_per_rank, sh->n, (const fe*)(r.arena + sh->lay.fr), r.rank,
+    shard_fp_partial_kernel<<<grid_for(sh->n), 256, 0, s>>>(sh->bufs[li].evals_ptrs_dev, (int)sh->polys_per_rank, sh->n, (const fe*)(r.arena + sh->lay.fr), r.rank,
                                                             sh->world, peers_of(sh), sh->lay.stage, sh->slice);
     MLB_KERNEL_CHECK();
     return signal(sh, r, P3, -1, s);
 }
 // ---- S3: reduce the own slice into rank 0's matrix
-int stage_fp_reduce(ml_shard* sh, ShardRank& r) {
+int stage_fp_reduce(ml_shard* sh, PeerRank& r) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     MLB_TRY(wait(sh, r, P3, -1, s));
@@ -373,7 +356,7 @@ int stage_fp_reduce(ml_shard* sh, ShardRank& r) {
     return signal(sh, r, P4, 0, s);
 }
 // ---- S5: first fold of the own rows into rank 0's `next`
-int stage_first_fold(ml_shard* sh, ShardRank& r) {
+int stage_first_fold(ml_shard* sh, PeerRank& r) {
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     const int log_n0 = (int)sh->n_vars + ML_LOG_BLOWUP;
@@ -388,28 +371,14 @@ int stage_first_fold(ml_shard* sh, ShardRank& r) {
     return signal(sh, r, P6, 0, s);
 }
 
-// phase boundary on the first local rank's main stream
-void mark_phase(ml_shard* sh, int idx) {
-    if (idx >= ml_shard::N_MARKS || sh->local.empty()) return;
-    ShardRank& r = sh->local[0];
-    cudaSetDevice(r.device);
-    if (!sh->mark[idx] && cudaEventCreate(&sh->mark[idx]) != cudaSuccess) { cudaGetLastError(); return; }
-    cudaEventRecord(sh->mark[idx], r.st.main);
-    if (idx + 1 > sh->n_marks) sh->n_marks = idx + 1;
-}
-ShardRank* rank0_of(ml_shard* sh) {
-    for (auto& r : sh->local)
-        if (r.rank == 0) return &r;
-    return nullptr;
-}
-
-int check_ready(ml_shard* sh) { return peer_check_ready(sh->grp, "ml_shard"); }
 // upload the per-call small inputs of a rank through its pinned staging block (asynchronous, stream ordered)
-int upload_inputs(ml_shard* sh, ShardRank& r, const HostSha256* tr, const uint8_t* outputs, const void* const* evals) {
+int upload_inputs(ml_shard* sh, size_t li, const HostSha256* tr, const uint8_t* outputs, const void* const* evals) {
+    PeerRank& r = sh->local[li];
+    ShardBufs& x = sh->bufs[li];
     MLB_CUDA(cudaSetDevice(r.device));
     cudaStream_t s = r.st.main;
     MLB_CUDA(cudaStreamSynchronize(s));  // the staging block of the previous call is free (calls on one handle are sequential anyway)
-    uint8_t* h = r.pinned;
+    uint8_t* h = x.pinned;
     const size_t o_tr = 0, o_out = 128, o_ptr = 128 + align_up(sh->B * 16);
     if (tr) {
         memcpy(h + o_tr, tr, sizeof(DevTranscript));
@@ -420,14 +389,14 @@ int upload_inputs(ml_shard* sh, ShardRank& r, const HostSha256* tr, const uint8_
         MLB_CUDA(cudaMemcpyAsync(r.arena + sh->lay.outputs, h + o_out, sh->B * 16, cudaMemcpyHostToDevice, s));
     }
     memcpy(h + o_ptr, evals, sh->polys_per_rank * sizeof(void*));
-    MLB_CUDA(cudaMemcpyAsync((void*)r.evals_ptrs_dev, h + o_ptr, sh->polys_per_rank * sizeof(void*), cudaMemcpyHostToDevice, s));
+    MLB_CUDA(cudaMemcpyAsync((void*)x.evals_ptrs_dev, h + o_ptr, sh->polys_per_rank * sizeof(void*), cudaMemcpyHostToDevice, s));
     MLB_CUDA(cudaMemsetAsync(status_at(sh, r), 0, 16, s));
     return ML_OK;
 }
-int read_status(ml_shard* sh, ShardRank& r) { return peer_read_status(sh->grp, r, "ml_shard"); }
+int read_status(ml_shard* sh, PeerRank& r) { return peer_read_status(sh->grp, r, "ml_shard"); }
 
 // batch layer openings + the rest of the proof on rank 0 (batched_fri.rs:207-225, 296-308)
-int shard_assemble(ml_shard* sh, ShardRank& r0, ml_fri* fri, ml_transcript* t, ml_bfri_proof* p, const uint8_t batch_root[32]) {
+int shard_assemble(ml_shard* sh, PeerRank& r0, ml_fri* fri, ml_transcript* t, ml_bfri_proof* p, const uint8_t batch_root[32]) {
     cudaStream_t s = r0.st.main;
     const size_t N = 2 * sh->n, L = sh->n, B = sh->B;
     if (fri->layers.empty()) { set_error("open_query_at: no folded layer (domain too small)"); return ML_ERR_OUT_OF_RANGE; }
@@ -469,6 +438,25 @@ int shard_assemble(ml_shard* sh, ShardRank& r0, ml_fri* fri, ml_transcript* t, m
 
 }  // namespace
 
+ml_shard::~ml_shard() {
+    DeviceGuard guard;
+    for (size_t i = 0; i < bufs.size(); i++) {
+        ShardBufs& x = bufs[i];
+        cudaSetDevice(local[i].device);
+        cudaDeviceSynchronize();
+        for (int b = 0; b < 2; b++) {
+            if (x.code[b]) cudaFree(x.code[b]);
+            if (x.ev_done[b]) cudaEventDestroy(x.ev_done[b]);
+            if (x.ev_free[b]) cudaEventDestroy(x.ev_free[b]);
+        }
+        if (x.ev_fork) cudaEventDestroy(x.ev_fork);
+        if (x.ev_enc2) cudaEventDestroy(x.ev_enc2);
+        if (x.ev_side) cudaEventDestroy(x.ev_side);
+        if (x.evals_ptrs_dev) cudaFree((void*)x.evals_ptrs_dev);
+        if (x.pinned) cudaFreeHost(x.pinned);
+    }
+}
+
 extern "C" {
 
 int ml_shard_create(int world, int n_local, const int* local_ranks, const int* local_devices, size_t n_polys, size_t n_vars, ml_shard** out) {
@@ -481,38 +469,26 @@ int ml_shard_create(int world, int n_local, const int* local_ranks, const int* l
     }
     DeviceGuard guard;
     ml_shard* sh = new ml_shard();
-    sh->world = world; sh->B = n_polys; sh->n_vars = n_vars; sh->n = n;
+    sh->who = "ml_shard";
+    sh->B = n_polys; sh->n_vars = n_vars; sh->n = n;
     sh->rows = n / world; sh->slice = n / world; sh->polys_per_rank = n_polys / world;
     sh->lay = make_layout(n_polys, n, world);
-    sh->grp.world = world;
-    sh->grp.arena_bytes = sh->lay.total;
-    sh->grp.off_flags = sh->lay.flags;
-    sh->grp.off_status = sh->lay.status;
-    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
     if (const char* e = getenv("MLB_SHARD_PACK_CTAS")) sh->pack_ctas = (unsigned)atoi(e);
-    int st = ML_OK;
-    for (int i = 0; i < n_local && st == ML_OK; i++) {
-        ShardRank r;
-        r.rank = local_ranks[i];
-        r.device = local_devices[i];
-        st = peer_rank_init(sh->grp, r, "ml_shard_create", sh->lay.pairs);
-        if (st != ML_OK && st != ML_ERR_ALLOC) break;
-        bool ok = st == ML_OK && cudaMalloc((void**)&r.code[0], 2 * n * 16) == cudaSuccess && cudaMalloc((void**)&r.code[1], 2 * n * 16) == cudaSuccess &&
-                  cudaMalloc((void**)&r.evals_ptrs_dev, sh->polys_per_rank * sizeof(void*)) == cudaSuccess &&
-                  cudaMallocHost((void**)&r.pinned, 128 + align_up(n_polys * 16) + sh->polys_per_rank * sizeof(void*)) == cudaSuccess;
+    int st = sh->init(world, n_local, local_ranks, local_devices, sh->lay.total, sh->lay.flags, sh->lay.status, sh->lay.pairs);
+    sh->bufs.resize(sh->local.size());
+    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
+        ShardBufs& x = sh->bufs[i];
+        cudaSetDevice(sh->local[i].device);
+        bool ok = cudaMalloc((void**)&x.code[0], 2 * n * 16) == cudaSuccess && cudaMalloc((void**)&x.code[1], 2 * n * 16) == cudaSuccess &&
+                  cudaMalloc((void**)&x.evals_ptrs_dev, sh->polys_per_rank * sizeof(void*)) == cudaSuccess &&
+                  cudaMallocHost((void**)&x.pinned, 128 + align_up(n_polys * 16) + sh->polys_per_rank * sizeof(void*)) == cudaSuccess;
         for (int b = 0; b < 2 && ok; b++)
-            ok = cudaEventCreateWithFlags(&r.ev_done[b], cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&r.ev_free[b], cudaEventDisableTiming) == cudaSuccess;
-        ok = ok && cudaEventCreateWithFlags(&r.ev_fork, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&r.ev_enc2, cudaEventDisableTiming) == cudaSuccess &&
-             cudaEventCreateWithFlags(&r.ev_side, cudaEventDisableTiming) == cudaSuccess;
-        sh->local.push_back(r);
-        if (!ok) { cudaGetLastError(); set_error("ml_shard_create: allocation of %zu bytes on device %d failed", sh->lay.total, r.device); st = ML_ERR_ALLOC; }
+            ok = cudaEventCreateWithFlags(&x.ev_done[b], cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&x.ev_free[b], cudaEventDisableTiming) == cudaSuccess;
+        ok = ok && cudaEventCreateWithFlags(&x.ev_fork, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&x.ev_enc2, cudaEventDisableTiming) == cudaSuccess &&
+             cudaEventCreateWithFlags(&x.ev_side, cudaEventDisableTiming) == cudaSuccess;
+        if (!ok) { cudaGetLastError(); set_error("ml_shard_create: allocation of %zu bytes on device %d failed", sh->lay.total, sh->local[i].device); st = ML_ERR_ALLOC; }
     }
-    if (st == ML_OK && n_local == world) {
-        std::vector<PeerRank*> ranks;
-        for (auto& r : sh->local) ranks.push_back(&r);
-        st = peer_link_local(sh->grp, ranks, "ml_shard_create");
-    }
-    if (st != ML_OK) { ml_shard_free(sh); return st; }
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
@@ -520,57 +496,31 @@ int ml_shard_create(int world, int n_local, const int* local_ranks, const int* l
 // INSTRUMENTATION (include/multilinear_b200_instr.h): device time between the phase marks of the last call on the first local
 // rank's main stream, in ms: commit: [S0 encode+pack, S1 subtree, S2 root]; prove: [S0, S1, S2 root+rho, S2 fingerprint partials,
 // S3 reduce, S4 wait for the matrix (rank 0), chain incl. S5 first fold (rank 0), openings + proof (rank 0)].  Returns the count.
-int ml_shard_phase_ms(const ml_shard* sh, double* out, int cap) {
-    int n = 0;
-    for (int i = 0; i + 1 < sh->n_marks && n < cap; i++) {
-        float ms = 0;
-        if (!sh->mark[i] || !sh->mark[i + 1] || cudaEventElapsedTime(&ms, sh->mark[i], sh->mark[i + 1]) != cudaSuccess) { cudaGetLastError(); ms = -1.f; }
-        out[n++] = ms;
-    }
-    return n;
-}
+int ml_shard_phase_ms(const ml_shard* sh, double* out, int cap) { return sh->phase_ms(out, cap); }
 
-void ml_shard_free(ml_shard* sh) {
-    if (!sh) return;
-    DeviceGuard guard;
-    for (int i = 0; i < ml_shard::N_MARKS; i++)
-        if (sh->mark[i]) cudaEventDestroy(sh->mark[i]);
-    for (auto& r : sh->local) free_rank(r);
-    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
-    delete sh;
-}
+void ml_shard_free(ml_shard* sh) { delete sh; }
 
 /* one record per local rank: int32 rank | int32 reserved | 64-byte CUDA IPC handle of the arena */
 size_t ml_shard_record_bytes(void) { return PEER_RECORD_BYTES; }
 int ml_shard_num_local(const ml_shard* sh) { return (int)sh->local.size(); }
-int ml_shard_export(ml_shard* sh, uint8_t* records_out) {
-    std::vector<PeerRank*> ranks;
-    for (auto& r : sh->local) ranks.push_back(&r);
-    return peer_export(ranks, records_out);
-}
-int ml_shard_connect(ml_shard* sh, const uint8_t* records, size_t n_records) {
-    if (sh->local.size() != 1) { set_error("ml_shard_connect: only for handles that host one rank"); return ML_ERR_ARG; }
-    return peer_connect(sh->grp, sh->local[0], records, n_records, "ml_shard_connect");
-}
-void* ml_shard_stream(const ml_shard* sh, int local_index) {
-    if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
-    return (void*)sh->local[local_index].st.main;
-}
+int ml_shard_export(ml_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_shard_connect(ml_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_shard_stream(const ml_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_shard_arena_bytes(const ml_shard* sh) { return sh->lay.total; }
 
 // Merkle::batch_commit of the encoded batch (batched_fri.rs:62-77 after batched_pcs.rs:144-149): phases S0-S2a.
 // local_evals_dev: for every local rank in handle order, its polynomials in increasing global index (rank, rank+G, ...).
 int ml_shard_batch_commit_dev(ml_shard* sh, const void* const* local_evals_dev, uint8_t root_out[32]) {
-    MLB_TRY(check_ready(sh));
+    MLB_TRY(sh->check_ready());
     DeviceGuard guard;
     sh->grp.epoch++;
     const size_t ppr = sh->polys_per_rank;
-    for (size_t i = 0; i < sh->local.size(); i++) MLB_TRY(upload_inputs(sh, sh->local[i], nullptr, nullptr, local_evals_dev + i * ppr));
+    for (size_t i = 0; i < sh->local.size(); i++) MLB_TRY(upload_inputs(sh, i, nullptr, nullptr, local_evals_dev + i * ppr));
     sh->n_marks = 0;
-    mark_phase(sh, 0);
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_encode_pack(sh, sh->local[i], local_evals_dev + i * ppr)); if (i == 0) mark_phase(sh, 1); }
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_subtree(sh, sh->local[i])); if (i == 0) mark_phase(sh, 2); }
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_root(sh, sh->local[i], false)); if (i == 0) mark_phase(sh, 3); }
+    sh->mark_phase(0);
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_encode_pack(sh, i, local_evals_dev + i * ppr)); if (i == 0) sh->mark_phase(1); }
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_subtree(sh, sh->local[i])); if (i == 0) sh->mark_phase(2); }
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_root(sh, sh->local[i], false)); if (i == 0) sh->mark_phase(3); }
     int st = ML_OK;
     for (auto& r : sh->local) {
         MLB_CUDA(cudaSetDevice(r.device));
@@ -585,7 +535,7 @@ int ml_shard_batch_commit_dev(ml_shard* sh, const void* const* local_evals_dev, 
 // proof comes out on the process that hosts rank 0 (*out = NULL elsewhere); every transcript ends in the same state.
 int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t* outputs, size_t n_polys,
                                    const void* const* local_evals_dev, ml_transcript* t, ml_bpcs_proof** out) {
-    MLB_TRY(check_ready(sh));
+    MLB_TRY(sh->check_ready());
     if (n_vars != sh->n_vars || n_polys != sh->B) { set_error("ml_shard_batched_pcs_prove: claim does not match the handle's shape"); return ML_ERR_SIZE; }
     DeviceGuard guard;
     *out = nullptr;
@@ -594,12 +544,12 @@ int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n
     // BatchedPCSProverData::init (:37-77): the claim enters the transcript first
     t->sha.update(inputs, n_vars * 16);    // :44-46
     t->sha.update(outputs, n_polys * 16);  // :47-49
-    ShardRank* r0 = rank0_of(sh);
+    PeerRank* r0 = sh->rank0();
     ml_sumcheck* sc = nullptr;
     std::vector<hfe> pts(n_vars), outs(n_polys);
     for (size_t i = 0; i < n_vars; i++) pts[i] = hfe_load(inputs + 16 * i);
     for (size_t i = 0; i < n_polys; i++) outs[i] = hfe_load(outputs + 16 * i);
-    for (size_t i = 0; i < sh->local.size(); i++) MLB_TRY(upload_inputs(sh, sh->local[i], &t->sha, outputs, local_evals_dev + i * ppr));
+    for (size_t i = 0; i < sh->local.size(); i++) MLB_TRY(upload_inputs(sh, i, &t->sha, outputs, local_evals_dev + i * ppr));
     if (r0) {  // the eq table does not depend on anything (:66-67): build it while the stream is idle
         MLB_CUDA(cudaSetDevice(r0->device));
         sc = new ml_sumcheck();
@@ -614,23 +564,23 @@ int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n
     struct ScGuard { ml_sumcheck* p; ~ScGuard() { free_sumcheck(p); } } sc_guard{sc};
 
     sh->n_marks = 0;
-    mark_phase(sh, 0);
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_encode_pack(sh, sh->local[i], local_evals_dev + i * ppr)); if (i == 0) mark_phase(sh, 1); }  // S0
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_subtree(sh, sh->local[i])); if (i == 0) mark_phase(sh, 2); }                                  // S1
+    sh->mark_phase(0);
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_encode_pack(sh, i, local_evals_dev + i * ppr)); if (i == 0) sh->mark_phase(1); }  // S0
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_subtree(sh, sh->local[i])); if (i == 0) sh->mark_phase(2); }                                  // S1
     for (size_t i = 0; i < sh->local.size(); i++) {                                                                                                              // S2
         MLB_TRY(stage_root(sh, sh->local[i], true));
-        if (i == 0) mark_phase(sh, 3);
-        MLB_TRY(stage_fp_partial(sh, sh->local[i]));
-        if (i == 0) mark_phase(sh, 4);
+        if (i == 0) sh->mark_phase(3);
+        MLB_TRY(stage_fp_partial(sh, i));
+        if (i == 0) sh->mark_phase(4);
     }
-    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_fp_reduce(sh, sh->local[i])); if (i == 0) mark_phase(sh, 5); }                               // S3
+    for (size_t i = 0; i < sh->local.size(); i++) { MLB_TRY(stage_fp_reduce(sh, sh->local[i])); if (i == 0) sh->mark_phase(5); }                               // S3
 
     int st = ML_OK;
     if (r0) {
         MLB_CUDA(cudaSetDevice(r0->device));
         cudaStream_t s = r0->st.main;
         MLB_TRY(wait(sh, *r0, P4, -1, s));  // S4: the sumcheck matrix is complete
-        if (r0 == &sh->local[0]) mark_phase(sh, 6);
+        if (r0 == &sh->local[0]) sh->mark_phase(6);
         ml_fri* fri = new ml_fri();
         fri->log_n0 = (int)ilog2(domain);
         fri->stream = s;
@@ -650,12 +600,12 @@ int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n
         const size_t num_steps = ilog2(domain) - ML_LOG_BLOWUP;  // :90
         p->sumcheck.resize(2 * num_steps);
         st = fold_chain_dev(r0->ctx, fri, &hooks, sc, 0, p->sumcheck.data(), 0, false, t, s);  // :100-123
-        if (r0 == &sh->local[0]) mark_phase(sh, 7);
+        if (r0 == &sh->local[0]) sh->mark_phase(7);
         uint8_t batch_root[32];
         if (st == ML_OK) st = d2h_sync(batch_root, r0->arena + sh->lay.root_out, 32, s);
         if (st == ML_OK) st = read_status(sh, *r0);
         if (st == ML_OK) st = shard_assemble(sh, *r0, fri, t, &p->fri, batch_root);              // :155-173
-        if (r0 == &sh->local[0]) mark_phase(sh, 8);
+        if (r0 == &sh->local[0]) sh->mark_phase(8);
         free_fri(fri);
         if (st == ML_OK) {  // final transcript to everybody; also releases the other ranks' buffers for the next call
             Scratch trd(s);
@@ -690,29 +640,9 @@ int ml_shard_batched_pcs_prove_dev(ml_shard* sh, const uint8_t* inputs, size_t n
 // host-pointer convenience for a single-process handle: evals[j] are the n_polys evaluation tables on the host
 int ml_shard_batched_pcs_prove(ml_shard* sh, const uint8_t* inputs, size_t n_vars, const uint8_t* outputs, size_t n_polys,
                                const uint8_t* const* evals, ml_transcript* t, ml_bpcs_proof** out) {
-    if ((int)sh->local.size() != sh->world) { set_error("ml_shard_batched_pcs_prove: host-pointer entry needs a handle that hosts every rank"); return ML_ERR_ARG; }
     if (n_polys != sh->B || n_vars != sh->n_vars) { set_error("ml_shard_batched_pcs_prove: claim does not match the handle's shape"); return ML_ERR_SIZE; }
-    DeviceGuard guard;
-    const size_t ppr = sh->polys_per_rank;
-    std::vector<void*> dev(n_polys, nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        ShardRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        for (size_t l = 0; l < ppr && st == ML_OK; l++) {
-            void*& d = dev[i * ppr + l];
-            st = pmalloc(&d, sh->n * 16, r.st.main);
-            if (st == ML_OK) st = h2d(d, evals[(size_t)r.rank + l * sh->world], sh->n * 16, r.st.main);
-        }
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK) st = ml_shard_batched_pcs_prove_dev(sh, inputs, n_vars, outputs, n_polys, dev.data(), t, out);
-    for (size_t i = 0; i < sh->local.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        for (size_t l = 0; l < ppr; l++) pfree(dev[i * ppr + l], sh->local[i].st.main);
-    }
-    return st;
+    return sh->host_call("ml_shard_batched_pcs_prove", sh->polys_per_rank, sh->n * 16, [&](int rank, size_t l) { return evals[(size_t)rank + l * sh->world]; },
+                         [&](const void* const* dev) { return ml_shard_batched_pcs_prove_dev(sh, inputs, n_vars, outputs, n_polys, dev, t, out); });
 }
 
 }  // extern "C"

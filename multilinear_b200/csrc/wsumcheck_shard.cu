@@ -16,8 +16,6 @@
 //   Tail: wait PG; wchain_tail_kernel on T rows, identically on every rank; one D2H of the coefficients, randoms and transcript.
 //   G = 1 takes no post or wait: the block is copied into the local tables and the rounds run exactly as the single-GPU path.
 // Field sums are exact, so summing per rank first does not change any value.
-#include <cstdlib>
-
 #include "pcs_shard.h"
 #include "reduce.cuh"
 
@@ -100,12 +98,10 @@ __global__ void __launch_bounds__(256) wsc_post_kernel(const fe* __restrict__ pa
 
 }  // namespace
 
-struct ml_wsumcheck_shard {
-    int world = 1, L = 0;
+struct ml_wsumcheck_shard : PeerHandle {
+    int L = 0;
     size_t n_vars = 0, h = 0, nloc = 0, width = 0, n_terms = 0, n_cols = 0;
     WLayout lay;
-    std::vector<PeerRank> local;
-    PeerGroup grp;
 };
 
 namespace {
@@ -235,56 +231,19 @@ int ml_wsumcheck_shard_create(int world, int n_local, const int* local_ranks, co
     }
     DeviceGuard guard;
     ml_wsumcheck_shard* sh = new ml_wsumcheck_shard();
-    sh->world = world; sh->L = L; sh->n_vars = n_vars; sh->h = (size_t)1 << n_vars; sh->nloc = sh->h / world; sh->width = width;
+    sh->who = WHO;
+    sh->L = L; sh->n_vars = n_vars; sh->h = (size_t)1 << n_vars; sh->nloc = sh->h / world; sh->width = width;
     sh->lay = make_layout(sh->h, width, world);
-    sh->grp.world = world;
-    sh->grp.arena_bytes = sh->lay.total;
-    sh->grp.off_flags = sh->lay.flags;
-    sh->grp.off_status = sh->lay.status;
-    if (const char* e = getenv("MLB_SHARD_TIMEOUT_S")) sh->grp.timeout_ns = (unsigned long long)(atof(e) * 1e9);
-    int st = ML_OK;
-    for (int i = 0; i < n_local && st == ML_OK; i++) {
-        PeerRank r;
-        r.rank = local_ranks[i];
-        r.device = local_devices[i];
-        st = peer_rank_init(sh->grp, r, "ml_wsumcheck_shard_create", sh->lay.hdr);
-        if (st == ML_OK || st == ML_ERR_ALLOC) sh->local.push_back(r);
-    }
-    if (st == ML_OK && n_local == world) {
-        std::vector<PeerRank*> ranks;
-        for (auto& r : sh->local) ranks.push_back(&r);
-        st = peer_link_local(sh->grp, ranks, "ml_wsumcheck_shard_create");
-    }
-    if (st != ML_OK) { ml_wsumcheck_shard_free(sh); return st; }
+    int st = sh->init(world, n_local, local_ranks, local_devices, sh->lay.total, sh->lay.flags, sh->lay.status, sh->lay.hdr);
+    if (st != ML_OK) { delete sh; return st; }
     *out = sh;
     return ML_OK;
 }
 
-void ml_wsumcheck_shard_free(ml_wsumcheck_shard* sh) {
-    if (!sh) return;
-    DeviceGuard guard;
-    for (auto& r : sh->local) {
-        cudaSetDevice(r.device);
-        cudaDeviceSynchronize();
-        peer_rank_free(r);
-    }
-    peer_group_release(sh->grp, sh->local.empty() ? guard.prev : sh->local[0].device);
-    delete sh;
-}
-
-int ml_wsumcheck_shard_export(ml_wsumcheck_shard* sh, uint8_t* records_out) {
-    std::vector<PeerRank*> ranks;
-    for (auto& r : sh->local) ranks.push_back(&r);
-    return peer_export(ranks, records_out);
-}
-int ml_wsumcheck_shard_connect(ml_wsumcheck_shard* sh, const uint8_t* records, size_t n_records) {
-    if (sh->local.size() != 1) { set_error("ml_wsumcheck_shard_connect: only for handles that host one rank"); return ML_ERR_ARG; }
-    return peer_connect(sh->grp, sh->local[0], records, n_records, "ml_wsumcheck_shard_connect");
-}
-void* ml_wsumcheck_shard_stream(const ml_wsumcheck_shard* sh, int local_index) {
-    if (local_index < 0 || (size_t)local_index >= sh->local.size()) return nullptr;
-    return (void*)sh->local[local_index].st.main;
-}
+void ml_wsumcheck_shard_free(ml_wsumcheck_shard* sh) { delete sh; }
+int ml_wsumcheck_shard_export(ml_wsumcheck_shard* sh, uint8_t* records_out) { return sh->export_records(records_out); }
+int ml_wsumcheck_shard_connect(ml_wsumcheck_shard* sh, const uint8_t* records, size_t n_records) { return sh->connect(records, n_records); }
+void* ml_wsumcheck_shard_stream(const ml_wsumcheck_shard* sh, int local_index) { return sh->stream(local_index); }
 size_t ml_wsumcheck_shard_arena_bytes(const ml_wsumcheck_shard* sh) { return sh->lay.total; }
 
 int ml_wsumcheck_shard_set_composition(ml_wsumcheck_shard* sh, size_t n_terms, const uint8_t* coefs, const uint32_t* term_lens, const uint32_t* term_cols) {
@@ -316,7 +275,7 @@ int ml_wsumcheck_shard_compute_polynomials_dev(ml_wsumcheck_shard* sh, const uin
         set_error("%s: composition_degree %zu, at most %d", WHO, composition_degree, W_MAX_TD - 1);
         return ML_ERR_ARG;
     }
-    MLB_TRY(peer_check_ready(sh->grp, WHO));
+    MLB_TRY(sh->check_ready());
     if (n_vars != sh->n_vars) { set_error("%s: the row point has %zu variables, the handle %zu", WHO, n_vars, sh->n_vars); return ML_ERR_SIZE; }
     DeviceGuard guard;
     const int td = (int)composition_degree + 1, v = (int)n_vars;
@@ -370,28 +329,13 @@ int ml_wsumcheck_shard_compute_polynomials_dev(ml_wsumcheck_shard* sh, const uin
 int ml_wsumcheck_shard_compute_polynomials(ml_wsumcheck_shard* sh, const uint8_t* row_point, size_t n_vars, const uint8_t* matrix, size_t width,
                                            size_t height, size_t composition_degree, ml_transcript* t, const uint8_t sum[16], uint8_t* coeffs_out,
                                            uint8_t* randoms_out) {
-    if ((int)sh->local.size() != sh->world) { set_error("ml_wsumcheck_shard_compute_polynomials: host-pointer entry needs a handle that hosts every rank"); return ML_ERR_ARG; }
     if (width != sh->width) { set_error("ml_wsumcheck_shard_compute_polynomials: trace width %zu, the handle's %zu", width, sh->width); return ML_ERR_ARG; }
     if (n_vars != sh->n_vars || height != sh->h) { set_error("ml_wsumcheck_shard_compute_polynomials: need 2^n_vars == height == the handle's"); return ML_ERR_SIZE; }
-    DeviceGuard guard;
     const size_t bytes = sh->nloc * width * 16;
-    std::vector<void*> dev(sh->local.size(), nullptr);
-    int st = ML_OK;
-    for (size_t i = 0; i < sh->local.size() && st == ML_OK; i++) {
-        PeerRank& r = sh->local[i];
-        if (cudaSetDevice(r.device) != cudaSuccess) { st = ML_ERR_CUDA; break; }
-        st = pmalloc(&dev[i], bytes, r.st.main);
-        if (st == ML_OK) st = h2d(dev[i], matrix + (size_t)r.rank * bytes, bytes, r.st.main);
-        if (st == ML_OK && cudaStreamSynchronize(r.st.main) != cudaSuccess) st = ML_ERR_CUDA;
-    }
-    if (st == ML_OK)
-        st = ml_wsumcheck_shard_compute_polynomials_dev(sh, row_point, n_vars, dev.data(), composition_degree, t, sum, coeffs_out, randoms_out);
-    for (size_t i = 0; i < sh->local.size(); i++) {
-        cudaSetDevice(sh->local[i].device);
-        cudaStreamSynchronize(sh->local[i].st.main);
-        pfree(dev[i], sh->local[i].st.main);
-    }
-    return st;
+    return sh->host_call("ml_wsumcheck_shard_compute_polynomials", 1, bytes, [&](int rank, size_t) { return matrix + (size_t)rank * bytes; },
+                         [&](const void* const* dev) {
+                             return ml_wsumcheck_shard_compute_polynomials_dev(sh, row_point, n_vars, dev, composition_degree, t, sum, coeffs_out, randoms_out);
+                         });
 }
 
 }  // extern "C"

@@ -18,39 +18,15 @@ import ctypes as C
 import json
 import os
 import statistics
-import subprocess
-import sys
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import torch
+from shard_harness import gpu_info, timed
 
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
 
 L_ = load()
 PHASES = ["S0_transpose_encode_exchange", "S1_combine_batch_tree", "S2_batch_root", "sharded_rounds", "tail_chain", "openings_proof"]
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=60).stdout
-        return [l.strip() for l in out.splitlines() if l.strip()]
-    except Exception as e:  # noqa: BLE001
-        return ["nvidia-smi unavailable: %s" % e]
-
-
-def timed(streams, fn):
-    """fn() under CUDA events on every (device, stream); returns (result, max ms over the streams)"""
-    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in streams]
-    for (d, s), (a, _) in zip(streams, ev):
-        a.record(s)
-    out = fn()
-    for (d, s), (_, b) in zip(streams, ev):
-        b.record(s)
-    for d, _ in streams:
-        torch.cuda.synchronize(d)
-    return out, max(a.elapsed_time(b) for a, b in ev)
 
 
 def med(xs):

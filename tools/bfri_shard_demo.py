@@ -12,9 +12,7 @@ import json
 import os
 import sys
 
-sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
-import torch
-import torch.distributed as dist
+from shard_harness import Ranks
 
 from multilinear_b200 import api as ml
 
@@ -23,29 +21,11 @@ B = int(sys.argv[2]) if len(sys.argv) > 2 else 4
 check = sys.argv[3] if len(sys.argv) > 3 else "gpu"
 reps = int(sys.argv[4]) if len(sys.argv) > 4 else 3
 n = 1 << log_n
-world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
-torch.cuda.set_device(local)
-ml.set_device(local)
-dev = torch.device("cuda", local)
-if world > 1:
-    dist.init_process_group("nccl", device_id=dev)
-
-
-def barrier():
-    torch.cuda.synchronize()
-    if world > 1:
-        dist.barrier()
-
-
-sh = ml.ShardedBatchedFriProver.one_rank(rank, world, local, B, log_n)
-if world > 1:
-    sh.connect_over(dist, dev)
-else:
-    sh.connect(sh.export())
+ranks = Ranks()
+world, rank = ranks.world, ranks.rank
+sh = ranks.connect(ml.ShardedBatchedFriProver.one_rank(rank, world, ranks.local, B, log_n))
 coeffs = [ml.synthetic_elements_dev(0xBF0 + j, n) for j in range(B)]
 blocks = [c.ptr.value + rank * (n // world) * 16 for c in coeffs]
-torch.cuda.synchronize()
-stream = torch.cuda.ExternalStream(sh.stream(0), device=dev)
 state = {}
 
 
@@ -56,28 +36,9 @@ def prove():
     return p
 
 
-barrier()
-prove()  # warm-up
-barrier()
-e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-e0.record(stream)
-for _ in range(reps):
-    proof = prove()
-e1.record(stream)
-barrier()
-ms = e0.elapsed_time(e1) / reps
+ms, proof = ranks.timed(sh, prove, reps)
 phases = sh.phase_ms()
-tr = torch.tensor(list(state["t"]), dtype=torch.uint8, device=dev)
-agree = True
-if world > 1:
-    t = torch.tensor([ms], device=dev, dtype=torch.float64)
-    dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    ms = float(t[0])
-    tr0 = tr.clone()
-    dist.broadcast(tr0, 0)
-    flag = torch.tensor([int(torch.equal(tr, tr0))], device=dev)
-    dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-    agree = bool(int(flag[0]))
+agree = ranks.agree(state["t"])
 
 if rank == 0:
     blob = proof.serialize()
@@ -104,8 +65,4 @@ if rank == 0:
         del single
     print(json.dumps(line), flush=True)
 del proof
-barrier()
-sh.free()
-if world > 1:
-    dist.barrier()
-    dist.destroy_process_group()
+ranks.close(sh)

@@ -15,11 +15,9 @@ import ctypes as C
 import json
 import os
 import statistics
-import subprocess
-import sys
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import torch
+from shard_harness import gpu_info, pool_stats
 
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
@@ -27,22 +25,6 @@ from multilinear_b200 import load
 L_ = load()
 PHASES = ["S0_transpose_encode_exchange", "S1_combine", "sharded_rounds", "tail_chain", "openings_proof"]
 SINGLE_MAX_LOG_N = 27
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=60).stdout
-        return [l.strip() for l in out.splitlines() if l.strip()]
-    except Exception as e:  # noqa: BLE001
-        return ["nvidia-smi unavailable: %s" % e]
-
-
-def pool_reserved(dev):
-    ml.set_device(dev)
-    r, u = C.c_uint64(), C.c_uint64()
-    ml.check(L_.ml_pool_stats(C.byref(r), C.byref(u)))
-    return r.value
 
 
 def run(G, log_n, reps):
@@ -105,7 +87,7 @@ def run(G, log_n, reps):
         row["proof_equals_single_gpu_every_call"] = all(same)
     row["rank0_phase_ms_median"] = {k: statistics.median(ph[i] for ph in phases) for i, k in enumerate(PHASES) if all(len(ph) > i for ph in phases)}
     row["arena_bytes_per_rank"] = sh.arena_bytes()
-    row["pool_reserved_bytes_per_rank"] = [pool_reserved(d) for d in range(G)]
+    row["pool_reserved_bytes_per_rank"] = [pool_stats(d)[0] for d in range(G)]
     row["coefficient_bytes_per_gpu"] = 16 * n
     sh.free()
     for b in coeffs:

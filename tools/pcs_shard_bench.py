@@ -15,34 +15,16 @@ import ctypes as C
 import json
 import os
 import statistics
-import subprocess
-import sys
 import time
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import torch
+from shard_harness import gpu_info, pool_stats
 
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
 
 L_ = load()
 M = (1 << 128) - 45 * (1 << 40) + 1  # the field modulus
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=60).stdout
-        return [l.strip() for l in out.splitlines() if l.strip()]
-    except Exception as e:  # noqa: BLE001
-        return ["nvidia-smi unavailable: %s" % e]
-
-
-def pool_stats(dev):
-    ml.set_device(dev)
-    r, u = C.c_uint64(), C.c_uint64()
-    ml.check(L_.ml_pool_stats(C.byref(r), C.byref(u)))
-    return r.value, u.value
 
 
 def synthetic_on(dev, seed, n):

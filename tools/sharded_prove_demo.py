@@ -11,10 +11,10 @@ import json
 import os
 import sys
 
-sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
 import numpy as np
 import torch
 import torch.distributed as dist
+from shard_harness import Ranks
 
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
@@ -24,12 +24,8 @@ B = int(sys.argv[2]) if len(sys.argv) > 2 else 8
 check = sys.argv[3] if len(sys.argv) > 3 else "gpu"
 reps = int(sys.argv[4]) if len(sys.argv) > 4 else 3
 n = 1 << nv
-world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
-torch.cuda.set_device(local)
-ml.set_device(local)
-dev = torch.device("cuda", local)
-if world > 1:
-    dist.init_process_group("nccl", device_id=dev)
+ranks = Ranks()
+world, rank, dev = ranks.world, ranks.rank, ranks.dev
 L = load()
 
 
@@ -39,17 +35,7 @@ def poly(j):
     return t
 
 
-def barrier():
-    torch.cuda.synchronize()
-    if world > 1:
-        dist.barrier()
-
-
-sh = ml.ShardedBatchedProver.one_rank(rank, world, local, B, nv)
-if world > 1:
-    sh.connect_over(dist, dev)
-else:
-    sh.connect(sh.export())
+sh = ranks.connect(ml.ShardedBatchedProver.one_rank(rank, world, ranks.local, B, nv))
 mine = [poly(j) for j in sh.local_polys()]
 ptrs = [t.data_ptr() for t in mine]
 torch.cuda.synchronize()
@@ -68,28 +54,7 @@ if world > 1:
 else:
     outputs = outs_local
 
-stream = torch.cuda.ExternalStream(sh.stream(0), device=dev)
-
-
-def timed(fn):
-    barrier()
-    fn()  # warm-up: tables, pools
-    barrier()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(stream)
-    for _ in range(reps):
-        out = fn()
-    e1.record(stream)
-    barrier()
-    ms = e0.elapsed_time(e1) / reps
-    if world > 1:
-        t = torch.tensor([ms], device=dev, dtype=torch.float64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        ms = float(t[0])
-    return ms, out
-
-
-commit_ms, root = timed(lambda: sh.batch_commit_dev(ptrs))
+commit_ms, root = ranks.timed(sh, lambda: sh.batch_commit_dev(ptrs), reps)
 commit_phases = sh.phase_ms()
 state = {}
 
@@ -101,19 +66,9 @@ def prove():
     return p
 
 
-prove_ms, proof = timed(prove)
+prove_ms, proof = ranks.timed(sh, prove, reps)
 prove_phases = sh.phase_ms()
-# every rank's transcript must end in rank 0's final state
-tr = torch.tensor(list(state["t"]), dtype=torch.uint8, device=dev)
-if world > 1:
-    tr0 = tr.clone()
-    dist.broadcast(tr0, 0)
-    transcripts_agree = bool(torch.equal(tr, tr0))
-    flag = torch.tensor([int(transcripts_agree)], device=dev)
-    dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-    transcripts_agree = bool(int(flag[0]))
-else:
-    transcripts_agree = True
+transcripts_agree = ranks.agree(state["t"])  # every rank's transcript must end in rank 0's final state
 
 fixture = None
 try:
@@ -153,8 +108,4 @@ if rank == 0:
         del single, allp
     print(json.dumps(line), flush=True)
 del proof
-barrier()
-sh.free()
-if world > 1:
-    dist.barrier()
-    dist.destroy_process_group()
+ranks.close(sh)

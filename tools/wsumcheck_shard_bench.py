@@ -15,43 +15,16 @@ import ctypes as C
 import json
 import os
 import statistics
-import subprocess
 import sys
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import torch
+from shard_harness import gpu_info, timed
 
 from multilinear_b200 import api as ml
 from multilinear_b200 import load
 from oracle.pyref import M
 
 L_ = load()
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=60).stdout
-        return [l.strip() for l in out.splitlines() if l.strip()]
-    except Exception as e:  # noqa: BLE001
-        return ["nvidia-smi unavailable: %s" % e]
-
-
-def timed(streams, fn):
-    """fn() under CUDA events on every (device, stream); returns (result, max ms over the streams)"""
-    evs = []
-    for dev, s in streams:
-        with torch.cuda.device(dev):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(s)
-            evs.append((dev, s, e0, e1))
-    out = fn()
-    for dev, s, e0, e1 in evs:
-        with torch.cuda.device(dev):
-            e1.record(s)
-    for dev, _, _, _ in evs:
-        torch.cuda.synchronize(dev)
-    return out, max(e0.elapsed_time(e1) for _, _, e0, e1 in evs)
 
 
 def composition(width, degree):
