@@ -20,6 +20,7 @@
  *     results in HBM.  There is no CPU fallback: without a usable CUDA device every compute entry
  *     point fails with ML_ERR_CUDA.
  *   - Handles are opaque, own device memory, are not thread-safe, and are released with their *_free.
+ *   - Aliasing: a `_dev` entry with separate element input and output buffers says next to it whether in == out is allowed.
  */
 #ifndef MULTILINEAR_B200_H
 #define MULTILINEAR_B200_H
@@ -74,6 +75,9 @@ int ml_stream_create(void **out);
 int ml_stream_destroy(void *stream);
 int ml_stream_synchronize(void *stream);
 int ml_set_thread_stream(void *stream, int enable);
+/* A handle made by a `_dev` entry (ml_fri_*, ml_merkle_*, ml_sumcheck_*, ml_wsumcheck_*) records that entry's stream and frees its
+ * device memory on it: free the handle before destroying its stream.  The handle's methods run on the library stream
+ * (ml_wsumcheck_* on the recorded one) and return once their results are complete. */
 
 /* Device memory the library caches.  Scratch and handle-owned buffers are stream-ordered allocations: streams made by
  * ml_stream_create get a private cudaMemPool (destroyed by ml_stream_destroy); any other stream (caller-owned, e.g. a
@@ -120,20 +124,21 @@ int ml_pow2_generator_powers_dev(uint64_t log_size, void *out_dev, void *stream)
 int ml_bit_reverse_permutation(uint8_t *values, size_t n, size_t elem_bytes); /* bit_reverse_permutation :113-123 */
 int ml_ntt(const uint8_t *coeffs, size_t n, const uint8_t gen[16], uint8_t *evals);   /* Polynomial::ntt :69-110 */
 int ml_intt(const uint8_t *evals, size_t n, const uint8_t gen[16], uint8_t *coeffs);  /* LagrangePolynomial::intt :132-173 */
-int ml_ntt_dev(const void *coeffs_dev, size_t n, const uint8_t gen[16], void *evals_dev, void *stream);
-int ml_intt_dev(const void *evals_dev, size_t n, const uint8_t gen[16], void *coeffs_dev, void *stream);
+int ml_ntt_dev(const void *coeffs_dev, size_t n, const uint8_t gen[16], void *evals_dev, void *stream);   /* in place allowed */
+int ml_intt_dev(const void *evals_dev, size_t n, const uint8_t gen[16], void *coeffs_dev, void *stream);   /* in place allowed */
 int ml_poly_evaluate(const uint8_t *coeffs, size_t n, const uint8_t x[16], uint8_t out[16]); /* Polynomial::evaluate :62-67 */
 /* univariate helpers of src/polynomials.rs on the domain 0..n-1 (the sumcheck round polynomials, n <= 4 in the crate) */
 int ml_poly_interpolate(const uint8_t *evals, size_t n, uint8_t *coeffs_out);          /* PolynomialEvals::interpolate :51-86 (host scalars, n <= 2^14) */
 int ml_poly_evaluate_over_domain(const uint8_t *coeffs, size_t n, uint8_t *evals_out);  /* Polynomial::evaluate_over_domain :16-28 */
 int ml_reed_solomon(const uint8_t *coeffs, size_t n, const uint8_t gen[16], uint8_t *code /* 2n */); /* src/fri/mod.rs:19-28 */
+/* in place allowed: code_dev == coeffs_dev, a buffer of 2n elements whose first n are the coefficients */
 int ml_reed_solomon_dev(const void *coeffs_dev, size_t n, const uint8_t gen[16], void *code_dev, void *stream);
 
 /* ---- multilinear polynomials (src/polynomials.rs) ---- */
 int ml_mle_to_coefficient(const uint8_t *evals, size_t len, uint8_t *coeffs);   /* MultilinearPolynomialEvals::to_coefficient :150-163 */
 int ml_mle_to_evaluation(const uint8_t *coeffs, size_t len, uint8_t *evals);    /* MultilinearPolynomial::to_evaluation :111-124 */
-int ml_mle_to_coefficient_dev(const void *evals_dev, size_t len, void *coeffs_dev, void *stream);
-int ml_mle_to_evaluation_dev(const void *coeffs_dev, size_t len, void *evals_dev, void *stream);
+int ml_mle_to_coefficient_dev(const void *evals_dev, size_t len, void *coeffs_dev, void *stream);   /* in place allowed */
+int ml_mle_to_evaluation_dev(const void *coeffs_dev, size_t len, void *evals_dev, void *stream);    /* in place allowed */
 int ml_mle_evals_evaluate(const uint8_t *evals, size_t len, const uint8_t *args, size_t n_args, uint8_t out[16]);   /* :165-187 */
 int ml_mle_coeffs_evaluate(const uint8_t *coeffs, size_t len, const uint8_t *args, size_t n_args, uint8_t out[16]); /* :126-146 */
 int ml_mle_evals_evaluate_dev(const void *evals_dev, size_t len, const uint8_t *args, size_t n_args, uint8_t out[16], void *stream);
@@ -151,7 +156,9 @@ int ml_transcript_next_challenge(ml_transcript *t, uint8_t out[16]);            
 typedef struct ml_merkle ml_merkle;
 int ml_merkle_commit(const uint8_t *data, size_t item_bytes, size_t n_items, ml_merkle **out);  /* Merkle::commit :65-85 */
 int ml_merkle_batch_commit(const uint8_t *const *data, size_t n_batches, size_t item_bytes, size_t n_items, ml_merkle **out); /* batch_commit :92-131 */
-/* leaves are ReedSolomonPairs (code[i], code[i + n/2]) of a device-resident code — commit_rs_code, src/fri/mod.rs:45-55 */
+/* leaves are ReedSolomonPairs (code[i], code[i + n/2]) of a device-resident code — commit_rs_code, src/fri/mod.rs:45-55.
+ * The tree keeps code_dev (ml_merkle_open reads the values from it): the code must stay allocated and unchanged until
+ * ml_merkle_free. */
 int ml_merkle_commit_rs_code_dev(const void *code_dev, size_t n, void *stream, ml_merkle **out);
 void ml_merkle_free(ml_merkle *m);
 int ml_merkle_root(const ml_merkle *m, uint8_t out[32]);                        /* root :27-29 */
@@ -486,17 +493,21 @@ int ml_wsumcheck_shard_compute_polynomials(ml_wsumcheck_shard *sh, const uint8_t
  * Writes the subtree root of the range (leaf_count a power of two); ranks then all-gather the roots
  * and call ml_merkle_top_from_roots. */
 int ml_batched_leaf_subtree_dev(const void *const *pairs_dev, size_t n_codes, size_t leaf_count, void *stream, uint8_t root_out[32]);
-/* pairs (code[i], code[i+n/2]) of one local code written in exchange order [dest rank][local poly][row][32 B] */
+/* pairs (code[i], code[i+n/2]) of one local code written in exchange order [dest rank][local poly][row][32 B]; an out_dev
+ * buffer (n_local_polys * n_code * 16 bytes) that overlaps the code is ML_ERR_ARG */
 int ml_pack_pairs_dev(const void *code_dev, size_t n_code, size_t n_ranks, size_t n_local_polys, size_t local_index, void *out_dev, void *stream);
-/* to_coefficient + bit_reverse + reed_solomon of one polynomial given by evaluations (batched_pcs.rs:144-149); code_dev holds 2n elements */
+/* to_coefficient + bit_reverse + reed_solomon of one polynomial given by evaluations (batched_pcs.rs:144-149); code_dev holds 2n elements.
+ * In place allowed: code_dev == evals_dev, a buffer of 2n elements whose first n are the evaluations. */
 int ml_pcs_encode_dev(const void *evals_dev, size_t n, void *code_dev, void *stream);
 int ml_merkle_top_from_roots(const uint8_t *roots, size_t n_roots, uint8_t root_out[32]);
-/* the subtree root left in device memory (32 bytes at root_dev) for the all-gather, no host round trip */
+/* the subtree root left in device memory (32 bytes at root_dev) for the all-gather, no host round trip; root_dev may lie inside
+ * the pairs (it is written after the subtree is complete) */
 int ml_batched_leaf_subtree_root_dev(const void *const *pairs_dev, size_t n_codes, size_t leaf_count, void *root_dev, void *stream);
 /* Exchange fused into the pack pass: pairs of one code stored straight into the leaf-range owners' receive buffers
  * through NVLink peer mappings (no send buffer, no collective).  peer_bases[g] is rank g's receive buffer
  * ([global polynomial][row][32 B], rows = n_code/2/n_ranks) as mapped into this process (own buffer for g == rank);
- * max_ctas bounds the grid so the store pass shares the GPU with the next polynomial's NTT (0 = default). */
+ * max_ctas bounds the grid so the store pass shares the GPU with the next polynomial's NTT (0 = default).  A destination slice
+ * (rows pairs of global_poly) that overlaps the code is ML_ERR_ARG. */
 int ml_pack_pairs_peer_dev(const void *code_dev, size_t n_code, size_t n_ranks, size_t global_poly, void *const *peer_bases, unsigned max_ctas, void *stream);
 /* peer-visible device buffers (CUDA IPC): owner allocates + publishes the 64-byte handle; peers map / unmap it */
 int ml_ipc_alloc(size_t bytes, void **dev_out, uint8_t handle_out[64]);

@@ -2022,6 +2022,9 @@ int ml_pack_pairs_dev(const void* code_dev, size_t n_code, size_t n_ranks, size_
     (void)ctx;
     const size_t half = n_code / 2;
     if (!is_pow2(n_code) || n_ranks == 0 || half % n_ranks != 0 || local_index >= n_local_polys) { set_error("ml_pack_pairs_dev: bad partition"); return ML_ERR_SIZE; }
+    // threads read pairs other threads' stores may already have overwritten: the output must not overlap the code
+    const uintptr_t c0 = (uintptr_t)code_dev, c1 = c0 + n_code * 16, o0 = (uintptr_t)out_dev, o1 = o0 + n_code * 16 * n_local_polys;
+    if (o0 < c1 && c0 < o1) { set_error("ml_pack_pairs_dev: the output buffer overlaps the code"); return ML_ERR_ARG; }
     size_t blocks = (half + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     pack_pairs_kernel<<<(unsigned)blocks, 256, 0, ST(stream)>>>((const fe*)code_dev, half, half / n_ranks, n_local_polys, local_index, (uint4*)out_dev);
@@ -2068,8 +2071,14 @@ int ml_pack_pairs_peer_dev(const void* code_dev, size_t n_code, size_t n_ranks, 
     (void)ctx;
     const size_t half = n_code / 2;
     if (!is_pow2(n_code) || n_ranks == 0 || n_ranks > ML_MAX_PEERS || half % n_ranks != 0) { set_error("ml_pack_pairs_peer_dev: bad partition"); return ML_ERR_SIZE; }
+    const size_t slice = half / n_ranks * 32;
+    const uintptr_t c0 = (uintptr_t)code_dev, c1 = c0 + n_code * 16;
     PeerBases pb;
-    for (size_t g = 0; g < ML_MAX_PEERS; g++) pb.base[g] = g < n_ranks ? (uint4*)peer_bases[g] : nullptr;
+    for (size_t g = 0; g < ML_MAX_PEERS; g++) {
+        pb.base[g] = g < n_ranks ? (uint4*)peer_bases[g] : nullptr;
+        const uintptr_t o0 = (uintptr_t)pb.base[g] + global_poly * slice;
+        if (g < n_ranks && o0 < c1 && c0 < o0 + slice) { set_error("ml_pack_pairs_peer_dev: a destination overlaps the code"); return ML_ERR_ARG; }
+    }
     size_t blocks = (half + 255) / 256;
     const size_t cap = max_ctas ? max_ctas : 148 * 8;
     if (blocks > cap) blocks = cap;
