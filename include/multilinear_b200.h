@@ -242,6 +242,50 @@ const ml_fri_proof *ml_pcs_proof_fri(const ml_pcs_proof *p);
 size_t ml_pcs_proof_num_rounds(const ml_pcs_proof *p);
 int ml_pcs_proof_sumcheck_coeffs(const ml_pcs_proof *p, uint8_t *out /* rounds*2*16 */);    /* SumcheckPolynomial.nonzero_coeffs */
 
+/* ---- stream-ordered provers: FriProof::prove / PCSProof::prove enqueued on a caller's stream ----
+ * The transcript state as bytes: the 104-byte running SHA-256 state (eight state words, the 64-byte block buffer, the u64 byte
+ * count), laid out identically on the host and on the device.  A state exported here can be copied into device memory and handed
+ * to the calls below, and a state they leave in device memory can be copied back and imported. */
+size_t ml_transcript_state_bytes(void);                                   /* 104 */
+int ml_transcript_export(const ml_transcript *t, uint8_t *state_out);
+int ml_transcript_import(const uint8_t *state, ml_transcript **out);
+/* A plan owns every device buffer one prove of a 2^log_domain code needs (N = 2^log_domain): the code and Merkle tree of every
+ * FRI layer (N, N/2, ... 4), the fold chain's scratch and the query phase's buffers, plus the sumcheck tables with pcs != 0.  It
+ * is allocated once at creation on the current device with cudaMalloc, not from the stream pools, so ml_trim_pools never touches
+ * it; creation also builds the root and NTT pass tables of the size.  ml_prove_plan_device_bytes is what it holds (about 96 N
+ * bytes, 112 N with pcs).  ml_prove_plan_create: ML_ERR_SIZE for log_domain outside 2..40, ML_ERR_ALLOC when the plan does not
+ * fit (nothing is left allocated), ML_ERR_CUDA without a device.  ml_prove_plan_free synchronises the plan's device.
+ *
+ * Each call computes what its blocking twin computes and leaves it in device memory, in stream order on `stream`:
+ *   ml_rs_fri_prove_async = ml_rs_fri_prove_dev (coeffs_dev: N/2 coefficients),
+ *   ml_fri_prove_async    = ml_fri_prove_dev    (code_dev: N elements),
+ *   ml_pcs_prove_async    = ml_pcs_prove_dev    (inputs_dev: n_vars = log_domain - 1 points, output_dev: the claim, 1 element,
+ *                                                evals_dev: N/2 evaluations); needs a plan made with pcs != 0.
+ *   proof_dev (ml_prove_plan_proof_bytes bytes) receives the FriProof bincode blob, byte-identical to ml_fri_proof_serialize of
+ *   the blocking twin's proof (for the PCS call: of ml_pcs_proof_fri); sumcheck_dev (2 * n_vars elements) receives
+ *   ml_pcs_proof_sumcheck_coeffs; transcript_dev holds ml_transcript_state_bytes() of state on entry and is updated in place to
+ *   the state the host transcript has after the blocking call; *status_dev receives ML_OK, or ML_ERR_NOT_RS_CODE when the code's
+ *   last fold is not constant (the proof and transcript contents are then unspecified; the plan proves normally next time).
+ * Inputs are only read.
+ * Host-side rejections enqueue nothing and return: ML_ERR_ARG for a NULL plan or buffer, a device buffer that is not 16-byte
+ * aligned, an output range (transcript, proof, sumcheck, status) overlapping any other buffer of the call, a PCS call on a plan
+ * made with pcs = 0, or a current device other than the plan's.
+ * No host work during an enqueue call: it makes no device allocation, no synchronisation, no host->device copy from host memory
+ * and no host read of device data, so it returns once its kernels are enqueued and may be captured into a CUDA graph with
+ * cudaStreamCaptureModeGlobal.  (A kernel launch error is returned as ML_ERR_CUDA; work enqueued before it stays enqueued.)
+ * One proof in flight per plan: calls on one plan must be ordered by the caller (calls on one stream are); for overlap use one
+ * plan per stream.  A captured graph keeps the pointers it was captured with, so each replay proves what those buffers hold at
+ * replay time. */
+typedef struct ml_prove_plan ml_prove_plan;
+int ml_prove_plan_create(size_t log_domain, int pcs, ml_prove_plan **out);
+void ml_prove_plan_free(ml_prove_plan *p);
+size_t ml_prove_plan_device_bytes(const ml_prove_plan *p);
+size_t ml_prove_plan_proof_bytes(const ml_prove_plan *p);   /* == ml_fri_proof_serialized_len of the proof it writes */
+int ml_rs_fri_prove_async(ml_prove_plan *p, const void *coeffs_dev, void *transcript_dev, void *proof_dev, int *status_dev, void *stream);
+int ml_fri_prove_async(ml_prove_plan *p, const void *code_dev, void *transcript_dev, void *proof_dev, int *status_dev, void *stream);
+int ml_pcs_prove_async(ml_prove_plan *p, const void *inputs_dev, const void *output_dev, const void *evals_dev, void *transcript_dev,
+                       void *proof_dev, void *sumcheck_dev, int *status_dev, void *stream);
+
 /* ---- batched FRI / PCS (src/fri/batched_fri.rs, src/fri/batched_pcs.rs) ---- */
 typedef struct ml_bfri_proof ml_bfri_proof; /* BatchedFriProof batched_fri.rs:21-27 */
 int ml_fingerprint(const uint8_t r[16], const uint8_t *coeffs, size_t n, uint8_t out[16]);  /* fingerprint batched_fri.rs:30-38 (host, tiny) */

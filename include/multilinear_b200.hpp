@@ -138,8 +138,21 @@ class Transcript {
         return out;
     }
     ml_transcript* handle() { return h_; }
+    // the running state (ml_transcript_state_bytes() bytes), as the stream-ordered provers take it in device memory
+    std::vector<uint8_t> export_state() const {
+        std::vector<uint8_t> out(ml_transcript_state_bytes());
+        check(ml_transcript_export(h_, out.data()));
+        return out;
+    }
+    static Transcript import_state(const std::vector<uint8_t>& state) {
+        if (state.size() != ml_transcript_state_bytes()) throw Panic(ML_ERR_SIZE, "transcript state of the wrong size");
+        ml_transcript* h = nullptr;
+        check(ml_transcript_import(state.data(), &h));
+        return Transcript(h);
+    }
 
   private:
+    explicit Transcript(ml_transcript* h) : h_(h) {}
     ml_transcript* h_ = nullptr;
 };
 
@@ -403,6 +416,30 @@ class ShardedFriProver {
 
   private:
     ml_fri_shard* h_ = nullptr;
+};
+// Stream-ordered FriProof / PCSProof provers of one domain size (ml_prove_plan_*, csrc/plan.cu): every buffer is caller-owned
+// device memory; a call only enqueues on `stream` and leaves the bincode blob, transcript state and status there.
+class ProvePlan {
+  public:
+    ProvePlan(size_t log_domain, bool pcs) { check(ml_prove_plan_create(log_domain, pcs ? 1 : 0, &h_)); }
+    ProvePlan(const ProvePlan&) = delete;
+    ProvePlan& operator=(const ProvePlan&) = delete;
+    ~ProvePlan() { ml_prove_plan_free(h_); }
+    size_t proof_bytes() const { return ml_prove_plan_proof_bytes(h_); }
+    size_t device_bytes() const { return ml_prove_plan_device_bytes(h_); }
+    void rs_fri_prove_async(const void* coeffs_dev, void* transcript_dev, void* proof_dev, int* status_dev, void* stream) {
+        check(ml_rs_fri_prove_async(h_, coeffs_dev, transcript_dev, proof_dev, status_dev, stream));
+    }
+    void fri_prove_async(const void* code_dev, void* transcript_dev, void* proof_dev, int* status_dev, void* stream) {
+        check(ml_fri_prove_async(h_, code_dev, transcript_dev, proof_dev, status_dev, stream));
+    }
+    void pcs_prove_async(const void* inputs_dev, const void* output_dev, const void* evals_dev, void* transcript_dev, void* proof_dev,
+                         void* sumcheck_dev, int* status_dev, void* stream) {
+        check(ml_pcs_prove_async(h_, inputs_dev, output_dev, evals_dev, transcript_dev, proof_dev, sumcheck_dev, status_dev, stream));
+    }
+
+  private:
+    ml_prove_plan* h_ = nullptr;
 };
 // src/fri/batched_fri.rs:284-398
 class BatchedFriProof {

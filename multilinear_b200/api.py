@@ -319,6 +319,22 @@ class Transcript:
         check(load().ml_transcript_next_challenge(self.h, _p(out)))
         return _int(out)
 
+    def export(self):
+        """the running state as ml_transcript_state_bytes() bytes (what the stream-ordered provers take in device memory)"""
+        out = np.empty(load().ml_transcript_state_bytes(), dtype=np.uint8)
+        check(load().ml_transcript_export(self.h, _p(out)))
+        return out.tobytes()
+
+    @staticmethod
+    def import_(state):
+        """a transcript continuing from an exported state"""
+        b = np.frombuffer(bytes(state), dtype=np.uint8).copy()
+        if b.size != load().ml_transcript_state_bytes():
+            raise SizeMismatch(2, "a transcript state has %d bytes, not %d" % (load().ml_transcript_state_bytes(), b.size))
+        h = C.c_void_p()
+        check(load().ml_transcript_import(_p(b), C.byref(h)))
+        return Transcript(h)
+
     def __del__(self):
         try:
             load().ml_transcript_free(self.h)
@@ -762,6 +778,57 @@ class PCSProof:
             (load().ml_bpcs_proof_free if self.batched else load().ml_pcs_proof_free)(self.h)
         except Exception:
             pass
+
+
+class ProvePlan:
+    """Stream-ordered FriProof / PCSProof provers of one domain size (ml_prove_plan_*): every buffer is device memory the caller
+    owns, passed as a raw pointer (int); `stream` is a cudaStream_t as an int (None: the legacy stream).  The calls only enqueue:
+    read proof_dev / transcript_dev / sumcheck_dev / status_dev after the stream has reached them."""
+
+    def __init__(self, h, log_domain, pcs):
+        self.h, self.log_domain, self.pcs = h, log_domain, pcs
+
+    @staticmethod
+    def create(log_domain, pcs=False):
+        h = C.c_void_p()
+        check(load().ml_prove_plan_create(_sz(log_domain), C.c_int(1 if pcs else 0), C.byref(h)))
+        return ProvePlan(h, log_domain, pcs)
+
+    @property
+    def proof_bytes(self):
+        return load().ml_prove_plan_proof_bytes(self.h)
+
+    @property
+    def device_bytes(self):
+        return load().ml_prove_plan_device_bytes(self.h)
+
+    def rs_fri_prove_async(self, coeffs_dev, transcript_dev, proof_dev, status_dev, stream=None):
+        """reed_solomon + FriProof::prove of N/2 coefficients (= ml_rs_fri_prove_dev)"""
+        check(load().ml_rs_fri_prove_async(self.h, _vp(coeffs_dev), _vp(transcript_dev), _vp(proof_dev), _vp(status_dev), _vp(stream)))
+
+    def fri_prove_async(self, code_dev, transcript_dev, proof_dev, status_dev, stream=None):
+        """FriProof::prove of a code of N elements (= ml_fri_prove_dev)"""
+        check(load().ml_fri_prove_async(self.h, _vp(code_dev), _vp(transcript_dev), _vp(proof_dev), _vp(status_dev), _vp(stream)))
+
+    def pcs_prove_async(self, inputs_dev, output_dev, evals_dev, transcript_dev, proof_dev, sumcheck_dev, status_dev, stream=None):
+        """PCSProof::prove of N/2 evaluations (= ml_pcs_prove_dev)"""
+        check(load().ml_pcs_prove_async(self.h, _vp(inputs_dev), _vp(output_dev), _vp(evals_dev), _vp(transcript_dev), _vp(proof_dev),
+                                        _vp(sumcheck_dev), _vp(status_dev), _vp(stream)))
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_prove_plan_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+def _vp(x):
+    return C.c_void_p(x if x is None else int(x))
 
 
 class BatchedFriProof:

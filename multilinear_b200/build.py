@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libmultilinear_b200.so")
-SOURCES = ["core.cu", "field_ops.cu", "ntt.cu", "merkle.cu", "fri.cu", "sumcheck.cu", "mle.cu", "prover.cu", "chain.cu", "peer.cu", "shard.cu", "pcs_shard.cu", "bpcs_shard.cu", "wsumcheck_shard.cu", "fri_shard.cu", "bfri_shard.cu"]
+SOURCES = ["core.cu", "field_ops.cu", "ntt.cu", "merkle.cu", "fri.cu", "sumcheck.cu", "mle.cu", "prover.cu", "chain.cu", "peer.cu", "shard.cu", "pcs_shard.cu", "bpcs_shard.cu", "wsumcheck_shard.cu", "fri_shard.cu", "bfri_shard.cu", "plan.cu"]
 # instrumentation (integer-pipe speed-of-light loops for bench.py / tools): its own library, not part of the product ABI
 INSTR_OUT = os.path.join(HERE, "libmlb_instr.so")
 INSTR_SOURCES = ["microbench.cu"]

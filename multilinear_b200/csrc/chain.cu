@@ -103,6 +103,40 @@ __global__ void __launch_bounds__(256) chain_sumcheck_finish_kernel(const fe* __
     *tr = t;
 }
 
+// FriProof::prove's query phase (src/fri/mod.rs:268-277) on one thread, from the transcript the fold chain left in HBM:
+// 128 times idx = LE u64 of the digest's first 8 bytes mod N/2 (a mask: N/2 is a power of two), then absorb idx as 8 LE bytes;
+// last_random = the digest after the last absorb.  The transcript's final state goes to tr_out.
+__global__ void fri_query_indices_kernel(const DevTranscript* tr_in, DevTranscript* tr_out, int log_half, unsigned long long* indices,
+                                         uint8_t* last_random) {
+    if (threadIdx.x != 0) return;
+    DevTranscript t = *tr_in;
+    const unsigned long long mask = (1ull << log_half) - 1ull;
+    uint32_t st[8];
+    for (int q = 0; q < ML_NUM_QUERIES; q++) {
+        dt_digest_words(&t, st);
+        // digest bytes are the big-endian state words: bytes 0..7 read as LE u64 -> bswap(st[0]) | bswap(st[1]) << 32
+        const unsigned long long idx = ((unsigned long long)sha_bswap(st[0]) | ((unsigned long long)sha_bswap(st[1]) << 32)) & mask;
+        indices[q] = idx;
+        uint8_t b[8];
+#pragma unroll
+        for (int i = 0; i < 8; i++) b[i] = (uint8_t)(idx >> (8 * i));
+        dt_absorb(&t, b, 8);
+    }
+    dt_digest_words(&t, st);
+    for (int i = 0; i < 8; i++) {
+        last_random[4 * i] = (uint8_t)(st[i] >> 24); last_random[4 * i + 1] = (uint8_t)(st[i] >> 16);
+        last_random[4 * i + 2] = (uint8_t)(st[i] >> 8); last_random[4 * i + 3] = (uint8_t)st[i];
+    }
+    *tr_out = t;
+}
+int fri_query_indices_launch(const DevTranscript* tr_in, DevTranscript* tr_out, int log_half, unsigned long long* indices, uint8_t* last_random,
+                             cudaStream_t s) {
+    ProfScope prof(PROF_TRANSCRIPT, 0.0, s);
+    fri_query_indices_kernel<<<1, 32, 0, s>>>(tr_in, tr_out, log_half, indices, last_random);
+    MLB_KERNEL_CHECK();
+    return ML_OK;
+}
+
 // ------------------------------------------------------------------ fused tail
 __global__ void __launch_bounds__(1024, 1) chain_tail_kernel(TailArgs a) {
     __shared__ DevTranscript tr;

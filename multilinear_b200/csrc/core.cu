@@ -556,5 +556,18 @@ int ml_transcript_next_challenge(ml_transcript* t, uint8_t out[16]) {
     hfe_store(out, hfe_new(hfe_load(d)));
     return ML_OK;
 }
+size_t ml_transcript_state_bytes(void) { return sizeof(HostSha256); }
+int ml_transcript_export(const ml_transcript* t, uint8_t* state_out) {
+    if (!t || !state_out) { set_error("ml_transcript_export: null pointer"); return ML_ERR_ARG; }
+    memcpy(state_out, &t->sha, sizeof(HostSha256));
+    return ML_OK;
+}
+int ml_transcript_import(const uint8_t* state, ml_transcript** out) {
+    if (!state || !out) { set_error("ml_transcript_import: null pointer"); return ML_ERR_ARG; }
+    ml_transcript* t = new ml_transcript();
+    memcpy(&t->sha, state, sizeof(HostSha256));
+    *out = t;
+    return ML_OK;
+}
 
 }  // extern "C"

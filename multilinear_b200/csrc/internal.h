@@ -146,8 +146,11 @@ int dev_free_async(void* p, cudaStream_t s);
 
 // ------------------------------------------------------------------ kernels (launchers)
 // ntt.cu
-// bitrev_in: the n live coefficients are stored bit-reversed (PCS encode); fused into pass 0, multi-pass sizes only
-int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs_zero_padded, cudaStream_t s, bool bitrev_in = false);
+// bitrev_in: the n live coefficients are stored bit-reversed (PCS encode); fused into pass 0, multi-pass sizes only.
+// tmp: 2^log_n elements of scratch for the multi-pass plans (nullptr: a stream-ordered allocation per call)
+int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs_zero_padded, cudaStream_t s, bool bitrev_in = false,
+               fe* tmp = nullptr);
+int ntt_prepare(Ctx* ctx, int log_n, cudaStream_t s);
 static inline bool ntt_fuses_bitrev(int log_n) { return log_n > 12; }
 int powers_launch(Ctx* ctx, int log_n, fe* out, cudaStream_t s);
 int bit_reverse_launch(const void* in, void* out, size_t n, size_t elem_bytes, cudaStream_t s);
@@ -161,7 +164,9 @@ int synthetic_launch(uint64_t seed, size_t n, fe* out, cudaStream_t s);
 int mobius_launch(const fe* in, fe* out, size_t len, bool subtract, cudaStream_t s);
 int mle_evals_evaluate_launch(Ctx* ctx, const fe* evals, size_t len, const hfe* args, size_t n_args, hfe* out, cudaStream_t s);
 int mle_coeffs_evaluate_launch(Ctx* ctx, const fe* coeffs, size_t len, const hfe* args, size_t n_args, hfe* out, cudaStream_t s);
-int eq_table_launch(Ctx* ctx, const hfe* inputs, size_t n_vars, fe* delta, cudaStream_t s);
+// points_dev: the n_vars points already in HBM (inputs unused, no upload); scratch: eq_weights_elems(n_vars) elements (nullptr: allocated)
+int eq_table_launch(Ctx* ctx, const hfe* inputs, size_t n_vars, fe* delta, cudaStream_t s, const fe* points_dev = nullptr, fe* scratch = nullptr);
+size_t eq_weights_elems(size_t n_vars);
 int poly_eval_launch(Ctx* ctx, const fe* coeffs, size_t n, hfe x, hfe* out, cudaStream_t s);
 // merkle.cu — digests buffer holds all layers back to back: layer l starts at digest index 2L - (2L >> l)
 static inline size_t merkle_layer_offset(size_t n_leaves, size_t layer) { return 2 * n_leaves - ((2 * n_leaves) >> layer); }
@@ -233,6 +238,9 @@ int chain_sumcheck_finish_launch(const fe* partials, int nb, fe* prev, DevTransc
 int chain_tail_launch(const TailArgs& a, cudaStream_t s);
 int chain_sumcheck_tail_launch(fe* m, fe* d, size_t height, fe* prev, DevTranscript* tr, fe* sc_out, fe* r_out, cudaStream_t s);
 int chain_last_launch(const fe* two, DevTranscript* tr, fe* last_out, int* status, cudaStream_t s);
+// the 128 query indices of a domain of 2^(log_half+1) and last_random from the transcript at tr_in; final state to tr_out
+int fri_query_indices_launch(const DevTranscript* tr_in, DevTranscript* tr_out, int log_half, unsigned long long* indices, uint8_t* last_random,
+                             cudaStream_t s);
 // width-w sumcheck rounds on the device (sumcheck.rs:174-202): lag = the (td+1) x (td+1) Lagrange coefficient matrix over x = 0..td
 static const int WTAIL_LOG = 12;  // the tail kernel runs every remaining round once the tables have <= 2^WTAIL_LOG rows
 int wchain_finish_launch(const fe* partials, int nb, int td, const fe* lag, fe* prev, DevTranscript* tr, fe* coef_out, fe* r_store, fe* r_dev,

@@ -200,17 +200,32 @@ __global__ void __launch_bounds__(256) sum_partials_kernel(const fe* __restrict_
     if (threadIdx.x == 0) fe_store(out, a);
 }
 
-// builds WH (2^(nv-lb) entries) and WL (2^lb entries) in one scratch allocation; caller frees *scratch
-static int build_weights(const hfe* points, size_t n_vars, int mode, cudaStream_t s, fe** scratch, fe** wh, fe** wl, int* lb_out) {
+// builds WH (2^(nv-lb) entries) and WL (2^lb entries); points from the host (uploaded into the scratch) or already in HBM
+// (points_dev).  The scratch is allocated (*scratch, the caller frees it) unless given in scratch_in.
+static void weight_split(size_t n_vars, int* lb, int* hb) {
+    *lb = (int)n_vars < 12 ? (int)n_vars : 12;
+    *hb = (int)n_vars - *lb;
+}
+size_t eq_weights_elems(size_t n_vars) {
+    int lb, hb;
+    weight_split(n_vars, &lb, &hb);
+    return n_vars + ((size_t)1 << lb) + ((size_t)1 << hb);
+}
+static int build_weights(const hfe* points, size_t n_vars, int mode, cudaStream_t s, fe** scratch, fe** wh, fe** wl, int* lb_out,
+                         const fe* points_dev = nullptr, fe* scratch_in = nullptr) {
     const int nv = (int)n_vars;
-    const int lb = nv < 12 ? nv : 12;
-    const int hb = nv - lb;
-    const size_t total = n_vars + ((size_t)1 << lb) + ((size_t)1 << hb);
-    MLB_TRY(dev_alloc_async((void**)scratch, total * 16, s));
-    fe* pts = *scratch;
+    int lb, hb;
+    weight_split(n_vars, &lb, &hb);
+    *scratch = nullptr;
+    fe* pts = scratch_in;
+    if (!pts) {
+        MLB_TRY(dev_alloc_async((void**)scratch, eq_weights_elems(n_vars) * 16, s));
+        pts = *scratch;
+    }
     *wl = pts + n_vars;
     *wh = *wl + ((size_t)1 << lb);
-    if (n_vars) MLB_CUDA(cudaMemcpyAsync(pts, points, n_vars * 16, cudaMemcpyHostToDevice, s));
+    if (points_dev) pts = (fe*)points_dev;
+    else if (n_vars) MLB_CUDA(cudaMemcpyAsync(pts, points, n_vars * 16, cudaMemcpyHostToDevice, s));
     weight_table_kernel<<<((1u << lb) + 255) / 256, 256, 0, s>>>(pts, nv, 0, lb, mode, *wl);
     MLB_KERNEL_CHECK();
     weight_table_kernel<<<((1u << hb) + 255) / 256, 256, 0, s>>>(pts, nv, lb, hb, mode, *wh);
@@ -254,17 +269,17 @@ int mle_coeffs_evaluate_launch(Ctx* ctx, const fe* coeffs, size_t len, const hfe
     return mle_evaluate(ctx, coeffs, len, args, n_args, 1, out, s);
 }
 // delta table of SumcheckTables::build_tables_for_pcs (sumcheck.rs:133-138)
-int eq_table_launch(Ctx* ctx, const hfe* inputs, size_t n_vars, fe* delta, cudaStream_t s) {
+int eq_table_launch(Ctx* ctx, const hfe* inputs, size_t n_vars, fe* delta, cudaStream_t s, const fe* points_dev, fe* scratch_in) {
     fe *scratch, *wh, *wl;
     int lb;
-    MLB_TRY(build_weights(inputs, n_vars, 0, s, &scratch, &wh, &wl, &lb));
+    MLB_TRY(build_weights(inputs, n_vars, 0, s, &scratch, &wh, &wl, &lb, points_dev, scratch_in));
     const size_t n = (size_t)1 << n_vars;
     size_t blocks = (n + 255) / 256;
     if (blocks > (size_t)ctx->sm_count * 16) blocks = (size_t)ctx->sm_count * 16;
     ProfScope prof(PROF_EQ_TABLE, 16.0 * (double)n, s);
     outer_product_kernel<<<(unsigned)blocks, 256, 0, s>>>(wh, wl, lb, n, delta);
     MLB_KERNEL_CHECK();
-    return dev_free_async(scratch, s);
+    return scratch ? dev_free_async(scratch, s) : ML_OK;
 }
 // Polynomial::evaluate (src/ntt/mod.rs:62-67): sum_i c_i x^i with x^i = XH[i >> 12] * XL[i & 4095]
 int poly_eval_launch(Ctx* ctx, const fe* coeffs, size_t n, hfe x, hfe* out, cudaStream_t s) {

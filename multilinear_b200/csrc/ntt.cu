@@ -330,7 +330,7 @@ int powers_launch(Ctx* ctx, int log_n, fe* out, cudaStream_t s) {
 // Natural-order NTT of size 2^log_n with the domain generator pow_2_generator(log_n) (or its inverse, with the
 // 1/N scaling of intt).  rs_zero_padded: `in` holds N/2 coefficients, the upper half of the input is zero
 // (reed_solomon's resize, src/fri/mod.rs:24).  in == out is allowed for P == 1 only when not zero padded.
-int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs_zero_padded, cudaStream_t s, bool bitrev_in) {
+int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs_zero_padded, cudaStream_t s, bool bitrev_in, fe* tmp_in) {
     if (bitrev_in && !(rs_zero_padded && !inverse && log_n > TILE_LOG)) { set_error("ntt: bit-reversed input needs a multi-pass RS encode"); return ML_ERR_ARG; }
     MLB_CUDA(cudaFuncSetAttribute(ntt_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
     const RootTables* rt;
@@ -351,8 +351,8 @@ int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs
         explicit TmpGuard(cudaStream_t st) : s(st) {}
         ~TmpGuard() { if (p) cudaFreeAsync(p, s); }
     } tmp_guard(s);
-    if (n_passes > 1) MLB_TRY(dev_alloc_async((void**)&tmp_guard.p, ((size_t)16) << log_n, s));
-    fe* const tmp = tmp_guard.p;
+    if (n_passes > 1 && !tmp_in) MLB_TRY(dev_alloc_async((void**)&tmp_guard.p, ((size_t)16) << log_n, s));
+    fe* const tmp = tmp_in ? tmp_in : tmp_guard.p;
 
     const double nbytes = 16.0 * (double)((size_t)1 << log_n);
     ProfScope prof(PROF_NTT_PASS, rs_zero_padded ? 1.5 * nbytes : 2.0 * nbytes, s);  // read input once + write output once
@@ -388,6 +388,23 @@ int ntt_launch(Ctx* ctx, const fe* in, fe* out, int log_n, bool inverse, bool rs
         ntt_pass_kernel<<<(unsigned)tiles, NTT_THREADS, smem, s>>>(a);
         MLB_KERNEL_CHECK();
         log_a += a.log_r;
+    }
+    return ML_OK;
+}
+
+// every table a forward transform of 2^log_n reads (root, small and inter-pass tables), built now so that later launches of
+// that size only read them: a prove plan calls this at creation, and its enqueue path then never synchronises or allocates
+int ntt_prepare(Ctx* ctx, int log_n, cudaStream_t s) {
+    const RootTables* rt;
+    MLB_TRY(get_root_tables(ctx, log_n, s, &rt));
+    const int n_passes = log_n <= TILE_LOG ? 1 : (log_n + 8) / 9;
+    if (n_passes > 4) { set_error("NTT size 2^%d not supported", log_n); return ML_ERR_ARG; }
+    int log_a = 0;
+    for (int p = 0; p + 1 < n_passes; p++) {
+        const int log_r = log_n / n_passes + (p < log_n % n_passes ? 1 : 0);
+        const fe* tab;
+        MLB_TRY(get_pass_table(ctx, log_n, false, p, log_a, log_r, log_n - log_a - log_r, s, &tab));
+        log_a += log_r;
     }
     return ML_OK;
 }

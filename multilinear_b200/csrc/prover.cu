@@ -155,7 +155,6 @@ int d2h_sync(void* dst, const void* src, size_t bytes, cudaStream_t s) {
     if (bytes) MLB_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s));
     return stream_wait_blocking(s);
 }
-int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree);
 void absorb_fe(ml_transcript* t, hfe x) {
     uint8_t b[16];
     hfe_store(b, x);
@@ -219,11 +218,13 @@ void free_merkle(ml_merkle* m) {
     pfree(m->data_ptrs_dev, m->stream);
     delete m;
 }
-int new_merkle(size_t n_leaves, cudaStream_t s, ml_merkle** out) {
+// digests: a buffer of 2 * n_leaves digests the tree uses without owning it (nullptr: allocated from the stream's pool)
+int new_merkle(size_t n_leaves, cudaStream_t s, ml_merkle** out, uint8_t* digests = nullptr) {
     ml_merkle* m = new ml_merkle();
     m->n_leaves = n_leaves;
     m->stream = s;
-    if (pmalloc((void**)&m->digests, (2 * n_leaves) * 32, s) != ML_OK) { delete m; return ML_ERR_ALLOC; }
+    if (digests) { m->digests = digests; m->owns_digests = false; }
+    else if (pmalloc((void**)&m->digests, (2 * n_leaves) * 32, s) != ML_OK) { delete m; return ML_ERR_ALLOC; }
     cudaGetDevice(&m->device);
     *out = m;
     return ML_OK;
@@ -478,17 +479,20 @@ int sumcheck_build(Ctx* ctx, const uint8_t* inputs, size_t n_vars, const void* e
 
 // evals -> to_coefficient -> bit_reverse -> reed_solomon (multilinear_pcs.rs:101-107): returns a new owned code of 2n elements
 // writes the code of one polynomial given by evaluations into `code` (2n elements)
-int encode_into(Ctx* ctx, const fe* evals_dev, size_t n, fe* code, cudaStream_t s) {
+// work: 3n elements of scratch (nullptr: stream-ordered allocations per call)
+int encode_into(Ctx* ctx, const fe* evals_dev, size_t n, fe* code, cudaStream_t s, fe* work) {
     const int log_domain = (int)ilog2(n) + ML_LOG_BLOWUP;
     Scratch coeffs(s);
-    MLB_TRY(coeffs.alloc(n * 16));
-    MLB_TRY(mobius_launch(evals_dev, coeffs.as<fe>(), n, true, s));
+    fe* c = work;
+    if (!c) { MLB_TRY(coeffs.alloc(n * 16)); c = coeffs.as<fe>(); }
+    MLB_TRY(mobius_launch(evals_dev, c, n, true, s));
     if (ntt_fuses_bitrev(log_domain))  // bit_reverse_permutation (:104) folded into the first NTT pass's addressing
-        return ntt_launch(ctx, coeffs.as<fe>(), code, log_domain, false, true, s, true);
+        return ntt_launch(ctx, c, code, log_domain, false, true, s, true, work ? work + n : nullptr);
     Scratch rev(s);
-    MLB_TRY(rev.alloc(n * 16));
-    MLB_TRY(bit_reverse_launch(coeffs.p, rev.p, n, 16, s));
-    return ntt_launch(ctx, rev.as<fe>(), code, log_domain, false, true, s);
+    fe* r = work ? work + n : nullptr;
+    if (!r) { MLB_TRY(rev.alloc(n * 16)); r = rev.as<fe>(); }
+    MLB_TRY(bit_reverse_launch(c, r, n, 16, s));
+    return ntt_launch(ctx, r, code, log_domain, false, true, s);
 }
 int encode_poly(Ctx* ctx, const fe* evals_dev, size_t n, fe** code_out, cudaStream_t s) {
     fe* code;
@@ -502,9 +506,9 @@ int encode_poly(Ctx* ctx, const fe* evals_dev, size_t n, fe** code_out, cudaStre
 // ------------------------------------------------------------------ sync-free fold chain (device transcript)
 
 // build the tree of a layer without reading the root back (the chain absorbs it on the device)
-int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree) {
+int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree, uint8_t* digests) {
     ml_merkle* m;
-    MLB_TRY(new_merkle(n / 2, s, &m));
+    MLB_TRY(new_merkle(n / 2, s, &m, digests));
     m->kind = ml_merkle::RS_CODE;
     m->item_bytes = 32;
     m->data.push_back(code);
@@ -523,36 +527,39 @@ uint8_t* layer_root_ptr(const ml_fri::Layer& L) {
     return L.tree->digests + 32 * merkle_layer_offset(leaves, (int)ilog2(leaves));
 }
 
-// Runs fold steps k_start.. to the end with the transcript advanced on the device.
+size_t chain_scratch_bytes() { return CHAIN_OFF_PART + (size_t)(2 * sumcheck_max_blocks() + 2) * 16; }
+
+// the next layer's buffers: a prove plan's (ChainHooks::layer_code / layer_digests) or a pool allocation the layer owns
+static int chain_layer_bufs(const ml_fri* f, const ChainHooks* hooks, size_t n, fe** code, uint8_t** digests, bool* owns, cudaStream_t s) {
+    if (hooks && hooks->layer_code) {
+        *code = hooks->layer_code[f->layers.size()];
+        *digests = hooks->layer_digests[f->layers.size()];
+        *owns = false;
+        return ML_OK;
+    }
+    *digests = nullptr;
+    *owns = true;
+    return pmalloc((void**)code, n * 16, s);
+}
+
+// Enqueues fold steps k_start.. to the end with the transcript advanced on the device; nothing is read back.
 //   f       : FriProverData; its last layer is the current code (tree built).  Empty only with `b` (batched first fold).
 //   pending : the last layer's root has not been absorbed yet
 //   sc/prev : sumcheck tables + running claim for the PCS interleave (nullptr/unused for plain FRI)
-//   sc_out  : host array receiving (c1, c2) per round from k_start on
-// On return every layer root, last_element and the host transcript are up to date.
-int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, hfe* sc_out, size_t k_start, bool pending,
-                   ml_transcript* t, cudaStream_t s) {
+//   base    : chain_scratch_bytes() of device memory; on completion it holds the state listed at CHAIN_OFF_*
+// Needs k_start < the number of fold steps.
+int fold_chain_enqueue(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, size_t k_start, bool pending,
+                       ml_transcript* t, uint8_t* base, ChainRun* run, cudaStream_t s) {
     const size_t total_steps = (size_t)f->log_n0 - ML_LOG_BLOWUP;
-    if (k_start >= total_steps) {
-        if (!f->has_last) { set_error("fold: last_element is None"); return ML_ERR_SIZE; }
-        return ML_OK;
-    }
-    // one scratch block: transcript | r, r/2 | prev | last[2] | status | roots[64] | sc[2*64] | partials
-    const int max_nb = sumcheck_max_blocks();
-    Scratch blk(s);
-    const size_t off_tr = 0, off_r = 128, off_prev = off_r + 32, off_last = off_prev + 16, off_status = off_last + 32,
-                 off_roots = off_status + 16, off_sc = off_roots + 64 * 32, off_part = off_sc + 2 * 64 * 16,
-                 total = off_part + (size_t)(2 * max_nb + 2) * 16;
-    MLB_TRY(blk.alloc(total));
-    uint8_t* base = blk.as<uint8_t>();
-    DevTranscript* tr_dev = (DevTranscript*)(base + off_tr);
-    fe* r_dev = (fe*)(base + off_r);
-    fe* prev_dev = (fe*)(base + off_prev);
-    fe* last_dev = (fe*)(base + off_last);
-    int* status_dev = (int*)(base + off_status);
-    uint8_t* roots_dev = base + off_roots;
-    fe* sc_dev = (fe*)(base + off_sc);
-    fe* partials = (fe*)(base + off_part);
-    MLB_CUDA(cudaMemsetAsync(base, 0, off_part, s));
+    DevTranscript* tr_dev = (DevTranscript*)(base + CHAIN_OFF_TR);
+    fe* r_dev = (fe*)(base + CHAIN_OFF_R);
+    fe* prev_dev = (fe*)(base + CHAIN_OFF_PREV);
+    fe* last_dev = (fe*)(base + CHAIN_OFF_LAST);
+    int* status_dev = (int*)(base + CHAIN_OFF_STATUS);
+    uint8_t* roots_dev = base + CHAIN_OFF_ROOTS;
+    fe* sc_dev = (fe*)(base + CHAIN_OFF_SC);
+    fe* partials = (fe*)(base + CHAIN_OFF_PART);
+    MLB_CUDA(cudaMemsetAsync(base, 0, CHAIN_OFF_PART, s));
     if (hooks && hooks->tr_dev) MLB_CUDA(cudaMemcpyAsync(tr_dev, hooks->tr_dev, sizeof(DevTranscript), cudaMemcpyDeviceToDevice, s));
     else MLB_TRY(h2d(tr_dev, &t->sha, sizeof(DevTranscript), s));
     if (sc) {
@@ -567,8 +574,9 @@ int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc
     const RootTables* rt;
     MLB_TRY(get_root_tables(ctx, f->log_n0, s, &rt));
 
-    const size_t first_new_layer = f->layers.size() - (pending ? 1 : 0);  // roots to fetch afterwards: layers >= this index
-    bool used_tail = false, have_partials = false;
+    run->first_new_layer = f->layers.size() - (pending ? 1 : 0);  // roots to fetch afterwards: layers >= this index
+    run->used_tail = false;
+    bool have_partials = false;
     int sc_nb = 0;
     size_t k = k_start;
     for (; k < total_steps; k++) {
@@ -595,16 +603,18 @@ int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc
             int i = 1;
             for (size_t m = half_n; m > 2; m >>= 1, i++) {  // committed tail layers: sizes half_n .. 4
                 fe* code;
-                MLB_TRY(pmalloc((void**)&code, m * 16, s));
-                int st = fri_push_layer(f, code, m, true, s, false);
-                if (st != ML_OK) { pfree(code, s); return st; }
+                uint8_t* digests;
+                bool owns;
+                MLB_TRY(chain_layer_bufs(f, hooks, m, &code, &digests, &owns, s));
+                int st = fri_push_layer(f, code, m, owns, s, false, digests);
+                if (st != ML_OK) { if (owns) pfree(code, s); return st; }
                 a.codes[i] = code;
                 a.digests[i] = f->layers.back().tree->digests;
             }
             MLB_TRY(chain_tail_launch(a, s));
             if (sc) { size_t rounds = ilog2(n) - 1; sc->height >>= rounds; }
             pending = false;
-            used_tail = true;
+            run->used_tail = true;
             k = total_steps;
             break;
         }
@@ -626,45 +636,64 @@ int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc
         pending = false;
         // ---- fold
         fe* next = nullptr;
+        uint8_t* next_digests = nullptr;
         bool owns_next = true;
         if (batched_round) {
             if (!hooks || !hooks->first_fold) { set_error("fold chain: empty FriProverData without a first-fold hook"); return ML_ERR_ARG; }
             MLB_TRY(hooks->first_fold(r_dev, &next, &owns_next));
         } else {
-            MLB_TRY(pmalloc((void**)&next, half_n * 16, s));
+            MLB_TRY(chain_layer_bufs(f, hooks, half_n, &next, &next_digests, &owns_next, s));
             int st = fri_fold_launch(ctx, f->layers.back().code, n, next, 0, r_dev, k, f->log_n0, s);
-            if (st != ML_OK) { pfree(next, s); return st; }
+            if (st != ML_OK) { if (owns_next) pfree(next, s); return st; }
         }
         if (half_n == ((size_t)1 << ML_LOG_BLOWUP)) {  // only reachable from a batched first fold of a 4-element domain
             int st = chain_last_launch(next, tr_dev, last_dev, status_dev, s);
             if (owns_next) pfree(next, s);
             MLB_TRY(st);
-            used_tail = true;
+            run->used_tail = true;
             k = total_steps;
             break;
         }
-        int st = fri_push_layer(f, next, half_n, owns_next, s, true);
+        int st = fri_push_layer(f, next, half_n, owns_next, s, true, next_digests);
         if (st != ML_OK) { if (owns_next) pfree(next, s); return st; }
         pending = true;
     }
     if (pending) {  // chain ended on a committed layer (cannot happen for well-formed sizes, kept for safety)
         MLB_TRY(chain_challenge_launch(tr_dev, layer_root_ptr(f->layers.back()), 32, roots_dev + 32 * (f->layers.size() - 1), r_dev, false, s));
     }
+    return ML_OK;
+}
+
+// Runs fold steps k_start.. to the end (fold_chain_enqueue) and reads the result back.
+//   sc_out  : host array receiving (c1, c2) per round from k_start on
+// On return every layer root, last_element and the host transcript are up to date.
+int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, hfe* sc_out, size_t k_start, bool pending,
+                   ml_transcript* t, cudaStream_t s) {
+    const size_t total_steps = (size_t)f->log_n0 - ML_LOG_BLOWUP;
+    if (k_start >= total_steps) {
+        if (!f->has_last) { set_error("fold: last_element is None"); return ML_ERR_SIZE; }
+        return ML_OK;
+    }
+    Scratch blk(s);
+    MLB_TRY(blk.alloc(chain_scratch_bytes()));
+    uint8_t* base = blk.as<uint8_t>();
+    ChainRun run;
+    MLB_TRY(fold_chain_enqueue(ctx, f, hooks, sc, prev, k_start, pending, t, base, &run, s));
     // ---- single synchronisation point: roots, last element, status, coefficients, transcript
     trace("enqueued");
-    std::vector<uint8_t> host(off_part);
-    MLB_TRY(d2h_sync(host.data(), base, off_part, s));
+    std::vector<uint8_t> host(CHAIN_OFF_PART);
+    MLB_TRY(d2h_sync(host.data(), base, CHAIN_OFF_PART, s));
     int status = 0;
-    memcpy(&status, host.data() + off_status, sizeof status);
+    memcpy(&status, host.data() + CHAIN_OFF_STATUS, sizeof status);
     if (status != 0) { set_error("not an RS code"); return status; }
-    for (size_t j = first_new_layer; j < f->layers.size(); j++) memcpy(f->layers[j].tree->root, host.data() + off_roots + 32 * j, 32);
-    if (used_tail) {
-        f->last = hfe_load(host.data() + off_last);
+    for (size_t j = run.first_new_layer; j < f->layers.size(); j++) memcpy(f->layers[j].tree->root, host.data() + CHAIN_OFF_ROOTS + 32 * j, 32);
+    if (run.used_tail) {
+        f->last = hfe_load(host.data() + CHAIN_OFF_LAST);
         f->has_last = true;
     }
     if (sc && sc_out)
-        for (size_t i = 0; i < 2 * (total_steps - k_start); i++) sc_out[i] = hfe_load(host.data() + off_sc + 16 * i);
-    memcpy(&t->sha, host.data() + off_tr, sizeof(DevTranscript));
+        for (size_t i = 0; i < 2 * (total_steps - k_start); i++) sc_out[i] = hfe_load(host.data() + CHAIN_OFF_SC + 16 * i);
+    memcpy(&t->sha, host.data() + CHAIN_OFF_TR, sizeof(DevTranscript));
     if (!f->has_last) { set_error("fold: last_element is None"); return ML_ERR_SIZE; }
     return ML_OK;
 }

@@ -32,11 +32,13 @@ void absorb_fe(ml_transcript* t, hfe x);
 hfe challenge(ml_transcript* t);
 void free_fri(ml_fri* f);
 void free_sumcheck(ml_sumcheck* s);
-int encode_into(Ctx* ctx, const fe* evals_dev, size_t n, fe* code, cudaStream_t s);
+// evals (n) -> to_coefficient -> bit_reverse -> reed_solomon into code (2n); work: 3n elements of scratch or nullptr
+int encode_into(Ctx* ctx, const fe* evals_dev, size_t n, fe* code, cudaStream_t s, fe* work = nullptr);
 void derive_indices(ml_transcript* t, size_t domain_size, std::vector<size_t>& idx);
 void fill_dirs(PathH& p, size_t index, int depth);
-// appends layer `code` (n elements) to f with its Merkle tree (build_tree) but without reading the root back
-int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree);
+// appends layer `code` (n elements) to f with its Merkle tree (build_tree) but without reading the root back; digests: the
+// tree's buffer (2 * n/2 digests, not owned) or nullptr for a pool allocation
+int fri_push_layer(ml_fri* f, fe* code, size_t n, bool owns_code, cudaStream_t s, bool build_tree, uint8_t* digests = nullptr);
 int fri_open_queries(const ml_fri* f, const std::vector<size_t>& indices, std::vector<QueryH>& out, cudaStream_t s);
 // the RESTRICTION on a caller's gen_pows (include/multilinear_b200.h): NULL, or the powers of pow_2_generator(log_n0)
 int check_gen_pows(int log_n0, const uint8_t* gen_pows, size_t gen_pows_len);
@@ -53,7 +55,22 @@ struct ChainHooks {
     std::function<int(const fe* r_dev, fe** next, bool* owns)> first_fold;
     const DevTranscript* tr_dev = nullptr;  // transcript state already in HBM (device copy instead of uploading the host state)
     const fe* prev_dev = nullptr;           // running sumcheck claim already in HBM
+    // buffers of a prove plan, indexed by layer: the code and the Merkle digests of every layer the chain commits (instead of
+    // pool allocations; the layers do not own them)
+    fe* const* layer_code = nullptr;
+    uint8_t* const* layer_digests = nullptr;
 };
+// the fold chain's scratch block: transcript | r, r/2 | prev | last[2] | status | roots[64] | sc[2*64] | sumcheck partials
+static const size_t CHAIN_OFF_TR = 0, CHAIN_OFF_R = 128, CHAIN_OFF_PREV = CHAIN_OFF_R + 32, CHAIN_OFF_LAST = CHAIN_OFF_PREV + 16,
+                    CHAIN_OFF_STATUS = CHAIN_OFF_LAST + 32, CHAIN_OFF_ROOTS = CHAIN_OFF_STATUS + 16, CHAIN_OFF_SC = CHAIN_OFF_ROOTS + 64 * 32,
+                    CHAIN_OFF_PART = CHAIN_OFF_SC + 2 * 64 * 16;
+size_t chain_scratch_bytes();
+struct ChainRun {
+    size_t first_new_layer = 0;  // layers whose roots the chain wrote at CHAIN_OFF_ROOTS
+    bool used_tail = false;      // the chain produced last_element (at CHAIN_OFF_LAST)
+};
+int fold_chain_enqueue(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, size_t k_start, bool pending,
+                       ml_transcript* t, uint8_t* base, ChainRun* run, cudaStream_t s);
 int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, hfe* sc_out, size_t k_start, bool pending,
                    ml_transcript* t, cudaStream_t s);
 

@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard, MlBfriShard);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard, MlBfriShard, MlProvePlan);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -112,6 +112,7 @@ extern "C" {
     pub fn ml_fri_proof_serialize(p: *const MlFriProof, out: *mut u8) -> c_int;
     pub fn ml_fri_proof_serialized_len(p: *const MlFriProof) -> usize;
     pub fn ml_fri_prove(code: *const u8, n: usize, gen_pows: *const u8, gen_pows_len: usize, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_fri_prove_async(p: *mut MlProvePlan, code_dev: *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_fri_prove_dev(code_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlFriProof) -> c_int;
     pub fn ml_fri_shard_arena_bytes(sh: *const MlFriShard) -> usize;
     pub fn ml_fri_shard_connect(sh: *mut MlFriShard, records: *const u8, n_records: usize) -> c_int;
@@ -166,6 +167,7 @@ extern "C" {
     pub fn ml_pcs_proof_num_rounds(p: *const MlPcsProof) -> usize;
     pub fn ml_pcs_proof_sumcheck_coeffs(p: *const MlPcsProof, out: *mut u8) -> c_int;
     pub fn ml_pcs_prove(inputs: *const u8, n_vars: usize, output: *const u8, evals: *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlPcsProof) -> c_int;
+    pub fn ml_pcs_prove_async(p: *mut MlProvePlan, inputs_dev: *const c_void, output_dev: *const c_void, evals_dev: *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, sumcheck_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_pcs_prove_dev(inputs: *const u8, n_vars: usize, output: *const u8, evals_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlPcsProof) -> c_int;
     pub fn ml_pcs_shard_arena_bytes(sh: *const MlPcsShard) -> usize;
     pub fn ml_pcs_shard_connect(sh: *mut MlPcsShard, records: *const u8, n_records: usize) -> c_int;
@@ -183,11 +185,16 @@ extern "C" {
     pub fn ml_pow2_generator(log_size: u64, out: *mut u8) -> c_int;
     pub fn ml_pow2_generator_powers(log_size: u64, out: *mut u8) -> c_int;
     pub fn ml_pow2_generator_powers_dev(log_size: u64, out_dev: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn ml_prove_plan_create(log_domain: usize, pcs: c_int, out: *mut *mut MlProvePlan) -> c_int;
+    pub fn ml_prove_plan_device_bytes(p: *const MlProvePlan) -> usize;
+    pub fn ml_prove_plan_free(p: *mut MlProvePlan);
+    pub fn ml_prove_plan_proof_bytes(p: *const MlProvePlan) -> usize;
     pub fn ml_reed_solomon(coeffs: *const u8, n: usize, gen_: *const u8, code: *mut u8) -> c_int;
     pub fn ml_reed_solomon_dev(coeffs_dev: *const c_void, n: usize, gen_: *const u8, code_dev: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn ml_release_pools() -> c_int;
     pub fn ml_rs_fri_fold_dev(coeffs_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlFri) -> c_int;
     pub fn ml_rs_fri_prove(coeffs: *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlFriProof) -> c_int;
+    pub fn ml_rs_fri_prove_async(p: *mut MlProvePlan, coeffs_dev: *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_rs_fri_prove_dev(coeffs_dev: *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlFriProof) -> c_int;
     pub fn ml_set_device(device: c_int) -> c_int;
     pub fn ml_set_pool_release_threshold(bytes: u64) -> c_int;
@@ -219,10 +226,13 @@ extern "C" {
     pub fn ml_synthetic_elements_dev(seed: u64, n: usize, out_dev: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn ml_transcript_absorb(t: *mut MlTranscript, bytes: *const u8, len: usize) -> c_int;
     pub fn ml_transcript_clone(t: *const MlTranscript, out: *mut *mut MlTranscript) -> c_int;
+    pub fn ml_transcript_export(t: *const MlTranscript, state_out: *mut u8) -> c_int;
     pub fn ml_transcript_free(t: *mut MlTranscript);
+    pub fn ml_transcript_import(state: *const u8, out: *mut *mut MlTranscript) -> c_int;
     pub fn ml_transcript_new(out: *mut *mut MlTranscript) -> c_int;
     pub fn ml_transcript_next_challenge(t: *mut MlTranscript, out: *mut u8) -> c_int;
     pub fn ml_transcript_random(t: *const MlTranscript, out: *mut u8) -> c_int;
+    pub fn ml_transcript_state_bytes() -> usize;
     pub fn ml_trim_pools(keep_bytes: usize) -> c_int;
     pub fn ml_version() -> *const c_char;
     pub fn ml_wsumcheck_build(row_point: *const u8, n_vars: usize, matrix: *const u8, width: usize, height: usize, out: *mut *mut MlWSumcheck) -> c_int;
@@ -365,6 +375,19 @@ impl Transcript {
         let mut le = [0u8; 16];
         check(unsafe { ml_transcript_next_challenge(self.h, le.as_mut_ptr()) });
         T::from(u128::from_le_bytes(le))
+    }
+    /// the running SHA-256 state (ml_transcript_state_bytes() bytes), as the stream-ordered provers take it in device memory
+    pub fn export_state(&self) -> Vec<u8> {
+        let mut out = vec![0u8; unsafe { ml_transcript_state_bytes() }];
+        check(unsafe { ml_transcript_export(self.h, out.as_mut_ptr()) });
+        out
+    }
+    /// a transcript continuing from an exported state (e.g. one a stream-ordered prove left in device memory)
+    pub fn import_state(state: &[u8]) -> Self {
+        assert_eq!(state.len(), unsafe { ml_transcript_state_bytes() });
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_transcript_import(state.as_ptr(), &mut h) });
+        Self { h }
     }
 }
 impl Default for Transcript {
@@ -662,6 +685,55 @@ impl ShardedFriProver {
 impl Drop for ShardedFriProver {
     fn drop(&mut self) {
         unsafe { ml_fri_shard_free(self.h) }
+    }
+}
+/// Stream-ordered `FriProof::prove` / `PCSProof::prove` of one domain size 2^log_domain (ml_prove_plan_*, csrc/plan.cu): the plan
+/// owns every device buffer a prove needs; a call only enqueues kernels on `stream` (e.g. a cudarc stream's raw handle) and writes
+/// the bincode blob, the final transcript state and the status into the caller's device buffers.  One proof in flight per plan.
+pub struct ProvePlan {
+    h: *mut MlProvePlan,
+}
+impl ProvePlan {
+    pub fn new(log_domain: usize, pcs: bool) -> Self {
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_prove_plan_create(log_domain, pcs as c_int, &mut h) });
+        Self { h }
+    }
+    /// bytes of the FriProof blob a call writes (`bincode` of the proof, fri/mod.rs:367-369)
+    pub fn proof_bytes(&self) -> usize {
+        unsafe { ml_prove_plan_proof_bytes(self.h) }
+    }
+    pub fn device_bytes(&self) -> usize {
+        unsafe { ml_prove_plan_device_bytes(self.h) }
+    }
+    /// `reed_solomon` + `FriProof::prove` of N/2 coefficients in HBM.
+    /// # Safety
+    /// Every pointer is device memory of the size include/multilinear_b200.h states, 16-byte aligned, and stays valid until the
+    /// stream has passed the call.
+    pub unsafe fn rs_fri_prove_async(&mut self, coeffs_dev: *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void,
+                                     status_dev: *mut c_int, stream: *mut c_void) {
+        check(ml_rs_fri_prove_async(self.h, coeffs_dev, transcript_dev, proof_dev, status_dev, stream));
+    }
+    /// `FriProof::prove` of a code of N elements in HBM.
+    /// # Safety
+    /// As for `rs_fri_prove_async`.
+    pub unsafe fn fri_prove_async(&mut self, code_dev: *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void,
+                                  status_dev: *mut c_int, stream: *mut c_void) {
+        check(ml_fri_prove_async(self.h, code_dev, transcript_dev, proof_dev, status_dev, stream));
+    }
+    /// `PCSProof::prove` of N/2 evaluations in HBM (a plan made with `pcs`); sumcheck_dev receives 2 * n_vars coefficients.
+    /// # Safety
+    /// As for `rs_fri_prove_async`.
+    #[allow(clippy::too_many_arguments)]
+    pub unsafe fn pcs_prove_async(&mut self, inputs_dev: *const c_void, output_dev: *const c_void, evals_dev: *const c_void,
+                                  transcript_dev: *mut c_void, proof_dev: *mut c_void, sumcheck_dev: *mut c_void, status_dev: *mut c_int,
+                                  stream: *mut c_void) {
+        check(ml_pcs_prove_async(self.h, inputs_dev, output_dev, evals_dev, transcript_dev, proof_dev, sumcheck_dev, status_dev, stream));
+    }
+}
+impl Drop for ProvePlan {
+    fn drop(&mut self) {
+        unsafe { ml_prove_plan_free(self.h) }
     }
 }
 /// `BatchedFriProof` does not derive `Deserialize`; its blob is the bincode encoding of its parts in field order, and the parts
