@@ -312,6 +312,9 @@ int ml_bfri_proof_commitments(const ml_bfri_proof *p, uint8_t *out);
 int ml_bfri_proof_last(const ml_bfri_proof *p, uint8_t last_elem[16], uint8_t last_random[32]);
 size_t ml_bfri_proof_serialized_len(const ml_bfri_proof *p);
 int ml_bfri_proof_serialize(const ml_bfri_proof *p, uint8_t *out);
+/* inverse of ml_bfri_proof_serialize (a blob made by the Rust crate, by ml_batched_*_prove_async or by the serializer): ML_ERR_ARG on
+ * malformed input (truncated or trailing bytes, a wrong length prefix, a direction above 1, a non-canonical field element) */
+int ml_bfri_proof_deserialize(const uint8_t *blob, size_t len, ml_bfri_proof **out);
 
 typedef struct ml_bpcs_proof ml_bpcs_proof; /* BatchedPCSProof batched_pcs.rs:22-29 */
 int ml_batched_pcs_prove(const uint8_t *inputs, size_t n_vars, const uint8_t *outputs, size_t n_polys,
@@ -323,6 +326,44 @@ void ml_bpcs_proof_free(ml_bpcs_proof *p);
 const ml_bfri_proof *ml_bpcs_proof_fri(const ml_bpcs_proof *p);
 size_t ml_bpcs_proof_num_rounds(const ml_bpcs_proof *p);
 int ml_bpcs_proof_sumcheck_coeffs(const ml_bpcs_proof *p, uint8_t *out);
+
+/* ---- stream-ordered batched provers: BatchedFriProof::prove / BatchedPCSProof::prove enqueued on a caller's stream ----
+ * The batched counterpart of the stream-ordered provers above, for B = n_codes codes of N = 2^log_domain elements.  A plan is
+ * made for one kind of call:
+ *   ML_BPLAN_CODES: ml_batched_fri_prove_async    = ml_batched_fri_prove (codes_dev: B device pointers, N elements each; the
+ *                   codes are read in place),
+ *   ML_BPLAN_RS:    ml_batched_rs_fri_prove_async = reed_solomon of each + ml_batched_fri_prove, as ml_bfri_shard_rs_prove_dev
+ *                   at one rank (coeffs_dev: B device pointers, N/2 coefficients each),
+ *   ML_BPLAN_PCS:   ml_batched_pcs_prove_async    = ml_batched_pcs_prove_dev (inputs_dev: n_vars = log_domain - 1 points,
+ *                   outputs_dev: B claimed values, evals_dev: B device pointers, N/2 evaluations each).
+ * codes_dev / coeffs_dev / evals_dev are HOST arrays of device pointers, as ml_batched_pcs_prove_dev takes them; the call reads
+ * the array before it returns.  A plan owns, in one cudaMalloc outside the stream pools: the batch tree (32 N bytes, also the
+ * encodes' scratch), FRI layers N/2 .. 4 with their trees, for RS and PCS plans the B codes (16 B N bytes: 8 GiB at 64 x 2^22),
+ * for PCS plans the sumcheck tables, and the chain and query buffers; ml_batched_prove_plan_device_bytes is the total.
+ * ml_batched_prove_plan_create: ML_ERR_SIZE for log_domain outside 3..40 or n_codes outside 1..2^20, ML_ERR_ARG for an unknown
+ * kind, ML_ERR_ALLOC when the plan does not fit (nothing is left allocated), ML_ERR_CUDA without a device.
+ *
+ * proof_dev (ml_batched_prove_plan_proof_bytes bytes) receives the BatchedFriProof bincode blob, byte-identical to
+ * ml_bfri_proof_serialize of the blocking twin's proof (for PCS: of ml_bpcs_proof_fri); sumcheck_dev (2 * n_vars elements)
+ * receives ml_bpcs_proof_sumcheck_coeffs; transcript_dev and *status_dev as for the single provers (ML_ERR_NOT_RS_CODE is possible
+ * only for ML_BPLAN_CODES).  Inputs are only read.
+ * Host-side rejections enqueue nothing and return ML_ERR_ARG: a NULL plan, buffer, array or pointer in the array; a device buffer
+ * that is not 16-byte aligned; an output (transcript, proof, sumcheck, status) overlapping any input, including each of the
+ * n_codes pointed-to buffers, or another output; a call of another kind than the plan's; a current device other than the plan's.
+ * An enqueue makes no allocation, no synchronisation, no host->device copy from host memory and no host read of device data, and
+ * may be captured into a CUDA graph with cudaStreamCaptureModeGlobal.  One proof in flight per plan, as above. */
+enum { ML_BPLAN_CODES = 0, ML_BPLAN_RS = 1, ML_BPLAN_PCS = 2 };
+typedef struct ml_batched_prove_plan ml_batched_prove_plan;
+int ml_batched_prove_plan_create(size_t log_domain, size_t n_codes, int kind, ml_batched_prove_plan **out);
+void ml_batched_prove_plan_free(ml_batched_prove_plan *p);
+size_t ml_batched_prove_plan_device_bytes(const ml_batched_prove_plan *p);
+size_t ml_batched_prove_plan_proof_bytes(const ml_batched_prove_plan *p);  /* == ml_bfri_proof_serialized_len of its proof */
+int ml_batched_fri_prove_async(ml_batched_prove_plan *p, const void *const *codes_dev, void *transcript_dev, void *proof_dev, int *status_dev,
+                               void *stream);
+int ml_batched_rs_fri_prove_async(ml_batched_prove_plan *p, const void *const *coeffs_dev, void *transcript_dev, void *proof_dev,
+                                  int *status_dev, void *stream);
+int ml_batched_pcs_prove_async(ml_batched_prove_plan *p, const void *inputs_dev, const void *outputs_dev, const void *const *evals_dev,
+                               void *transcript_dev, void *proof_dev, void *sumcheck_dev, int *status_dev, void *stream);
 
 /* ---- sumcheck tables of arbitrary trace width (System path; SURVEY.md §8f row 4).
  * Replaces SumcheckTables as built by System::build_tables (src/constraint_system/sumcheck.rs:22-38) with

@@ -441,6 +441,29 @@ class ProvePlan {
   private:
     ml_prove_plan* h_ = nullptr;
 };
+// stream-ordered BatchedFriProof / BatchedPCSProof provers (ml_batched_prove_plan_*); the per-code arguments are device pointers
+class BatchedProvePlan {
+  public:
+    BatchedProvePlan(size_t log_domain, size_t n_codes, int kind /* ML_BPLAN_* */) { check(ml_batched_prove_plan_create(log_domain, n_codes, kind, &h_)); }
+    BatchedProvePlan(const BatchedProvePlan&) = delete;
+    BatchedProvePlan& operator=(const BatchedProvePlan&) = delete;
+    ~BatchedProvePlan() { ml_batched_prove_plan_free(h_); }
+    size_t proof_bytes() const { return ml_batched_prove_plan_proof_bytes(h_); }
+    size_t device_bytes() const { return ml_batched_prove_plan_device_bytes(h_); }
+    void batched_fri_prove_async(const std::vector<const void*>& codes_dev, void* transcript_dev, void* proof_dev, int* status_dev, void* stream) {
+        check(ml_batched_fri_prove_async(h_, codes_dev.data(), transcript_dev, proof_dev, status_dev, stream));
+    }
+    void batched_rs_fri_prove_async(const std::vector<const void*>& coeffs_dev, void* transcript_dev, void* proof_dev, int* status_dev, void* stream) {
+        check(ml_batched_rs_fri_prove_async(h_, coeffs_dev.data(), transcript_dev, proof_dev, status_dev, stream));
+    }
+    void batched_pcs_prove_async(const void* inputs_dev, const void* outputs_dev, const std::vector<const void*>& evals_dev, void* transcript_dev,
+                                 void* proof_dev, void* sumcheck_dev, int* status_dev, void* stream) {
+        check(ml_batched_pcs_prove_async(h_, inputs_dev, outputs_dev, evals_dev.data(), transcript_dev, proof_dev, sumcheck_dev, status_dev, stream));
+    }
+
+  private:
+    ml_batched_prove_plan* h_ = nullptr;
+};
 // src/fri/batched_fri.rs:284-398
 class BatchedFriProof {
   public:
@@ -449,6 +472,11 @@ class BatchedFriProof {
         for (auto& c : codes) ptrs.push_back(raw(c));
         BatchedFriProof p;
         check(ml_batched_fri_prove(ptrs.data(), codes.size(), codes.empty() ? 0 : codes[0].size(), raw(gen_pows), gen_pows.size(), t.handle(), &p.h_));
+        return p;
+    }
+    static BatchedFriProof deserialize(const std::vector<uint8_t>& blob) {  // inverse of serialize()
+        BatchedFriProof p;
+        check(ml_bfri_proof_deserialize(blob.data(), blob.size(), &p.h_));
         return p;
     }
     BatchedFriProof(BatchedFriProof&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }

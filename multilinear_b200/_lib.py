@@ -41,12 +41,12 @@ _SIZE_T_FUNCS = ["ml_merkle_num_layers", "ml_merkle_layer_len", "ml_fri_num_tree
                  "ml_bfri_proof_serialized_len", "ml_bpcs_proof_num_rounds", "ml_shard_record_bytes", "ml_shard_arena_bytes", "ml_bfri_num_codes",
                  "ml_pcs_shard_arena_bytes", "ml_bpcs_shard_arena_bytes", "ml_wsumcheck_shard_arena_bytes",
                  "ml_fri_shard_arena_bytes", "ml_bfri_shard_arena_bytes", "ml_transcript_state_bytes", "ml_prove_plan_device_bytes",
-                 "ml_prove_plan_proof_bytes"]
+                 "ml_prove_plan_proof_bytes", "ml_batched_prove_plan_device_bytes", "ml_batched_prove_plan_proof_bytes"]
 _PTR_FUNCS = ["ml_pcs_proof_fri", "ml_bpcs_proof_fri", "ml_shard_stream", "ml_bfri_fri_data", "ml_bfri_batch_layer", "ml_pcs_shard_stream", "ml_bpcs_shard_stream", "ml_wsumcheck_shard_stream",
               "ml_fri_shard_stream", "ml_bfri_shard_stream"]
 _VOID_FUNCS = ["ml_transcript_free", "ml_merkle_free", "ml_fri_free", "ml_fri_proof_free", "ml_sumcheck_free", "ml_wsumcheck_free", "ml_pcs_proof_free",
                "ml_bfri_proof_free", "ml_bpcs_proof_free", "ml_shard_free", "ml_bfri_free", "ml_pcs_shard_free", "ml_bpcs_shard_free", "ml_wsumcheck_shard_free",
-               "ml_fri_shard_free", "ml_bfri_shard_free", "ml_prove_plan_free"]
+               "ml_fri_shard_free", "ml_bfri_shard_free", "ml_prove_plan_free", "ml_batched_prove_plan_free"]
 
 
 def lib_path():

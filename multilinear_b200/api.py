@@ -831,6 +831,60 @@ def _vp(x):
     return C.c_void_p(x if x is None else int(x))
 
 
+def _ptr_array(ptrs):
+    return (C.c_void_p * max(len(ptrs), 1))(*[None if x is None else int(x) for x in ptrs])
+
+
+class BatchedProvePlan:
+    """Stream-ordered BatchedFriProof / BatchedPCSProof provers of n_codes codes of 2^log_domain elements (ml_batched_prove_plan_*),
+    made for one kind of call: "codes" (batched_fri_prove_async), "rs" (batched_rs_fri_prove_async) or "pcs"
+    (batched_pcs_prove_async).  Buffers are device pointers as ints; the per-code arguments are lists of them.  `stream` is a
+    cudaStream_t as an int (None: the legacy stream).  The calls only enqueue: read the outputs after the stream has reached them."""
+    KINDS = {"codes": 0, "rs": 1, "pcs": 2}
+
+    def __init__(self, h, log_domain, n_codes, kind):
+        self.h, self.log_domain, self.n_codes, self.kind = h, log_domain, n_codes, kind
+
+    @staticmethod
+    def create(log_domain, n_codes, kind):
+        h = C.c_void_p()
+        check(load().ml_batched_prove_plan_create(_sz(log_domain), _sz(n_codes), C.c_int(BatchedProvePlan.KINDS[kind]), C.byref(h)))
+        return BatchedProvePlan(h, log_domain, n_codes, kind)
+
+    @property
+    def proof_bytes(self):
+        return load().ml_batched_prove_plan_proof_bytes(self.h)
+
+    @property
+    def device_bytes(self):
+        return load().ml_batched_prove_plan_device_bytes(self.h)
+
+    def batched_fri_prove_async(self, codes_dev, transcript_dev, proof_dev, status_dev, stream=None):
+        """BatchedFriProof::prove of n_codes codes of N elements each (= ml_batched_fri_prove)"""
+        check(load().ml_batched_fri_prove_async(self.h, _ptr_array(codes_dev), _vp(transcript_dev), _vp(proof_dev), _vp(status_dev), _vp(stream)))
+
+    def batched_rs_fri_prove_async(self, coeffs_dev, transcript_dev, proof_dev, status_dev, stream=None):
+        """reed_solomon of each of n_codes polynomials of N/2 coefficients + BatchedFriProof::prove"""
+        check(load().ml_batched_rs_fri_prove_async(self.h, _ptr_array(coeffs_dev), _vp(transcript_dev), _vp(proof_dev), _vp(status_dev),
+                                                   _vp(stream)))
+
+    def batched_pcs_prove_async(self, inputs_dev, outputs_dev, evals_dev, transcript_dev, proof_dev, sumcheck_dev, status_dev, stream=None):
+        """BatchedPCSProof::prove of n_codes polynomials of N/2 evaluations each (= ml_batched_pcs_prove_dev)"""
+        check(load().ml_batched_pcs_prove_async(self.h, _vp(inputs_dev), _vp(outputs_dev), _ptr_array(evals_dev), _vp(transcript_dev),
+                                                _vp(proof_dev), _vp(sumcheck_dev), _vp(status_dev), _vp(stream)))
+
+    def free(self):
+        if self.h is not None and self.h.value:
+            load().ml_batched_prove_plan_free(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class BatchedFriProof:
     @staticmethod
     def prove(codes, gen_pows, transcript):
@@ -845,6 +899,14 @@ class BatchedFriProof:
         h = C.c_void_p()
         check(load().ml_batched_fri_prove(ptrs, _sz(len(cs)), _sz(cs[0].shape[0]), _p(gp) if gp is not None else None,
                                           _sz(gp.shape[0] if gp is not None else 0), transcript.h, C.byref(h)))
+        return FriProof(h, batched=True)
+
+    @staticmethod
+    def deserialize(blob):
+        """a BatchedFriProof from its bincode bytes (batched_fri.rs:21-27) — e.g. one made by the Rust crate or by BatchedProvePlan"""
+        b = np.frombuffer(bytes(blob), dtype=np.uint8).copy()
+        h = C.c_void_p()
+        check(load().ml_bfri_proof_deserialize(_p(b), _sz(len(b)), C.byref(h)))
         return FriProof(h, batched=True)
 
 

@@ -7,11 +7,11 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libmultilinear_b200.so")
-SOURCES = ["core.cu", "field_ops.cu", "ntt.cu", "merkle.cu", "fri.cu", "sumcheck.cu", "mle.cu", "prover.cu", "chain.cu", "peer.cu", "shard.cu", "pcs_shard.cu", "bpcs_shard.cu", "wsumcheck_shard.cu", "fri_shard.cu", "bfri_shard.cu", "plan.cu"]
+SOURCES = ["core.cu", "field_ops.cu", "ntt.cu", "merkle.cu", "fri.cu", "sumcheck.cu", "mle.cu", "prover.cu", "chain.cu", "peer.cu", "shard.cu", "pcs_shard.cu", "bpcs_shard.cu", "wsumcheck_shard.cu", "fri_shard.cu", "bfri_shard.cu", "plan.cu", "bplan.cu"]
 # instrumentation (integer-pipe speed-of-light loops for bench.py / tools): its own library, not part of the product ABI
 INSTR_OUT = os.path.join(HERE, "libmlb_instr.so")
 INSTR_SOURCES = ["microbench.cu"]
-HEADERS = ["field.cuh", "sha256.cuh", "reduce.cuh", "transcript.cuh", "internal.h", "handles.h", "prover_internal.h", "peer.h", "pcs_shard.h", os.path.join("..", "..", "include", "multilinear_b200.h"),
+HEADERS = ["field.cuh", "sha256.cuh", "reduce.cuh", "transcript.cuh", "internal.h", "handles.h", "prover_internal.h", "peer.h", "pcs_shard.h", "plan.h", os.path.join("..", "..", "include", "multilinear_b200.h"),
            os.path.join("..", "..", "include", "multilinear_b200_instr.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--expt-relaxed-constexpr",

@@ -103,8 +103,10 @@ int fri_fold_launch(Ctx* ctx, const fe* cur, size_t n_cur, fe* next, hfe r, cons
 // batched first fold (batched_fri.rs:124-150): a, b are Horner fingerprints over the batch, acc = acc*rho + c_j
 __global__ void __launch_bounds__(256) fri_batched_fold_kernel(const fe* const* __restrict__ codes, int n_codes, size_t half_n,
                                                                fe* __restrict__ next, fe rho, fe r_half, const fe* __restrict__ r_dev,
-                                                               int log_n0, const fe* __restrict__ lo, const fe* __restrict__ hi) {
+                                                               int log_n0, const fe* __restrict__ lo, const fe* __restrict__ hi,
+                                                               const fe* __restrict__ rho_dev) {
     if (r_dev) r_half = fe_load(r_dev + 1);
+    if (rho_dev) rho = fe_load(rho_dev);
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     const size_t n0 = (size_t)1 << log_n0;
@@ -122,13 +124,13 @@ __global__ void __launch_bounds__(256) fri_batched_fold_kernel(const fe* const* 
     }
 }
 int fri_batched_fold_launch(Ctx* ctx, const fe* const* codes, size_t n_codes, size_t n, fe* next, hfe fingerprint_r, hfe r,
-                            const fe* r_dev, int log_n0, cudaStream_t s) {
+                            const fe* r_dev, int log_n0, cudaStream_t s, const fe* rho_dev) {
     const RootTables* rt;
     MLB_TRY(get_root_tables(ctx, log_n0, s, &rt));
     const size_t half_n = n / 2;
     ProfScope prof(PROF_FRI_FOLD, 16.0 * (double)n * (double)n_codes + 8.0 * (double)n, s);
     fri_batched_fold_kernel<<<grid_for(half_n), 256, 0, s>>>(codes, (int)n_codes, half_n, next, to_dev_fe(fingerprint_r),
-                                                              to_dev_fe(hfe_half(r)), r_dev, log_n0, rt->lo, rt->hi);
+                                                              to_dev_fe(hfe_half(r)), r_dev, log_n0, rt->lo, rt->hi, rho_dev);
     MLB_KERNEL_CHECK();
     return ML_OK;
 }

@@ -178,8 +178,9 @@ int merkle_batched_pairs_strided_launch(const uint8_t* pairs_base, size_t n_code
 int merkle_upper_launch(uint8_t* digests, size_t n_leaves, cudaStream_t s);  // layers 1.. from layer 0
 // fri.cu — r_dev (optional): device pointer to {r, r/2} written by a transcript kernel; overrides the host value r
 int fri_fold_launch(Ctx* ctx, const fe* cur, size_t n_cur, fe* next, hfe r, const fe* r_dev, size_t k, int log_n0, cudaStream_t s);
+// rho_dev (optional): the fingerprint challenge read from HBM instead of fingerprint_r
 int fri_batched_fold_launch(Ctx* ctx, const fe* const* codes_dev_ptrs, size_t n_codes, size_t n, fe* next, hfe fingerprint_r, hfe r,
-                            const fe* r_dev, int log_n0, cudaStream_t s);
+                            const fe* r_dev, int log_n0, cudaStream_t s, const fe* rho_dev = nullptr);
 // r_dev: rho read from HBM instead of r
 int fingerprint_rows_launch(const fe* const* polys_dev_ptrs, size_t n_polys, size_t n, hfe r, fe* out, cudaStream_t s, const fe* r_dev = nullptr);
 // sumcheck.cu

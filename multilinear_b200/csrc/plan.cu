@@ -8,27 +8,16 @@
 //   provers run, with its layers in the plan)  ->  fri_query_indices_kernel  ->  fri_proof_write_kernel  ->  status copy.
 // The blocking provers read the chain's state back and open the queries on the host (assemble_fri_proof); here the query indices
 // are derived on the device and the proof writer gathers the openings straight into the bincode blob.
-#include "prover_internal.h"
+#include "plan.h"
 
 using namespace mlb;
 using namespace mlbp;
 
 namespace {
 
-const int MAX_LAYERS = 40;  // log_domain <= 40: at most 39 committed layers
+const int MAX_LAYERS = PLAN_MAX_LAYERS;
 
-// The bincode wire format of a FriProof (fri/mod.rs:239-249, :367-369; Writer in prover.cu) at log_domain D, N = 2^D:
-//   u64 nc | nc x 32 B commitments | u64 128 | 128 queries | Field128 last_element (u64 16 + 16 B) | 32 B last_random
-// nc = D - 1 (layers N .. 4), query = u64 nc | nc paths; path j (depth d_j = D - 1 - j) =
-//   u64 16 | value 16 B | u64 16 | minus_value 16 B | u64 d_j | d_j x (32 B sibling digest | u32 direction)
-// Every offset depends on D alone.  Writer (prover.cu) states the same format for ml_fri_proof objects; the parity tests of
-// tests/test_prove_plan.py compare the two byte for byte at every size.
-__host__ __device__ inline size_t path_offset(int D, int j) {  // within a query
-    const size_t jj = (size_t)j;
-    return 8 + 56 * jj + 36 * (jj * (size_t)(D - 1) - jj * (jj - 1) / 2);
-}
-__host__ __device__ inline size_t query_bytes(int D) { return path_offset(D, D - 1); }
-__host__ __device__ inline size_t header_bytes(int D) { return 16 + 32 * (size_t)(D - 1); }
+// the FriProof wire format: plan.h
 size_t proof_bytes(int D) { return header_bytes(D) + (size_t)ML_NUM_QUERIES * query_bytes(D) + 56; }
 
 struct WriteArgs {
@@ -41,13 +30,7 @@ struct WriteArgs {
     uint8_t* out;
     int log_domain;
 };
-// every field of the blob starts at a multiple of 4 bytes from its 16-byte aligned start
-__device__ __forceinline__ void put32(uint8_t* p, uint32_t v) { *reinterpret_cast<uint32_t*>(p) = v; }
-__device__ __forceinline__ void put64(uint8_t* p, unsigned long long v) { put32(p, (uint32_t)v); put32(p + 4, (uint32_t)(v >> 32)); }
-__device__ __forceinline__ uint32_t word(const void* p, int i) { return reinterpret_cast<const uint32_t*>(p)[i]; }
-
-// CTA q < 128 writes query q: one warp per layer, lane 0..7 the value pair and lengths, every lane one sibling digest of the path
-// (open_query_at, fri/mod.rs:154-174; sibling and direction as merkle_tree/mod.rs:43-55).  CTA 128 writes the rest.
+// CTA q < 128 writes query q (write_fri_query, plan.h), CTA 128 writes the rest.
 __global__ void __launch_bounds__(256) fri_proof_write_kernel(WriteArgs a) {
     const int D = a.log_domain, nc = D - 1;
     const size_t qbytes = query_bytes(D), header = header_bytes(D);
@@ -61,52 +44,41 @@ __global__ void __launch_bounds__(256) fri_proof_write_kernel(WriteArgs a) {
         if (tid >= 32 && tid < 40) put32(tail + 24 + 4 * (tid - 32), word(a.last_random, tid - 32));
         return;
     }
-    uint8_t* qo = a.out + header + (size_t)blockIdx.x * qbytes;
-    const unsigned long long idx0 = a.indices[blockIdx.x];
-    if (tid == 0) put64(qo, (unsigned long long)nc);
-    const int lane = tid & 31;
-    for (int j = tid >> 5; j < nc; j += blockDim.x >> 5) {
-        const int depth = D - 1 - j;
-        const unsigned long long L = 1ull << depth, idx = idx0 & (L - 1);  // the index folds with the domain (cur %= cur_n)
-        uint8_t* po = qo + path_offset(D, j);
-        if (lane == 0) { put64(po, 16); put64(po + 24, 16); put64(po + 48, (unsigned long long)depth); }
-        if (lane < 4) put32(po + 8 + 4 * lane, word(a.code[j] + idx, lane));
-        else if (lane < 8) put32(po + 32 + 4 * (lane - 4), word(a.code[j] + idx + L, lane - 4));
-        for (int t = lane; t < depth; t += 32) {
-            const uint8_t* src = a.digests[j] + 32 * ((2 * L - ((2 * L) >> t)) + ((idx >> t) ^ 1ull));
-            uint8_t* dst = po + 56 + 36 * (size_t)t;
-#pragma unroll
-            for (int w = 0; w < 8; w++) put32(dst + 4 * w, word(src, w));
-            put32(dst + 32, ((idx >> t) & 1ull) ? 0u : 1u);  // even index: the sibling is on the Right
-        }
-    }
+    write_fri_query(a.out + header + (size_t)blockIdx.x * qbytes, a.code, a.digests, D, a.indices[blockIdx.x]);
 }
 
 size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
-bool misaligned(const void* p) { return ((uintptr_t)p & 15) != 0; }
-
-struct Buf {
-    const void* p;
-    size_t bytes;
-    bool out;
-    const char* name;
-};
-// null, misaligned and overlapping buffers (an output may overlap nothing else): ML_ERR_ARG before anything is enqueued
-int check_bufs(const Buf* b, int n) {
-    for (int i = 0; i < n; i++) {
-        if (!b[i].p) { set_error("prove plan: %s is NULL", b[i].name); return ML_ERR_ARG; }
-        if (misaligned(b[i].p)) { set_error("prove plan: %s is not 16-byte aligned", b[i].name); return ML_ERR_ARG; }
-    }
-    for (int i = 0; i < n; i++)
-        for (int j = i + 1; j < n; j++) {
-            if (!b[i].out && !b[j].out) continue;
-            const uintptr_t a0 = (uintptr_t)b[i].p, a1 = a0 + b[i].bytes, c0 = (uintptr_t)b[j].p, c1 = c0 + b[j].bytes;
-            if (a0 < c1 && c0 < a1) { set_error("prove plan: %s overlaps %s", b[i].name, b[j].name); return ML_ERR_ARG; }
-        }
-    return ML_OK;
-}
 
 }  // namespace
+
+int mlbp::plan_check_bufs(const PlanBuf* b, size_t n) {
+    char name[64];
+    auto label = [&](const PlanBuf& x) -> const char* {
+        if (x.index < 0) return x.name;
+        snprintf(name, sizeof name, "%s[%ld]", x.name, x.index);
+        return name;
+    };
+    for (size_t i = 0; i < n; i++) {
+        if (!b[i].p) { set_error("prove plan: %s is NULL", label(b[i])); return ML_ERR_ARG; }
+        if ((uintptr_t)b[i].p & 15) { set_error("prove plan: %s is not 16-byte aligned", label(b[i])); return ML_ERR_ARG; }
+    }
+    // outputs are few: compare each with every other buffer (inputs may overlap each other)
+    for (size_t i = 0; i < n; i++) {
+        if (!b[i].out) continue;
+        const uintptr_t a0 = (uintptr_t)b[i].p, a1 = a0 + b[i].bytes;
+        for (size_t j = 0; j < n; j++) {
+            if (j == i || (b[j].out && j < i)) continue;
+            const uintptr_t c0 = (uintptr_t)b[j].p, c1 = c0 + b[j].bytes;
+            if (a0 < c1 && c0 < a1) {
+                char other[64];
+                snprintf(other, sizeof other, "%s", label(b[j]));
+                set_error("prove plan: %s overlaps %s", b[i].name, other);
+                return ML_ERR_ARG;
+            }
+        }
+    }
+    return ML_OK;
+}
 
 struct ml_prove_plan {
     int device = -1;
@@ -243,9 +215,9 @@ int ml_rs_fri_prove_async(ml_prove_plan* p, const void* coeffs_dev, void* transc
     Ctx* ctx;
     MLB_TRY(check_plan(p, &ctx));
     const size_t N = (size_t)1 << p->log_domain;
-    const Buf b[] = {{coeffs_dev, 16 * (N / 2), false, "coeffs_dev"}, {transcript_dev, sizeof(DevTranscript), true, "transcript_dev"},
+    const PlanBuf b[] = {{coeffs_dev, 16 * (N / 2), false, "coeffs_dev"}, {transcript_dev, sizeof(DevTranscript), true, "transcript_dev"},
                      {proof_dev, proof_bytes(p->log_domain), true, "proof_dev"}, {status_dev, sizeof(int), true, "status_dev"}};
-    MLB_TRY(check_bufs(b, 4));
+    MLB_TRY(plan_check_bufs(b, 4));
     cudaStream_t s = (cudaStream_t)stream;
     // reed_solomon (fri/mod.rs:19-28) into layer 0; the multi-pass NTT's temporary is layer 0's digest buffer, which the tree
     // of layer 0 overwrites only after the NTT
@@ -257,9 +229,9 @@ int ml_fri_prove_async(ml_prove_plan* p, const void* code_dev, void* transcript_
     Ctx* ctx;
     MLB_TRY(check_plan(p, &ctx));
     const size_t N = (size_t)1 << p->log_domain;
-    const Buf b[] = {{code_dev, 16 * N, false, "code_dev"}, {transcript_dev, sizeof(DevTranscript), true, "transcript_dev"},
+    const PlanBuf b[] = {{code_dev, 16 * N, false, "code_dev"}, {transcript_dev, sizeof(DevTranscript), true, "transcript_dev"},
                      {proof_dev, proof_bytes(p->log_domain), true, "proof_dev"}, {status_dev, sizeof(int), true, "status_dev"}};
-    MLB_TRY(check_bufs(b, 4));
+    MLB_TRY(plan_check_bufs(b, 4));
     // the caller's code is layer 0 itself: the kernels only read it
     return enqueue_prove(ctx, p, (const fe*)code_dev, nullptr, nullptr, transcript_dev, proof_dev, nullptr, status_dev, (cudaStream_t)stream);
 }
@@ -271,10 +243,10 @@ int ml_pcs_prove_async(ml_prove_plan* p, const void* inputs_dev, const void* out
     if (!p->pcs) { set_error("ml_pcs_prove_async: the plan was made with pcs = 0"); return ML_ERR_ARG; }
     const int D = p->log_domain;
     const size_t N = (size_t)1 << D, n_vars = (size_t)D - 1;
-    const Buf b[] = {{inputs_dev, 16 * n_vars, false, "inputs_dev"}, {output_dev, 16, false, "output_dev"}, {evals_dev, 16 * (N / 2), false, "evals_dev"},
+    const PlanBuf b[] = {{inputs_dev, 16 * n_vars, false, "inputs_dev"}, {output_dev, 16, false, "output_dev"}, {evals_dev, 16 * (N / 2), false, "evals_dev"},
                      {transcript_dev, sizeof(DevTranscript), true, "transcript_dev"}, {proof_dev, proof_bytes(D), true, "proof_dev"},
                      {sumcheck_dev, 2 * 16 * n_vars, true, "sumcheck_dev"}, {status_dev, sizeof(int), true, "status_dev"}};
-    MLB_TRY(check_bufs(b, 7));
+    MLB_TRY(plan_check_bufs(b, 7));
     cudaStream_t s = (cudaStream_t)stream;
     // encode (multilinear_pcs.rs:101-107) into layer 0, its scratch in layer 0's digest buffer as above
     MLB_TRY(encode_into(ctx, (const fe*)evals_dev, N / 2, p->code[0], s, (fe*)p->digests[0]));

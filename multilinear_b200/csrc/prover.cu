@@ -641,6 +641,7 @@ int fold_chain_enqueue(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck
         if (batched_round) {
             if (!hooks || !hooks->first_fold) { set_error("fold chain: empty FriProverData without a first-fold hook"); return ML_ERR_ARG; }
             MLB_TRY(hooks->first_fold(r_dev, &next, &owns_next));
+            if (hooks->layer_digests) next_digests = hooks->layer_digests[f->layers.size()];
         } else {
             MLB_TRY(chain_layer_bufs(f, hooks, half_n, &next, &next_digests, &owns_next, s));
             int st = fri_fold_launch(ctx, f->layers.back().code, n, next, 0, r_dev, k, f->log_n0, s);
@@ -882,6 +883,62 @@ void write_bfri_proof(const ml_bfri_proof* p, Writer& w) {
     hfe_store(le, p->last_elem);
     w.febytes(le);
     w.bytes(p->last_random, 32);
+}
+
+// inverse of write_bfri_proof (batched_fri.rs:21-27 through the same derives): false on malformed input.  Every field element must
+// be canonical (< the modulus).
+bool read_bfri_proof(Reader& r, ml_bfri_proof* p) {
+    auto canonical = [](const uint8_t* b) { return hfe_load(b) < HFE_M; };
+    if (!r.take(p->batch_commitment, 32)) return false;
+    const uint64_t nc = r.u64();
+    if (!r.ok || nc > 64) return false;
+    p->commitments.resize(32 * nc);
+    r.take(p->commitments.data(), 32 * nc);
+    const uint64_t nq = r.u64();
+    if (!r.ok || nq > 4096) return false;
+    p->queries.resize(nq);
+    for (BQueryH& q : p->queries) {
+        const uint64_t nb = r.u64();
+        if (!r.ok || nb > (r.n - r.o) / 48) return false;  // every batch value pair takes 48 bytes
+        PathH& bp = q.batch_path;
+        bp.value.resize(32 * nb);
+        for (uint64_t j = 0; j < nb; j++)
+            if (!r.febytes(&bp.value[32 * j]) || !r.febytes(&bp.value[32 * j + 16]) || !canonical(&bp.value[32 * j]) ||
+                !canonical(&bp.value[32 * j + 16]))
+                return false;
+        const uint64_t len = r.u64();
+        if (!r.ok || len > 64) return false;
+        bp.digests.resize(32 * len);
+        bp.dirs.resize(len);
+        for (uint64_t i = 0; i < len; i++) {
+            r.take(&bp.digests[32 * i], 32);
+            const uint32_t d = r.u32();
+            if (!r.ok || d > 1) return false;
+            bp.dirs[i] = (uint8_t)d;
+        }
+        const uint64_t np = r.u64();
+        if (!r.ok || np > 64) return false;
+        q.query.paths.resize(np);
+        for (PathH& ph : q.query.paths) {
+            ph.value.resize(32);
+            if (!r.febytes(ph.value.data()) || !r.febytes(ph.value.data() + 16) || !canonical(ph.value.data()) || !canonical(ph.value.data() + 16))
+                return false;
+            const uint64_t plen = r.u64();
+            if (!r.ok || plen > 64) return false;
+            ph.digests.resize(32 * plen);
+            ph.dirs.resize(plen);
+            for (uint64_t i = 0; i < plen; i++) {
+                r.take(&ph.digests[32 * i], 32);
+                const uint32_t d = r.u32();
+                if (!r.ok || d > 1) return false;
+                ph.dirs[i] = (uint8_t)d;
+            }
+        }
+    }
+    uint8_t le[16];
+    if (!r.febytes(le) || !canonical(le)) return false;
+    p->last_elem = hfe_load(le);
+    return r.take(p->last_random, 32);
 }
 
 // ------------------------------------------------------------------ batched FRI prover data (batched_fri.rs:9-14)
@@ -1921,6 +1978,15 @@ int ml_bfri_proof_last(const ml_bfri_proof* p, uint8_t last_elem[16], uint8_t la
 }
 size_t ml_bfri_proof_serialized_len(const ml_bfri_proof* p) { Writer w(nullptr); write_bfri_proof(p, w); return w.n; }
 int ml_bfri_proof_serialize(const ml_bfri_proof* p, uint8_t* out) { Writer w(out); write_bfri_proof(p, w); return ML_OK; }
+int ml_bfri_proof_deserialize(const uint8_t* blob, size_t len, ml_bfri_proof** out) {
+    if (!out || (!blob && len)) { set_error("ml_bfri_proof_deserialize: NULL argument"); return ML_ERR_ARG; }
+    *out = nullptr;
+    ml_bfri_proof* p = new ml_bfri_proof();
+    Reader r(blob, len);
+    if (!read_bfri_proof(r, p) || r.o != len) { delete p; set_error("BatchedFriProof blob is malformed"); return ML_ERR_ARG; }
+    *out = p;
+    return ML_OK;
+}
 
 int ml_batched_pcs_prove_dev(const uint8_t* inputs, size_t n_vars, const uint8_t* outputs, size_t n_polys, const void* const* evals_dev,
                              size_t n, ml_transcript* t, void* stream, ml_bpcs_proof** out) {

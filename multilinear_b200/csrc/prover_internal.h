@@ -56,7 +56,8 @@ struct ChainHooks {
     const DevTranscript* tr_dev = nullptr;  // transcript state already in HBM (device copy instead of uploading the host state)
     const fe* prev_dev = nullptr;           // running sumcheck claim already in HBM
     // buffers of a prove plan, indexed by layer: the code and the Merkle digests of every layer the chain commits (instead of
-    // pool allocations; the layers do not own them)
+    // pool allocations; the layers do not own them).  In a batched chain layer 0 is first_fold's output, whose tree goes to
+    // layer_digests[0].
     fe* const* layer_code = nullptr;
     uint8_t* const* layer_digests = nullptr;
 };
@@ -71,6 +72,12 @@ struct ChainRun {
 };
 int fold_chain_enqueue(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, size_t k_start, bool pending,
                        ml_transcript* t, uint8_t* base, ChainRun* run, cudaStream_t s);
+// BatchedPCSProverData::init's claim (batched_pcs.rs:44-49) and BatchedFriProverData::init after the batch tree
+// (batched_fri.rs:80-86) on one thread: transcript from tr_in; with absorb_claim, absorb inputs (n_inputs) then outputs
+// (n_outputs); absorb the root, draw rho and absorb it; transcript to tr_out (may equal tr_in).  rho_out = rho; prev_out
+// (optional) = fingerprint(rho, outputs); r_out (optional) = {r_0, r_0 / 2}, the next challenge (batched_fri.rs:194).
+int batch_root_launch(const DevTranscript* tr_in, DevTranscript* tr_out, const uint8_t* root, const fe* inputs, int n_inputs, const fe* outputs,
+                      int n_outputs, bool absorb_claim, fe* rho_out, fe* prev_out, fe* r_out, cudaStream_t s);
 int fold_chain_dev(Ctx* ctx, ml_fri* f, const ChainHooks* hooks, ml_sumcheck* sc, hfe prev, hfe* sc_out, size_t k_start, bool pending,
                    ml_transcript* t, cudaStream_t s);
 

@@ -23,7 +23,7 @@ use crate::ntt::{LagrangePolynomial, Polynomial};
 use crate::polynomials::{MultilinearPolynomial, MultilinearPolynomialEvals};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard, MlBfriShard, MlProvePlan);
+opaque!(MlTranscript, MlMerkle, MlFri, MlFriProof, MlSumcheck, MlWSumcheck, MlPcsProof, MlBfriProof, MlBpcsProof, MlShard, MlBfri, MlPcsShard, MlBpcsShard, MlWSumcheckShard, MlFriShard, MlBfriShard, MlProvePlan, MlBatchedProvePlan);
 
 const _: () = assert!(std::mem::size_of::<Field128>() == 16 && std::mem::align_of::<Field128>() == 16);
 const _: () = assert!(std::mem::size_of::<ReedSolomonPair<Field128>>() == 32); // #[repr(C)], src/fri/mod.rs:30-35
@@ -34,12 +34,19 @@ const _: () = assert!(cfg!(target_endian = "little"));
 extern "C" {
     // ---- GENERATED from include/multilinear_b200.h by tools/abi_tools.py (do not edit by hand)
     pub fn ml_batched_fri_prove(codes: *const *const u8, n_codes: usize, n: usize, gen_pows: *const u8, gen_pows_len: usize, t: *mut MlTranscript, out: *mut *mut MlBfriProof) -> c_int;
+    pub fn ml_batched_fri_prove_async(p: *mut MlBatchedProvePlan, codes_dev: *const *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_batched_fri_verify(p: *const MlBfriProof) -> c_int;
     pub fn ml_batched_leaf_subtree_dev(pairs_dev: *const *const c_void, n_codes: usize, leaf_count: usize, stream: *mut c_void, root_out: *mut u8) -> c_int;
     pub fn ml_batched_leaf_subtree_root_dev(pairs_dev: *const *const c_void, n_codes: usize, leaf_count: usize, root_dev: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn ml_batched_pcs_prove(inputs: *const u8, n_vars: usize, outputs: *const u8, n_polys: usize, evals: *const *const u8, n: usize, t: *mut MlTranscript, out: *mut *mut MlBpcsProof) -> c_int;
+    pub fn ml_batched_pcs_prove_async(p: *mut MlBatchedProvePlan, inputs_dev: *const c_void, outputs_dev: *const c_void, evals_dev: *const *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, sumcheck_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_batched_pcs_prove_dev(inputs: *const u8, n_vars: usize, outputs: *const u8, n_polys: usize, evals_dev: *const *const c_void, n: usize, t: *mut MlTranscript, stream: *mut c_void, out: *mut *mut MlBpcsProof) -> c_int;
     pub fn ml_batched_pcs_verify(p: *const MlBpcsProof, t: *mut MlTranscript) -> c_int;
+    pub fn ml_batched_prove_plan_create(log_domain: usize, n_codes: usize, kind: c_int, out: *mut *mut MlBatchedProvePlan) -> c_int;
+    pub fn ml_batched_prove_plan_device_bytes(p: *const MlBatchedProvePlan) -> usize;
+    pub fn ml_batched_prove_plan_free(p: *mut MlBatchedProvePlan);
+    pub fn ml_batched_prove_plan_proof_bytes(p: *const MlBatchedProvePlan) -> usize;
+    pub fn ml_batched_rs_fri_prove_async(p: *mut MlBatchedProvePlan, coeffs_dev: *const *const c_void, transcript_dev: *mut c_void, proof_dev: *mut c_void, status_dev: *mut c_int, stream: *mut c_void) -> c_int;
     pub fn ml_bfri_batch_layer(h: *const MlBfri) -> *const MlMerkle;
     pub fn ml_bfri_batched_fold_step(h: *mut MlBfri, gen_pows: *const u8, gen_pows_len: usize, r: *const u8, t: *mut MlTranscript) -> c_int;
     pub fn ml_bfri_fingerprint_r(h: *const MlBfri, out: *mut u8) -> c_int;
@@ -51,6 +58,7 @@ extern "C" {
     pub fn ml_bfri_open_query_at(h: *const MlBfri, index: usize, batch_values: *mut u8, batch_digests: *mut u8, batch_dirs: *mut u8, batch_path_len: *mut usize, values: *mut u8, digests: *mut u8, dirs: *mut u8, path_lens: *mut usize) -> c_int;
     pub fn ml_bfri_proof_batch_commitment(p: *const MlBfriProof, out: *mut u8) -> c_int;
     pub fn ml_bfri_proof_commitments(p: *const MlBfriProof, out: *mut u8) -> c_int;
+    pub fn ml_bfri_proof_deserialize(blob: *const u8, len: usize, out: *mut *mut MlBfriProof) -> c_int;
     pub fn ml_bfri_proof_free(p: *mut MlBfriProof);
     pub fn ml_bfri_proof_last(p: *const MlBfriProof, last_elem: *mut u8, last_random: *mut u8) -> c_int;
     pub fn ml_bfri_proof_num_commitments(p: *const MlBfriProof) -> usize;
@@ -734,6 +742,64 @@ impl ProvePlan {
 impl Drop for ProvePlan {
     fn drop(&mut self) {
         unsafe { ml_prove_plan_free(self.h) }
+    }
+}
+/// Stream-ordered `BatchedFriProof::prove` / `BatchedPCSProof::prove` of n_codes codes of 2^log_domain elements
+/// (ml_batched_prove_plan_*, csrc/bplan.cu), for one kind of call: from codes, from coefficients (reed_solomon of each first) or
+/// from evaluations (PCS).  A call only enqueues kernels on `stream` and writes the bincode blob, the final transcript state, the
+/// status and (PCS) the sumcheck coefficients into the caller's device buffers.  One proof in flight per plan.
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub enum BatchedPlanKind {
+    Codes = 0,
+    Rs = 1,
+    Pcs = 2,
+}
+pub struct BatchedProvePlan {
+    h: *mut MlBatchedProvePlan,
+}
+impl BatchedProvePlan {
+    pub fn new(log_domain: usize, n_codes: usize, kind: BatchedPlanKind) -> Self {
+        let mut h = std::ptr::null_mut();
+        check(unsafe { ml_batched_prove_plan_create(log_domain, n_codes, kind as c_int, &mut h) });
+        Self { h }
+    }
+    /// bytes of the BatchedFriProof blob a call writes (`bincode` of the proof)
+    pub fn proof_bytes(&self) -> usize {
+        unsafe { ml_batched_prove_plan_proof_bytes(self.h) }
+    }
+    pub fn device_bytes(&self) -> usize {
+        unsafe { ml_batched_prove_plan_device_bytes(self.h) }
+    }
+    /// `BatchedFriProof::prove` of n_codes codes of N elements in HBM (a `Codes` plan).
+    /// # Safety
+    /// Every pointer (those in `codes_dev` too) is device memory of the size include/multilinear_b200.h states, 16-byte aligned,
+    /// and stays valid until the stream has passed the call.
+    pub unsafe fn batched_fri_prove_async(&mut self, codes_dev: &[*const c_void], transcript_dev: *mut c_void, proof_dev: *mut c_void,
+                                          status_dev: *mut c_int, stream: *mut c_void) {
+        check(ml_batched_fri_prove_async(self.h, codes_dev.as_ptr(), transcript_dev, proof_dev, status_dev, stream));
+    }
+    /// `reed_solomon` of each of n_codes polynomials of N/2 coefficients in HBM + `BatchedFriProof::prove` (an `Rs` plan).
+    /// # Safety
+    /// As for `batched_fri_prove_async`.
+    pub unsafe fn batched_rs_fri_prove_async(&mut self, coeffs_dev: &[*const c_void], transcript_dev: *mut c_void, proof_dev: *mut c_void,
+                                             status_dev: *mut c_int, stream: *mut c_void) {
+        check(ml_batched_rs_fri_prove_async(self.h, coeffs_dev.as_ptr(), transcript_dev, proof_dev, status_dev, stream));
+    }
+    /// `BatchedPCSProof::prove` of n_codes polynomials of N/2 evaluations in HBM (a `Pcs` plan); sumcheck_dev receives 2 * n_vars
+    /// coefficients.
+    /// # Safety
+    /// As for `batched_fri_prove_async`.
+    #[allow(clippy::too_many_arguments)]
+    pub unsafe fn batched_pcs_prove_async(&mut self, inputs_dev: *const c_void, outputs_dev: *const c_void, evals_dev: &[*const c_void],
+                                          transcript_dev: *mut c_void, proof_dev: *mut c_void, sumcheck_dev: *mut c_void,
+                                          status_dev: *mut c_int, stream: *mut c_void) {
+        check(ml_batched_pcs_prove_async(self.h, inputs_dev, outputs_dev, evals_dev.as_ptr(), transcript_dev, proof_dev, sumcheck_dev,
+                                         status_dev, stream));
+    }
+}
+impl Drop for BatchedProvePlan {
+    fn drop(&mut self) {
+        unsafe { ml_batched_prove_plan_free(self.h) }
     }
 }
 /// `BatchedFriProof` does not derive `Deserialize`; its blob is the bincode encoding of its parts in field order, and the parts

@@ -12,7 +12,7 @@ HANDLES = {"ml_transcript": "MlTranscript", "ml_merkle": "MlMerkle", "ml_fri": "
            "ml_wsumcheck": "MlWSumcheck", "ml_pcs_proof": "MlPcsProof", "ml_bfri_proof": "MlBfriProof", "ml_bpcs_proof": "MlBpcsProof",
            "ml_shard": "MlShard", "ml_bfri": "MlBfri", "ml_pcs_shard": "MlPcsShard", "ml_bpcs_shard": "MlBpcsShard",
            "ml_wsumcheck_shard": "MlWSumcheckShard", "ml_fri_shard": "MlFriShard", "ml_bfri_shard": "MlBfriShard",
-           "ml_prove_plan": "MlProvePlan"}
+           "ml_prove_plan": "MlProvePlan", "ml_batched_prove_plan": "MlBatchedProvePlan"}
 SCALARS = {"int": "c_int", "unsigned": "c_uint", "size_t": "usize", "uint64_t": "u64", "int64_t": "i64", "uint32_t": "u32", "uint8_t": "u8",
            "double": "f64", "char": "c_char", "void": "c_void"}
 BEGIN, END = "    // ---- GENERATED from include/multilinear_b200.h by tools/abi_tools.py (do not edit by hand)\n", "    // ---- END GENERATED\n"
